@@ -17,6 +17,12 @@ fwd + loss + bwd + all-reduce.  N>1: one process per GPU (torchrun), every rank 
 shape (weak scaling; sequences are independent, the only collective is the training gradient all-reduce).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--legs cfg2,cfg5_bf16,...]
+                  [--dump-outputs DIR]
+
+Both timed regions of every leg run exactly K steps: from inputs resident in HBM, then end to end from pinned host
+buffers (the roofline / kernel-alone passes that follow are separate).  The inputs are seeded, so the same
+arguments give the same inputs on every run; `--dump-outputs DIR` writes what the last timed step of each leg returned
+to its caller (see OutputDump) so that two builds can be compared output for output.
 
 `--impl reference` times the UNMODIFIED reference classes (oracle/_ref, vendored by oracle/make_ref.py) on the host
 cores; it never imports the product package.
@@ -59,7 +65,12 @@ def parse():
     ap.add_argument('--infer-chunks', type=int, default=4, help='streams the graphed inference body forks into (1 = single stream)')
     ap.add_argument('--cpu-sample', type=int, default=4096, help='sequences of the batch the CPU reference runs (baseline + tag check)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write the outputs of the last timed step of every leg as DIR/<leg>_<name>.npy')
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    return a
 
 
 def flops_per_position(S, R, D, Cp, farnn):
@@ -231,6 +242,8 @@ class Ctx:
         self.local = int(os.environ.get('LOCAL_RANK', '0'))
         self.flush = None
         self.peaks = load_peaks()
+        self.dump = OutputDump(a.dump_outputs, self.rank == 0)
+        self.last_output = None
 
     def barrier(self):
         if self.world > 1:
@@ -239,18 +252,23 @@ class Ctx:
 
     def timed(self, fn, steps):
         """K steps, each bracketed by CUDA events on the current stream, an L2 flush (256 MB write) before each, a
-        barrier + synchronize on both sides.  -> per-step ms list of this rank."""
+        barrier + synchronize on both sides.  -> per-step ms list of this rank; what the last step returned is kept in
+        self.last_output (earlier steps' results are dropped as they come, as a caller looping over batches would)."""
         torch = self.torch
         if self.flush is None:
             self.flush = torch.empty(256 * 1024 * 1024 // 4, dtype=torch.float32, device='cuda')   # > 126 MB L2
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
+        self.last_output = None
         self.barrier()
         for i in range(steps):
             self.flush.zero_()
             ev[i][0].record()
-            fn()
+            out = fn()
             ev[i][1].record()
+            if i + 1 < steps:
+                out = None
         self.barrier()
+        self.last_output = out
         return [s.elapsed_time(e) for s, e in ev]
 
     def reduce(self, total_ms, tokens):
@@ -266,6 +284,38 @@ class Ctx:
 
 def stats(ms):
     return {'min': float(np.min(ms)), 'median': float(np.median(ms)), 'max': float(np.max(ms)), 'argmax': int(np.argmax(ms))}
+
+
+class OutputDump:
+    """--dump-outputs DIR: the arrays the last timed step of a leg handed to its caller, one DIR/<leg>_<name>.npy each,
+    float64 where the output is float64 and float32 otherwise (tags and labels are small integers, exact in float32).
+    An array of more than CAP elements is stored as a fixed sample of its flattened values: the positions
+    np.sort(np.random.RandomState(0).choice(size, CAP, replace=False)).  With CAP, the default legs write about 14 MB.
+    Every rank counts the bytes (the legs have the same shapes on every rank) and only rank 0 writes, so going over
+    LIMIT stops all ranks at the same leg instead of leaving the others waiting in a collective."""
+    CAP = 1 << 19
+    LIMIT = 64 << 20
+
+    def __init__(self, path, writer):
+        self.path, self.writer, self.bytes = path, writer, 0
+        if path and writer:
+            os.makedirs(path, exist_ok=True)
+
+    def write(self, leg, arrays):
+        if not self.path:
+            return
+        for name, t in arrays.items():
+            if t is None:
+                continue
+            a = t.detach().cpu().numpy() if hasattr(t, 'detach') else np.asarray(t)
+            a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+            if a.size > self.CAP:
+                a = a.reshape(-1)[np.sort(np.random.RandomState(0).choice(a.size, self.CAP, replace=False))]
+            self.bytes += a.nbytes
+            if self.bytes > self.LIMIT:
+                raise SystemExit('--dump-outputs: the outputs exceed %d MB' % (self.LIMIT >> 20))
+            if self.writer:
+                np.save(os.path.join(self.path, '%s_%s.npy' % (leg, name)), a)
 
 
 # ---- decompose inference leg ------------------------------------------------------------------------------------------
@@ -335,6 +385,10 @@ def leg_decompose(ctx, name, cfg, precision, farnn, steps, warmup, batch=0, ref_
     l0 = ops.launches()
     ms1 = ctx.timed(step_device, steps)
     launches_total = ops.launches() - l0
+    loss_o, pred_o, true_o = ctx.last_output
+    ctx.dump.write(name, {'loss': loss_o, 'pred': pred_o, 'true': true_o})
+    del loss_o, pred_o, true_o
+    ctx.last_output = None
 
     # ---- roofline pass: the SAME configuration (CUDA graph, chunk streams) with every recurrence launch bracketed by
     # CUDA events recorded inside the library on the launching stream (external event nodes inside the graph) ---------
@@ -472,16 +526,16 @@ def leg_train(ctx, cfg, farnn, steps, warmup):
 
     def train_step(xg, yg, lg):
         bucket.zero_grad()
-        loss, pred, _ = m.forward_local(xg, yg, lg, train=True)
+        loss, pred, true = m.forward_local(xg, yg, lg, train=True)
         loss.backward()
         bucket.all_reduce()                # one all-reduce(SUM) of the flat gradient bucket (NCCL when N>1)
-        return loss
+        return loss, pred, true
 
     def step_device():
         return train_step(xd, yd, ld)
 
     def step_e2e():
-        loss = train_step(xh.cuda(non_blocking=True), yh.cuda(non_blocking=True), lh.cuda(non_blocking=True))
+        loss, _, _ = train_step(xh.cuda(non_blocking=True), yh.cuda(non_blocking=True), lh.cuda(non_blocking=True))
         loss_host.copy_(loss.detach(), non_blocking=True)
 
     for _ in range(max(warmup, 3)):
@@ -492,6 +546,11 @@ def leg_train(ctx, cfg, farnn, steps, warmup):
     ms1 = ctx.timed(step_device, steps)
     launches_total = ops.launches() - l0
     clocks = sampler.stop()
+    loss_o, pred_o, true_o = ctx.last_output           # the gradients of this step are still in the bucket
+    ctx.dump.write('%s_train' % cfg, dict({'loss': loss_o, 'pred': pred_o, 'true': true_o},
+                                          **{'grad.' + k: v.grad for k, v in m.named_parameters() if v.grad is not None}))
+    del loss_o, pred_o, true_o
+    ctx.last_output = None
     for _ in range(2):
         step_e2e()
     ms2 = ctx.timed(step_e2e, steps)
@@ -557,6 +616,10 @@ def leg_onehot(ctx, name, V, S, C, B, Lmax, fixed, steps, warmup, note):
     l0 = ops.launches()
     ms1 = ctx.timed(step_device, steps)
     launches_total = ops.launches() - l0
+    loss_o, pred_o, true_o = ctx.last_output
+    ctx.dump.write(name, {'loss': loss_o, 'pred': pred_o, 'true': true_o})
+    del loss_o, pred_o, true_o
+    ctx.last_output = None
     # dominant kernel alone: CUDA events around the recurrence launch
     alone = []
     with torch.no_grad():
@@ -622,7 +685,6 @@ def main():
     ref_sample = 0 if a.no_cpu_baseline else a.cpu_sample
     results = {}
     for leg in legs:
-        ksteps = a.steps
         if leg == 'custom':
             results[leg] = leg_decompose(ctx, leg, a.config, a.precision, a.farnn, a.steps, a.warmup, batch=a.batch,
                                          ref_sample=ref_sample, ref_repeats=3, want_cpu_baseline=want_cpu)
@@ -633,17 +695,17 @@ def main():
             results[leg] = leg_decompose(ctx, leg, 'cfg2', a.precision, 2, a.steps, a.warmup, ref_sample=min(ref_sample, 256),
                                          ref_repeats=1)
         elif leg == 'cfg4':                # configs[3]: ATIS-ZH-shaped long recurrence (S=512, R=256, len<=128, B=4096)
-            results[leg] = leg_decompose(ctx, leg, 'cfg4', a.precision, 0, max(3, min(ksteps, 10)), 3,
+            results[leg] = leg_decompose(ctx, leg, 'cfg4', a.precision, 0, a.steps, 3,
                                          ref_sample=min(ref_sample, 128), ref_repeats=1)
         elif leg in ('cfg5_bf16', 'cfg5_parity'):
-            results[leg] = leg_decompose(ctx, leg, 'cfg5', 'bf16' if leg == 'cfg5_bf16' else 'auto', 0, max(3, min(ksteps, 5)), 3,
+            results[leg] = leg_decompose(ctx, leg, 'cfg5', 'bf16' if leg == 'cfg5_bf16' else 'auto', 0, a.steps, 3,
                                          ref_sample=min(ref_sample, 128), ref_repeats=1)
         elif leg == 'cfg3_train':
             results[leg] = leg_train(ctx, 'cfg3', a.farnn, a.steps, a.warmup)
         elif leg == 'cfg1_onehot':
             results[leg] = leg_onehot(ctx, leg, 900, 300, 127, 32, 46, False, a.steps, a.warmup, '')
         elif leg == 'cfg5_onehot':
-            results[leg] = leg_onehot(ctx, leg, 900, 1024, 128, 1024, 64, True, max(3, min(ksteps, 5)), 3,
+            results[leg] = leg_onehot(ctx, leg, 900, 1024, 128, 1024, 64, True, a.steps, 3,
                                       ' -- B reduced from 65536: the dense gather moves 8*S^2 = 8.4 MB per position, '
                                       '65536 x 64 positions would be 35 PB per batch')
         else:

@@ -42,6 +42,36 @@ def rel_err(a, b):
     return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
 
 
+# ---- a stand-in reference tree for the `src_seq` shadow package (shim/) ------------------------------
+# The reference's module layout and the names its drivers import, each defined in a placeholder module.  The shadow
+# package's import mechanics (which name resolves to which tree) are tested against it, so those tests do not need an
+# RE2NN-SEQ checkout.
+_STAND_IN = {
+    '__init__.py': '',
+    'val.py': 'def val_onehot(*a, **k):\n    raise NotImplementedError\n',
+    'utils.py': '',
+    'farnn/__init__.py': '',
+    'farnn/model_decompose_single.py': 'class FARNN_S_D_W_I_S:\n    pass\n\n\nclass FARNN_S_SF:\n    pass\n',
+    'farnn/model_onehot.py': 'class FARNN_S_O:\n    pass\n\n\nclass FARNN_S_O_I:\n    pass\n\n\nclass FARNN_S_O_I_S:\n    pass\n',
+    'farnn/model_decompose.py': 'class FARNN_S_D_W:\n    pass\n',
+    'farnn/model_decompose_independent.py': 'class FARNN_S_D_W_I:\n    pass\n',
+    'farnn/priority.py': 'class PriorityLayer:\n    pass\n',
+    'baselines/__init__.py': '',
+    'baselines/crf.py': 'class CRF:\n    pass\n',
+    'baselines/KD.py': 'def KD_loss(*a, **k):\n    raise NotImplementedError\n',
+}
+
+
+def stand_in_reference(root):
+    """Write the stand-in reference tree under `root` (root/src_seq/...) -> root."""
+    for rel, text in _STAND_IN.items():
+        path = os.path.join(root, 'src_seq', rel)
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        with open(path, 'w') as f:
+            f.write(text)
+    return str(root)
+
+
 # ---- building product modules from fixtures --------------------------------------------------------
 def golden_seed(name):
     """Seed used by tests/golden/make_golden.py for this case (see its main())."""

@@ -5,7 +5,9 @@ box, /root/reference does not).  Each test first runs the pure reference on the 
 function -- val.val_onehot (src_seq/val.py:7-43) and the training loop of train_decompose.py:170-193 -- with
 shim/ ahead on sys.path, so `from src_seq.farnn.model_decompose_single import FARNN_S_D_W_I_S` inside the
 reference code resolves to the B200 implementation while src_seq.val / src_seq.utils / src_seq.metrics stay the
-reference's files.  Tags and the metric dictionary must be identical, losses agree to 1e-5 relative."""
+reference's files.  Tags and the metric dictionary must be identical, losses agree to 1e-5 relative.
+test_reference_val_onehot_runs_on_the_dropins needs that reference checkout and skips without it; the training loop runs through the shadow package
+on a stand-in reference tree and compares with stored oracle values (the repository does not contain the reference)."""
 import os
 import sys
 
@@ -37,9 +39,9 @@ def _use_reference():
     make_ref.import_reference()
 
 
-def _use_shim():
+def _use_shim(ref=REF):
     _purge()
-    os.environ['RE2NN_REFERENCE_ROOT'] = REF
+    os.environ['RE2NN_REFERENCE_ROOT'] = ref
     sys.path.insert(0, SHIM)
 
 
@@ -119,27 +121,35 @@ def _train_like_reference(m, args, batches, steps, cuda):
 
 
 @pytest.mark.parametrize('farnn,crf', [(0, 1), (2, 1)])
-def test_reference_training_loop_runs_on_the_dropins(farnn, crf):
-    _use_reference()
-    m, args, x, lens, lab = _decompose_model(farnn, crf, 8, False)
-    want_l, want_p = _train_like_reference(m, args, _batches(x, lens, lab, 16), 4, False)
-    _use_shim()
-    m2, args2, x2, lens2, lab2 = _decompose_model(farnn, crf, 8, True)
-    m2 = m2.cuda()
-    got_l, got_p = _train_like_reference(m2, args2, _batches(x2, lens2, lab2, 16), 4, True)
+def test_training_loop_through_shim_vs_oracle(farnn, crf, tmp_path):
+    """The training loop above on the drop-in that the shadow package resolves (against the stand-in reference tree of
+    helpers.stand_in_reference), against the same loop on the float32 torch oracle, stored by
+    tests/golden/make_golden_oracle.py.  The repository does not contain the reference, so the expected values come
+    from the oracle, not from the reference classes."""
+    from helpers import GOLDEN, stand_in_reference
+    z = np.load(os.path.join(GOLDEN, 'oracle_train_f%d_crf%d.npz' % (farnn, crf)))
+    _use_shim(stand_in_reference(tmp_path))
+    m, args, x, lens, lab = _decompose_model(farnn, crf, 8, True)
+    assert type(m).__module__.startswith('re2nn_seq_b200')
+    m = m.cuda()
+    got_l, got_p = _train_like_reference(m, args, _batches(x, lens, lab, 16), 4, True)
+    want_l = z['losses']
     for a, b in zip(got_l, want_l):
         assert abs(a - b) <= 2e-5 * abs(b), (got_l, want_l)
-    np.testing.assert_array_equal(got_p[0], want_p[0])                  # same parameters -> same decoded tags
+    np.testing.assert_array_equal(got_p[0], z['pred0'])                 # same parameters -> same decoded tags
     _purge()
 
 
-def test_shim_off_switch_falls_through_to_reference():
-    _use_shim()
+def test_shim_off_switch_falls_through_to_reference(tmp_path):
+    """Against the stand-in reference tree of helpers.stand_in_reference (the reference's layout and names)."""
+    from helpers import stand_in_reference
+    ref = stand_in_reference(tmp_path)
+    _use_shim(ref)
     os.environ['RE2NN_SHIM'] = 'off'
     try:
         from src_seq.farnn.model_decompose_single import FARNN_S_D_W_I_S
         assert FARNN_S_D_W_I_S.__module__ == 'src_seq.farnn.model_decompose_single'
-        assert os.path.abspath(sys.modules[FARNN_S_D_W_I_S.__module__].__file__).startswith(REF)
+        assert os.path.abspath(sys.modules[FARNN_S_D_W_I_S.__module__].__file__).startswith(ref)
     finally:
         del os.environ['RE2NN_SHIM']
         _purge()

@@ -1,13 +1,13 @@
 """CPU: import mechanics of the `src_seq` shadow package (no kernels run): shadowed modules resolve to the drop-in
-classes, everything else to the reference's own files, RE2NN_SHIM=off falls through."""
+classes, everything else to the reference tree's own files, RE2NN_SHIM=off falls through.  The reference tree is the
+stand-in of helpers.stand_in_reference (the reference's layout and names), written to a temporary directory."""
 import os
 import subprocess
 import sys
 
-import pytest
+from helpers import stand_in_reference
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, 'oracle', '_ref')
 
 CODE = r'''
 import os, sys
@@ -26,12 +26,8 @@ print(src_seq.val.__file__ + '|' + src_seq.utils.__file__ + '|' + KD_loss.__modu
 '''
 
 
-def _run(shim_on):
-    from oracle import make_ref
-    why = make_ref.verify()
-    if why:
-        pytest.skip(why)
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, 'shim'), ROOT]), RE2NN_REFERENCE_ROOT=REF,
+def _run(shim_on, ref):
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, 'shim'), ROOT]), RE2NN_REFERENCE_ROOT=ref,
                RE2NN_SHIM='on' if shim_on else 'off')
     r = subprocess.run([sys.executable, '-c', CODE], env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True,
                        timeout=300)
@@ -39,14 +35,15 @@ def _run(shim_on):
     return r.stdout.strip().splitlines()[-2:]
 
 
-def test_shim_resolves_dropins_and_reference_files():
-    mods, files = _run(True)
+def test_shim_resolves_dropins_and_reference_files(tmp_path):
+    ref = stand_in_reference(tmp_path)
+    mods, files = _run(True, ref)
     assert all(m.startswith('re2nn_seq_b200') for m in mods.split('|')), mods
     val_file, utils_file, kd_mod = files.split('|')
-    assert os.path.abspath(val_file).startswith(REF) and os.path.abspath(utils_file).startswith(REF)
+    assert os.path.abspath(val_file).startswith(ref) and os.path.abspath(utils_file).startswith(ref)
     assert kd_mod == 'src_seq.baselines.KD'
 
 
-def test_shim_off_is_the_reference():
-    mods, _ = _run(False)
+def test_shim_off_is_the_reference(tmp_path):
+    mods, _ = _run(False, stand_in_reference(tmp_path))
     assert all(m.startswith('src_seq.') for m in mods.split('|')), mods

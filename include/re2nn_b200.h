@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define RE2NN_ABI_VERSION 2
+#define RE2NN_ABI_VERSION 3
 
 /* update_nonlinear / additional_nonlinear (model_decompose_single.py:184-191, model_decompose.py:228-237) */
 enum { RE2NN_NL_NONE = 0, RE2NN_NL_RELU = 1, RE2NN_NL_TANH = 2, RE2NN_NL_RELUTANH = 3, RE2NN_NL_SIGMOID = 4 };
@@ -74,21 +74,12 @@ int re2nn_debug_set_tc_cta_group(int cta_group);
 /* debug / calibration: 1 (default) = inference without gates runs the whole recurrence in one resident launch
  * (a CTA pair per 128-row tile iterates over all steps); 0 = one launch per step GEMM. */
 int re2nn_debug_set_resident(int on);
-/* debug / calibration: training on resident launches in the split tensor-core precisions.  bit 0 = the forward that
- * keeps the BPTT slabs (re2nn_decompose_recurrence with save_for_backward), bit 1 = the BPTT sweep of
- * re2nn_decompose_backward (farnn = 0: one launch for all steps instead of five per step).  Default 0 = per-step
- * launches: the resident variants are parity-identical but measured slower at B = 1024 and equal at B = 4096. */
-int re2nn_debug_set_resident_train(int on);
 /* debug / calibration: 1 (default) = the weight-gradient GEMMs (X^T Y over every (step, sequence) row) run on tcgen05 in
  * 3xTF32 with the operands transposed on the fly; 0 = the CUDA-core kernel. */
 int re2nn_debug_set_tn_tc(int on);
 /* debug / calibration: 1 (default) = the CRF backward sweep gives each sequence three warps (one transition row per
  * lane, named barriers between them) when the tag set has at most 96 entries; 0 = one warp per sequence. */
 int re2nn_debug_set_crf_backward_split(int on);
-/* debug / calibration: 1 = large bf16 step GEMMs (N a multiple of 512) run on clusters of 2 x 2 CTAs that TMA-
- * multicast their A row blocks and B column tiles (a quarter fewer operand bytes requested from L2); 0 (default) =
- * CTA pairs (cta_group::2) only -- the multicast variant measured 5-10 % slower on B200. */
-int re2nn_debug_set_tc_multicast(int on);
 int re2nn_profile_read(double* ms_out_host, int64_t* count_out_host);
 /* Per-launch [start, end] of kernel class `cls` in ms relative to the earliest start of the class, for up to
  * `cap` launches recorded since the last clearing read.  The event pairs also work inside stream capture (they

@@ -97,10 +97,8 @@ SYMBOLS = {
     're2nn_debug_set_tc_timeline': (C.c_int, [vp]),
     're2nn_debug_set_tc_cta_group': (C.c_int, [C.c_int]),
     're2nn_debug_set_resident': (C.c_int, [C.c_int]),
-    're2nn_debug_set_resident_train': (C.c_int, [C.c_int]),
     're2nn_debug_set_tn_tc': (C.c_int, [C.c_int]),
     're2nn_debug_set_crf_backward_split': (C.c_int, [C.c_int]),
-    're2nn_debug_set_tc_multicast': (C.c_int, [C.c_int]),
     're2nn_debug_set_backward_tc': (C.c_int, [C.c_int]),
     're2nn_debug_set_viterbi_seqs': (C.c_int, [C.c_int]),
     're2nn_profile_read': (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_int64)]),

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libre2nn_b200.so')
-SOURCES = ['recurrence.cu', 'recurrence_train.cu', 'crf.cu', 'onehot.cu', 'backward.cu', 'maxprod.cu', 'fst.cu']
+SOURCES = ['recurrence.cu', 'crf.cu', 'onehot.cu', 'backward.cu', 'maxprod.cu', 'fst.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '--use_fast_math=false', '-Xcompiler', '-fPIC', '-Xptxas', '-v', '--split-compile', '0']
 

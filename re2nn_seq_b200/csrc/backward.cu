@@ -15,14 +15,12 @@
 // After the sweep every weight gradient is ONE large transposed GEMM over all (step, sequence) rows
 // (K = 2*L*B) -- on tcgen05 with the operands transposed on the fly (gemm_tn_tc.cuh), CUDA cores for short reductions --
 // reduced deterministically (split-K partials + ordered sum); bias / vector gradients are deterministic column sums
-// of the per-step slabs.  The whole sweep also exists as ONE resident launch (ResidentBackward below): parity-
-// identical, slower at the benchmarked batch, off by default.
+// of the per-step slabs.
 #include <algorithm>
 #include <memory>
 
 #include "gemm_simt.cuh"
 #include "gemm_tc.cuh"
-#include "recurrence_resident.cuh"
 #include "gemm_tn_tc.cuh"
 
 namespace re2nn {
@@ -256,9 +254,6 @@ struct BwdCtx {
   void* DZop[2]; void* DRop[2];                      // farnn >= 1: dz / dr of this step (A operands of the gate GEMM)
   int ldS, ldR;
   size_t da_plane, du_plane;
-  // resident sweep: second DA operand buffer (ping-pong between steps) and the per-tile last live step
-  void* DAop1[2];
-  int* tile_last[2];
   void* DrawOp; void* CmatOp;                        // tensor-core label-score backward: operand-format draw / C_mat^T
 };
 
@@ -508,208 +503,9 @@ struct EpiTokenBwd {
   }
 };
 
-// ---- resident BPTT sweep (farnn = 0): the kernel of recurrence_resident.cuh run backwards -----------------------------
-// The sweep has the shape of the forward recurrence with the weights transposed: per step a GEMM of width R
-// (dq = DA[k] @ S2|S1) and one of width S with two K segments (dhb = DU[k] @ S1^T|S2^T + DA[k] @ W^T|W); what the
-// three elementwise kernels E1 / E2 / E3 do between them becomes the two fused epilogues below, and a CTA pair keeps
-// one 128-row tile for all steps: one launch instead of five per step, no grid-wide dependency between steps.
-//   epilogue of dq   (step k)   = E2(k):            DU[k], Q[k], dvtab, the DU operand of this step
-//   epilogue of dhb  (step k)   = E3(k) + E1(k-1):  carry g, d_o products, DA[k-1] and the DA operand of step k-1
-// E1 of a tile's first step (its last live step) runs in bwd_resident_init_kernel, which also zeroes the slabs of the
-// steps the tile never executes (the weight-gradient GEMMs read every step of every row).
-struct EpiBwdQ {
-  static constexpr bool kRows = false;
-  const float* vtab; const float* u;          // token table; u = hbar @ S of this step (forward save)
-  float* DU; float* Qs; float* dvtab;
-  void* DUop;
-  int R, ldR;
-  size_t du_plane;
-  __device__ __forceinline__ Col col(int) const { return Col{0.f, 0.f}; }
-  __device__ __forceinline__ Pre prefetch(const RowCtx& r, int m, int n) const {
-    return Pre{__ldg(vtab + (size_t)((uint32_t)r.vrow * (uint32_t)R + (uint32_t)n)), u[(uint32_t)m * (uint32_t)R + (uint32_t)n]};
-  }
-  __device__ __forceinline__ float compute(const Col&, float acc, const Pre& pre) const { return acc * pre.a; }
-  __device__ __forceinline__ void store(const Col&, const RowCtx& r, int m, int n, float du, float dq, const Pre& pre) const {
-    const uint32_t i = (uint32_t)m * (uint32_t)R + (uint32_t)n;
-    DU[i] = du;
-    Qs[i] = pre.b * pre.a;
-    OperandFmt<RE2NN_PREC_TF32X3>::store(DUop, (uint32_t)m * (uint32_t)ldR + (uint32_t)n, du_plane, du);
-    const float dv = dq * pre.b;
-    if (dv != 0.f) atomicAdd(dvtab + (size_t)((uint32_t)r.vrow * (uint32_t)R + (uint32_t)n), dv);
-  }
-  __device__ __forceinline__ void apply(const Col& c, const RowCtx& r, int m, int n, float acc, const Pre& pre) const {
-    store(c, r, m, n, compute(c, acc, pre), acc, pre);
-  }
-};
-
-// RowCtx here: orow = output row of step k-1 (-1: the row is not alive at k-1, or k = 0)
-template <int NL> struct EpiBwdH {
-  static constexpr bool kRows = false;
-  const float* o; const float* dout;          // d alpha (z = 0) / d beta (z = 1), B x L x S
-  const float* second;                        // z = 0: pre-activation a of step k-1 ; z = 1: state after step k-1 (= h~ of step k)
-  float* DAprev; float* DOprod; float* gout;  // DA slab of step k-1 ; d_o products (z = 0: step k-1, z = 1: step k) ; carry at k = 0
-  void* DAop;
-  int L, S, ldS, z, has_prev, nl_rt;
-  size_t da_plane;
-  __device__ __forceinline__ int nl() const { return NL >= 0 ? NL : nl_rt; }
-  __device__ __forceinline__ Col col(int n) const { return Col{__ldg(o + n), 0.f}; }
-  __device__ __forceinline__ Pre prefetch(const RowCtx& r, int m, int n) const {
-    Pre q{0.f, 0.f};
-    if (r.orow >= 0) q.a = __ldg(dout + ((size_t)m * (uint32_t)L + (uint32_t)r.orow) * (uint32_t)S + (uint32_t)n);
-    if (second) q.b = second[(uint32_t)m * (uint32_t)S + (uint32_t)n];
-    return q;
-  }
-  // -> d pre-activation of step k-1 (or the final carry when there is no step k-1)
-  __device__ __forceinline__ float compute(const Col& c, float dhb, const Pre& pre) const {
-    const float g = z == 1 ? dhb * c.a : dhb;
-    if (!has_prev) return g;
-    const float G = g + pre.a;
-    const float hhat = z == 0 ? apply_nl(pre.b * c.a, nl()) : pre.b;
-    return G * nl_grad_from_out(hhat, nl());
-  }
-  __device__ __forceinline__ void store(const Col& c, const RowCtx&, int m, int n, float v, float dhb, const Pre& pre) const {
-    const uint32_t si = (uint32_t)m * (uint32_t)S + (uint32_t)n;
-    if (z == 1) DOprod[si] = dhb * pre.b;
-    if (!has_prev) {
-      gout[si] = v;
-      return;
-    }
-    const float da = z == 0 ? v * c.a : v;
-    DAprev[si] = da;
-    if (z == 0) DOprod[si] = v * pre.b;
-    OperandFmt<RE2NN_PREC_TF32X3>::store(DAop, (uint32_t)m * (uint32_t)ldS + (uint32_t)n, da_plane, da);
-  }
-  __device__ __forceinline__ void apply(const Col& c, const RowCtx& r, int m, int n, float acc, const Pre& pre) const {
-    store(c, r, m, n, compute(c, acc, pre), acc, pre);
-  }
-};
-
-// Both epilogues read slabs nobody has touched since the forward pass wrote them (HBM latency), from an SM whose L1 is
-// all but given away to shared memory: the loads of a chunk then trickle in at the few lines L1 can keep in flight
-// (measured: 12k cycles per 16 rows).  Pulling the lines into L2 while the step's MMAs run cuts the latency each of
-// those slots is held for.  Rows are not 128-byte aligned (pitch 4*S): a 32-column segment straddles two lines.
-template <> struct EpiL2Prefetch<EpiBwdQ> {
-  static constexpr bool kOn = true;
-  __device__ static __forceinline__ void issue(const EpiBwdQ& e, const RowCtx&, int m, int n) {
-    const float* u = e.u + (uint32_t)m * (uint32_t)e.R + (uint32_t)n;
-    l2_prefetch(u);
-    l2_prefetch(u + min(31, e.R - 1 - n));
-  }
-};
-template <int NL> struct EpiL2Prefetch<EpiBwdH<NL>> {
-  static constexpr bool kOn = true;
-  __device__ static __forceinline__ void issue(const EpiBwdH<NL>& e, const RowCtx& r, int m, int n) {
-    const int last = min(31, e.S - 1 - n);
-    if (r.orow >= 0) {
-      const float* d = e.dout + ((size_t)m * (uint32_t)e.L + (uint32_t)r.orow) * (uint32_t)e.S + (uint32_t)n;
-      l2_prefetch(d);
-      l2_prefetch(d + last);
-    }
-    if (e.second) {
-      const float* s2 = e.second + (uint32_t)m * (uint32_t)e.S + (uint32_t)n;
-      l2_prefetch(s2);
-      l2_prefetch(s2 + last);
-    }
-  }
-};
-
-template <int NL> struct ResidentBackward {
-  static constexpr int kPrec = RE2NN_PREC_TF32X3, kFarnn = 0, kEpiWarps = 8;
-  using E1 = EpiBwdQ;
-  using E2 = EpiBwdH<NL>;
-  using EG = EpiBwdQ;     // no gate phases
-  BwdCtx c;
-  struct Tile { int z, k, par; };
-  __device__ __forceinline__ int M() const { return c.B; }
-  __device__ __forceinline__ int S() const { return c.S; }
-  __device__ __forceinline__ int R() const { return c.R; }
-  __device__ __forceinline__ int nsteps(int z, int mt, int steps) const { return min(steps, __ldg(c.tile_last[z] + mt) + 1); }
-  __device__ __forceinline__ void begin(Tile& t, int z) const { t.z = z; }
-  __device__ __forceinline__ void step(Tile& t, int i, int ns) const {      // the i-th executed step is step ns-1-i
-    t.k = ns - 1 - i;
-    t.par = i & 1;
-  }
-  __device__ __forceinline__ RowCtx row(const Tile& t, int m) const {
-    const int n = (int)c.len[m];
-    int tpos, orow, tp2, oprev = -1;
-    bool alive, al2;
-    step_pos(t.z, t.k, n, 0, tpos, orow, alive);
-    if (t.k >= 1) step_pos(t.z, t.k - 1, n, 0, tp2, oprev, al2);
-    const int vrow = c.v_mode == RE2NN_V_TOKEN ? (int)c.x[(size_t)m * c.Lpad + tpos] : m * c.Lpad + tpos;
-    return RowCtx{vrow, oprev, oprev >= 0};
-  }
-  __device__ __forceinline__ EG eg(const Tile& t) const { return e1(t); }
-  __device__ __forceinline__ E1 e1(const Tile& t) const {
-    const size_t sl = slab(c, t.z, t.k, c.R);
-    return E1{c.vtab, c.u_save + sl, c.DU + sl, c.Qs + sl, c.dvtab, c.DUop[t.z], c.R, c.ldR, c.du_plane};
-  }
-  __device__ __forceinline__ E2 e2(const Tile& t) const {
-    const bool prev = t.k >= 1;
-    const size_t sk = slab(c, t.z, t.k, c.S), sp = prev ? slab(c, t.z, t.k - 1, c.S) : 0;
-    E2 e;
-    e.o = c.o;
-    e.dout = t.z == 0 ? c.dalpha : c.dbeta;
-    e.second = t.z == 0 ? (prev ? c.a_save + sp : nullptr) : c.hst_save + slab1(c, t.z, t.k, c.S);
-    e.DAprev = prev ? c.DA + sp : nullptr;
-    e.DOprod = t.z == 0 ? (prev ? c.DOprod + sp : nullptr) : c.DOprod + sk;
-    e.gout = c.g + (size_t)t.z * c.B * c.S;
-    e.DAop = t.par == 0 ? c.DAop1[t.z] : c.DAop[t.z];      // this step reads parity par, the next one par ^ 1
-    e.L = c.L; e.S = c.S; e.ldS = c.ldS; e.z = t.z; e.has_prev = prev ? 1 : 0; e.nl_rt = c.nl;
-    e.da_plane = c.da_plane;
-    return e;
-  }
-};
-
-// grid (2 * m-tiles, L): block (tile, k).  k above the tile's last live step: zero the rows of the step slabs the sweep
-// never writes; k = last live step: E1 with a zero carry (DA, d_o product, the parity-0 DA operand); below: nothing.
-__global__ void __launch_bounds__(256) bwd_resident_init_kernel(const BwdCtx c) {
-  const int m_tiles = (c.B + 127) / 128;
-  const int z = blockIdx.x / m_tiles, mt = blockIdx.x - z * m_tiles, k = blockIdx.y;
-  const int ks = c.tile_last[z][mt];
-  if (k < ks) return;
-  const int m0 = mt * 128, nrows = min(128, c.B - m0);
-  if (k > ks) {
-    float* da = c.DA + slab(c, z, k, c.S) + (size_t)m0 * c.S;
-    float* dp = c.DOprod + slab(c, z, k, c.S) + (size_t)m0 * c.S;
-    float* du = c.DU + slab(c, z, k, c.R) + (size_t)m0 * c.R;
-    float* qs = c.Qs + slab(c, z, k, c.R) + (size_t)m0 * c.R;
-    for (int i = threadIdx.x; i < nrows * c.S; i += blockDim.x) { da[i] = 0.f; dp[i] = 0.f; }
-    for (int i = threadIdx.x; i < nrows * c.R; i += blockDim.x) { du[i] = 0.f; qs[i] = 0.f; }
-    return;
-  }
-  for (int i = threadIdx.x; i < nrows * c.S; i += blockDim.x) {
-    const int r = i / c.S, s = i - r * c.S, b = m0 + r;
-    int tpos, orow;
-    bool alive;
-    step_pos(z, k, (int)c.len[b], 0, tpos, orow, alive);
-    const size_t e = (size_t)b * c.S + s;
-    const size_t sl = slab(c, z, k, c.S) + e;
-    float da = 0.f, dop = 0.f;
-    if (alive) {
-      const float* dout = z == 0 ? c.dalpha : c.dbeta;
-      const float G = orow >= 0 ? dout[((size_t)b * c.L + orow) * c.S + s] : 0.f;
-      const float a = c.a_save[sl];
-      const float on = c.o[s];
-      const float hhat = apply_nl(z == 0 ? a * on : a, c.nl);
-      const float dpre = G * nl_grad_from_out(hhat, c.nl);
-      da = z == 0 ? dpre * on : dpre;
-      dop = dpre * a;
-    }
-    c.DA[sl] = da;
-    if (z == 0) c.DOprod[sl] = dop;
-    OperandFmt<RE2NN_PREC_TF32X3>::store(c.DAop[z], (size_t)b * c.ldS + s, c.da_plane, da);
-  }
-}
-
 // The two GEMMs of every BPTT step (dq = DA @ S, dhbar = DU @ S^T + DA @ W^T) run on the tensor cores in 3xTF32
 // (fp32-grade products, 8-bit exponent: safe for gradients of any magnitude) when tcgen05 is there.
 static bool g_bwd_tc = true;
-// this translation unit's copy of the phase-trace pointer (re2nn_debug_set_tc_trace sets both)
-cudaError_t backward_set_trace(unsigned long long* device_buf) {
-  return cudaMemcpyToSymbol(g_tc_trace, &device_buf, sizeof(device_buf));
-}
-extern int g_resident_train_on;       // recurrence.cu (re2nn_debug_set_resident_train)
-cudaError_t launch_tile_last(const int64_t* len, int B, int* fwd, int* bwd, cudaStream_t st);      // recurrence.cu
 extern "C" int re2nn_has_tcgen05(void);
 static bool bwd_uses_tc() { return g_bwd_tc && re2nn_has_tcgen05() != 0; }
 
@@ -749,8 +545,6 @@ static size_t bwd_carve(const re2nn_backward_args& a, char* base, BwdCtx* c, flo
     for (int z = 0; z < 2; ++z) {
       x.DAop[z] = take(operand_bytes(P, B, (int)S) / 4);
       x.DUop[z] = take(operand_bytes(P, B, (int)R) / 4);
-      x.DAop1[z] = take(operand_bytes(P, B, (int)S) / 4);
-      x.tile_last[z] = (int*)take((B + 127) / 128);
     }
     if (a.C > 0) {        // label-score backward on tensor cores: draw (B*L x C) and C_mat^T (S x C) in operand format
       x.DrawOp = take(operand_bytes(P, B * L, a.C) / 4);
@@ -905,40 +699,7 @@ static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
       if (int rc = tc_make_launch<P>(gg, tg.get())) return rc;
     }
   }
-  // farnn = 0 on tensor cores: the whole sweep in one resident launch (see ResidentBackward)
-  const bool resident = tc && a.farnn == 0 && !a.full_pad && (g_resident_train_on & 2) && resident_supported(2, S, R, true);
-  if (resident) {
-    constexpr int P = RE2NN_PREC_TF32X3;
-    RE2NN_CUDA(launch_tile_last(a.lengths, B, c.tile_last[0], c.tile_last[1], st));
-    bwd_resident_init_kernel<<<dim3(2 * cdiv(B, 128), L), 256, 0, st>>>(c);
-    RE2NN_LAUNCH_CHECK();
-    std::unique_ptr<ResidentLaunch> rl(new ResidentLaunch);
-    memset(rl.get(), 0, sizeof(ResidentLaunch));
-    const int bn1 = resident_part(R), bn2 = resident_part(S);
-    for (int par = 0; par < 2; ++par) {
-      GemmProblem gq, gh;
-      memset(&gq, 0, sizeof(gq));
-      memset(&gh, 0, sizeof(gh));
-      gq.M = B; gq.N = R; gq.nseg = 1; gq.ndir = 2;
-      gh.M = B; gh.N = S; gh.nseg = 2; gh.ndir = 2;
-      for (int z = 0; z < 2; ++z) {
-        void* da = par == 0 ? c.DAop[z] : c.DAop1[z];
-        gq.seg[z][0] = wp.seg_g1(1 - z, da, c.ldS, c.da_plane);               // DA @ S2 (fwd) | DA @ S1 (bwd)
-        gh.seg[z][0] = wp.seg_g2q(1 - z, c.DUop[z], c.ldR, c.du_plane);       // DU @ S1^T (fwd) | DU @ S2^T (bwd)
-        gh.seg[z][1] = wp.seg_g2w(1 - z, da, c.ldS, c.da_plane);              // DA @ W^T (fwd) | DA @ W (bwd)
-      }
-      if (int rc = tc_make_launch<P>(gq, &rl->g1[par], bn1)) return rc;
-      if (int rc = tc_make_launch<P>(gh, &rl->g2[par], bn2)) return rc;
-    }
-    rl->steps = L;
-    rl->q_first = 1;
-    rl->alias_tbuf = resident_alias(2, true) ? 1 : 0;
-    rl->stage_bytes = resident_stage_bytes(2, S, R);
-    rl->stages = resident_stages(2, S, R, true);
-    if (a.update_nonlinear == RE2NN_NL_TANH) RE2NN_CUDA(launch_resident_policy(*rl, ResidentBackward<RE2NN_NL_TANH>{c}, B, st));
-    else RE2NN_CUDA(launch_resident_policy(*rl, ResidentBackward<-1>{c}, B, st));
-  }
-  for (int k = L - 1; k >= 0 && !resident; --k) {
+  for (int k = L - 1; k >= 0; --k) {
     c.k = k;
     if (k == L - 1 || a.farnn >= 1) {      // without gates E1 of the later steps rides in bwd_e31_kernel
       bwd_e1_kernel<<<grid_for((size_t)2 * B * S), 256, 0, st>>>(c);

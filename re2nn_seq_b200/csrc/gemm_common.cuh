@@ -213,7 +213,7 @@ struct StepParams {
     HbarSaveNext[0] = HbarSaveNext[z]; HbarSaveCur[0] = HbarSaveCur[z];
   }
   // bind_const(): selects between CONSTANT indices, so the copy is scalarised into registers.  For the kernels with
-  // registers to spare (eight epilogue warps: gates, training saves): their epilogues touch most fields, and with
+  // registers to spare (eight epilogue warps: the gated recurrences): their epilogues touch most fields, and with
   // 225 KB of the SM given to shared memory there is next to no L1 left to catch local-memory loads.
   __device__ __forceinline__ void bind_const(int zt) {
     const bool one = (zt + dir_base) != 0;

@@ -33,14 +33,12 @@ struct __align__(64) TcLaunch {
   int nseg, nmaps, M, N, BN, ndir;
   int bn;   // effective n-tile width (multiple of 16, <= BN): MMA N, TMA box rows of B, grid.y = ceil(N / bn)
   int cg;   // 1: one CTA per 128 x bn tile; 2: CTA pair per 256 x bn tile (B box rows = bn / 2)
-  int mc;   // 1: multicast variant: clusters of 2 x 2 CTAs on 256 x 512 super-tiles (cg = 1, bn = 256; A box 64 rows, B box 128)
   int launch_id;   // debug trace: index of this launch since tracing was switched on
 };
 typedef TcLaunch TcStepMaps;
 static int g_tc_trace_launches = -1;  // debug: >= 0 while a phase-trace buffer is installed (next launch index)
 static int g_tc_force_cg = 0;        // debug: 0 = cost model picks, 1 / 2 = force the CTA-group size
 static bool g_tc_use_pdl = true;     // programmatic dependent launch between consecutive tcgen05 step kernels
-static int g_tc_multicast = 0;       // 1 = large bf16 GEMMs on 2 x 2 multicast clusters (measured 5-10 % SLOWER than CTA pairs: see tc_make_launch)
 struct TcRecurrenceMaps { TcLaunch gate, g1[2], g2[2]; };
 
 // ---- host: tensor maps ---------------------------------------------------------------------------------
@@ -120,21 +118,7 @@ inline int tc_make_launch(const GemmProblem& g, TcLaunch* out, int force_bn = 0)
     tc_pick_shape(g.M, g.N, g.ndir, OperandFmt<PREC>::kPlanes, OperandFmt<PREC>::kPlanes == 2 ? 3 : 1, &out->bn, &out->BN,
                   &out->cg);
   }
-  // Multicast variant (bf16 only: two planes do not leave room for three stages): large GEMMs run at the L2 -> SM
-  // crossbar ceiling, and a 2 x 2 cluster that multicasts its A row blocks and B column tiles requests 24 KB per CTA
-  // and k-block from L2 instead of 32 KB.  Needs an even number of full 256-column tiles and enough row tiles.
-  // MEASURED (tools/test_mc.py, M=65536 N=1024 K=1536 bf16): correct, but 0.58 vs 0.53 ms per call -- the bytes
-  // DELIVERED to each SM are the same, clusters of four strand SMs (GPCs of 16 / 18 / 20) and leave three stages
-  // instead of four.  Off by default (re2nn_debug_set_tc_multicast).
-  out->mc = 0;
-  if (PREC == RE2NN_PREC_BF16 && force_bn == 0 && g_tc_multicast && out->bn == 256 && g.N % 512 == 0 &&
-      (long)cdiv(g.M, 256) * (g.N / 512) * g.ndir >= 2L * (sm_count() / 4)) {
-    out->mc = 1;
-    out->cg = 1;
-    out->BN = 256;
-  }
-  const int b_box = out->mc ? 128 : out->bn / out->cg;
-  const int a_box = out->mc ? 64 : 128;
+  const int b_box = out->bn / out->cg;
   constexpr int kpb = 128 / OperandFmt<PREC>::kElemBytes;   // K elements per 128-byte block
   int nm = 0;
   for (int z = 0; z < g.ndir; ++z) {
@@ -145,13 +129,13 @@ inline int tc_make_launch(const GemmProblem& g, TcLaunch* out, int force_bn = 0)
       const int kb = cdiv(sg.K, kpb);
       RE2NN_CHECK(nm + 2 * OperandFmt<PREC>::kPlanes <= kTcMaxMaps, "too many tensor maps");
       const int a_hi = nm++;
-      if (int rc = make_operand_map<PREC>(&out->maps[a_hi], sg.A, 0, g.M, sg.K, sg.lda, a_box)) return rc;
+      if (int rc = make_operand_map<PREC>(&out->maps[a_hi], sg.A, 0, g.M, sg.K, sg.lda, 128)) return rc;
       const int b_hi = nm++;
       if (int rc = make_operand_map<PREC>(&out->maps[b_hi], sg.B, 0, g.N, sg.K, sg.ldb, b_box)) return rc;
       int a_lo = -1, b_lo = -1;
       if (OperandFmt<PREC>::kPlanes == 2) {
         a_lo = nm++;
-        if (int rc = make_operand_map<PREC>(&out->maps[a_lo], sg.A, sg.a_plane, g.M, sg.K, sg.lda, a_box)) return rc;
+        if (int rc = make_operand_map<PREC>(&out->maps[a_lo], sg.A, sg.a_plane, g.M, sg.K, sg.lda, 128)) return rc;
         b_lo = nm++;
         if (int rc = make_operand_map<PREC>(&out->maps[b_lo], sg.B, sg.b_plane, g.N, sg.K, sg.ldb, b_box)) return rc;
       }
@@ -208,19 +192,6 @@ __device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(dst), "l"((uint64_t)map), "r"(leader_bar), "r"(c0), "r"(c1)
       : "memory");
-}
-// multicast load: the box lands at the same offset in every CTA of `mask`, each of their barriers (same offset) gets the bytes
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(dst), "l"((uint64_t)map), "r"(bar), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-// commit that arrives on the barrier at this offset in every CTA of `mask`
-__device__ __forceinline__ void tc_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"(mask)
-               : "memory");
 }
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
@@ -580,31 +551,25 @@ __device__ __forceinline__ void tc_epilogue_quads(const Epi epi, int M, int N, i
 
 // Persistent kernel: CTA c works on tiles c, c + gridDim.x, ...; tile id -> (direction z, m-tile, n-tile) with the
 // n-tile fastest so concurrently running CTAs share A tiles in L2.
-template <int PREC, int BN, int CG, class Epi, bool MC = false>
+template <int PREC, int BN, int CG, class Epi>
 __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_constant__ TcLaunch L, const Epi epi_in) {
   using Cfg = TcCfg<PREC, BN, CG>;
   constexpr bool PAIR = CG == 2;
-  static_assert(!MC || CG == 1, "the multicast variant issues its own MMAs per CTA");
   constexpr bool TF32 = PREC == RE2NN_PREC_TF32X3;
   constexpr bool SPLIT = Cfg::kPlanes == 2;
   constexpr bool TWOACC = Cfg::kAccs == 2;
   constexpr bool OVERLAP = Cfg::kOverlap;
   constexpr int kpb = 128 / OperandFmt<PREC>::kElemBytes;
   const int bn = L.bn;
-  // MC: a cluster of 2 x 2 CTAs works on a 256 x (2 bn) super-tile: CTA (ci, cj) owns rows ci*128.. of it and column
-  // tile cj; it loads HALF of its A row block (multicast to the CTA with the other cj) and HALF of its B column tile
-  // (multicast to the CTA with the other ci).  Every barrier is CTA-local; a stage is free when this CTA and both
-  // partners have consumed it (three multicast commits arrive on every empty barrier).
-  constexpr int kTileM = MC ? 256 : 128 * CG;            // rows of one (pair / cluster) tile
-  const int m_tiles = (L.M + kTileM - 1) / kTileM, n_tiles = MC ? (L.N + 2 * bn - 1) / (2 * bn) : (L.N + bn - 1) / bn;
+  constexpr int kTileM = 128 * CG;                       // rows of one (pair) tile
+  const int m_tiles = (L.M + kTileM - 1) / kTileM, n_tiles = (L.N + bn - 1) / bn;
   const int tiles_per_dir = m_tiles * n_tiles, total_tiles = tiles_per_dir * L.ndir;
-  const int cr4 = MC ? (int)cluster_ctarank() : 0, ci = cr4 & 1, cj = cr4 >> 1;
   const int crank = PAIR ? (int)cluster_ctarank() : 0;   // 0 = leader (issues the MMAs), 1 = peer
-  const int worker = MC ? (int)(blockIdx.x >> 2) : (PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x);
-  const int nworkers = MC ? (int)(gridDim.x >> 2) : (PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x);
+  const int worker = PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
+  const int nworkers = PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x;
   // a 128-row block past the end of M (second half of the last pair tile) is simply dead
   auto alive = [&](int z, int mt) -> bool {
-    if (!PAIR && !MC) return epi_in.tile_alive(z, mt);
+    if (!PAIR) return epi_in.tile_alive(z, mt);
     const int last = (L.M + 127) / 128 - 1;
     return epi_in.tile_alive(z, 2 * mt) || (2 * mt + 1 <= last && epi_in.tile_alive(z, 2 * mt + 1));
   };
@@ -646,7 +611,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
       }
     for (int s = 0; s < Cfg::kStages; ++s) {
       mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), MC ? 3 : 1);
+      mbar_init(empty_bar(s), 1);
     }
     for (int s = 0; s < 2; ++s) {
       mbar_init(tfull_bar(s), 1);
@@ -666,7 +631,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
     }
   }
   tc_fence_before();
-  if (PAIR || MC) cluster_sync_all();     // the peers' barriers must exist before anything arrives on them remotely
+  if (PAIR) cluster_sync_all();     // the peer's barriers must exist before anything arrives on them remotely
   else __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot_p;
@@ -684,8 +649,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
       const int z = tile / tiles_per_dir, rem = tile - z * tiles_per_dir;
       const int mt = rem / n_tiles, nt = rem - mt * n_tiles;
       if (!alive(z, mt)) continue;
-      const int m0 = MC ? mt * 256 + ci * 128 : mt * kTileM + crank * 128;
-      const int n0 = MC ? (2 * nt + cj) * bn : nt * bn + crank * (int)bbox;
+      const int m0 = mt * kTileM + crank * 128, n0 = nt * bn + crank * (int)bbox;
       if (lane == 0) {
         for (int s = 0; s < nseg; ++s) {
           const TcSeg sg = L.seg[z][s];
@@ -696,12 +660,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
             const uint32_t ph = (it / Cfg::kStages) & 1;
             mbar_wait(empty_bar(st), ph ^ 1);
             const uint32_t sa = base + st * Cfg::kStageBytes;
-            if (MC) {
-              const uint16_t mask_a = (uint16_t)((1u << cr4) | (1u << (cr4 ^ 2))), mask_b = (uint16_t)((1u << cr4) | (1u << (cr4 ^ 1)));
-              mbar_expect_tx(full_bar(st), (uint32_t)(Cfg::kPlanes * (Cfg::kATile + BN * 128)));
-              tma_load_2d_mc(sa + (uint32_t)cj * 64u * 128u, ma, full_bar(st), kb * kpb, m0 + cj * 64, mask_a);
-              tma_load_2d_mc(sa + Cfg::kABytes + (uint32_t)ci * 128u * 128u, mb, full_bar(st), kb * kpb, n0 + ci * 128, mask_b);
-            } else if (PAIR) {
+            if (PAIR) {
               const uint32_t fb = mapa_shared(full_bar(st), 0);         // the leader's barrier collects both CTAs' bytes
               if (crank == 0) mbar_expect_tx(full_bar(st), 2u * cta_bytes);
               tma_load_2d_pair(sa, ma, fb, kb * kpb, m0);
@@ -731,7 +690,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
     // instruction descriptor: D=f32, A/B = f16 (0) / bf16 (1) / tf32 (2), both K-major, N>>3, M>>4
     const uint32_t fmt = TF32 ? 2u : (PREC == RE2NN_PREC_FP16X3 ? 0u : 1u);
     const uint32_t idesc =
-        (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(bn >> 3) << 17) | (((uint32_t)(128 * CG) >> 4) << 24);
+        (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(bn >> 3) << 17) | (((uint32_t)kTileM >> 4) << 24);
     int it = 0, tcount = 0;
     griddep_wait();
     if (lane == 0) tc_stamp(trace, 1);   // previous grid complete
@@ -773,7 +732,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
             }
           }
           if (PAIR) tc_commit_pair(empty_bar(st));   // frees this slot in both CTAs once the MMAs have read it
-          else if (MC) tc_commit_mc(empty_bar(st), (uint16_t)((1u << cr4) | (1u << (cr4 ^ 1)) | (1u << (cr4 ^ 2))));
           else tc_commit(empty_bar(st));
         }
         if (PAIR) tc_commit_pair(tfull_bar(as));     // accumulator complete (each CTA's epilogue waits on its own)
@@ -799,8 +757,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
       const int z = tile / tiles_per_dir, rem = tile - z * tiles_per_dir;
       const int mt = rem / n_tiles, nt = rem - mt * n_tiles;
       if (!alive(z, mt)) continue;
-      const int m0 = MC ? mt * 256 + ci * 128 : mt * kTileM + crank * 128;
-      const int n0 = MC ? (2 * nt + cj) * bn : nt * bn;
+      const int m0 = mt * kTileM + crank * 128, n0 = nt * bn;
       const Epi epi = epi_in.for_dir(z);    // direction-bound copy: plain members, no per-element z indexing
       const int mrow0 = m0 + q * 32;
       const int as = OVERLAP ? (tcount & 1) : 0;
@@ -834,7 +791,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) tc_gemm_kernel(const __grid_con
     }
   }
   tc_fence_before();
-  if (PAIR || MC) cluster_sync_all();     // no CTA may retire while the cluster still touches its smem / TMEM
+  if (PAIR) cluster_sync_all();     // neither CTA may retire while the pair still touches its smem / TMEM
   else __syncthreads();
   if (threadIdx.x == 0) tc_stamp(trace, 7);
   if (tl_idx < 4096) g_tc_timeline[2 * tl_idx + 1] = globaltimer_ns();
@@ -884,59 +841,12 @@ inline cudaError_t launch_tc_bn(const TcLaunch& L, const Epi& epi, cudaStream_t 
   return cudaLaunchKernelEx(&cfg, tc_gemm_kernel<PREC, BN, CG, Epi>, L, epi);
 }
 
-// multicast variant: clusters of four (2 x 2), as many as can be co-resident (GPCs of 16 / 18 / 20 SMs strand a few SMs)
-template <int PREC, class Epi>
-inline cudaError_t launch_tc_mc(const TcLaunch& L, const Epi& epi, cudaStream_t st) {
-  using Cfg = TcCfg<PREC, 256, 1>;
-  auto kern = tc_gemm_kernel<PREC, 256, 1, Epi, true>;
-  static int configured[kMaxDevices];
-  static int max_clusters[kMaxDevices];
-  if (cudaError_t e = ensure_dynamic_smem(kern, Cfg::kSmem, configured)) return e;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.blockDim = dim3(kTcThreads);
-  cfg.dynamicSmemBytes = Cfg::kSmem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 4;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  int na = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = na;
-  const int d = device_slot();
-  if (max_clusters[d] == 0) {
-    cfg.gridDim = dim3((unsigned)(sm_count() / 4 * 4));
-    int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess || n <= 0) n = sm_count() / 4 - 4;
-    max_clusters[d] = n;
-  }
-  const long tiles = (long)cdiv(L.M, 256) * cdiv(L.N, 512) * L.ndir;
-  cfg.gridDim = dim3((unsigned)(std::min<long>(tiles, max_clusters[d]) * 4));
-  if (g_tc_use_pdl) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  cfg.numAttrs = na;
-  if (g_tc_trace_launches >= 0) {
-    TcLaunch Lt = L;
-    Lt.launch_id = g_tc_trace_launches++;
-    return cudaLaunchKernelEx(&cfg, kern, Lt, epi);
-  }
-  return cudaLaunchKernelEx(&cfg, kern, L, epi);
-}
-
 template <int PREC, class Epi>
 inline cudaError_t launch_tc_gemm(const GemmProblem&, const Epi& epi, const TcStepMaps* L, cudaStream_t st) {
   if constexpr (PREC == RE2NN_PREC_FP32) {
     return cudaErrorNotSupported;
   } else {
     if (L == nullptr) return cudaErrorInvalidValue;
-    if constexpr (PREC == RE2NN_PREC_BF16) {
-      if (L->mc) return launch_tc_mc<PREC>(*L, epi, st);
-    }
     if (L->cg == 2) {
       switch (L->BN) {
         case 64: return launch_tc_bn<PREC, 64, 2>(*L, epi, st);

@@ -79,12 +79,6 @@ __global__ void __launch_bounds__(128) tile_last_kernel(const int64_t* __restric
   }
 }
 
-cudaError_t backward_set_trace(unsigned long long* device_buf);      // backward.cu
-cudaError_t launch_tile_last(const int64_t* len, int B, int* fwd, int* bwd, cudaStream_t st) {
-  tile_last_kernel<<<cdiv(B, 128), 128, 0, st>>>(len, B, fwd, bwd);
-  return cudaGetLastError();
-}
-
 // ---- init: step "-1" ------------------------------------------------------------------------------
 template <int PREC>
 __global__ void rec_init_kernel(int B, int L, int S, int farnn, const int64_t* len, const float* h0, const float* hT,
@@ -115,11 +109,7 @@ __global__ void rec_init_kernel(int B, int L, int S, int farnn, const int64_t* l
 
 // ---- optional per-launch timing ------------------------------------------------------------------------
 struct ProfPair { cudaEvent_t a, b; };
-static bool g_resident_on = true;    // run the whole recurrence in one resident launch (tensor-core precisions)
-// training on resident launches: bit 0 = the forward that keeps the BPTT slabs, bit 1 = the BPTT sweep (backward.cu).
-// Off by default: measured slower than the per-step launches at the benchmarked batch (cfg3, B = 1024: 6.8 vs 5.25 ms
-// per training step) and within 3 % of them at B = 4096 (12.3 vs 12.65 ms) -- see DESIGN.md section 3.
-int g_resident_train_on = 0;
+static bool g_resident_on = true;    // inference: run the whole recurrence in one resident launch (tensor-core precisions)
 static bool g_prof_on = false;
 static std::vector<ProfPair> g_prof_pool;        // all event pairs ever created
 static std::vector<int> g_prof_used[4];          // indices into the pool, per kernel class (3 = resident recurrence)
@@ -234,10 +224,8 @@ static int run_recurrence(const re2nn_recurrence_args& a, cudaStream_t st) {
   for (int z = 0; z < 2; ++z) { p.Q[z] = w.Q[z]; p.Hst[z] = w.Hst[z]; p.H[z] = w.H[z]; }
 
   if constexpr (PREC != RE2NN_PREC_FP32) {
-    // One resident launch (a CTA pair per 128-row tile runs all steps; recurrence_resident.cuh): inference in every
-    // tensor-core precision, training (save slabs for BPTT) in the split formats
-    const bool train_res = a.save_for_backward && (g_resident_train_on & 1) && PREC != RE2NN_PREC_BF16;
-    if (g_resident_on && (!a.save_for_backward || train_res) &&
+    // Inference: one resident launch (a CTA pair per 128-row tile runs all steps; recurrence_resident.cuh)
+    if (g_resident_on && !a.save_for_backward &&
         resident_supported(OperandFmt<PREC>::kPlanes, S, R, PREC != RE2NN_PREC_BF16)) {
       std::unique_ptr<ResidentLaunch> rl(new ResidentLaunch);
       memset(rl.get(), 0, sizeof(ResidentLaunch));
@@ -266,23 +254,7 @@ static int run_recurrence(const re2nn_recurrence_args& a, cudaStream_t st) {
       const int pi = prof_begin(3, st);
       const bool th = a.update_nonlinear == RE2NN_NL_TANH;
       cudaError_t e;
-      if (train_res) {
-        // save pointers of step 0; the kernel advances them by one slab per step (same layout as the per-step path below)
-        const size_t sS = (size_t)B * S, sR = (size_t)B * R;
-        for (int z = 0; z < 2; ++z) {
-          float* hb0 = a.hbar_save + (size_t)z * (L + 1) * sS;
-          float* hs0 = a.hst_save + (size_t)z * (L + 1) * sS;
-          p.HstNext[z] = hs0 + sS;
-          p.HbarSaveNext[z] = hb0 + sS;
-          p.HbarSaveCur[z] = hb0;
-          p.Usave[z] = a.u_save + (size_t)z * L * sR;
-          p.Asave[z] = a.a_save + (size_t)z * L * sS;
-          if (a.farnn >= 1) p.Z[z] = a.zsave + (size_t)z * L * sS;
-          p.Rg[z] = a.farnn == 2 ? a.rsave + (size_t)z * L * sS : nullptr;
-        }
-        e = launch_resident_train(PREC, th ? RE2NN_NL_TANH : -1, a.farnn, *rl, p, sS, sR, B, st);
-      }
-      else if (a.farnn == 0) e = th ? launch_resident<PREC, RE2NN_NL_TANH, 0>(*rl, p, B, st) : launch_resident<PREC, -1, 0>(*rl, p, B, st);
+      if (a.farnn == 0) e = th ? launch_resident<PREC, RE2NN_NL_TANH, 0>(*rl, p, B, st) : launch_resident<PREC, -1, 0>(*rl, p, B, st);
       else if (a.farnn == 1) e = th ? launch_resident<PREC, RE2NN_NL_TANH, 1>(*rl, p, B, st) : launch_resident<PREC, -1, 1>(*rl, p, B, st);
       else e = th ? launch_resident<PREC, RE2NN_NL_TANH, 2>(*rl, p, B, st) : launch_resident<PREC, -1, 2>(*rl, p, B, st);
       prof_end(pi, st);
@@ -520,7 +492,6 @@ int re2nn_abi_version(void) { return RE2NN_ABI_VERSION; }
 
 int re2nn_debug_set_tc_trace(unsigned long long* device_buf) {
   RE2NN_CUDA(cudaMemcpyToSymbol(g_tc_trace, &device_buf, sizeof(device_buf)));
-  RE2NN_CUDA(backward_set_trace(device_buf));
   g_tc_trace_launches = device_buf ? 0 : -1;
   return 0;
 }
@@ -540,20 +511,8 @@ int re2nn_debug_set_tc_cta_group(int cta_group) {
   return 0;
 }
 
-int re2nn_debug_set_tc_multicast(int on) {
-#ifdef RE2NN_HAVE_TC
-  g_tc_multicast = on != 0;
-#endif
-  return 0;
-}
-
 int re2nn_debug_set_resident(int on) {
   g_resident_on = on != 0;
-  return 0;
-}
-
-int re2nn_debug_set_resident_train(int on) {
-  g_resident_train_on = on;
   return 0;
 }
 
@@ -624,8 +583,7 @@ size_t re2nn_decompose_recurrence_workspace(const re2nn_recurrence_args* a) {
 
 // does this call take the resident single-launch path?  (mirrors the test in run_recurrence)
 static bool takes_resident_path(const re2nn_recurrence_args& a) {
-  if (a.precision == RE2NN_PREC_FP32 || !g_resident_on) return false;
-  if (a.save_for_backward && (!(g_resident_train_on & 1) || a.precision == RE2NN_PREC_BF16)) return false;
+  if (a.precision == RE2NN_PREC_FP32 || !g_resident_on || a.save_for_backward) return false;
   const int planes = a.precision == RE2NN_PREC_BF16 ? 1 : 2;
   return resident_supported(planes, a.S, a.R, a.precision != RE2NN_PREC_BF16);
 }

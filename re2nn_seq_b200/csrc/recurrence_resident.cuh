@@ -1,7 +1,4 @@
-// Resident decompose recurrence (farnn = 0 / 1 / 2): ONE launch runs every step of both directions.  Inference is the
-// default user; the same kernel takes the training forward (save slabs) and the BPTT sweep as epilogue policies
-// (ResidentForward<.., TRAIN>, backward.cu: ResidentBackward) -- measured slower than per-step launches at B = 1024 and
-// therefore off by default (re2nn_debug_set_resident_train).
+// Resident decompose recurrence for inference (farnn = 0 / 1 / 2): ONE launch runs every step of both directions.
 //
 // The per-step launches of recurrence.cu are bound by what happens BETWEEN the GEMMs, not by the GEMMs: every
 // step boundary is a grid-wide dependency (drain the epilogue stores, resolve the launch, refill the operand
@@ -38,93 +35,30 @@ struct __align__(64) ResidentLaunch {
 };
 
 constexpr int kResEpiWarps = 12;        // at most three epilogue warps per TMEM lane quarter (shared-memory sizing)
-// epilogue warps actually launched: Policy::kEpiWarps (12 for plain inference, 8 otherwise)
+// epilogue warps actually launched: twelve leave 128 registers per thread, enough for the epilogues without gates
+// only.  The gate epilogues spill at that budget, and with 225 KB of the SM given to shared memory the spill traffic
+// misses L1 on every access, so the gated kernels run 8
+__host__ __device__ constexpr int resident_epi_warps(int farnn) { return farnn == 0 ? 12 : 8; }
 constexpr int kResThreads = 64 + 32 * kResEpiWarps;
 constexpr int kResTbufBytes = kResEpiWarps * kTcTbufWords * 4;
 constexpr int kResCtxBytes = kResEpiWarps * kTcCtxWords * 4;
 constexpr int kResTbufPerStage = 7;     // 7 x 4608 B fit the 32 KB A region (two planes) of one stage
 constexpr uint32_t kResCorrOff = 256;   // TMEM column of the second (residual) accumulator of the fp16 split
 
-// What the epilogue warps do with the two (three, four with gates) accumulators of a step is a policy: the forward
-// recurrence (inference or training saves) below, the BPTT sweep in backward.cu.  A policy provides
-//   kPrec, kFarnn (gate phases per step), M() / S() / R(), nsteps(z, m-tile, L),
-//   Tile (per-tile state of an epilogue warp), begin(tile, z), step(tile, i, ns)  -- i counts executed steps --,
-//   row(tile, m) -> RowCtx of row m for this step, and the epilogue functors eg / e1 / e2 of the step.
-template <int PREC, int NL, int FARNN, bool TRAIN = false> struct ResidentForward {
-  static constexpr int kPrec = PREC, kFarnn = FARNN;
-  // twelve epilogue warps leave 128 registers per thread: enough for the plain inference epilogues only.  The gate
-  // epilogues and the ones that write the training slabs spill at that budget, and with 225 KB of the SM given to
-  // shared memory the spill traffic misses L1 on every access (measured: the BPTT sweep ran 3x slower) -> 8 warps
-  static constexpr int kEpiWarps = (FARNN == 0 && !TRAIN) ? 12 : 8;
-  using E1 = EpiQ<PREC, TRAIN>;
-  using E2 = EpiH<PREC, NL, FARNN, TRAIN>;
-  using EG = EpiGate<PREC, TRAIN>;
-  StepParams p;          // Hbar_cur / Hbar_next = parity-0 / parity-1 operand buffers; TRAIN: the save pointers of step 0
-  size_t sS, sR;         // TRAIN: elements between the slabs of consecutive steps (B*S, B*R)
-  struct Tile {
-    StepParams ps;
-    void *hbar0, *hbar1;
-    float *u0, *a0, *hst0, *hbn0, *hbc0, *z0, *r0;
-  };
-  __device__ __forceinline__ int M() const { return p.B; }
-  __device__ __forceinline__ int S() const { return p.S; }
-  __device__ __forceinline__ int R() const { return p.R; }
-  // steps this tile runs: rows past their length are never observed (tile_last: last step any row is alive)
-  __device__ __forceinline__ int nsteps(int z, int mt, int steps) const {
-    if (p.full_pad) return steps;
-    return min(steps, __ldg(p.tile_last[z] + mt) + 1);
-  }
-  __device__ __forceinline__ void begin(Tile& t, int z) const {
-    t.ps = p;
-    if constexpr (kEpiWarps == 12) {      // see StepParams::bind / bind_const
-      t.hbar0 = p.Hbar_cur[z];
-      t.hbar1 = p.Hbar_next[z];
-      t.ps.bind(z);
-    } else {
-      t.hbar0 = z ? p.Hbar_cur[1] : p.Hbar_cur[0];
-      t.hbar1 = z ? p.Hbar_next[1] : p.Hbar_next[0];
-      t.ps.bind_const(z);
-    }
-    if constexpr (TRAIN) {
-      t.u0 = t.ps.Usave[0]; t.a0 = t.ps.Asave[0]; t.hst0 = t.ps.HstNext[0];
-      t.hbn0 = t.ps.HbarSaveNext[0]; t.hbc0 = t.ps.HbarSaveCur[0]; t.z0 = t.ps.Z[0]; t.r0 = t.ps.Rg[0];
-    }
-  }
-  __device__ __forceinline__ void step(Tile& t, int k, int) const {
-    t.ps.k = k;
-    t.ps.Hbar_cur[0] = (k & 1) ? t.hbar1 : t.hbar0;
-    t.ps.Hbar_next[0] = (k & 1) ? t.hbar0 : t.hbar1;
-    if constexpr (TRAIN) {      // step-major save slabs (recurrence.cu lays them out; rows that are finished get zeros)
-      t.ps.Usave[0] = t.u0 + (size_t)k * sR;
-      t.ps.Asave[0] = t.a0 + (size_t)k * sS;
-      t.ps.HstNext[0] = t.hst0 + (size_t)k * sS;
-      t.ps.HbarSaveNext[0] = t.hbn0 + (size_t)k * sS;
-      t.ps.HbarSaveCur[0] = t.hbc0 + (size_t)k * sS;
-      if (FARNN >= 1) t.ps.Z[0] = t.z0 + (size_t)k * sS;
-      if (FARNN == 2) t.ps.Rg[0] = t.r0 + (size_t)k * sS;
-    }
-  }
-  __device__ __forceinline__ RowCtx row(const Tile& t, int m) const { return make_row(t.ps, t.ps.dir, m); }
-  __device__ __forceinline__ EG eg(const Tile& t) const { return EG{t.ps}; }
-  __device__ __forceinline__ E1 e1(const Tile& t) const { return E1{t.ps}; }
-  __device__ __forceinline__ E2 e2(const Tile& t) const { return E2{t.ps}; }
-};
-
-template <class Pol>
-__global__ void __launch_bounds__(64 + 32 * Pol::kEpiWarps, 1) tc_resident_kernel(const __grid_constant__ ResidentLaunch RL,
-                                                                                                  const Pol pol) {
-  constexpr int PREC = Pol::kPrec, FARNN = Pol::kFarnn;
+template <int PREC, int NL, int FARNN>
+__global__ void __launch_bounds__(64 + 32 * resident_epi_warps(FARNN), 1) tc_resident_kernel(const __grid_constant__ ResidentLaunch RL,
+                                                                    const StepParams p_in) {
   constexpr bool TF32 = PREC == RE2NN_PREC_TF32X3;
   constexpr int kPlanes = OperandFmt<PREC>::kPlanes;
   constexpr bool SPLIT = kPlanes == 2;
   constexpr bool TWOACC = PREC == RE2NN_PREC_FP16X3;
   constexpr int kpb = 128 / OperandFmt<PREC>::kElemBytes;
   constexpr int kATile = 128 * 128;
-  constexpr int EW = Pol::kEpiWarps;
+  constexpr int EW = resident_epi_warps(FARNN);
 
   const int crank = (int)cluster_ctarank();
   const int worker = (int)(blockIdx.x >> 1), nworkers = (int)(gridDim.x >> 1);
-  const int M = pol.M(), S = pol.S(), R = pol.R();
+  const int M = p_in.B, S = p_in.S, R = p_in.R;
   const int m_tiles = (M + 127) / 128, total_tiles = 2 * m_tiles;
   const int stages = RL.stages;
   const uint32_t stage_bytes = (uint32_t)RL.stage_bytes;
@@ -192,7 +126,11 @@ __global__ void __launch_bounds__(64 + 32 * Pol::kEpiWarps, 1) tc_resident_kerne
   const uint32_t tmem_base = *tmem_slot_p;
   if (threadIdx.x == 0) tc_stamp(trace, 2);
 
-  auto nsteps = [&](int z, int mt) -> int { return pol.nsteps(z, mt, RL.steps); };
+  // steps this tile runs: rows past their length are never observed (tile_last: last step any row is alive)
+  auto nsteps = [&](int z, int mt) -> int {
+    if (p_in.full_pad) return RL.steps;
+    return min(RL.steps, __ldg(p_in.tile_last[z] + mt) + 1);
+  };
 
   if (warp == 0) {
     // ---- TMA producer ------------------------------------------------------------------------------------
@@ -333,21 +271,33 @@ __global__ void __launch_bounds__(64 + 32 * Pol::kEpiWarps, 1) tc_resident_kerne
       const int z = tile / m_tiles, mt = tile - z * m_tiles;
       const int ns = nsteps(z, mt);
       const int mrow0 = mt * 128 + q * 32;
-      typename Pol::Tile tl;
-      pol.begin(tl, z);
+      StepParams ps = p_in;
+      void* hbar0;      // host: Hbar_cur = parity-0 buffer, Hbar_next = parity-1 buffer
+      void* hbar1;
+      if constexpr (EW == 12) {      // see StepParams::bind / bind_const
+        hbar0 = p_in.Hbar_cur[z];
+        hbar1 = p_in.Hbar_next[z];
+        ps.bind(z);
+      } else {
+        hbar0 = z ? p_in.Hbar_cur[1] : p_in.Hbar_cur[0];
+        hbar1 = z ? p_in.Hbar_next[1] : p_in.Hbar_next[0];
+        ps.bind_const(z);
+      }
       for (int k = 0; k < ns; ++k) {
-        pol.step(tl, k, ns);
-        const typename Pol::E1 e1 = pol.e1(tl);
+        ps.k = k;
+        ps.Hbar_cur[0] = (k & 1) ? hbar1 : hbar0;
+        ps.Hbar_next[0] = (k & 1) ? hbar0 : hbar1;
+        const EpiQ<PREC> e1{ps};
         {
           RowCtx mine{0, -1, false};
-          if (mrow0 + lane < M) mine = pol.row(tl, mrow0 + lane);
+          if (mrow0 + lane < M) mine = e1.row(mrow0 + lane);
           ctx[lane] = mine.vrow;
           ctx[32 + lane] = mine.orow;
         }
         __syncwarp();
         const bool tr = tile == worker && k == 2 && ew == 0 && lane == 0;
         if constexpr (FARNN >= 1) {
-          const typename Pol::EG eg = pol.eg(tl);
+          const EpiGate<PREC> eg{ps};
           tc_epilogue_chunks<TWOACC, EW / 4>(eg, M, S, mrow0, crank * bn2, bn2, tmem_rows, kResCorrOff, half, lane,
                                                        tbuf, ctx, tfull_bar, acc & 1u, nullptr);
           release_and_publish();
@@ -357,7 +307,7 @@ __global__ void __launch_bounds__(64 + 32 * Pol::kEpiWarps, 1) tc_resident_kerne
             release_and_publish();
           }
         }
-        if constexpr (EpiHasRows<typename Pol::E1>::value)
+        if constexpr (EpiHasRows<EpiQ<PREC>>::value)
           tc_epilogue_quads<TWOACC, EW / 4>(e1, M, R, mrow0, crank * bn1, bn1, tmem_rows, kResCorrOff, half, lane, tbuf, ctx,
                                             tfull_bar, acc & 1u);
         else
@@ -365,8 +315,8 @@ __global__ void __launch_bounds__(64 + 32 * Pol::kEpiWarps, 1) tc_resident_kerne
                                              tfull_bar, acc & 1u, nullptr);
         if (tr) tc_stamp(trace, 18);
         release_and_publish();
-        const typename Pol::E2 e2 = pol.e2(tl);
-        if constexpr (EpiHasRows<typename Pol::E2>::value)
+        const EpiH<PREC, NL, FARNN> e2{ps};
+        if constexpr (EpiHasRows<EpiH<PREC, NL, FARNN>>::value)
           tc_epilogue_quads<TWOACC, EW / 4>(e2, M, S, mrow0, crank * bn2, bn2, tmem_rows, kResCorrOff, half, lane, tbuf, ctx,
                                             tfull_bar, acc & 1u, tr ? trace : nullptr);
         else
@@ -408,16 +358,16 @@ inline bool resident_supported(int planes, int S, int R, bool q_first) {
   return resident_part(S) <= 256 && resident_part(R) <= 256 && st >= 2;
 }
 
-template <class Pol>
-inline cudaError_t launch_resident_policy(const ResidentLaunch& RL, const Pol& pol, int B, cudaStream_t st) {
-  const int smem = resident_smem_bytes(OperandFmt<Pol::kPrec>::kPlanes, RL.stages, RL.stage_bytes, RL.q_first != 0);
+template <int PREC, int NL, int FARNN>
+inline cudaError_t launch_resident(const ResidentLaunch& RL, const StepParams& p, int B, cudaStream_t st) {
+  const int smem = resident_smem_bytes(OperandFmt<PREC>::kPlanes, RL.stages, RL.stage_bytes, RL.q_first != 0);
   static int configured[kMaxDevices];
-  if (cudaError_t e = ensure_dynamic_smem(tc_resident_kernel<Pol>, smem, configured)) return e;
+  if (cudaError_t e = ensure_dynamic_smem(tc_resident_kernel<PREC, NL, FARNN>, smem, configured)) return e;
   const long tiles = 2L * cdiv(B, 128);
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)(std::min<long>(tiles, sm_count() / 2) * 2));   // one CTA pair per SM pair
-  cfg.blockDim = dim3(64 + 32 * Pol::kEpiWarps);
+  cfg.blockDim = dim3(64 + 32 * resident_epi_warps(FARNN));
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
@@ -427,16 +377,7 @@ inline cudaError_t launch_resident_policy(const ResidentLaunch& RL, const Pol& p
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, tc_resident_kernel<Pol>, RL, pol);
+  return cudaLaunchKernelEx(&cfg, tc_resident_kernel<PREC, NL, FARNN>, RL, p);
 }
-
-template <int PREC, int NL, int FARNN>
-inline cudaError_t launch_resident(const ResidentLaunch& RL, const StepParams& p, int B, cudaStream_t st) {
-  return launch_resident_policy(RL, ResidentForward<PREC, NL, FARNN, false>{p, 0, 0}, B, st);
-}
-
-// training forward (save slabs): instantiated in recurrence_train.cu (tf32x3 / fp16x3; update_nonlinear tanh or generic)
-cudaError_t launch_resident_train(int prec, int nl, int farnn, const ResidentLaunch& RL, const StepParams& p, size_t sS,
-                                  size_t sR, int B, cudaStream_t st);
 
 }  // namespace re2nn

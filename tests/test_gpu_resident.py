@@ -253,44 +253,6 @@ def test_graph_policy_over_an_evaluation_sweep():
     assert len(m._graphs) == 0
 
 
-def _set_resident_train(on):
-    from re2nn_seq_b200 import _lib
-    _lib.check(_lib.fn['re2nn_debug_set_resident_train'](3 if on else 0), 'resident_train')
-
-
-@pytest.mark.parametrize('tp', ['fp16x3', 'tf32x3'])
-@pytest.mark.parametrize('farnn,B,S,R,L,nl,crf', [(0, 300, 300, 200, 14, 'tanh', 1), (0, 1500, 96, 48, 9, 'relu', 0),
-                                                  (2, 260, 128, 64, 8, 'tanh', 1), (1, 200, 64, 40, 7, 'tanh', 0)])
-def test_training_resident_matches_per_step(farnn, B, S, R, L, nl, crf, tp):
-    """Training on resident launches (forward with the BPTT slabs; for farnn = 0 the BPTT sweep itself) against the
-    per-step launches: same loss, same gradients (the sweep only reorders the atomic adds of the token-table gradient)."""
-    from test_gpu_parity import _random_decompose
-    _need_tc()
-    m, args, x, lens, lab = _random_decompose(21, 400, S, R, 20, 50, B, L, farnn=farnn, use_crf=crf, update_nonlinear=nl,
-                                              beta=0.1, train_h0=1, train_hT=1)
-    lens[:3] = [L, 1, 2][:3]                 # a full-length row, and rows that are done after one / two steps
-    m.train_precision = tp
-    xt, lt, yt = _t(x), _t(lens), _t(lab)
-    out = {}
-    try:
-        for on in (True, False):
-            _set_resident_train(on)
-            m.zero_grad(set_to_none=True)
-            loss, _, _ = m.forward_local(xt, yt, lt, train=True)
-            loss.backward()
-            torch.cuda.synchronize()
-            out[on] = (loss.item(), {k: v.grad.detach().clone() for k, v in m.named_parameters() if v.grad is not None})
-    finally:
-        _set_resident_train(False)          # the default: per-step launches (resident training measured slower at B = 1024)
-    assert out[True][0] == out[False][0], (out[True][0], out[False][0])
-    assert set(out[True][1]) == set(out[False][1]) and len(out[True][1]) >= 5
-    for k, g in out[True][1].items():
-        ref = out[False][1][k]
-        scale = ref.abs().max().item() + 1e-30
-        err = (g - ref).abs().max().item() / scale
-        assert err < 2e-6, '%s: %.3e' % (k, err)
-
-
 @pytest.mark.parametrize('farnn,B,S,R,L', [(0, 700, 300, 200, 13), (2, 520, 136, 72, 9), (0, 333, 64, 40, 14)])
 def test_weight_gradient_gemm_on_tensor_cores_matches_cuda_cores(farnn, B, S, R, L):
     """The weight gradients (X^T Y over every (step, sequence) row, gemm_tn_tc.cuh: 3xTF32 with on-the-fly transposition,

@@ -343,7 +343,7 @@ int re2nn_crf_viterbi(const float* feats, const float* transitions, const int64_
                       int64_t o_idx, int64_t* padded_path, int64_t* flat_pred, float* part_ws,
                       void* stream);
 
-/* debug / calibration: sequences one warp of the Viterbi sweep decodes together (0 = pick by batch size; 1, 2, 4). */
+/* debug / calibration: sequences one warp of the Viterbi sweep decodes together (0 = pick by batch size; 1, 2). */
 int re2nn_debug_set_viterbi_seqs(int ns);
 
 /* ---- CRF negative log-likelihood ---------------------------------------------------------------------
@@ -355,7 +355,8 @@ int re2nn_crf_nll(const float* feats, const float* transitions, const int64_t* l
                   float* part_save, void* stream);
 
 /* d loss / d feats (B x L x T, zero at pads) and d loss / d transitions (T x T), scaled by *gscale
- * (device scalar, the upstream gradient). */
+ * (device scalar, the upstream gradient).  T <= 225: a larger tag set returns an error ("tag set too large"),
+ * since one sequence's T x T accumulator no longer fits in shared memory. */
 int re2nn_crf_nll_backward(const float* feats, const float* transitions, const int64_t* lengths,
                            const int64_t* tags, const float* part_save, const float* gscale,
                            int B, int L, int Ltags, int T, float* dfeats, float* dtrans, void* stream);

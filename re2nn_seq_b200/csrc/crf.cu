@@ -6,6 +6,15 @@
 // the running partition is exchanged through a per-warp shared buffer.  Arithmetic order follows the
 // reference exactly where it decides an argmax: cur = (feat_j + trans_ij) + part_i, strict ">" keeps
 // the first maximal index like torch.max(dim).
+//
+// Kernel by tag-set width T = tagset + 2 (shared memory capped at kSmemLimit = 200 KB):
+//   re2nn_crf_nll            3-32 crf_nll_exp_kernel<1>, 33-64 <2>, 65-96 <3>, 97-128 <4>, 129-153 <5>,
+//                            154-218 crf_nll_kernel<true>, >= 219 crf_nll_kernel<false>
+//   re2nn_crf_nll_backward   3-96 crf_nll_backward_exp3_kernel, 97-111 crf_nll_backward_exp_kernel,
+//                            112-159 crf_nll_backward_kernel<true>, 160-225 <false>, >= 226 error "tag set too large"
+//                            (re2nn_debug_set_crf_backward_split(0): 3-111 crf_nll_backward_exp_kernel)
+//   re2nn_crf_viterbi        3-160 crf_viterbi_kernel<cdiv(T, 32), NS> (NS = 2 for large batches, else 1),
+//                            161-216 crf_viterbi_kernel<0, 1>, >= 217 crf_viterbi_global_kernel
 #include <algorithm>
 
 #include "common.cuh"
@@ -54,6 +63,68 @@ __host__ __device__ inline int viterbi_pitch(int T) {
   return 4 * q;
 }
 
+// trans[i][j] as the Viterbi kernels hold it: the transposed shared-memory table of pitch Tq, or the row-major
+// matrix in global memory
+struct TransposedTrans {
+  const float* p;
+  int Tq;
+  __device__ __forceinline__ float operator()(int i, int j) const { return p[j * Tq + i]; }
+};
+struct RowMajorTrans {
+  const float* p;
+  int T;
+  __device__ __forceinline__ float operator()(int i, int j) const { return p[i * T + j]; }
+};
+
+// part_0[j] = feat_0[j] + trans[START][j]
+template <class Tr>
+__device__ __forceinline__ float viterbi_start(Tr tr, const float* f0, int j, int T, int clamp_col, float thr) {
+  return clamped_feat(f0, j, clamp_col, thr) + tr(T - 2, j);
+}
+
+// Backtrace of sequence b (n tags) from its partition history hs, all lanes of the warp cooperating.  Each pointer on
+// the best path is the first maximal source tag over i of (f + trans[i][j]) + part[i], or part[i] + trans[i][j] for
+// the STOP step (crf.py:166-175, torch.max tie-break).
+template <class Tr>
+__device__ __forceinline__ void viterbi_backtrace(Tr tr, const float* fs, const float* hs, int n, int b, int L, int T,
+                                                  int lane, int clamp_col, float thr, int64_t o_idx,
+                                                  const int64_t* offsets, int64_t* padded, int64_t* flat) {
+  if (n <= 0) {   // empty sequence: no tags; the padded row is all zeros like the reference's masked back-pointers
+    if (padded)
+      for (int t = lane; t < L; t += 32) padded[(size_t)b * L + t] = 0;
+    return;
+  }
+  auto best_source = [&](const float* part, float f, int j, bool with_f) -> int {
+    float best = -INFINITY;
+    int bi = 0x7fffffff;
+    for (int i = lane; i < T; i += 32) {
+      const float v = with_f ? (f + tr(i, j)) + part[i] : part[i] + tr(i, j);
+      if (v > best) { best = v; bi = i; }
+    }
+    if (bi == 0x7fffffff) bi = lane;   // nothing above -inf in this lane: keep order so index 0 wins a full tie
+    warp_argmax_first(best, bi);
+    if (best == -INFINITY) bi = 0;
+    return bi;
+  };
+  int ptr = best_source(hs + (size_t)(n - 1) * T, 0.f, T - 1, false);
+  const int64_t off = offsets ? offsets[b] : 0;
+  auto emit = [&](int t, int tag) {
+    if (lane == 0) {
+      if (padded) padded[(size_t)b * L + t] = tag;
+      if (flat) flat[off + t] = (tag == clamp_col) ? o_idx : (int64_t)tag;
+    }
+  };
+  if (padded && lane == 0) {   // reference leaves pads at 0 and the final pointer in the last column
+    for (int t = n; t < L - 1; ++t) padded[(size_t)b * L + t] = 0;
+    if (n < L) padded[(size_t)b * L + (L - 1)] = ptr;
+  }
+  emit(n - 1, ptr);
+  for (int t = n - 1; t >= 1; --t) {
+    ptr = best_source(hs + (size_t)(t - 1) * T, clamped_feat(fs + (size_t)t * T, ptr, clamp_col, thr), ptr, true);
+    emit(t - 1, ptr);
+  }
+}
+
 // dynamic smem: trT[T][Tq] (trT[j][i] = trans[i][j], source tags i >= T hold -inf), then kCrfWarps * NS * 2 * Tq
 // partitions.  One warp sweeps NS neighbouring sequences together: every transition value read from shared memory
 // (the binding resource once the compare/select sweep is gone: each candidate needs its own 4-byte trans[i][j])
@@ -91,12 +162,13 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_viterbi_kernel(
   const size_t seq = (size_t)L * T;
   const float* fb = feats + (size_t)b0 * seq;
   float* hb = hist + (size_t)b0 * seq;
+  const TransposedTrans tr{trT, Tq};
 
 #pragma unroll
   for (int s = 0; s < NS; ++s) {
     if (n[s] > 0)
       for (int j = lane; j < T; j += 32) {
-        const float v = clamped_feat(fb + s * seq, j, clamp_col, thr) + trT[j * Tq + (T - 2)];
+        const float v = viterbi_start(tr, fb + s * seq, j, T, clamp_col, thr);
         pa[s * Tq + j] = v;
         hb[s * seq + j] = v;
       }
@@ -183,110 +255,129 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_viterbi_kernel(
       float* tmp = pa; pa = pb; pb = tmp;
     }
   }
-  __syncwarp();
-  // first maximal source tag over i of (f + trans[i][j]) + part[i]  (with_f)  or  part[i] + trans[i][j]  (STOP step,
-  // crf.py:166-175), all lanes cooperating (torch.max tie-break)
-  auto best_source = [&](const float* part, float f, int j, bool with_f) -> int {
-    const float* row = trT + j * Tq;
-    float best = -INFINITY;
-    int bi = 0x7fffffff;
-    for (int i = lane; i < T; i += 32) {
-      const float v = with_f ? (f + row[i]) + part[i] : part[i] + row[i];
-      if (v > best) { best = v; bi = i; }
-    }
-    if (bi == 0x7fffffff) bi = lane;   // nothing above -inf in this lane: keep order so index 0 wins a full tie
-    warp_argmax_first(best, bi);
-    if (best == -INFINITY) bi = 0;
-    return bi;
-  };
+  __syncwarp();      // the history rows are read back by every lane
 #pragma unroll 1
-  for (int s = 0; s < NS; ++s) {
-    const int b = b0 + s;
-    if (b >= B) break;
-    const int ns = n[s];
-    if (ns <= 0) {   // empty sequence: no tags; the padded row is all zeros like the reference's masked back-pointers
-      if (padded)
-        for (int t = lane; t < L; t += 32) padded[(size_t)b * L + t] = 0;
-      continue;
-    }
-    const float* fs = fb + s * seq;
-    const float* hs = hb + s * seq;      // written by this warp (ordered by __syncwarp)
-    int ptr = best_source(hs + (size_t)(ns - 1) * T, 0.f, T - 1, false);
-    const int64_t off = offsets ? offsets[b] : 0;
-    auto emit = [&](int t, int tag) {
-      if (lane == 0) {
-        if (padded) padded[(size_t)b * L + t] = tag;
-        if (flat) flat[off + t] = (tag == clamp_col) ? o_idx : (int64_t)tag;
-      }
-    };
-    if (padded && lane == 0) {   // reference leaves pads at 0 and the final pointer in the last column
-      for (int t = ns; t < L - 1; ++t) padded[(size_t)b * L + t] = 0;
-      if (ns < L) padded[(size_t)b * L + (L - 1)] = ptr;
-    }
-    emit(ns - 1, ptr);
-    for (int t = ns - 1; t >= 1; --t) {
-      ptr = best_source(hs + (size_t)(t - 1) * T, clamped_feat(fs + (size_t)t * T, ptr, clamp_col, thr), ptr, true);
-      emit(t - 1, ptr);
-    }
-  }
+  for (int s = 0; s < NS && b0 + s < B; ++s)
+    viterbi_backtrace(tr, fb + s * seq, hb + s * seq, n[s], b0 + s, L, T, lane, clamp_col, thr, o_idx, offsets, padded,
+                      flat);
 }
 
 // transitions too large for shared memory: same algorithm straight from global memory
 __global__ void __launch_bounds__(kCrfWarps * 32) crf_viterbi_global_kernel(
-    const float* __restrict__ feats, const float* __restrict__ tr, const int64_t* __restrict__ len,
+    const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len,
     const int64_t* __restrict__ offsets, int B, int L, int T, int clamp_col, float thr, int64_t o_idx,
     int64_t* __restrict__ padded, int64_t* __restrict__ flat, float* hist) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * kCrfWarps + warp;
   if (b >= B) return;
   const int n = min((int)len[b], L);
-  if (n <= 0) {
-    if (padded)
-      for (int t = lane; t < L; t += 32) padded[(size_t)b * L + t] = 0;
-    return;
-  }
+  const RowMajorTrans tr{trans_g, T};
   const float* fb = feats + (size_t)b * L * T;
   float* hb = hist + (size_t)b * L * T;
-  for (int j = lane; j < T; j += 32) hb[j] = clamped_feat(fb, j, clamp_col, thr) + tr[(T - 2) * T + j];
+  if (n > 0)
+    for (int j = lane; j < T; j += 32) hb[j] = viterbi_start(tr, fb, j, T, clamp_col, thr);
   __syncwarp();
   for (int t = 1; t < n; ++t) {
     const float* pa = hb + (size_t)(t - 1) * T;
     for (int j = lane; j < T; j += 32) {
       const float f = clamped_feat(fb + (size_t)t * T, j, clamp_col, thr);
       float best = -INFINITY;
-      for (int i = 0; i < T; ++i) best = fmaxf(best, (f + tr[i * T + j]) + pa[i]);
+      for (int i = 0; i < T; ++i) best = fmaxf(best, (f + tr(i, j)) + pa[i]);
       hb[(size_t)t * T + j] = best;
     }
     __syncwarp();
   }
-  auto first_max = [&](const float* part, float f, int j, bool with_f) -> int {
-    float best = -INFINITY;
-    int bi = 0x7fffffff;
-    for (int i = lane; i < T; i += 32) {
-      const float v = with_f ? (f + tr[i * T + j]) + part[i] : part[i] + tr[i * T + j];
-      if (v > best) { best = v; bi = i; }
-    }
-    if (bi == 0x7fffffff) bi = lane;
-    warp_argmax_first(best, bi);
-    if (best == -INFINITY) bi = 0;
-    return bi;
-  };
-  int ptr = first_max(hb + (size_t)(n - 1) * T, 0.f, T - 1, false);
-  const int64_t off = offsets ? offsets[b] : 0;
-  auto emit = [&](int t, int tag) {
-    if (lane == 0) {
-      if (padded) padded[(size_t)b * L + t] = tag;
-      if (flat) flat[off + t] = (tag == clamp_col) ? o_idx : (int64_t)tag;
-    }
-  };
-  if (padded && lane == 0) {
-    for (int t = n; t < L - 1; ++t) padded[(size_t)b * L + t] = 0;
-    if (n < L) padded[(size_t)b * L + (L - 1)] = ptr;
+  viterbi_backtrace(tr, fb, hb, n, b, L, T, lane, clamp_col, thr, o_idx, offsets, padded, flat);
+}
+
+// ---- per-sequence pieces of the NLL kernels (crf.py:48-99, 202-251); tr is the row-major T x T matrix -------------
+// logZ = LSE_i(trans[i][STOP] + part[i]) over the last partition, one warp
+__device__ __forceinline__ float crf_log_z(const float* tr, const float* part, int T, int lane) {
+  float m = -INFINITY;
+  for (int i = lane; i < T; i += 32) m = fmaxf(m, tr[i * T + (T - 1)] + part[i]);
+  m = warp_max(m);
+  float s = 0.f;
+  for (int i = lane; i < T; i += 32) s += expf((tr[i * T + (T - 1)] + part[i]) - m);
+  s = warp_sum(s);
+  return m + logf(s);
+}
+
+// per_seq = logZ - (score of the gold path of the n tags tg), one warp
+__device__ __forceinline__ void crf_store_nll(const float* tr, const float* part, const float* fb, const int64_t* tg,
+                                              int n, int T, int lane, float* per_seq) {
+  const float logZ = crf_log_z(tr, part, T, lane);
+  float g = 0.f;
+  for (int t = lane; t < n; t += 32) {
+    int cur = (int)tg[t];
+    int prev = t == 0 ? T - 2 : (int)tg[t - 1];
+    g += __ldg(fb + (size_t)t * T + cur) + tr[prev * T + cur];
   }
-  emit(n - 1, ptr);
-  for (int t = n - 1; t >= 1; --t) {
-    ptr = first_max(hb + (size_t)(t - 1) * T, clamped_feat(fb + (size_t)t * T, ptr, clamp_col, thr), ptr, true);
-    emit(t - 1, ptr);
+  g = warp_sum(g);
+  if (lane == 0) {
+    g += tr[(int)tg[n - 1] * T + (T - 1)];
+    *per_seq = logZ - g;
+  }
+}
+
+// exact log-domain LSE_i((f + trans[i][j]) + part[i]) of column j
+__device__ __forceinline__ float crf_column_lse(const float* tr, const float* part, float f, int j, int T) {
+  float m = -INFINITY;
+  for (int i = 0; i < T; ++i) m = fmaxf(m, (f + tr[i * T + j]) + part[i]);
+  float s = 0.f;
+  for (int i = 0; i < T; ++i) s += expf(((f + tr[i * T + j]) + part[i]) - m);
+  return m + logf(s);
+}
+
+// Exact log-domain backward row i (tri = trans[i][.]): returns beta_{t-1}[i] = LSE_j((trans[i][j] + feat_t[j]) +
+// beta_t[j]) and adds the pairwise marginals gs * exp(pi + e_ij), pi = part_{t-1}[i] - logZ, to the accumulator row dwi.
+__device__ __forceinline__ float crf_backward_row_exact(const float* tri, const float* ft, const float* beta, float pi,
+                                                        float gs, float* dwi, int T) {
+  float mx = -INFINITY;
+  for (int j = 0; j < T; ++j) mx = fmaxf(mx, (tri[j] + __ldg(ft + j)) + beta[j]);
+  float sm = 0.f;
+  for (int j = 0; j < T; ++j) {
+    const float e = (tri[j] + __ldg(ft + j)) + beta[j];
+    sm += expf(e - mx);
+    dwi[j] += gs * expf(pi + e);
+  }
+  return mx + logf(sm);
+}
+
+// Shared-memory tables of the scaled-exponential backward kernels, built by the whole CTA: tr = trans_g (T x T),
+// rmax[i] = max_j trans[i][j] (-inf for T <= i < Tp), te[i * pitch + j] = exp(trans[i][j] - rmax[i]), 0 in the pad
+// columns j >= T.  (crf_nll_exp_kernel keeps its column-maximum table inline: built through a shared function, its
+// T <= 32 instantiation spilled 8 bytes.)
+__device__ __forceinline__ void crf_exp_row_table(const float* trans_g, int T, int Tp, int pitch, float* tr, float* te,
+                                                  float* rmax) {
+  for (int i = threadIdx.x; i < T * T; i += blockDim.x) tr[i] = trans_g[i];
+  __syncthreads();
+  for (int i = threadIdx.x; i < Tp; i += blockDim.x) {
+    float m = -INFINITY;
+    if (i < T)
+      for (int j = 0; j < T; ++j) m = fmaxf(m, tr[i * T + j]);
+    rmax[i] = m;
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < T * pitch; i += blockDim.x) {
+    const int r = i / pitch, c = i - r * pitch;
+    te[i] = c < T ? expf(tr[r * T + c] - rmax[r]) : 0.f;
+  }
+  __syncthreads();
+}
+
+// dfeats rows from..L-1 of one sequence are zero (pads; every row of an empty sequence); `stride` threads from `tid`
+__device__ __forceinline__ void crf_zero_rows(float* df, int from, int L, int T, int tid, int stride) {
+  for (int i = from * T + tid; i < L * T; i += stride) df[i] = 0.f;
+}
+
+// Sum of the CTA's nacc private dtrans accumulators (T x T at row pitch Tq) into dtrans, one atomicAdd per element
+__device__ __forceinline__ void crf_fold_dtrans(const float* s_dtr, int nacc, int T, int Tq, float* dtrans) {
+  __syncthreads();
+  for (int i = threadIdx.x; i < T * T; i += blockDim.x) {
+    const int r = i / T, c = i - r * T;
+    float v = 0.f;
+    for (int w = 0; w < nacc; ++w) v += s_dtr[(size_t)w * T * Tq + r * Tq + c];
+    if (v != 0.f) atomicAdd(dtrans + i, v);
   }
 }
 
@@ -327,39 +418,14 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_kernel(
   for (int t = 1; t < n; ++t) {
     const float* ft = fb + (size_t)t * T;
     for (int j = lane; j < T; j += 32) {
-      const float f = __ldg(ft + j);
-      float m = -INFINITY;
-      for (int i = 0; i < T; ++i) m = fmaxf(m, (f + tr[i * T + j]) + pa[i]);
-      float s = 0.f;
-      for (int i = 0; i < T; ++i) s += expf(((f + tr[i * T + j]) + pa[i]) - m);
-      float v = m + logf(s);
+      const float v = crf_column_lse(tr, pa, __ldg(ft + j), j, T);
       pb[j] = v;
       if (ps) ps[(size_t)t * T + j] = v;
     }
     __syncwarp();
     float* tmp = pa; pa = pb; pb = tmp;
   }
-  // logZ = LSE_i(trans[i][STOP] + part_i)
-  float m = -INFINITY;
-  for (int i = lane; i < T; i += 32) m = fmaxf(m, tr[i * T + (T - 1)] + pa[i]);
-  m = warp_max(m);
-  float s = 0.f;
-  for (int i = lane; i < T; i += 32) s += expf((tr[i * T + (T - 1)] + pa[i]) - m);
-  s = warp_sum(s);
-  const float logZ = m + logf(s);
-  // gold path
-  const int64_t* tg = tags + (size_t)b * Ltags;
-  float g = 0.f;
-  for (int t = lane; t < n; t += 32) {
-    int cur = (int)tg[t];
-    int prev = t == 0 ? T - 2 : (int)tg[t - 1];
-    g += __ldg(fb + (size_t)t * T + cur) + tr[prev * T + cur];
-  }
-  g = warp_sum(g);
-  if (lane == 0) {
-    g += tr[(int)tg[n - 1] * T + (T - 1)];
-    per_seq[b] = logZ - g;
-  }
+  crf_store_nll(tr, pa, fb, tags + (size_t)b * Ltags, n, T, lane, per_seq + b);
 }
 
 // Same log-partition in the scaled exponential domain: with M = max_i part[i] and cmax[j] = max_i trans[i][j]
@@ -437,16 +503,8 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
       const int j = lane + 32 * q;
       if (j < T) {
         const float f = __ldg(ft + j);
-        float v;
-        if (acc[q] > 1e-30f) {
-          v = ((M + cmax[j]) + f) + logf(acc[q]);
-        } else {   // underflow: exact log-domain evaluation of this column
-          float m = -INFINITY;
-          for (int i = 0; i < T; ++i) m = fmaxf(m, (f + tr[i * T + j]) + pa[i]);
-          float sm = 0.f;
-          for (int i = 0; i < T; ++i) sm += expf(((f + tr[i * T + j]) + pa[i]) - m);
-          v = m + logf(sm);
-        }
+        // a column whose sum underflows is evaluated exactly in the log domain
+        const float v = acc[q] > 1e-30f ? ((M + cmax[j]) + f) + logf(acc[q]) : crf_column_lse(tr, pa, f, j, T);
         pb[j] = v;
         if (ps) ps[(size_t)t * T + j] = v;
       }
@@ -454,27 +512,7 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
     __syncwarp();
     float* tmp = pa; pa = pb; pb = tmp;
   }
-  // logZ = LSE_i(trans[i][STOP] + part_i)
-  float m = -INFINITY;
-  for (int i = lane; i < T; i += 32) m = fmaxf(m, tr[i * T + (T - 1)] + pa[i]);
-  m = warp_max(m);
-  float s = 0.f;
-  for (int i = lane; i < T; i += 32) s += expf((tr[i * T + (T - 1)] + pa[i]) - m);
-  s = warp_sum(s);
-  const float logZ = m + logf(s);
-  // gold path
-  const int64_t* tg = tags + (size_t)b * Ltags;
-  float g = 0.f;
-  for (int t = lane; t < n; t += 32) {
-    int cur = (int)tg[t];
-    int prev = t == 0 ? T - 2 : (int)tg[t - 1];
-    g += __ldg(fb + (size_t)t * T + cur) + tr[prev * T + cur];
-  }
-  g = warp_sum(g);
-  if (lane == 0) {
-    g += tr[(int)tg[n - 1] * T + (T - 1)];
-    per_seq[b] = logZ - g;
-  }
+  crf_store_nll(tr, pa, fb, tags + (size_t)b * Ltags, n, T, lane, per_seq + b);
 }
 
 // CRF backward: marginals by the backward recursion, reusing the saved forward partitions.
@@ -503,27 +541,15 @@ __global__ void crf_nll_backward_kernel(
   const float gs = gscale ? *gscale : 1.f;
   float* dw = s_dtr + (size_t)warp * T * Tq;
   const int b = blockIdx.x * nw + warp;
-  if (b < B && min((int)len[b], L) <= 0) {      // empty sequence: no marginals, zero feature gradient
-    float* df0 = dfeats + (size_t)b * L * T;
-    for (int i = lane; i < L * T; i += 32) df0[i] = 0.f;
-  }
-  if (b < B && min((int)len[b], L) > 0) {
-    const int n = min((int)len[b], L);
+  const int n = b < B ? min((int)len[b], L) : 0;
+  float* df = dfeats + (size_t)b * L * T;
+  if (n > 0) {
     float* ba = s_beta + warp * 2 * Tp;   // beta_t
     float* bb = ba + Tp;                  // beta_{t-1}
     const float* fb = feats + (size_t)b * L * T;
     const float* ps = part_save + (size_t)b * L * T;
-    float* df = dfeats + (size_t)b * L * T;
     const int64_t* tg = tags + (size_t)b * Ltags;
-    // logZ from the last saved partition
-    const float* pl = ps + (size_t)(n - 1) * T;
-    float m = -INFINITY;
-    for (int i = lane; i < T; i += 32) m = fmaxf(m, tr[i * T + (T - 1)] + pl[i]);
-    m = warp_max(m);
-    float s = 0.f;
-    for (int i = lane; i < T; i += 32) s += expf((tr[i * T + (T - 1)] + pl[i]) - m);
-    s = warp_sum(s);
-    const float logZ = m + logf(s);
+    const float logZ = crf_log_z(tr, ps + (size_t)(n - 1) * T, T, lane);
     for (int i = lane; i < T; i += 32) ba[i] = tr[i * T + (T - 1)];   // beta_{n-1}[i] = trans[i][STOP]
     __syncwarp();
     for (int t = n - 1; t >= 0; --t) {
@@ -545,32 +571,16 @@ __global__ void crf_nll_backward_kernel(
       const float* ft = fb + (size_t)t * T;
       const int gprev = (int)tg[t - 1];
       for (int i = lane; i < T; i += 32) {
-        float mx = -INFINITY;
-        for (int j = 0; j < T; ++j) mx = fmaxf(mx, (tr[i * T + j] + __ldg(ft + j)) + ba[j]);
-        float sm = 0.f;
-        const float pi = pp[i] - logZ;
         float* dwi = dw + i * Tq;
-        for (int j = 0; j < T; ++j) {
-          const float e = (tr[i * T + j] + __ldg(ft + j)) + ba[j];
-          sm += expf(e - mx);
-          dwi[j] += gs * expf(pi + e);
-        }
+        bb[i] = crf_backward_row_exact(tr + i * T, ft, ba, pp[i] - logZ, gs, dwi, T);
         if (i == gprev) dwi[gold] -= gs;
-        bb[i] = mx + logf(sm);
       }
       __syncwarp();
       float* tmp = ba; ba = bb; bb = tmp;
     }
-    // zero the pad rows of dfeats
-    for (int i = n * T + lane; i < L * T; i += 32) df[i] = 0.f;
   }
-  __syncthreads();
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) {
-    const int r = i / T, c = i - r * T;
-    float v = 0.f;
-    for (int w = 0; w < nw; ++w) v += s_dtr[(size_t)w * T * Tq + r * Tq + c];
-    if (v != 0.f) atomicAdd(dtrans + i, v);
-  }
+  if (b < B) crf_zero_rows(df, max(n, 0), L, T, lane, 32);
+  crf_fold_dtrans(s_dtr, nw, T, Tq, dtrans);
 }
 
 // CRF backward in the scaled exponential domain (see crf_nll_exp_kernel): with w_j = feat_t[j] + beta_t[j],
@@ -594,42 +604,21 @@ __global__ void crf_nll_backward_exp_kernel(
   float* s_dtr = rmax + Tp;
   float* s_vec = s_dtr + (size_t)nw * T * Tq;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) tr[i] = trans_g[i];
   for (int i = threadIdx.x; i < nw * T * Tq; i += blockDim.x) s_dtr[i] = 0.f;
-  __syncthreads();
-  for (int i = threadIdx.x; i < Tp; i += blockDim.x) {
-    float m = -INFINITY;
-    if (i < T)
-      for (int j = 0; j < T; ++j) m = fmaxf(m, tr[i * T + j]);
-    rmax[i] = m;
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) te[i] = expf(tr[i] - rmax[i / T]);
-  __syncthreads();
+  crf_exp_row_table(trans_g, T, Tp, T, tr, te, rmax);
   const float gs = gscale ? *gscale : 1.f;
   float* dw = s_dtr + (size_t)warp * T * Tq;
   const int b = blockIdx.x * nw + warp;
-  if (b < B && min((int)len[b], L) <= 0) {      // empty sequence: no marginals, zero feature gradient
-    float* df0 = dfeats + (size_t)b * L * T;
-    for (int i = lane; i < L * T; i += 32) df0[i] = 0.f;
-  }
-  if (b < B && min((int)len[b], L) > 0) {
-    const int n = min((int)len[b], L);
+  const int n = b < B ? min((int)len[b], L) : 0;
+  float* df = dfeats + (size_t)b * L * T;
+  if (n > 0) {
     float* ba = s_vec + warp * 3 * Tp;   // beta_t
     float* bb = ba + Tp;                 // beta_{t-1}
     float* W = bb + Tp;
     const float* fb = feats + (size_t)b * L * T;
     const float* ps = part_save + (size_t)b * L * T;
-    float* df = dfeats + (size_t)b * L * T;
     const int64_t* tg = tags + (size_t)b * Ltags;
-    const float* pl = ps + (size_t)(n - 1) * T;
-    float m = -INFINITY;
-    for (int i = lane; i < T; i += 32) m = fmaxf(m, tr[i * T + (T - 1)] + pl[i]);
-    m = warp_max(m);
-    float s = 0.f;
-    for (int i = lane; i < T; i += 32) s += expf((tr[i * T + (T - 1)] + pl[i]) - m);
-    s = warp_sum(s);
-    const float logZ = m + logf(s);
+    const float logZ = crf_log_z(tr, ps + (size_t)(n - 1) * T, T, lane);
     for (int i = lane; i < T; i += 32) ba[i] = tr[i * T + (T - 1)];
     __syncwarp();
     for (int t = n - 1; t >= 0; --t) {
@@ -662,112 +651,34 @@ __global__ void crf_nll_backward_exp_kernel(
       Mw = warp_max(Mw);
       for (int j = lane; j < T; j += 32) W[j] = expf((__ldg(ft + j) + ba[j]) - Mw);
       __syncwarp();
-      // lane owns source rows lane, lane + 32, lane + 64
-      auto row_exact = [&](int i) {      // underflow: exact log-domain evaluation of this row
+      for (int i = lane; i < T; i += 32) {
+        const float* tei = te + i * T;
         float* dwi = dw + i * Tq;
-        float mx = -INFINITY;
-        for (int j = 0; j < T; ++j) mx = fmaxf(mx, (tr[i * T + j] + __ldg(ft + j)) + ba[j]);
-        float sm = 0.f;
-        const float pi = pp[i] - logZ;
-        for (int j = 0; j < T; ++j) {
-          const float e = (tr[i * T + j] + __ldg(ft + j)) + ba[j];
-          sm += expf(e - mx);
-          dwi[j] += gs * expf(pi + e);
-        }
-        bb[i] = mx + logf(sm);
-      };
-      if (T <= 96) {
-        // the (up to) three rows of a lane side by side: three independent FMA chains per W[j] load instead of three
-        // dependent shared-memory round trips in sequence (the sweep is one latency-bound chain per sequence).  Every
-        // row keeps its own left-to-right summation order: same bits as the row-by-row form.
-        const int i0 = lane, i1 = lane + 32, i2 = lane + 64;
-        const bool v0 = i0 < T, v1 = i1 < T, v2 = i2 < T;
-        const float* t0 = te + (v0 ? i0 : 0) * T;
-        const float* t1 = te + (v1 ? i1 : 0) * T;
-        const float* t2 = te + (v2 ? i2 : 0) * T;
-        float S0 = 0.f, S1 = 0.f, S2 = 0.f;
-#pragma unroll 4
-        for (int j = 0; j < T; ++j) {
-          const float w = W[j];
-          S0 = fmaf(t0[j], w, S0);
-          S1 = fmaf(t1[j], w, S1);
-          S2 = fmaf(t2[j], w, S2);
-        }
-        const bool f0 = v0 && S0 > 1e-30f, f1 = v1 && S1 > 1e-30f, f2 = v2 && S2 > 1e-30f;
-        const float A0 = f0 ? gs * expf(((pp[i0] - logZ) + rmax[i0]) + Mw) : 0.f;
-        const float A1 = f1 ? gs * expf(((pp[i1] - logZ) + rmax[i1]) + Mw) : 0.f;
-        const float A2 = f2 ? gs * expf(((pp[i2] - logZ) + rmax[i2]) + Mw) : 0.f;
-        float* d0 = dw + (v0 ? i0 : 0) * Tq;
-        float* d1 = dw + (v1 ? i1 : 0) * Tq;
-        float* d2 = dw + (v2 ? i2 : 0) * Tq;
-        int j = 0;
-        for (; j + 4 <= T; j += 4) {     // all loads of a batch before its stores (stores may alias the next loads)
-          float a[4], b[4], c[4];
+        float S = 0.f;
+        for (int j = 0; j < T; ++j) S = fmaf(tei[j], W[j], S);
+        if (S > 1e-30f) {
+          const float A = gs * expf(((pp[i] - logZ) + rmax[i]) + Mw);
+          int j = 0;
+          for (; j + 8 <= T; j += 8) {
+            float d[8];
 #pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const float w = W[j + q];
-            a[q] = fmaf(A0 * t0[j + q], w, d0[j + q]);
-            b[q] = fmaf(A1 * t1[j + q], w, d1[j + q]);
-            c[q] = fmaf(A2 * t2[j + q], w, d2[j + q]);
+            for (int q = 0; q < 8; ++q) d[q] = fmaf(A * tei[j + q], W[j + q], dwi[j + q]);
+#pragma unroll
+            for (int q = 0; q < 8; ++q) dwi[j + q] = d[q];
           }
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            if (f0) d0[j + q] = a[q];
-            if (f1) d1[j + q] = b[q];
-            if (f2) d2[j + q] = c[q];
-          }
+          for (; j < T; ++j) dwi[j] = fmaf(A * tei[j], W[j], dwi[j]);
+          bb[i] = (rmax[i] + Mw) + logf(S);
+        } else {   // underflow: exact log-domain evaluation of this row
+          bb[i] = crf_backward_row_exact(tr + i * T, ft, ba, pp[i] - logZ, gs, dwi, T);
         }
-        for (; j < T; ++j) {
-          const float w = W[j];
-          if (f0) d0[j] = fmaf(A0 * t0[j], w, d0[j]);
-          if (f1) d1[j] = fmaf(A1 * t1[j], w, d1[j]);
-          if (f2) d2[j] = fmaf(A2 * t2[j], w, d2[j]);
-        }
-        if (f0) bb[i0] = (rmax[i0] + Mw) + logf(S0);
-        if (f1) bb[i1] = (rmax[i1] + Mw) + logf(S1);
-        if (f2) bb[i2] = (rmax[i2] + Mw) + logf(S2);
-        if (v0 && !f0) row_exact(i0);
-        if (v1 && !f1) row_exact(i1);
-        if (v2 && !f2) row_exact(i2);
-        if (v0 && i0 == gprev) d0[gold] -= gs;
-        if (v1 && i1 == gprev) d1[gold] -= gs;
-        if (v2 && i2 == gprev) d2[gold] -= gs;
-      } else {
-        for (int i = lane; i < T; i += 32) {
-          const float* tei = te + i * T;
-          float* dwi = dw + i * Tq;
-          float S = 0.f;
-          for (int j = 0; j < T; ++j) S = fmaf(tei[j], W[j], S);
-          if (S > 1e-30f) {
-            const float A = gs * expf(((pp[i] - logZ) + rmax[i]) + Mw);
-            int j = 0;
-            for (; j + 8 <= T; j += 8) {
-              float d[8];
-#pragma unroll
-              for (int q = 0; q < 8; ++q) d[q] = fmaf(A * tei[j + q], W[j + q], dwi[j + q]);
-#pragma unroll
-              for (int q = 0; q < 8; ++q) dwi[j + q] = d[q];
-            }
-            for (; j < T; ++j) dwi[j] = fmaf(A * tei[j], W[j], dwi[j]);
-            bb[i] = (rmax[i] + Mw) + logf(S);
-          } else {
-            row_exact(i);
-          }
-          if (i == gprev) dwi[gold] -= gs;
-        }
+        if (i == gprev) dwi[gold] -= gs;
       }
       __syncwarp();
       float* tmp = ba; ba = bb; bb = tmp;
     }
-    for (int i = n * T + lane; i < L * T; i += 32) df[i] = 0.f;
   }
-  __syncthreads();
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) {
-    const int r = i / T, c = i - r * T;
-    float v = 0.f;
-    for (int w = 0; w < nw; ++w) v += s_dtr[(size_t)w * T * Tq + r * Tq + c];
-    if (v != 0.f) atomicAdd(dtrans + i, v);
-  }
+  if (b < B) crf_zero_rows(df, max(n, 0), L, T, lane, 32);
+  crf_fold_dtrans(s_dtr, nw, T, Tq, dtrans);
 }
 
 // The same sweep with THREE warps per sequence (T <= 96): warp `part` of a sequence owns transition rows / tag columns
@@ -790,22 +701,9 @@ __global__ void crf_nll_backward_exp3_kernel(
   float* s_dtr = rmax + Tp;
   float* s_vec = s_dtr + (size_t)nseq * T * Tq;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) tr[i] = trans_g[i];
   for (int i = threadIdx.x; i < nseq * T * Tq; i += blockDim.x) s_dtr[i] = 0.f;
-  __syncthreads();
-  for (int i = threadIdx.x; i < Tp; i += blockDim.x) {
-    float m = -INFINITY;
-    if (i < T)
-      for (int j = 0; j < T; ++j) m = fmaxf(m, tr[i * T + j]);
-    rmax[i] = m;
-  }
-  __syncthreads();
-  for (int i = threadIdx.x; i < T * Tq; i += blockDim.x) {
-    const int r = i / Tq, c = i - r * Tq;
-    te[i] = c < T ? expf(tr[r * T + c] - rmax[r]) : 0.f;      // pad columns contribute exact zeros
-  }
   for (int i = threadIdx.x; i < nseq * 3 * Tp; i += blockDim.x) s_vec[i] = 0.f;   // W pad entries stay 0
-  __syncthreads();
+  crf_exp_row_table(trans_g, T, Tp, Tq, tr, te, rmax);      // pad columns of the table contribute exact zeros
   const float gs = gscale ? *gscale : 1.f;
   const int seq = warp / 3, part = warp - seq * 3;
   const int own = part * 32 + lane;            // the row / column this lane owns
@@ -814,28 +712,16 @@ __global__ void crf_nll_backward_exp3_kernel(
   auto seq_sync = [&]() { asm volatile("bar.sync %0, 96;" ::"r"(seq + 1) : "memory"); };
   float* dw = s_dtr + (size_t)seq * T * Tq;
   const int b = blockIdx.x * nseq + seq;
-  if (b < B && min((int)len[b], L) <= 0) {      // empty sequence: no marginals, zero feature gradient
-    float* df0 = dfeats + (size_t)b * L * T;
-    for (int i = tid96; i < L * T; i += 96) df0[i] = 0.f;
-  }
-  if (b < B && min((int)len[b], L) > 0) {       // uniform over the three warps of a sequence
-    const int n = min((int)len[b], L);
+  const int n = b < B ? min((int)len[b], L) : 0;
+  float* df = dfeats + (size_t)b * L * T;
+  if (n > 0) {       // uniform over the three warps of a sequence
     float* ba = s_vec + seq * 3 * Tp;    // beta_t
     float* bb = ba + Tp;                 // beta_{t-1}
     float* W = bb + Tp;
     const float* fb = feats + (size_t)b * L * T;
     const float* ps = part_save + (size_t)b * L * T;
-    float* df = dfeats + (size_t)b * L * T;
     const int64_t* tg = tags + (size_t)b * Ltags;
-    const float* pl = ps + (size_t)(n - 1) * T;
-    // log Z: every warp for itself (same operations, same result)
-    float m = -INFINITY;
-    for (int i = lane; i < T; i += 32) m = fmaxf(m, tr[i * T + (T - 1)] + pl[i]);
-    m = warp_max(m);
-    float s = 0.f;
-    for (int i = lane; i < T; i += 32) s += expf((tr[i * T + (T - 1)] + pl[i]) - m);
-    s = warp_sum(s);
-    const float logZ = m + logf(s);
+    const float logZ = crf_log_z(tr, ps + (size_t)(n - 1) * T, T, lane);   // every warp for itself, same result
     if (has) ba[own] = tr[own * T + (T - 1)];
     seq_sync();
     const float4* tei4 = reinterpret_cast<const float4*>(te + (has ? own : 0) * Tq);
@@ -918,31 +804,16 @@ __global__ void crf_nll_backward_exp3_kernel(
           }
           bb[own] = (rmax[own] + Mw) + logf(S);
         } else {                           // underflow: exact log-domain evaluation of this row
-          float mx = -INFINITY;
-          for (int j = 0; j < T; ++j) mx = fmaxf(mx, (tr[own * T + j] + __ldg(ft + j)) + ba[j]);
-          float sm = 0.f;
-          const float pi = ppv - logZ;
-          for (int j = 0; j < T; ++j) {
-            const float e = (tr[own * T + j] + __ldg(ft + j)) + ba[j];
-            sm += expf(e - mx);
-            dwi[j] += gs * expf(pi + e);
-          }
-          bb[own] = mx + logf(sm);
+          bb[own] = crf_backward_row_exact(tr + own * T, ft, ba, ppv - logZ, gs, dwi, T);
         }
         if (own == gprev) dwi[gold] -= gs;
       }
       seq_sync();                          // beta_{t-1} complete, nobody reads beta_t / W any more
       float* tmp = ba; ba = bb; bb = tmp;
     }
-    for (int i = n * T + tid96; i < L * T; i += 96) df[i] = 0.f;
   }
-  __syncthreads();
-  for (int i = threadIdx.x; i < T * T; i += blockDim.x) {
-    const int r = i / T, c = i - r * T;
-    float v = 0.f;
-    for (int w = 0; w < nseq; ++w) v += s_dtr[(size_t)w * T * Tq + r * Tq + c];
-    if (v != 0.f) atomicAdd(dtrans + i, v);
-  }
+  if (b < B) crf_zero_rows(df, max(n, 0), L, T, tid96, 96);
+  crf_fold_dtrans(s_dtr, nseq, T, Tq, dtrans);
 }
 
 // deterministic sum of n floats (double accumulation), scaled
@@ -1129,6 +1000,17 @@ __global__ void __launch_bounds__(1024) length_order_kernel(const int64_t* __res
 
 static const size_t kSmemLimit = 200 * 1024;
 static bool g_crf_bwd_split = true;      // CRF backward: three warps per sequence when T <= 96 (re2nn_debug_set_crf_backward_split)
+static int g_viterbi_ns = 0;             // sequences per Viterbi warp, 0 = by batch size (re2nn_debug_set_viterbi_seqs)
+
+// One launch of a CRF kernel; `configured` is that kernel's dynamic shared-memory state (ensure_dynamic_smem).
+template <class Kernel, class... Args>
+static int crf_launch(Kernel kernel, int (&configured)[kMaxDevices], int grid, int block, size_t smem, cudaStream_t st,
+                      Args... args) {
+  RE2NN_CUDA(ensure_dynamic_smem(kernel, (int)smem, configured));
+  kernel<<<grid, block, smem, st>>>(args...);
+  RE2NN_LAUNCH_CHECK();
+  return 0;
+}
 
 }  // namespace re2nn
 
@@ -1164,54 +1046,34 @@ int re2nn_length_order(const int64_t* lengths, int B, int L, int64_t* order, int
   return 0;
 }
 
-static int g_viterbi_ns = 0;      // debug: sequences per warp (0 = default)
-
 int re2nn_crf_viterbi(const float* feats, const float* transitions, const int64_t* lengths, const int64_t* offsets,
                       int B, int L, int T, int clamp_col, float threshold, int64_t o_idx, int64_t* padded_path,
                       int64_t* flat_pred, float* part_ws, void* stream) {
   RE2NN_CHECK(feats && transitions && lengths && part_ws, "crf_viterbi: null tensor");
   RE2NN_CHECK(B > 0 && L > 0 && T >= 3 && T <= 65535, "crf_viterbi: bad dims B=%d L=%d T=%d", B, L, T);
   RE2NN_CHECK(!flat_pred || offsets, "crf_viterbi: flat output needs offsets");
+  using Kernel = decltype(&crf_viterbi_global_kernel);
+  static const Kernel kernels[2][6] = {       // [NS - 1][NJ]
+      {crf_viterbi_kernel<0, 1>, crf_viterbi_kernel<1, 1>, crf_viterbi_kernel<2, 1>, crf_viterbi_kernel<3, 1>,
+       crf_viterbi_kernel<4, 1>, crf_viterbi_kernel<5, 1>},
+      {nullptr, crf_viterbi_kernel<1, 2>, crf_viterbi_kernel<2, 2>, crf_viterbi_kernel<3, 2>, crf_viterbi_kernel<4, 2>,
+       crf_viterbi_kernel<5, 2>}};
+  static int configured[2][6][kMaxDevices];
   const int Tq = viterbi_pitch(T);
-  cudaStream_t st = (cudaStream_t)stream;
+  const int nj = cdiv(T, 32) <= 5 ? cdiv(T, 32) : 0;
   // sequences per warp: two halve the shared-memory reads of the transition table per candidate (measured at T = 131,
   // B = 16384: 3.7 -> 2.9 ms; four run out of registers: 4.3 ms), as long as the batch still fills the machine with
   // warps (cfg2, B = 4096: one sequence per warp is fastest, 0.18 vs 0.20 ms)
   int ns = g_viterbi_ns ? g_viterbi_ns : (B >= sm_count() * kCrfWarps * 8 ? 2 : 1);
-  if (cdiv(T, 32) > 5) ns = 1;
-#define RE2NN_VIT(NJ, NS)                                                                                          \
-  do {                                                                                                             \
-    static int configured[kMaxDevices];                                                                            \
-    const size_t smem = ((size_t)T * Tq + (size_t)kCrfWarps * NS * 2 * Tq) * 4;                                    \
-    RE2NN_CUDA(ensure_dynamic_smem(crf_viterbi_kernel<NJ, NS>, (int)smem, configured));                            \
-    crf_viterbi_kernel<NJ, NS><<<cdiv(B, kCrfWarps * NS), kCrfWarps * 32, smem, st>>>(                             \
-        feats, transitions, lengths, offsets, B, L, T, clamp_col, threshold, o_idx, padded_path, flat_pred, part_ws); \
-  } while (0)
-#define RE2NN_VIT_NS(NJ)                                     \
-  do {                                                       \
-    if (ns == 4) RE2NN_VIT(NJ, 4);                           \
-    else if (ns == 2) RE2NN_VIT(NJ, 2);                      \
-    else RE2NN_VIT(NJ, 1);                                   \
-  } while (0)
-  const size_t smem_max = ((size_t)T * Tq + (size_t)kCrfWarps * ns * 2 * Tq) * 4;
-  if (smem_max <= kSmemLimit) {
-    switch (cdiv(T, 32)) {
-      case 1: RE2NN_VIT_NS(1); break;
-      case 2: RE2NN_VIT_NS(2); break;
-      case 3: RE2NN_VIT_NS(3); break;
-      case 4: RE2NN_VIT_NS(4); break;
-      case 5: RE2NN_VIT_NS(5); break;
-      default: RE2NN_VIT(0, 1); break;
-    }
-  } else {
-    crf_viterbi_global_kernel<<<cdiv(B, kCrfWarps), kCrfWarps * 32, 0, st>>>(feats, transitions, lengths, offsets, B, L, T,
-                                                                             clamp_col, threshold, o_idx, padded_path,
-                                                                             flat_pred, part_ws);
-  }
-#undef RE2NN_VIT
-#undef RE2NN_VIT_NS
-  RE2NN_LAUNCH_CHECK();
-  return 0;
+  if (nj == 0) ns = 1;
+  const size_t smem = ((size_t)T * Tq + (size_t)kCrfWarps * ns * 2 * Tq) * 4;
+  if (smem > kSmemLimit)      // no dynamic shared memory: ensure_dynamic_smem leaves `configured` alone
+    return crf_launch(crf_viterbi_global_kernel, configured[0][0], cdiv(B, kCrfWarps), kCrfWarps * 32, 0,
+                      (cudaStream_t)stream, feats, transitions, lengths, offsets, B, L, T, clamp_col, threshold, o_idx,
+                      padded_path, flat_pred, part_ws);
+  return crf_launch(kernels[ns - 1][nj], configured[ns - 1][nj], cdiv(B, kCrfWarps * ns), kCrfWarps * 32, smem,
+                    (cudaStream_t)stream, feats, transitions, lengths, offsets, B, L, T, clamp_col, threshold, o_idx,
+                    padded_path, flat_pred, part_ws);
 }
 
 int re2nn_debug_set_crf_backward_split(int on) {
@@ -1220,7 +1082,7 @@ int re2nn_debug_set_crf_backward_split(int on) {
 }
 
 int re2nn_debug_set_viterbi_seqs(int ns) {
-  RE2NN_CHECK(ns == 0 || ns == 1 || ns == 2 || ns == 4, "debug_set_viterbi_seqs: expected 0, 1, 2 or 4");
+  RE2NN_CHECK(ns == 0 || ns == 1 || ns == 2, "debug_set_viterbi_seqs: expected 0, 1 or 2");
   g_viterbi_ns = ns;
   return 0;
 }
@@ -1229,37 +1091,31 @@ int re2nn_crf_nll(const float* feats, const float* transitions, const int64_t* l
                   int L, int Ltags, int T, float* per_seq, float* loss, float* part_save, void* stream) {
   RE2NN_CHECK(feats && transitions && lengths && tags && per_seq, "crf_nll: null tensor");
   RE2NN_CHECK(B > 0 && L > 0 && T >= 3, "crf_nll: bad dims");
+  using Kernel = decltype(&crf_nll_kernel<true>);
+  static const Kernel kernels[7] = {crf_nll_exp_kernel<1>, crf_nll_exp_kernel<2>, crf_nll_exp_kernel<3>,
+                                    crf_nll_exp_kernel<4>, crf_nll_exp_kernel<5>, crf_nll_kernel<true>,
+                                    crf_nll_kernel<false>};
+  static int configured[7][kMaxDevices];
   const int Tp = (T + 31) & ~31;
   const size_t part = (size_t)kCrfWarps * 2 * Tp * 4;
   const size_t with_tr = part + (size_t)T * T * 4;
-  const int grid = cdiv(B, kCrfWarps);
-  cudaStream_t st = (cudaStream_t)stream;
   const size_t exp_smem = ((size_t)2 * T * T + kCrfOverrun + Tp + (size_t)kCrfWarps * 3 * Tp) * 4;
+  int k;           // exp<cdiv(T, 32)>, then the log-domain kernel with / without the transitions in shared memory
+  size_t smem;
   if (exp_smem <= kSmemLimit && T <= 160) {
-#define RE2NN_NLL(NJ)                                                                                              \
-  do {                                                                                                             \
-    RE2NN_CUDA(cudaFuncSetAttribute(crf_nll_exp_kernel<NJ>, cudaFuncAttributeMaxDynamicSharedMemorySize,          \
-                                    (int)exp_smem));                                                               \
-    crf_nll_exp_kernel<NJ><<<grid, kCrfWarps * 32, exp_smem, st>>>(feats, transitions, lengths, tags, B, L, Ltags, \
-                                                                   T, per_seq, part_save);                         \
-  } while (0)
-    switch (cdiv(T, 32)) {
-      case 1: RE2NN_NLL(1); break;
-      case 2: RE2NN_NLL(2); break;
-      case 3: RE2NN_NLL(3); break;
-      case 4: RE2NN_NLL(4); break;
-      default: RE2NN_NLL(5); break;
-    }
-#undef RE2NN_NLL
+    k = cdiv(T, 32) - 1;
+    smem = exp_smem;
   } else if (with_tr <= kSmemLimit) {
-    RE2NN_CUDA(cudaFuncSetAttribute(crf_nll_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)with_tr));
-    crf_nll_kernel<true><<<grid, kCrfWarps * 32, with_tr, st>>>(feats, transitions, lengths, tags, B, L, Ltags, T,
-                                                                per_seq, part_save);
+    k = 5;
+    smem = with_tr;
   } else {
-    crf_nll_kernel<false><<<grid, kCrfWarps * 32, part, st>>>(feats, transitions, lengths, tags, B, L, Ltags, T,
-                                                              per_seq, part_save);
+    k = 6;
+    smem = part;
   }
-  RE2NN_LAUNCH_CHECK();
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int rc = crf_launch(kernels[k], configured[k], cdiv(B, kCrfWarps), kCrfWarps * 32, smem, st, feats, transitions,
+                          lengths, tags, B, L, Ltags, T, per_seq, part_save))
+    return rc;
   if (loss) {
     reduce_sum_kernel<<<1, 1024, 0, st>>>(per_seq, (size_t)B, 1.0, loss);
     RE2NN_LAUNCH_CHECK();
@@ -1271,57 +1127,46 @@ int re2nn_crf_nll_backward(const float* feats, const float* transitions, const i
                            const float* part_save, const float* gscale, int B, int L, int Ltags, int T, float* dfeats,
                            float* dtrans, void* stream) {
   RE2NN_CHECK(feats && transitions && lengths && tags && part_save && dfeats && dtrans, "crf_nll_backward: null tensor");
+  using Kernel = decltype(&crf_nll_backward_exp_kernel);
+  static const Kernel kernels[4] = {crf_nll_backward_exp3_kernel, crf_nll_backward_exp_kernel,
+                                    crf_nll_backward_kernel<true>, crf_nll_backward_kernel<false>};
+  static int configured[4][kMaxDevices];
   const int Tp = (T + 31) & ~31, Tq = T | 1;
-  const size_t per_warp = ((size_t)T * Tq + 2 * Tp) * 4;
   const size_t tr_bytes = (size_t)T * T * 4;
+  // one CTA per SM either way (the per-sequence accumulators fill the shared memory): the scaled-exponential kernels
+  // take everything the SM has, so that e.g. B = 1024 at T = 74 is 147 CTAs of seven sequences = ONE wave instead of
+  // 171 CTAs of six = two
+  const size_t smem_all = 226 * 1024;
+  const size_t pw = ((size_t)T * Tq + 3 * Tp) * 4;             // per sequence of the scaled-exponential kernels
+  const size_t fixed = 2 * tr_bytes + (size_t)Tp * 4;
+  int k, nseq, block;       // kernel, sequences per CTA, threads per CTA
+  size_t smem;
+  if (fixed + 2 * pw <= kSmemLimit && T <= 96 && g_crf_bwd_split) {   // three warps per sequence
+    const int Tv = (T + 3) & ~3;                                         // 16-byte rows of the table and accumulators
+    const size_t fixed3 = ((((size_t)T * T + 3) & ~(size_t)3) + (size_t)T * Tv + Tp) * 4;
+    const size_t pw3 = ((size_t)T * Tv + 3 * Tp) * 4;
+    k = 0;
+    nseq = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed3) / pw3);
+    block = nseq * 96;
+    smem = fixed3 + nseq * pw3;
+  } else if (fixed + 2 * pw <= kSmemLimit) {        // transitions + table + at least two accumulators fit
+    k = 1;
+    nseq = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed) / pw);
+    block = nseq * 32;
+    smem = fixed + nseq * pw;
+  } else {   // log domain: as many warps as the accumulators allow, transitions in shared memory when they still fit
+    const size_t per_warp = ((size_t)T * Tq + 2 * Tp) * 4;
+    const bool ts = tr_bytes + per_warp <= kSmemLimit;
+    nseq = (int)std::min<size_t>(kCrfWarps, (kSmemLimit - (ts ? tr_bytes : 0)) / per_warp);
+    RE2NN_CHECK(nseq >= 1, "crf_nll_backward: tag set too large (T=%d)", T);
+    k = ts ? 2 : 3;
+    block = nseq * 32;
+    smem = (ts ? tr_bytes : 0) + nseq * per_warp;
+  }
   cudaStream_t st = (cudaStream_t)stream;
   RE2NN_CUDA(cudaMemsetAsync(dtrans, 0, tr_bytes, st));
-  {   // scaled-exponential kernel when transitions + table + at least two warps' accumulators fit
-    const size_t pw = ((size_t)T * Tq + 3 * Tp) * 4;
-    const size_t fixed = 2 * tr_bytes + (size_t)Tp * 4;
-    if (fixed + 2 * pw <= kSmemLimit) {
-      // one CTA per SM either way (the per-warp accumulators fill the shared memory): take everything the SM has, so
-      // that e.g. B = 1024 at T = 74 is 147 CTAs of seven sequences = ONE wave instead of 171 CTAs of six = two
-      const size_t smem_all = 226 * 1024;
-      const int nwe = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed) / pw);
-      if (T <= 96 && g_crf_bwd_split) {      // three warps per sequence: a third of the per-step latency
-        const int Tv = (T + 3) & ~3;           // 16-byte rows of the table and the accumulators
-        const size_t fixed3 = ((((size_t)T * T + 3) & ~(size_t)3) + (size_t)T * Tv + Tp) * 4;
-        const size_t pw3 = ((size_t)T * Tv + 3 * Tp) * 4;
-        const int nwe3 = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed3) / pw3);
-        const size_t smem_3 = fixed3 + nwe3 * pw3;
-        RE2NN_CUDA(cudaFuncSetAttribute(crf_nll_backward_exp3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_3));
-        crf_nll_backward_exp3_kernel<<<cdiv(B, nwe3), nwe3 * 96, smem_3, st>>>(feats, transitions, lengths, tags, part_save,
-                                                                             gscale, B, L, Ltags, T, dfeats, dtrans);
-        RE2NN_LAUNCH_CHECK();
-        return 0;
-      }
-      const size_t smem_e = fixed + nwe * pw;
-      RE2NN_CUDA(cudaFuncSetAttribute(crf_nll_backward_exp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_e));
-      crf_nll_backward_exp_kernel<<<cdiv(B, nwe), nwe * 32, smem_e, st>>>(feats, transitions, lengths, tags, part_save,
-                                                                          gscale, B, L, Ltags, T, dfeats, dtrans);
-      RE2NN_LAUNCH_CHECK();
-      return 0;
-    }
-  }
-  // as many warps (sequences) per CTA as the private accumulators allow, transitions in smem when they still fit
-  bool ts = tr_bytes + per_warp <= kSmemLimit;
-  size_t avail = kSmemLimit - (ts ? tr_bytes : 0);
-  int nw = (int)std::min<size_t>(kCrfWarps, avail / per_warp);
-  RE2NN_CHECK(nw >= 1, "crf_nll_backward: tag set too large (T=%d)", T);
-  const size_t smem = (ts ? tr_bytes : 0) + nw * per_warp;
-  const int grid = cdiv(B, nw);
-  if (ts) {
-    RE2NN_CUDA(cudaFuncSetAttribute(crf_nll_backward_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    crf_nll_backward_kernel<true><<<grid, nw * 32, smem, st>>>(feats, transitions, lengths, tags, part_save, gscale, B,
-                                                               L, Ltags, T, dfeats, dtrans);
-  } else {
-    RE2NN_CUDA(cudaFuncSetAttribute(crf_nll_backward_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    crf_nll_backward_kernel<false><<<grid, nw * 32, smem, st>>>(feats, transitions, lengths, tags, part_save, gscale,
-                                                                B, L, Ltags, T, dfeats, dtrans);
-  }
-  RE2NN_LAUNCH_CHECK();
-  return 0;
+  return crf_launch(kernels[k], configured[k], cdiv(B, nseq), block, smem, st, feats, transitions, lengths, tags,
+                    part_save, gscale, B, L, Ltags, T, dfeats, dtrans);
 }
 
 int re2nn_argmax_decode(const float* scores, const int64_t* lengths, const int64_t* offsets, int B, int L, int C,

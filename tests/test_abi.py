@@ -29,6 +29,8 @@ def test_version_and_error_channel():
     rc = _lib.fn['re2nn_decompose_recurrence'](None, None)
     assert rc != 0
     assert b'null args' in _lib.fn['re2nn_last_error']()
+    assert _lib.fn['re2nn_debug_set_viterbi_seqs'](4) != 0
+    assert b'expected 0, 1 or 2' in _lib.fn['re2nn_last_error']()
 
 
 def test_no_oracle_in_product():

@@ -229,45 +229,53 @@ def test_training_with_tensor_core_forward(farnn, crf, tp):
 
 def test_crf_hard_constraints_underflow_fallback():
     """Spiky features + forbidden (-1e4) transitions: the scaled-exponential CRF kernels underflow on some columns /
-    rows and must take their exact log-domain fallback; loss and gradients against a float64 autograd CRF."""
+    rows and must take their exact log-domain fallback; loss and gradients against a float64 autograd CRF.  T = 22,
+    100, 131, 170 and 225 land in every forward and backward kernel range of re2nn_crf_nll / _backward; at T = 226 the
+    loss still works and the backward reports that the tag set is too large."""
     import re2nn_seq_b200 as r
-    rs = np.random.RandomState(3)
-    ntag, B, L = 20, 37, 14
-    T = ntag + 2
-    feats = (rs.randn(B, L, T) * 12.0).astype(np.float32)
-    lens = rs.randint(2, L + 1, size=B).astype(np.int64)
-    lens[0] = L
-    tags = rs.randint(0, ntag, size=(B, L)).astype(np.int64)
-    trans = rs.randn(T, T).astype(np.float32)
-    trans[rs.rand(T, T) < 0.4] = -10000.0
-    trans[:, T - 2] = -10000.0
-    trans[T - 1, :] = -10000.0
-    crf = r.CRF(ntag, True).cuda()
-    with torch.no_grad():
-        crf.transitions.copy_(_t(trans))
-    f = _t(feats).requires_grad_(True)
-    mask = _t(orc.length_mask(lens, L))
-    loss = crf.neg_log_likelihood_loss(f, mask, _t(tags))
-    loss.backward()
-    # float64 reference (crf.py:48-99,202-251 in plain autograd)
-    f64 = torch.from_numpy(feats).double().requires_grad_(True)
-    t64 = torch.from_numpy(trans).double().requires_grad_(True)
-    total = 0.0
-    for b in range(B):
-        n = int(lens[b])
-        part = f64[b, 0] + t64[T - 2]
-        gold = f64[b, 0, tags[b, 0]] + t64[T - 2, tags[b, 0]]
-        for t in range(1, n):
-            part = torch.logsumexp(part[:, None] + t64, 0) + f64[b, t]
-            gold = gold + f64[b, t, tags[b, t]] + t64[tags[b, t - 1], tags[b, t]]
-        logz = torch.logsumexp(part + t64[:, T - 1], 0)
-        gold = gold + t64[tags[b, n - 1], T - 1]
-        total = total + (logz - gold)
-    total.backward()
-    assert rel_err(loss.item(), total.item()) < TOL
-    # log Z is a few hundred here: fp32 keeps ~3e-5 absolute on it, which is the relative error of every marginal
-    assert rel_err(f.grad.cpu().numpy(), f64.grad.numpy()) < 3e-4
-    assert rel_err(crf.transitions.grad.cpu().numpy(), t64.grad.numpy()) < 3e-4
+    for ntag in (20, 98, 129, 168, 223, 224):
+        rs = np.random.RandomState(3)
+        B, L = 37, 14
+        T = ntag + 2
+        feats = (rs.randn(B, L, T) * 12.0).astype(np.float32)
+        lens = rs.randint(2, L + 1, size=B).astype(np.int64)
+        lens[0] = L
+        tags = rs.randint(0, ntag, size=(B, L)).astype(np.int64)
+        trans = rs.randn(T, T).astype(np.float32)
+        trans[rs.rand(T, T) < 0.4] = -10000.0
+        trans[:, T - 2] = -10000.0
+        trans[T - 1, :] = -10000.0
+        crf = r.CRF(ntag, True).cuda()
+        with torch.no_grad():
+            crf.transitions.copy_(_t(trans))
+        f = _t(feats).requires_grad_(True)
+        mask = _t(orc.length_mask(lens, L))
+        loss = crf.neg_log_likelihood_loss(f, mask, _t(tags))
+        # float64 reference (crf.py:48-99,202-251 in plain autograd), all sequences at once
+        f64 = torch.from_numpy(feats).double().requires_grad_(True)
+        t64 = torch.from_numpy(trans).double().requires_grad_(True)
+        n = torch.from_numpy(lens)
+        tg = torch.from_numpy(tags)
+        part = f64[:, 0] + t64[T - 2]
+        for t in range(1, L):
+            nxt = torch.logsumexp(part[:, :, None] + t64, 1) + f64[:, t]
+            part = torch.where((t < n)[:, None], nxt, part)
+        logz = torch.logsumexp(part + t64[:, T - 1], 1)
+        prev = torch.cat([torch.full((B, 1), T - 2), tg[:, :-1]], 1)
+        steps = f64.gather(2, tg[:, :, None])[:, :, 0] + t64[prev, tg]
+        gold = (torch.where(torch.arange(L)[None, :] < n[:, None], steps, 0.0).sum(1)
+                + t64[tg[torch.arange(B), n - 1], T - 1])
+        total = (logz - gold).sum()
+        total.backward()
+        assert rel_err(loss.item(), total.item()) < TOL, 'T = %d' % T
+        if T > 225:
+            with pytest.raises(RuntimeError, match='tag set too large'):
+                loss.backward()
+            continue
+        loss.backward()
+        # log Z is a few hundred here: fp32 keeps ~3e-5 absolute on it, which is the relative error of every marginal
+        assert rel_err(f.grad.cpu().numpy(), f64.grad.numpy()) < 3e-4, 'T = %d' % T
+        assert rel_err(crf.transitions.grad.cpu().numpy(), t64.grad.numpy()) < 3e-4, 'T = %d' % T
 
 
 @pytest.mark.parametrize('B,ntag', [(2500, 12), (4801, 70)])
@@ -294,9 +302,9 @@ def test_crf_viterbi_large_batch(B, ntag):
 
 
 @pytest.mark.parametrize('seqs_per_warp', [1, 2])
-@pytest.mark.parametrize('B,ntag,L', [(700, 129, 12), (300, 198, 7), (90, 258, 6), (333, 34, 9)])
+@pytest.mark.parametrize('B,ntag,L', [(700, 129, 12), (500, 110, 10), (300, 198, 7), (90, 258, 6), (333, 34, 9)])
 def test_crf_viterbi_wide_tagsets(B, ntag, L, seqs_per_warp):
-    """T = 131 (cfg5: five target tags per lane), T = 200 (generic shared-memory sweep) and T = 260 (transition table
+    """T = 131 (cfg5: five target tags per lane), T = 112 (four), T = 200 (generic shared-memory sweep) and T = 260 (transition table
     beyond shared memory: global-memory kernel), real-valued features with many exact ties, one empty sequence:
     paths bit-exact against the restatement of crf.py:102-195."""
     import re2nn_seq_b200 as r

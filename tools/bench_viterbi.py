@@ -1,4 +1,4 @@
-"""Viterbi kernel alone: time per launch for 1 / 2 / 4 sequences per warp at the cfg2 and cfg5 tag-set sizes."""
+"""Viterbi kernel alone: time per launch for 1 / 2 sequences per warp at the cfg2 and cfg5 tag-set sizes."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -15,7 +15,7 @@ for name, B, L, T, fixed in (('cfg2', 4096, 35, 75, False), ('cfg5/4', 16384, 64
     tr = torch.from_numpy(synth.crf_transitions(0, T)).cuda()
     N = int(lens.sum())
     ref = None
-    for ns in (1, 2, 4):
+    for ns in (1, 2):
         _lib.check(_lib.fn['re2nn_debug_set_viterbi_seqs'](ns), 'ns')
         for _ in range(2):
             flat, _ = ops.crf_viterbi(feats, tr, lt, offs, N, want_flat=True, want_padded=False)

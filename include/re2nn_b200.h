@@ -30,7 +30,7 @@
 extern "C" {
 #endif
 
-#define RE2NN_ABI_VERSION 3
+#define RE2NN_ABI_VERSION 4
 
 /* update_nonlinear / additional_nonlinear (model_decompose_single.py:184-191, model_decompose.py:228-237) */
 enum { RE2NN_NL_NONE = 0, RE2NN_NL_RELU = 1, RE2NN_NL_TANH = 2, RE2NN_NL_RELUTANH = 3, RE2NN_NL_SIGMOID = 4 };
@@ -98,6 +98,23 @@ int re2nn_profile_enabled(void);
 size_t re2nn_gemm_nt_workspace(int precision, int M, int N, int K);
 int re2nn_gemm_nt(int precision, const float* A, const float* B, int M, int N, int K, float* C, void* ws,
                   size_t ws_bytes, void* stream);
+
+/* ---- stand-alone weight-gradient GEMM (unit-test / calibration entry) ---------------------------------
+ * C[P x Q] = sum_m X0[m, :]^T Y0[m, :] (m < rows0) + sum_m X1[m, :]^T Y1[m, :] (m < rows1), every operand fp32
+ * row-major with its own leading dimension (ldx >= P, ldy >= Q, any alignment); pair 1 is optional (X1 = NULL).
+ * Y2 (optional, single pair only, leading dimension ldy0): the right operand is Y0 * Y2 element-wise.  mask_len
+ * (optional, needs Y2): row m = b * mask_L + t only counts when t < mask_len[b], rows0 = B * mask_L; the pad rows of
+ * Y0 / Y2 may hold anything, NaN and Inf included (this is the dC product of the decompose backward).
+ * path: 0 = the kernel re2nn_decompose_backward picks for this shape (re2nn_gemm_tn_path), 1 = the CUDA-core split-K
+ * kernel, 2 = tcgen05 in 3xTF32 (fails without an sm_100 device or when P or Q is below 16).  ws: at least
+ * re2nn_gemm_tn_workspace(P, Q) bytes.  Deterministic: the same call gives the same bits.
+ * re2nn_gemm_tn_path: 1 or 2, the kernel the backward takes for a P x Q product over `rows` summed rows (has_y2: the
+ * dC layout; it takes the same path as a plain product). */
+int re2nn_gemm_tn_path(int P, int Q, int64_t rows, int has_y2);
+size_t re2nn_gemm_tn_workspace(int P, int Q);
+int re2nn_gemm_tn(int path, int P, int Q, const float* X0, const float* Y0, int ldx0, int ldy0, int64_t rows0, const float* X1,
+                  const float* Y1, int ldx1, int ldy1, int64_t rows1, const float* Y2, const int64_t* mask_len, int mask_L,
+                  float* C, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- generalised token factor table ------------------------------------------------------------
  * table[r, :] = V_embed[r,:]*beta_vec + phi_add(E[r,:] @ G) * (1 - beta_vec)   for r in [0, rows)

@@ -107,6 +107,10 @@ SYMBOLS = {
     're2nn_profile_enabled': (C.c_int, []),
     're2nn_gemm_nt_workspace': (sz, [C.c_int, C.c_int, C.c_int, C.c_int]),
     're2nn_gemm_nt': (C.c_int, [C.c_int, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, sz, vp]),
+    're2nn_gemm_tn_path': (C.c_int, [C.c_int, C.c_int, i64, C.c_int]),
+    're2nn_gemm_tn_workspace': (sz, [C.c_int, C.c_int]),
+    're2nn_gemm_tn': (C.c_int, [C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, C.c_int, i64, vp, vp, C.c_int, C.c_int, i64,
+                                vp, vp, C.c_int, vp, vp, sz, vp]),
     're2nn_token_table': (C.c_int, [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]),
     're2nn_gate_table': (C.c_int, [vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp, vp]),
     're2nn_output_vector_sum': (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp]),

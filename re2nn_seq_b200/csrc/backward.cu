@@ -169,20 +169,51 @@ __global__ void split_reduce_kernel(const float* __restrict__ partial, int nspli
 static bool g_tn_tc = true;      // long reductions on tcgen05 (gemm_tn_tc.cuh); re2nn_debug_set_tn_tc
 extern "C" int re2nn_has_tcgen05(void);
 
+enum { kTnPathCuda = 1, kTnPathTc = 2 };
+
+// The kernel a weight-gradient product of P x Q over `rows` summed rows runs on: tcgen05 once the reduction is long
+// enough to fill a pipeline per CTA, the CUDA-core kernel otherwise.
+static int tn_path(int P, int Q, size_t rows) {
+#ifdef RE2NN_HAVE_TC
+  if (g_tn_tc && re2nn_has_tcgen05() != 0 && rows >= 4096 && P >= 16 && Q >= 16) return kTnPathTc;
+#endif
+  return kTnPathCuda;
+}
+
+// out (+)= sum over pairs X^T Y.  path 0 = tn_path's choice; kTnPathTc requires tcgen05 and P, Q >= 16 (callers check).
+// The partial buffer holds kTnSplit slices of P x Q.
 template <class YLoad>
-static cudaError_t run_tn(const TnProblem& prob, float* partial, float* out, int accumulate, const YLoad& yl, cudaStream_t st) {
+static cudaError_t run_tn(const TnProblem& prob, float* partial, float* out, int accumulate, const YLoad& yl, cudaStream_t st,
+                          int path = 0) {
   const size_t n = (size_t)prob.P * prob.Q;
   size_t rows = 0;
   for (int i = 0; i < prob.npairs; ++i) rows += prob.pair[i].rows;
+  // the tensor-core kernel forms the right operand from a plain Y or from Y * Y2 (YLoadAlphaBeta without Y2: CUDA cores)
+  if (path == 0) path = (YLoad::kPlain || prob.Y2 != nullptr) ? tn_path(prob.P, prob.Q, rows) : kTnPathCuda;
 #ifdef RE2NN_HAVE_TC
-  // tensor cores once the reduction is long enough to fill a pipeline per CTA (the partial buffer holds kTnSplit slices)
-  if ((YLoad::kPlain || prob.Y2 != nullptr) && g_tn_tc && re2nn_has_tcgen05() != 0 && rows >= 4096 && prob.P >= 16 && prob.Q >= 16) {
-    const TnTcPlan pl = tn_tc_plan(prob, kTnSplit);
-    if (pl.stages >= 2) {
-      if (cudaError_t e = launch_tn_tc(prob, partial, pl, st)) return e;
-      split_reduce_kernel<<<(unsigned)std::min<size_t>((n + 255) / 256, 1184), 256, 0, st>>>(partial, pl.nsplit, n, out, accumulate);
-      return cudaGetLastError();
+  if (path == kTnPathTc) {
+    // Consecutive row chunks of at most kTnSplit * kTnMaxKb k-blocks (shared by the pairs), so that no split of any
+    // launch accumulates more than kTnMaxKb k-blocks; the later chunks add onto `out`.  Masked chunks start on a sequence.
+    size_t crows = (size_t)kTnSplit * kTnMaxKb * kTnKBlock / prob.npairs, longest = 0;
+    if (prob.mask_len != nullptr) crows = std::max<size_t>(crows / prob.mask_L, 1) * prob.mask_L;
+    for (int i = 0; i < prob.npairs; ++i) longest = std::max(longest, prob.pair[i].rows);
+    for (size_t c0 = 0; c0 == 0 || c0 < longest; c0 += crows) {
+      TnProblem sub = prob;         // one chunk: the problem itself
+      sub.npairs = 0;
+      for (int i = 0; i < prob.npairs; ++i) {
+        const TnPair& p = prob.pair[i];
+        if (c0 > 0 && p.rows <= c0) continue;
+        sub.pair[sub.npairs++] = TnPair{p.X + c0 * p.ldx, p.Y + c0 * p.ldy, p.ldx, p.ldy, std::min(p.rows - c0, crows)};
+      }
+      if (prob.Y2 != nullptr) sub.Y2 = prob.Y2 + c0 * prob.pair[0].ldy;     // Y2 goes with a single pair
+      if (prob.mask_len != nullptr) sub.mask_len = prob.mask_len + c0 / prob.mask_L;
+      const TnTcPlan pl = tn_tc_plan(sub, kTnSplit);
+      if (cudaError_t e = launch_tn_tc(sub, partial, pl, st)) return e;
+      split_reduce_kernel<<<(unsigned)std::min<size_t>((n + 255) / 256, 1184), 256, 0, st>>>(partial, pl.nsplit, n, out,
+                                                                                             c0 == 0 ? accumulate : 1);
+      if (cudaError_t e = cudaGetLastError()) return e;
     }
+    return cudaSuccess;
   }
 #endif
   dim3 grid(cdiv(prob.P, 64), cdiv(prob.Q, 64), kTnSplit);
@@ -844,6 +875,41 @@ int re2nn_debug_set_backward_tc(int on) {
 
 int re2nn_debug_set_tn_tc(int on) {
   g_tn_tc = on != 0;
+  return 0;
+}
+
+int re2nn_gemm_tn_path(int P, int Q, int64_t rows, int has_y2) {
+  (void)has_y2;                  // both kernels form Y * Y2 themselves: the dC layout takes the same path
+  return tn_path(P, Q, rows > 0 ? (size_t)rows : 0);
+}
+
+size_t re2nn_gemm_tn_workspace(int P, int Q) {
+  return P > 0 && Q > 0 ? align_up((size_t)kTnSplit * P * Q * 4, 256) : 0;
+}
+
+int re2nn_gemm_tn(int path, int P, int Q, const float* X0, const float* Y0, int ldx0, int ldy0, int64_t rows0, const float* X1,
+                  const float* Y1, int ldx1, int ldy1, int64_t rows1, const float* Y2, const int64_t* mask_len, int mask_L,
+                  float* C, void* ws, size_t ws_bytes, void* stream) {
+  RE2NN_CHECK(path >= 0 && path <= 2, "gemm_tn: path must be 0, 1 or 2");
+  RE2NN_CHECK(P > 0 && Q > 0 && X0 && Y0 && C && ldx0 >= P && ldy0 >= Q && rows0 >= 0, "gemm_tn: bad arguments");
+  RE2NN_CHECK(!X1 || (Y1 && ldx1 >= P && ldy1 >= Q && rows1 >= 0), "gemm_tn: bad second pair");
+  RE2NN_CHECK(!Y2 || (!X1 && Y2 != Y0), "gemm_tn: Y2 needs a single pair and must not alias Y0");
+  RE2NN_CHECK(!mask_len || (Y2 && mask_L > 0 && rows0 % mask_L == 0), "gemm_tn: a mask needs Y2 and rows0 = B * mask_L");
+  RE2NN_CHECK(ws && ws_bytes >= re2nn_gemm_tn_workspace(P, Q), "gemm_tn: workspace too small");
+  RE2NN_CHECK(path != kTnPathTc || (re2nn_has_tcgen05() != 0 && P >= 16 && Q >= 16),
+              "gemm_tn: the tcgen05 path needs an sm_100 device and P, Q >= 16");
+  TnProblem t;
+  memset(&t, 0, sizeof(t));
+  t.P = P; t.Q = Q; t.npairs = X1 ? 2 : 1;
+  t.pair[0] = TnPair{X0, Y0, ldx0, ldy0, (size_t)rows0};
+  if (X1) t.pair[1] = TnPair{X1, Y1, ldx1, ldy1, (size_t)rows1};
+  t.Y2 = Y2;
+  t.mask_len = mask_len;
+  t.mask_L = mask_len ? mask_L : 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  float* partial = (float*)ws;
+  if (Y2) RE2NN_CUDA(run_tn(t, partial, C, 0, YLoadAlphaBeta{Y2, mask_len, mask_len ? mask_L : 1, mask_len ? 0 : 1}, st, path));
+  else RE2NN_CUDA(run_tn(t, partial, C, 0, YLoadPlain{}, st, path));
   return 0;
 }
 

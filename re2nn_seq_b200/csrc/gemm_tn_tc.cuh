@@ -28,6 +28,14 @@ constexpr int kTnLoaderWarps = 8;
 // it never waits for the other warps; warps 0..3 drain TMEM at the end
 constexpr int kTnThreads = 32 * kTnLoaderWarps;
 constexpr int kTnKBlock = 32;                                 // reduction rows per pipeline stage: 128 bytes of tf32
+// k-blocks one split accumulates at most (1536 rows).  The TMEM accumulator truncates every add, so a split's error grows
+// with its chain, fastest on same-sign data where every truncation pulls the same way.  Measured on a B200 (max-norm
+// relative vs float64, uniform [0, 1) operands): 128 k-blocks per split 2.5-2.8e-5, a whole 2240-k-block reduction in
+// one split 5.3e-4; signed data about a third of that.  48 keeps every product within the 2e-5 gradient bound of
+// DESIGN.md section 2 and leaves every plan of the benchmarked cfg3 training step alone (its longest chain, dS1 / dS2,
+// is 46 k-blocks).  tn_tc_plan adds splits and run_tn reduces longer products in consecutive chunks so that no split
+// exceeds the cap.
+constexpr int kTnMaxKb = 48;
 
 // rows of pair `pr` that split `split` of `nsplit` reduces: whole k-blocks, so only a pair's last chunk has a ragged end
 __host__ __device__ inline void tn_split_range(size_t rows, int split, int nsplit, size_t* r0, size_t* r1) {
@@ -267,14 +275,27 @@ __global__ void __launch_bounds__(kTnThreads, 1) tn_tc_kernel(const TnProblem pr
   }
 }
 
-// tile width over Q, split count and pipeline depth of one problem
+// k-blocks the busiest split reduces when the problem is cut into `nsplit` splits (tn_split_range, summed over the pairs)
+inline size_t tn_chain_kb(const TnProblem& prob, int nsplit) {
+  size_t kb = 0;
+  for (int pi = 0; pi < prob.npairs; ++pi) {
+    const size_t k = (prob.pair[pi].rows + kTnKBlock - 1) / kTnKBlock;
+    kb += (k + nsplit - 1) / nsplit;
+  }
+  return kb;
+}
+
+// tile width over Q, split count and pipeline depth of one problem: one split per SM the tiles leave free, more when a
+// split would otherwise accumulate more than kTnMaxKb k-blocks (up to max_split)
 struct TnTcPlan { int bn, nt, nsplit, stages, smem; };
+static_assert(2 * 2 * (128 * 128 + 256 * 128) + 256 <= kTcSmemLimit, "tn_tc_kernel needs two pipeline stages at bn = 256");
 inline TnTcPlan tn_tc_plan(const TnProblem& prob, int max_split) {
   TnTcPlan pl;
   pl.nt = cdiv(prob.Q, 256);
   pl.bn = ((cdiv(prob.Q, pl.nt) + 15) / 16) * 16;
   const int tiles = cdiv(prob.P, 128) * pl.nt;
   pl.nsplit = std::max(1, std::min(max_split, sm_count() / tiles));
+  while (pl.nsplit < max_split && tn_chain_kb(prob, pl.nsplit) > (size_t)kTnMaxKb) ++pl.nsplit;
   const int stage_bytes = 2 * (128 * 128 + pl.bn * 128);
   pl.stages = std::min(4, (kTcSmemLimit - 256) / stage_bytes);
   pl.smem = pl.stages * stage_bytes + 256;

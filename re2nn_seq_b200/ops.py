@@ -362,6 +362,57 @@ def gemm_nt(A, B, precision='fp32'):
     return out
 
 
+_TN_PATH = {'auto': 0, 'cuda': 1, 'tc': 2}
+
+
+def gemm_tn_workspace(P, Q):
+    return fn['re2nn_gemm_tn_workspace'](P, Q)
+
+
+def gemm_tn_path(P, Q, rows, has_y2=False):
+    """'cuda' or 'tc': the kernel the decompose backward runs a P x Q weight gradient over `rows` summed rows on."""
+    return {1: 'cuda', 2: 'tc'}[fn['re2nn_gemm_tn_path'](P, Q, rows, int(has_y2))]
+
+
+def gemm_tn(X0, Y0, X1=None, Y1=None, Y2=None, mask_len=None, path='auto', ws=None):
+    """C = X0^T (Y0 [* Y2]) [+ X1^T Y1] through the weight-gradient GEMMs of the backward (test / calibration entry).
+    Operands are 2-D fp32 CUDA tensors whose rows are the reduction index; each may be a column slice of a wider slab
+    (unit column stride, any row stride).  mask_len (int64, B entries, needs Y2): row b * L + t of Y0 * Y2 counts only
+    when t < mask_len[b], with L = rows / B.  path: 'auto' (the backward's choice), 'cuda' or 'tc'.  ws: optional
+    uint8 scratch of gemm_tn_workspace(P, Q) bytes (the split-K partials)."""
+    def ld(t):
+        if t.dtype != torch.float32 or not t.is_cuda or t.dim() != 2 or (t.shape[0] > 1 and t.stride(1) != 1):
+            raise RuntimeError("re2nn_b200: gemm_tn operands are 2-D fp32 CUDA tensors with unit column stride")
+        return max(t.stride(0), t.shape[1])
+
+    def ptr(t):
+        return C.c_void_p(t.data_ptr()) if t is not None else None
+    rows0, P = X0.shape
+    Q = Y0.shape[1]
+    rows1 = X1.shape[0] if X1 is not None else 0
+    if Y0.shape[0] != rows0 or (X1 is not None and (Y1.shape[0] != rows1 or X1.shape[1] != P or Y1.shape[1] != Q)):
+        raise RuntimeError("re2nn_b200: gemm_tn operand shapes do not match")
+    if Y2 is not None and (Y2.shape != Y0.shape or ld(Y2) != ld(Y0)):
+        raise RuntimeError("re2nn_b200: gemm_tn Y2 must have Y0's shape and leading dimension")
+    mask_L = 0
+    if mask_len is not None:
+        if mask_len.numel() == 0 or rows0 % mask_len.numel() != 0:
+            raise RuntimeError("re2nn_b200: gemm_tn rows must be B * L with B = len(mask_len)")
+        mask_L = rows0 // mask_len.numel()
+    out = torch.empty((P, Q), dtype=torch.float32, device=X0.device)
+    need = gemm_tn_workspace(P, Q)
+    if ws is None:
+        ws = torch.empty((need,), dtype=torch.uint8, device=X0.device)
+    elif ws.numel() * ws.element_size() < need or not ws.is_cuda:
+        raise RuntimeError("re2nn_b200: gemm_tn workspace too small")
+    check(fn['re2nn_gemm_tn'](_TN_PATH[path], P, Q, ptr(X0), ptr(Y0), ld(X0), ld(Y0), rows0,
+                              ptr(X1), ptr(Y1), ld(X1) if X1 is not None else 0, ld(Y1) if Y1 is not None else 0, rows1,
+                              ptr(Y2), _i64(mask_len) if mask_len is not None else None, mask_L,
+                              _f32(out), C.c_void_p(ws.data_ptr()), need, _stream()), 'gemm_tn')
+    _count(2)
+    return out
+
+
 def batched_vecmat(h, T, transposed=False, max_semiring=False):
     """out[b,s] = (+|max)_j h[b,j] * T[b,j,s] (or T[b,s,j] when transposed); -> (out, argmax int32 or None)."""
     B, S = h.shape

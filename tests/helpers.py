@@ -42,6 +42,26 @@ def rel_err(a, b):
     return float(np.abs(a - b).max() / max(np.abs(b).max(), 1e-30))
 
 
+def oracle_gradient_errors(m, args, x, labels, lengths, loss, dense_v=None):
+    """After loss.backward() on module `m`: its loss and every trained parameter's gradient against the float64 autograd
+    oracle (oracle/re2nn_oracle_torch.py) over the same batch -> (loss rel err, {parameter name: max-norm rel err}).
+    A parameter the oracle's loss does not reach must get no gradient or a zero one (error 0, else inf)."""
+    from oracle import re2nn_oracle_torch as ot
+    p64 = {_RENAME.get(k, k): v.detach().cpu().numpy().astype(np.float64) for k, v in m.state_dict().items()}
+    names = [_RENAME.get(k, k) for k, v in m.named_parameters() if v.requires_grad]
+    o_loss, g64 = ot.grads(p64, x if dense_v is None else dense_v, labels, lengths, args, dense_v=dense_v, names=names)
+    errs = {}
+    for k, v in m.named_parameters():
+        if not v.requires_grad:
+            continue
+        ref = g64[_RENAME.get(k, k)]
+        if ref is None:
+            errs[k] = 0.0 if v.grad is None or not v.grad.any() else float('inf')
+        else:
+            errs[k] = rel_err(v.grad.cpu().numpy(), ref)
+    return rel_err(float(loss), o_loss), errs
+
+
 # ---- a stand-in reference tree for the `src_seq` shadow package (shim/) ------------------------------
 # The reference's module layout and the names its drivers import, each defined in a placeholder module.  The shadow
 # package's import mechanics (which name resolves to which tree) are tested against it, so those tests do not need an

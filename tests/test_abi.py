@@ -24,7 +24,7 @@ def test_header_symbols_exported():
 
 def test_version_and_error_channel():
     from re2nn_seq_b200 import _lib
-    assert _lib.fn["re2nn_abi_version"]() == 3
+    assert _lib.fn["re2nn_abi_version"]() == 4
     # argument validation happens before any CUDA call, so this is safe without a GPU
     rc = _lib.fn['re2nn_decompose_recurrence'](None, None)
     assert rc != 0
@@ -49,7 +49,7 @@ def test_torch_library_registration():
     import pytest
     import torch
     from re2nn_seq_b200 import _lib
-    assert int(_lib.tops.abi_version()) == 3
+    assert int(_lib.tops.abi_version()) == 4
     for name in ('ifst_decompose_forward', 'ifst_onehot_forward', 'label_scores', 'argmax_decode', 'crf_viterbi', 'crf_nll',
                  'crf_nll_backward'):
         assert hasattr(_lib.tops, name), name

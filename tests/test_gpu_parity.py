@@ -7,7 +7,7 @@ import pytest
 import torch
 
 from conftest import golden_files
-from helpers import args_of, build_module, golden_grads, load_golden, oracle_params, rel_err
+from helpers import args_of, build_module, golden_grads, load_golden, oracle_gradient_errors, oracle_params, rel_err
 from oracle import re2nn_oracle as orc
 
 pytestmark = pytest.mark.gpu
@@ -167,23 +167,14 @@ def test_decompose_gradients_golden(name):
 @pytest.mark.parametrize('farnn,crf', [(0, 1), (2, 1), (1, 0)])
 def test_decompose_gradients_cfg3_shapes_vs_oracle(farnn, crf):
     """SNIPS-shaped factors, gradients against the float64 autograd oracle within 1e-5 * max|grad| ... 1e-4."""
-    from oracle import re2nn_oracle_torch as ot
     m, args, x, lens, lab = _random_decompose(7, 500, 300, 200, 72, 100, 24, 20, farnn=farnn, use_crf=crf,
                                               update_nonlinear='tanh', beta=0.1, train_beta=1, train_h0=1, train_hT=1,
                                               train_V_embed=1, train_wildcard=1)
     loss, _, _ = m.forward_local(_t(x), _t(lab), _t(lens), train=True)
     loss.backward()
-    rename = {'embedding.weight': 'embedding', 'crf.transitions': 'crf_transitions',
-              'priority_layer.priority_mat': 'priority_mat', 'priority_layer.priority_bias': 'priority_bias'}
-    p64 = {rename.get(k, k): v.detach().cpu().numpy().astype(np.float64) for k, v in m.state_dict().items()}
-    names = [rename.get(k, k) for k, v in m.named_parameters() if v.requires_grad]
-    o_loss, g64 = ot.grads(p64, x, lab, lens, args, names=names)
-    assert rel_err(loss.item(), o_loss) < TOL
-    for k, v in m.named_parameters():
-        if not v.requires_grad:
-            continue
-        ref = g64[rename.get(k, k)]
-        err = rel_err(v.grad.cpu().numpy(), ref)
+    loss_err, errs = oracle_gradient_errors(m, args, x, lab, lens, loss.item())
+    assert loss_err < TOL
+    for k, err in errs.items():
         assert err < 1e-4, '%s: rel err %.3e' % (k, err)
 
 

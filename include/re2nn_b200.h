@@ -220,8 +220,10 @@ int re2nn_batched_vecmat(const float* h, const float* T, int B, int S, int trans
 /* ---- decompose i-FST backward (BPTT through both directions + label scores) ---------------------------
  * replaces torch.autograd over forward_local (train_decompose.py:192).  Input: d loss / d all_scores.
  * Outputs: gradients of every parameter the reference trains (NULL pointer = not wanted).
- * fp32 CUDA-core path; weight gradients are reduced deterministically (split-K partials + ordered sum),
- * token-table scatter-adds use float atomics. */
+ * fp32 data throughout.  On an sm_100 device the GEMMs of every BPTT step, the label-score GEMM and the long
+ * weight-gradient products run on tcgen05 in 3xTF32 (fp32-grade products), the rest on CUDA cores in fp32.
+ * Weight gradients are reduced deterministically (split-K partials + ordered sum), token-table scatter-adds use
+ * float atomics. */
 typedef struct re2nn_backward_args {
   int32_t B, Lpad, L, S, R, C;  /* C = columns of all_scores */
   int32_t farnn, update_nonlinear, v_mode, full_pad, ce1;

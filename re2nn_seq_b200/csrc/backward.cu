@@ -17,6 +17,7 @@
 // reduced deterministically (split-K partials + ordered sum); bias / vector gradients are deterministic column sums
 // of the per-step slabs.
 #include <algorithm>
+#include <initializer_list>
 #include <memory>
 
 #include "gemm_simt.cuh"
@@ -79,13 +80,11 @@ struct EpiDAB {
 // ---- transposed ("TN") GEMM: C[P x Q] = sum over pairs, rows m:  X[m, p] * Y[m, q]  ---------------------------
 // (TnPair / TnProblem: gemm_tn_tc.cuh, which holds the tcgen05 version of this kernel)
 
-// XLoad hook lets dC form (alpha*beta) on the fly
+// The right operand as the CUDA-core kernel reads it: Y itself, or the masked Y * Y2 of a problem with Y2 (run_tn)
 struct YLoadPlain {
-  static constexpr bool kPlain = true;
   __device__ __forceinline__ float operator()(const TnPair& pr, size_t m, int q) const { return __ldg(pr.Y + m * pr.ldy + q); }
 };
 struct YLoadAlphaBeta {
-  static constexpr bool kPlain = false;      // CUDA-core kernel: forms the masked alpha * beta itself (the tcgen05 one reads Y2 / mask_len)
   const float* beta; const int64_t* len; int L, full_pad;
   __device__ __forceinline__ float operator()(const TnPair& pr, size_t m, int q) const {
     int b = (int)(m / L), t = (int)(m - (size_t)b * L);
@@ -167,30 +166,23 @@ __global__ void split_reduce_kernel(const float* __restrict__ partial, int nspli
 }
 
 static bool g_tn_tc = true;      // long reductions on tcgen05 (gemm_tn_tc.cuh); re2nn_debug_set_tn_tc
-extern "C" int re2nn_has_tcgen05(void);
 
 enum { kTnPathCuda = 1, kTnPathTc = 2 };
 
 // The kernel a weight-gradient product of P x Q over `rows` summed rows runs on: tcgen05 once the reduction is long
 // enough to fill a pipeline per CTA, the CUDA-core kernel otherwise.
 static int tn_path(int P, int Q, size_t rows) {
-#ifdef RE2NN_HAVE_TC
   if (g_tn_tc && re2nn_has_tcgen05() != 0 && rows >= 4096 && P >= 16 && Q >= 16) return kTnPathTc;
-#endif
   return kTnPathCuda;
 }
 
 // out (+)= sum over pairs X^T Y.  path 0 = tn_path's choice; kTnPathTc requires tcgen05 and P, Q >= 16 (callers check).
 // The partial buffer holds kTnSplit slices of P x Q.
-template <class YLoad>
-static cudaError_t run_tn(const TnProblem& prob, float* partial, float* out, int accumulate, const YLoad& yl, cudaStream_t st,
-                          int path = 0) {
+static cudaError_t run_tn(const TnProblem& prob, float* partial, float* out, int accumulate, cudaStream_t st, int path = 0) {
   const size_t n = (size_t)prob.P * prob.Q;
   size_t rows = 0;
   for (int i = 0; i < prob.npairs; ++i) rows += prob.pair[i].rows;
-  // the tensor-core kernel forms the right operand from a plain Y or from Y * Y2 (YLoadAlphaBeta without Y2: CUDA cores)
-  if (path == 0) path = (YLoad::kPlain || prob.Y2 != nullptr) ? tn_path(prob.P, prob.Q, rows) : kTnPathCuda;
-#ifdef RE2NN_HAVE_TC
+  if (path == 0) path = tn_path(prob.P, prob.Q, rows);
   if (path == kTnPathTc) {
     // Consecutive row chunks of at most kTnSplit * kTnMaxKb k-blocks (shared by the pairs), so that no split of any
     // launch accumulates more than kTnMaxKb k-blocks; the later chunks add onto `out`.  Masked chunks start on a sequence.
@@ -215,13 +207,28 @@ static cudaError_t run_tn(const TnProblem& prob, float* partial, float* out, int
     }
     return cudaSuccess;
   }
-#endif
   dim3 grid(cdiv(prob.P, 64), cdiv(prob.Q, 64), kTnSplit);
-  tn_gemm_kernel<YLoad><<<grid, 256, 0, st>>>(prob, partial, yl);
+  if (prob.Y2 == nullptr) {
+    tn_gemm_kernel<<<grid, 256, 0, st>>>(prob, partial, YLoadPlain{});
+  } else {
+    const bool masked = prob.mask_len != nullptr;
+    const YLoadAlphaBeta yl{prob.Y2, prob.mask_len, masked ? prob.mask_L : 1, masked ? 0 : 1};
+    tn_gemm_kernel<<<grid, 256, 0, st>>>(prob, partial, yl);
+  }
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   split_reduce_kernel<<<(unsigned)std::min<size_t>((n + 255) / 256, 1184), 256, 0, st>>>(partial, kTnSplit, n, out, accumulate);
   return cudaGetLastError();
+}
+
+// out = sum over `pairs` X^T Y (nothing when out is NULL)
+static cudaError_t tn(float* out, int P, int Q, std::initializer_list<TnPair> pairs, float* partial, cudaStream_t st) {
+  if (out == nullptr) return cudaSuccess;
+  TnProblem t;
+  memset(&t, 0, sizeof(t));
+  t.P = P; t.Q = Q;
+  for (const TnPair& p : pairs) t.pair[t.npairs++] = p;
+  return run_tn(t, partial, out, 0, st);
 }
 
 // deterministic column sums: out[c] (+)= sum_r X[r, c].  grid (column blocks of 32, row splits): every CTA sums its
@@ -295,15 +302,72 @@ __device__ __forceinline__ size_t slab1(const BwdCtx& c, int z, int k, int width
   return ((size_t)z * (c.L + 1) + k) * c.B * width;
 }
 
-__global__ void bwd_e1_kernel(const BwdCtx c) {
-  const size_t total = (size_t)2 * c.B * c.S;
+// Grid-stride loop over the (direction z, sequence b, column) elements of step c.k, columns fastest, with the row's
+// step position: f(z, b, column, n = len[b], tpos, orow, alive).
+template <class F>
+__device__ __forceinline__ void for_each_elem(const BwdCtx& c, int width, const F& f) {
+  const size_t total = (size_t)2 * c.B * width;
   for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int s = (int)(i % c.S);
-    const size_t rr = i / c.S;
+    const int col = (int)(i % width);
+    const size_t rr = i / width;
     const int b = (int)(rr % c.B), z = (int)(rr / c.B);
+    const int n = (int)c.len[b];
     int tpos, orow;
     bool alive;
-    step_pos(z, c.k, (int)c.len[b], c.full_pad, tpos, orow, alive);
+    step_pos(z, c.k, n, c.full_pad, tpos, orow, alive);
+    f(z, b, col, n, tpos, orow, alive);
+  }
+}
+
+// E3 of element (z, b, s) at step c.k: DHb -> the carry g for step k-1 (GA + gB; GA = 0 without gates) and DOprod of the
+// backward direction; with the reset gate also Pinit and the reset-gate gradient.  A row that is not alive gets zeros
+// and keeps its carry (0 until the row's last live step).  Returns the carry.  kGates = true (bwd_e3_kernel): c.farnn
+// decides, the carry is stored; false (bwd_e31_kernel): farnn = 0 is known, the gate branches are compiled out and the
+// carry is stored only at k = 0, where it feeds dh0 / dhT.
+template <bool kGates>
+__device__ __forceinline__ float bwd_e3(const BwdCtx& c, int z, int b, int s, float on, bool alive) {
+  const size_t e = (size_t)b * c.S + s;
+  const size_t gi = (size_t)z * c.B * c.S + e;
+  // formed where it is used: inside `z == 1` the index is uniform (fewer registers in bwd_e31_kernel)
+  const auto sl = [&] { return slab(c, z, c.k, c.S) + e; };
+  const int gw = c.S * c.farnn;
+  const bool reset = kGates && c.farnn == 2;
+  if (!alive) {
+    const float g = c.g[gi];
+    if (z == 1) c.DOprod[sl()] = 0.f;
+    if (reset) {
+      c.Pinit[sl()] = 0.f;
+      c.DZR[slab(c, z, c.k, gw) + (size_t)b * gw + c.S + s] = 0.f;
+      if (c.DRop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DRop[z], (size_t)b * c.ldS + s, c.da_plane, 0.f);
+    }
+    return g;
+  }
+  const float dhb = c.DHb[gi];
+  const float hk = kGates ? c.hst_save[slab1(c, z, c.k, c.S) + e] : 0.f;   // without gates: loaded below, z = 1 only
+  const float hinit = z == 0 ? c.h0[s] : c.hT[s];
+  float rt = 1.f;
+  if (reset) rt = c.rsave[sl()];
+  const float htil = reset ? (1.f - rt) * hinit + rt * hk : hk;
+  float dht = dhb;
+  if (z == 1) {
+    dht = dhb * on;
+    c.DOprod[sl()] = dhb * (kGates ? htil : c.hst_save[slab1(c, z, c.k, c.S) + e]);
+  }
+  float gB = dht;
+  if (reset) {
+    gB = dht * rt;
+    c.Pinit[sl()] = dht * (1.f - rt);
+    const float drpre = dht * (hk - hinit) * rt * (1.f - rt) * c.kappa;
+    c.DZR[slab(c, z, c.k, gw) + (size_t)b * gw + c.S + s] = drpre;
+    if (c.DRop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DRop[z], (size_t)b * c.ldS + s, c.da_plane, drpre);
+  }
+  const float g = (kGates ? c.GA[gi] : 0.f) + gB;       // without gates: 0.f + gB, as GA + gB with GA = 0
+  if (kGates || c.k == 0) c.g[gi] = g;
+  return g;
+}
+
+__global__ void bwd_e1_kernel(const BwdCtx c) {
+  for_each_elem(c, c.S, [&](int z, int b, int s, int, int, int orow, bool alive) {
     const size_t e = (size_t)b * c.S + s;
     const size_t sl = slab(c, z, c.k, c.S) + e;
     const int gw = c.S * c.farnn;
@@ -316,7 +380,7 @@ __global__ void bwd_e1_kernel(const BwdCtx c) {
         if (c.DZop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DZop[z], (size_t)b * c.ldS + s, c.da_plane, 0.f);
       }
       c.GA[(size_t)z * c.B * c.S + e] = 0.f;
-      continue;
+      return;
     }
     const float* dout = z == 0 ? c.dalpha : c.dbeta;
     const float G = c.g[(size_t)z * c.B * c.S + e] + (orow >= 0 ? dout[((size_t)b * c.L + orow) * c.S + s] : 0.f);
@@ -339,32 +403,23 @@ __global__ void bwd_e1_kernel(const BwdCtx c) {
     if (z == 0) c.DOprod[sl] = dpre * a;
     if (c.DAop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DAop[z], (size_t)b * c.ldS + s, c.da_plane, da);
     c.GA[(size_t)z * c.B * c.S + e] = gA;
-  }
+  });
 }
 
 // bwd_e2 / bwd_e31 sit between two tcgen05 step GEMMs 35 times per sweep: they are launched with programmatic stream
 // serialization like the GEMMs, let the next GEMM begin its prologue (barrier init, TMEM allocation, descriptor
 // prefetch) right away and wait for the previous GEMM's results themselves.
 __global__ void bwd_e2_kernel(const BwdCtx c) {
-#ifdef RE2NN_HAVE_TC
   griddep_launch_dependents();
   griddep_wait();
-#endif
-  const size_t total = (size_t)2 * c.B * c.R;
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int r = (int)(i % c.R);
-    const size_t rr = i / c.R;
-    const int b = (int)(rr % c.B), z = (int)(rr / c.B);
-    int tpos, orow;
-    bool alive;
-    step_pos(z, c.k, (int)c.len[b], c.full_pad, tpos, orow, alive);
+  for_each_elem(c, c.R, [&](int z, int b, int r, int, int tpos, int, bool alive) {
     const size_t e = (size_t)b * c.R + r;
     const size_t sl = slab(c, z, c.k, c.R) + e;
     if (!alive) {
       c.DU[sl] = 0.f;
       c.Qs[sl] = 0.f;
       if (c.DUop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DUop[z], (size_t)b * c.ldR + r, c.du_plane, 0.f);
-      continue;
+      return;
     }
     const size_t vrow = c.v_mode == RE2NN_V_TOKEN ? (size_t)c.x[(size_t)b * c.Lpad + tpos] : (size_t)b * c.Lpad + tpos;
     const float v = c.vtab[vrow * c.R + r];
@@ -375,98 +430,35 @@ __global__ void bwd_e2_kernel(const BwdCtx c) {
     c.Qs[sl] = u * v;
     const float dv = dq * u;
     if (dv != 0.f) atomicAdd(c.dvtab + vrow * c.R + r, dv);
-  }
+  });
 }
 
 __global__ void bwd_e3_kernel(const BwdCtx c) {
-  const size_t total = (size_t)2 * c.B * c.S;
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int s = (int)(i % c.S);
-    const size_t rr = i / c.S;
-    const int b = (int)(rr % c.B), z = (int)(rr / c.B);
-    int tpos, orow;
-    bool alive;
-    step_pos(z, c.k, (int)c.len[b], c.full_pad, tpos, orow, alive);
-    const size_t e = (size_t)b * c.S + s;
-    const size_t sl = slab(c, z, c.k, c.S) + e;
-    const int gw = c.S * c.farnn;
-    if (!alive) {   // g keeps whatever it had (0 until the row's last live step)
-      if (z == 1) c.DOprod[sl] = 0.f;
-      if (c.farnn == 2) {
-        c.Pinit[sl] = 0.f;
-        c.DZR[slab(c, z, c.k, gw) + (size_t)b * gw + c.S + s] = 0.f;
-        if (c.DRop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DRop[z], (size_t)b * c.ldS + s, c.da_plane, 0.f);
-      }
-      continue;
-    }
-    const float dhb = c.DHb[(size_t)z * c.B * c.S + e];
-    const float on = c.o[s];
-    const float hk = c.hst_save[slab1(c, z, c.k, c.S) + e];
-    const float hinit = z == 0 ? c.h0[s] : c.hT[s];
-    float rt = 1.f;
-    if (c.farnn == 2) rt = c.rsave[sl];
-    const float htil = c.farnn == 2 ? (1.f - rt) * hinit + rt * hk : hk;
-    float dht = dhb;
-    if (z == 1) {
-      dht = dhb * on;
-      c.DOprod[sl] = dhb * htil;
-    }
-    float gB = dht;
-    if (c.farnn == 2) {
-      gB = dht * rt;
-      c.Pinit[sl] = dht * (1.f - rt);
-      const float drpre = dht * (hk - hinit) * rt * (1.f - rt) * c.kappa;
-      c.DZR[slab(c, z, c.k, gw) + (size_t)b * gw + c.S + s] = drpre;
-      if (c.DRop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DRop[z], (size_t)b * c.ldS + s, c.da_plane, drpre);
-    }
-    c.g[(size_t)z * c.B * c.S + e] = c.GA[(size_t)z * c.B * c.S + e] + gB;
-  }
+  for_each_elem(c, c.S, [&](int z, int b, int s, int, int, int, bool alive) {
+    bwd_e3<true>(c, z, b, s, c.o[s], alive);
+  });
 }
 
 // farnn = 0: E3 of step k and E1 of step k-1 touch the same element and nothing runs between them (no gate GEMM), so
 // they are one launch: the carry g stays in a register, the GA / g round trip disappears.  Same arithmetic, same order.
 __global__ void bwd_e31_kernel(const BwdCtx c) {
-#ifdef RE2NN_HAVE_TC
   griddep_launch_dependents();
   griddep_wait();
-#endif
-  const size_t total = (size_t)2 * c.B * c.S;
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int s = (int)(i % c.S);
-    const size_t rr = i / c.S;
-    const int b = (int)(rr % c.B), z = (int)(rr / c.B);
-    const int n = (int)c.len[b];
-    int tpos, orow;
-    bool alive;
-    step_pos(z, c.k, n, c.full_pad, tpos, orow, alive);
-    const size_t e = (size_t)b * c.S + s;
-    const size_t gi = (size_t)z * c.B * c.S + e;
+  for_each_elem(c, c.S, [&](int z, int b, int s, int n, int tpos, int orow, bool alive) {
     const float on = c.o[s];
-    // ---- E3 of step k
-    float g;
-    if (!alive) {
-      g = c.g[gi];                       // keeps whatever it had (0 until the row's last live step)
-      if (z == 1) c.DOprod[slab(c, z, c.k, c.S) + e] = 0.f;
-    } else {
-      const float dhb = c.DHb[gi];
-      g = dhb;
-      if (z == 1) {
-        g = dhb * on;
-        c.DOprod[slab(c, z, c.k, c.S) + e] = dhb * c.hst_save[slab1(c, z, c.k, c.S) + e];
-      }
-      g = 0.f + g;                       // the carry is GA + gB with GA = 0 without gates
-      if (c.k == 0) c.g[gi] = g;         // the final carry feeds dh0 / dhT
-    }
-    if (c.k == 0) continue;
-    // ---- E1 of step k-1
+    const float g = bwd_e3<false>(c, z, b, s, on, alive);
+    if (c.k == 0) return;
+    // ---- E1 of step k-1, without gates.  Written out here rather than shared with bwd_e1_kernel: a shared device
+    // helper compiled to 30-32 registers for this kernel instead of 28.
     const int k1 = c.k - 1;
     step_pos(z, k1, n, c.full_pad, tpos, orow, alive);
+    const size_t e = (size_t)b * c.S + s;
     const size_t sl = slab(c, z, k1, c.S) + e;
     if (!alive) {
       c.DA[sl] = 0.f;
       if (c.DAop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DAop[z], (size_t)b * c.ldS + s, c.da_plane, 0.f);
       if (z == 0) c.DOprod[sl] = 0.f;
-      continue;
+      return;
     }
     const float* dout = z == 0 ? c.dalpha : c.dbeta;
     const float G = g + (orow >= 0 ? dout[((size_t)b * c.L + orow) * c.S + s] : 0.f);
@@ -477,26 +469,19 @@ __global__ void bwd_e31_kernel(const BwdCtx c) {
     c.DA[sl] = da;
     if (z == 0) c.DOprod[sl] = dpre * a;
     if (c.DAop[0]) OperandFmt<RE2NN_PREC_TF32X3>::store(c.DAop[z], (size_t)b * c.ldS + s, c.da_plane, da);
-  }
+  });
 }
 
 // dgtab[token] += [dz | dr] of this step (after the gate slab is complete)
 __global__ void bwd_gate_scatter_kernel(const BwdCtx c) {
   const int gw = c.S * c.farnn;
-  const size_t total = (size_t)2 * c.B * gw;
-  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
-    const int col = (int)(i % gw);
-    const size_t rr = i / gw;
-    const int b = (int)(rr % c.B), z = (int)(rr / c.B);
-    int tpos, orow;
-    bool alive;
-    step_pos(z, c.k, (int)c.len[b], c.full_pad, tpos, orow, alive);
-    if (!alive) continue;
+  for_each_elem(c, gw, [&](int z, int b, int col, int, int tpos, int, bool alive) {
+    if (!alive) return;
     const float v = c.DZR[slab(c, z, c.k, gw) + (size_t)b * gw + col];
-    if (v == 0.f) continue;
+    if (v == 0.f) return;
     const size_t vrow = c.v_mode == RE2NN_V_TOKEN ? (size_t)c.x[(size_t)b * c.Lpad + tpos] : (size_t)b * c.Lpad + tpos;
     atomicAdd(c.dgtab + vrow * gw + col, v);
-  }
+  });
 }
 
 // dhT += sum_b dbeta[b, n_b - 1, :]   (beta_n = hT is emitted directly)
@@ -537,7 +522,6 @@ struct EpiTokenBwd {
 // The two GEMMs of every BPTT step (dq = DA @ S, dhbar = DU @ S^T + DA @ W^T) run on the tensor cores in 3xTF32
 // (fp32-grade products, 8-bit exponent: safe for gradients of any magnitude) when tcgen05 is there.
 static bool g_bwd_tc = true;
-extern "C" int re2nn_has_tcgen05(void);
 static bool bwd_uses_tc() { return g_bwd_tc && re2nn_has_tcgen05() != 0; }
 
 static size_t bwd_carve(const re2nn_backward_args& a, char* base, BwdCtx* c, float** draw, float** partial,
@@ -618,6 +602,53 @@ static cudaError_t launch_pdl(void (*kernel)(BwdCtx), int grid, cudaStream_t st,
 
 static int grid_for(size_t total) { return (int)std::min<size_t>((total + 255) / 256, (size_t)sm_count() * 16); }
 
+// One GEMM of a BPTT step: on tcgen05 in 3xTF32 when it has a launch plan (whose tensor maps name the operand-format
+// copies), else on CUDA cores over the fp32 operands of `g`.
+static cudaError_t step_gemm(const GemmProblem& g, const EpiStore2& epi, const TcLaunch* tl, cudaStream_t st) {
+  if (tl) return launch_tc_gemm<RE2NN_PREC_TF32X3>(g, epi, tl, st);
+  return launch_simt_gemm(g, epi, ALoadPlain{}, st);
+}
+
+// Label-score backward: undo the priority layer (draw = dscores @ P^T into draw_ws; draw = dscores without one), then
+// dAB = draw @ C_mat -> dalpha = dAB * beta, dbeta = dAB * alpha (EpiDAB).  Given operand-format buffers for draw and
+// C_mat^T, the second GEMM runs on tcgen05 in 3xTF32: it is tiny (K = C), what matters is the coalesced epilogue over
+// alpha / beta / dalpha / dbeta.  Without them it runs on CUDA cores.  draw_out (optional) receives draw.
+static int label_scores_bwd(const float* dscores, const float* priority_mat, float* draw_ws, const float* C_mat, int C,
+                            const EpiDAB& edab, int B, void* draw_op, void* cmat_op, cudaStream_t st,
+                            const float** draw_out) {
+  const int M = B * edab.L, S = edab.S;
+  const float* draw = dscores;
+  GemmProblem g;
+  if (priority_mat) {
+    memset(&g, 0, sizeof(g));
+    g.M = M; g.N = C; g.nseg = 1; g.ndir = 1;
+    g.seg[0][0] = GemmSeg{dscores, priority_mat, C, C, C, 1, 0, 0};
+    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{draw_ws, C, nullptr}, ALoadPlain{}, st));
+    draw = draw_ws;
+  }
+  memset(&g, 0, sizeof(g));
+  g.M = M; g.N = S; g.nseg = 1; g.ndir = 1;
+  if (draw_op) {
+    constexpr int P = RE2NN_PREC_TF32X3;
+    const int ldc = operand_ld(P, C);
+    const size_t pa = (size_t)M * ldc, pb = (size_t)S * ldc;
+    convert_weight_kernel<P><<<(unsigned)std::min<size_t>((pa + 255) / 256, (size_t)sm_count() * 32), 256, 0, st>>>(
+        draw, M, C, C, 0, draw_op, ldc, pa, 0);
+    RE2NN_LAUNCH_CHECK();
+    convert_weight_kernel<P><<<(unsigned)((pb + 255) / 256), 256, 0, st>>>(C_mat, S, C, S, 1, cmat_op, ldc, pb, 0);
+    RE2NN_LAUNCH_CHECK();
+    g.seg[0][0] = GemmSeg{draw_op, cmat_op, ldc, ldc, C, 1, pa, pb};
+    std::unique_ptr<TcLaunch> tl(new TcLaunch);
+    if (int rc = tc_make_launch<P>(g, tl.get())) return rc;
+    RE2NN_CUDA((launch_tc_gemm<P>(g, edab, tl.get(), st)));
+  } else {
+    g.seg[0][0] = GemmSeg{draw, C_mat, C, S, C, 0, 0, 0};
+    RE2NN_CUDA(launch_simt_gemm(g, edab, ALoadPlain{}, st));
+  }
+  if (draw_out) *draw_out = draw;
+  return 0;
+}
+
 static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
   BwdCtx c;
   float *draw_ws, *partial, *dalpha, *dbeta;
@@ -635,62 +666,33 @@ static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
   c.hst_save = a.hst_save; c.u_save = a.u_save; c.a_save = a.a_save; c.zsave = a.zsave; c.rsave = a.rsave;
   c.dvtab = a.dvtab;
 
-  // 0. undo the priority layer: draw = dscores @ P^T
-  const float* draw = a.dscores;
-  GemmProblem g;
   const bool direct = a.dalpha_in != nullptr && a.dbeta_in != nullptr;   // caller differentiated its own score stage
   if (direct) {
     c.dalpha = a.dalpha_in; c.dbeta = a.dbeta_in;
     dbeta = const_cast<float*>(a.dbeta_in);
-  }
-  if (!direct && a.priority_mat) {
-    memset(&g, 0, sizeof(g));
-    g.M = (int)M; g.N = C; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{a.dscores, a.priority_mat, C, C, C, 1, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{draw_ws, C, nullptr}, ALoadPlain{}, st));
-    draw = draw_ws;
-  }
-  // 1. dAB = draw @ C  ->  dAlpha, dBeta
-  if (!direct) {
-    const EpiDAB edab{a.alpha, a.beta, a.lengths, dalpha, dbeta, L, S, a.full_pad};
-    if (tc && c.DrawOp != nullptr) {
-      // 3xTF32 on tcgen05: the GEMM is tiny (K = C), what matters is the coalesced epilogue over alpha / beta / dalpha / dbeta
-      constexpr int P = RE2NN_PREC_TF32X3;
-      const int ldc = operand_ld(P, C);
-      const size_t pa = M * ldc, pb = (size_t)S * ldc;
-      convert_weight_kernel<P><<<(unsigned)std::min<size_t>((M * ldc + 255) / 256, (size_t)sm_count() * 32), 256, 0, st>>>(
-          draw, (int)M, C, C, 0, c.DrawOp, ldc, pa, 0);
-      RE2NN_LAUNCH_CHECK();
-      convert_weight_kernel<P><<<(unsigned)(((size_t)S * ldc + 255) / 256), 256, 0, st>>>(a.C_mat, S, C, S, 1, c.CmatOp, ldc, pb, 0);
-      RE2NN_LAUNCH_CHECK();
-      memset(&g, 0, sizeof(g));
-      g.M = (int)M; g.N = S; g.nseg = 1; g.ndir = 1;
-      g.seg[0][0] = GemmSeg{c.DrawOp, c.CmatOp, ldc, ldc, C, 1, pa, pb};
-      std::unique_ptr<TcLaunch> tl(new TcLaunch);
-      if (int rc = tc_make_launch<P>(g, tl.get())) return rc;
-      RE2NN_CUDA((launch_tc_gemm<P>(g, edab, tl.get(), st)));
-    } else {
-      memset(&g, 0, sizeof(g));
-      g.M = (int)M; g.N = S; g.nseg = 1; g.ndir = 1;
-      g.seg[0][0] = GemmSeg{draw, a.C_mat, C, S, C, 0, 0, 0};
-      RE2NN_CUDA(launch_simt_gemm(g, edab, ALoadPlain{}, st));
+  } else {
+    // 1. dscores -> dAlpha, dBeta (on tcgen05 when the carve made operand-format buffers for it)
+    const float* draw;
+    if (int rc = label_scores_bwd(a.dscores, a.priority_mat, draw_ws, a.C_mat, C,
+                                  EpiDAB{a.alpha, a.beta, a.lengths, dalpha, dbeta, L, S, a.full_pad}, B, c.DrawOp,
+                                  c.CmatOp, st, &draw))
+      return rc;
+    // 2. dC = draw^T @ (alpha * beta) over the valid positions: run_tn forms the masked product from Y2 / mask_len
+    if (a.dC) {
+      TnProblem t;
+      memset(&t, 0, sizeof(t));
+      t.P = C; t.Q = S; t.npairs = 1;
+      t.pair[0] = TnPair{draw, a.alpha, C, S, M};
+      t.Y2 = a.beta;
+      if (!a.full_pad) { t.mask_len = a.lengths; t.mask_L = L; }
+      RE2NN_CUDA(run_tn(t, partial, a.dC, 0, st));
     }
-  }
-  // 2. dC = draw^T @ (alpha * beta)   (the tensor-core kernel forms the masked product itself: Y2 / mask_len)
-  if (!direct && a.dC) {
-    TnProblem t;
-    memset(&t, 0, sizeof(t));
-    t.P = C; t.Q = S; t.npairs = 1;
-    t.pair[0] = TnPair{draw, a.alpha, C, S, M};
-    t.Y2 = a.beta;
-    if (!a.full_pad) { t.mask_len = a.lengths; t.mask_L = L; }
-    RE2NN_CUDA(run_tn(t, partial, a.dC, 0, YLoadAlphaBeta{a.beta, a.lengths, L, a.full_pad}, st));
   }
   // 3. sweep
   RE2NN_CUDA(cudaMemsetAsync(c.g, 0, (size_t)2 * B * S * 4, st));
   RE2NN_CUDA(cudaMemsetAsync(a.dvtab, 0, (size_t)a.table_rows * R * 4, st));
   if (a.farnn >= 1) RE2NN_CUDA(cudaMemsetAsync(c.dgtab, 0, (size_t)a.table_rows * gw * 4, st));
-  std::unique_ptr<TcLaunch> tq, th, tg;
+  std::unique_ptr<TcLaunch> tq, th, tg;      // launch plans of the three step GEMMs on tcgen05 (none: CUDA cores)
   if (tc) {
     // K-major operand-format copies of S1, S2, W (the same layouts the forward uses) + the tensor maps of the two
     // step GEMMs; the A operands are the per-step DAop / DUop buffers, rewritten every step
@@ -730,6 +732,7 @@ static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
       if (int rc = tc_make_launch<P>(gg, tg.get())) return rc;
     }
   }
+  GemmProblem g;
   for (int k = L - 1; k >= 0; --k) {
     c.k = k;
     if (k == L - 1 || a.farnn >= 1) {      // without gates E1 of the later steps rides in bwd_e31_kernel
@@ -741,10 +744,7 @@ static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
     g.M = B; g.N = R; g.nseg = 1; g.ndir = 2;
     for (int z = 0; z < 2; ++z)
       g.seg[z][0] = GemmSeg{c.DA + ((size_t)z * L + k) * B * S, z == 0 ? a.S2 : a.S1, S, R, S, 0, 0, 0};
-    if (tc)
-      RE2NN_CUDA((launch_tc_gemm<RE2NN_PREC_TF32X3>(g, EpiStore2{{c.DQ, c.DQ + (size_t)B * R}, R, 0}, tq.get(), st)));
-    else
-      RE2NN_CUDA(launch_simt_gemm(g, EpiStore2{{c.DQ, c.DQ + (size_t)B * R}, R, 0}, ALoadPlain{}, st));
+    RE2NN_CUDA(step_gemm(g, EpiStore2{{c.DQ, c.DQ + (size_t)B * R}, R, 0}, tq.get(), st));
     RE2NN_CUDA(launch_pdl(bwd_e2_kernel, grid_for((size_t)2 * B * R), st, c));
     // dhb = DU[k] @ S1^T + DA[k] @ W^T (fwd) | DU[k] @ S2^T + DA[k] @ W (bwd)
     memset(&g, 0, sizeof(g));
@@ -753,10 +753,7 @@ static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
       g.seg[z][0] = GemmSeg{c.DU + ((size_t)z * L + k) * B * R, z == 0 ? a.S1 : a.S2, R, R, R, 1, 0, 0};
       g.seg[z][1] = GemmSeg{c.DA + ((size_t)z * L + k) * B * S, a.W, S, S, S, z == 0 ? 1 : 0, 0, 0};
     }
-    if (tc)
-      RE2NN_CUDA((launch_tc_gemm<RE2NN_PREC_TF32X3>(g, EpiStore2{{c.DHb, c.DHb + (size_t)B * S}, S, 0}, th.get(), st)));
-    else
-      RE2NN_CUDA(launch_simt_gemm(g, EpiStore2{{c.DHb, c.DHb + (size_t)B * S}, S, 0}, ALoadPlain{}, st));
+    RE2NN_CUDA(step_gemm(g, EpiStore2{{c.DHb, c.DHb + (size_t)B * S}, S, 0}, th.get(), st));
     if (a.farnn == 0) RE2NN_CUDA(launch_pdl(bwd_e31_kernel, grid_for((size_t)2 * B * S), st, c));
     else {
       bwd_e3_kernel<<<grid_for((size_t)2 * B * S), 256, 0, st>>>(c);
@@ -771,10 +768,7 @@ static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
         g.seg[z][0] = GemmSeg{dzr, a.Wss1, gw, S, S, 1, 0, 0};
         if (a.farnn == 2) g.seg[z][1] = GemmSeg{dzr + S, a.Wss2, gw, S, S, 1, 0, 0};
       }
-      if (tc)
-        RE2NN_CUDA((launch_tc_gemm<RE2NN_PREC_TF32X3>(g, EpiStore2{{c.g, c.g + (size_t)B * S}, S, 1}, tg.get(), st)));
-      else
-        RE2NN_CUDA(launch_simt_gemm(g, EpiStore2{{c.g, c.g + (size_t)B * S}, S, 1}, ALoadPlain{}, st));
+      RE2NN_CUDA(step_gemm(g, EpiStore2{{c.g, c.g + (size_t)B * S}, S, 1}, tg.get(), st));
       bwd_gate_scatter_kernel<<<grid_for((size_t)2 * B * gw), 256, 0, st>>>(c);
       RE2NN_LAUNCH_CHECK();
     }
@@ -785,60 +779,20 @@ static int run_backward(const re2nn_backward_args& a, cudaStream_t st) {
   const float* Hb1 = a.hbar_save + (size_t)(L + 1) * B * S;
   const float *DA0 = c.DA, *DA1 = c.DA + rows1 * S, *DU0 = c.DU, *DU1 = c.DU + rows1 * R;
   const float *Q0 = c.Qs, *Q1 = c.Qs + rows1 * R;
-  TnProblem t;
-  if (a.dS1) {   // fwd: hbar^T du ; bwd: da^T q
-    memset(&t, 0, sizeof(t));
-    t.P = S; t.Q = R; t.npairs = 2;
-    t.pair[0] = TnPair{Hb0, DU0, S, R, rows1};
-    t.pair[1] = TnPair{DA1, Q1, S, R, rows1};
-    RE2NN_CUDA(run_tn(t, partial, a.dS1, 0, YLoadPlain{}, st));
-  }
-  if (a.dS2) {   // fwd: da^T q ; bwd: hbar^T du
-    memset(&t, 0, sizeof(t));
-    t.P = S; t.Q = R; t.npairs = 2;
-    t.pair[0] = TnPair{DA0, Q0, S, R, rows1};
-    t.pair[1] = TnPair{Hb1, DU1, S, R, rows1};
-    RE2NN_CUDA(run_tn(t, partial, a.dS2, 0, YLoadPlain{}, st));
-  }
-  if (a.dW) {    // fwd: hbar^T da ; bwd: da^T hbar
-    memset(&t, 0, sizeof(t));
-    t.P = S; t.Q = S; t.npairs = 2;
-    t.pair[0] = TnPair{Hb0, DA0, S, S, rows1};
-    t.pair[1] = TnPair{DA1, Hb1, S, S, rows1};
-    RE2NN_CUDA(run_tn(t, partial, a.dW, 0, YLoadPlain{}, st));
-  }
+  // dS1 = fwd hbar^T du + bwd da^T q ; dS2 = fwd da^T q + bwd hbar^T du ; dW = fwd hbar^T da + bwd da^T hbar
+  RE2NN_CUDA(tn(a.dS1, S, R, {{Hb0, DU0, S, R, rows1}, {DA1, Q1, S, R, rows1}}, partial, st));
+  RE2NN_CUDA(tn(a.dS2, S, R, {{DA0, Q0, S, R, rows1}, {Hb1, DU1, S, R, rows1}}, partial, st));
+  RE2NN_CUDA(tn(a.dW, S, S, {{Hb0, DA0, S, S, rows1}, {DA1, Hb1, S, S, rows1}}, partial, st));
   if (a.farnn >= 1) {
     const float* Hs0 = a.hst_save;
     const float* Hs1 = a.hst_save + (size_t)(L + 1) * B * S;
     const float* Z0 = c.DZR;
     const float* Z1 = c.DZR + rows1 * gw;
-    if (a.dWss1) {
-      memset(&t, 0, sizeof(t));
-      t.P = S; t.Q = S; t.npairs = 2;
-      t.pair[0] = TnPair{Hs0, Z0, S, gw, rows1};
-      t.pair[1] = TnPair{Hs1, Z1, S, gw, rows1};
-      RE2NN_CUDA(run_tn(t, partial, a.dWss1, 0, YLoadPlain{}, st));
-    }
-    if (a.farnn == 2 && a.dWss2) {
-      memset(&t, 0, sizeof(t));
-      t.P = S; t.Q = S; t.npairs = 2;
-      t.pair[0] = TnPair{Hs0, Z0 + S, S, gw, rows1};
-      t.pair[1] = TnPair{Hs1, Z1 + S, S, gw, rows1};
-      RE2NN_CUDA(run_tn(t, partial, a.dWss2, 0, YLoadPlain{}, st));
-    }
+    RE2NN_CUDA(tn(a.dWss1, S, S, {{Hs0, Z0, S, gw, rows1}, {Hs1, Z1, S, gw, rows1}}, partial, st));
+    if (a.farnn == 2) RE2NN_CUDA(tn(a.dWss2, S, S, {{Hs0, Z0 + S, S, gw, rows1}, {Hs1, Z1 + S, S, gw, rows1}}, partial, st));
     // token-side gate parameters through the gate table: Wrs = vtab^T dgtab, bs = colsum(dgtab), dvtab += dgtab Wrs^T
-    if (a.dWrs1) {
-      memset(&t, 0, sizeof(t));
-      t.P = R; t.Q = S; t.npairs = 1;
-      t.pair[0] = TnPair{a.vtab, c.dgtab, R, gw, (size_t)a.table_rows};
-      RE2NN_CUDA(run_tn(t, partial, a.dWrs1, 0, YLoadPlain{}, st));
-    }
-    if (a.farnn == 2 && a.dWrs2) {
-      memset(&t, 0, sizeof(t));
-      t.P = R; t.Q = S; t.npairs = 1;
-      t.pair[0] = TnPair{a.vtab, c.dgtab + S, R, gw, (size_t)a.table_rows};
-      RE2NN_CUDA(run_tn(t, partial, a.dWrs2, 0, YLoadPlain{}, st));
-    }
+    RE2NN_CUDA(tn(a.dWrs1, R, S, {{a.vtab, c.dgtab, R, gw, (size_t)a.table_rows}}, partial, st));
+    if (a.farnn == 2) RE2NN_CUDA(tn(a.dWrs2, R, S, {{a.vtab, c.dgtab + S, R, gw, (size_t)a.table_rows}}, partial, st));
     if (a.dbs1) RE2NN_CUDA(colsum_rows(c.dgtab, a.table_rows, S, gw, a.dbs1, 0, st, partial));
     if (a.farnn == 2 && a.dbs2) RE2NN_CUDA(colsum_rows(c.dgtab + S, a.table_rows, S, gw, a.dbs2, 0, st, partial));
     memset(&g, 0, sizeof(g));
@@ -906,10 +860,7 @@ int re2nn_gemm_tn(int path, int P, int Q, const float* X0, const float* Y0, int 
   t.Y2 = Y2;
   t.mask_len = mask_len;
   t.mask_L = mask_len ? mask_L : 0;
-  cudaStream_t st = (cudaStream_t)stream;
-  float* partial = (float*)ws;
-  if (Y2) RE2NN_CUDA(run_tn(t, partial, C, 0, YLoadAlphaBeta{Y2, mask_len, mask_len ? mask_L : 1, mask_len ? 0 : 1}, st, path));
-  else RE2NN_CUDA(run_tn(t, partial, C, 0, YLoadPlain{}, st, path));
+  RE2NN_CUDA(run_tn(t, (float*)ws, C, 0, (cudaStream_t)stream, path));
   return 0;
 }
 
@@ -937,21 +888,8 @@ int re2nn_label_scores_backward(const float* dscores, const float* alpha, const 
                                 int full_pad, float* dalpha, float* dbeta, float* ws, void* stream) {
   RE2NN_CHECK(dscores && alpha && beta && lengths && C_mat && dalpha && dbeta, "label_scores_backward: null tensor");
   RE2NN_CHECK(!priority_mat || ws, "label_scores_backward: priority needs a workspace");
-  cudaStream_t st = (cudaStream_t)stream;
-  const float* draw = dscores;
-  GemmProblem g;
-  if (priority_mat) {
-    memset(&g, 0, sizeof(g));
-    g.M = B * L; g.N = C; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{dscores, priority_mat, C, C, C, 1, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{ws, C, nullptr}, ALoadPlain{}, st));
-    draw = ws;
-  }
-  memset(&g, 0, sizeof(g));
-  g.M = B * L; g.N = S; g.nseg = 1; g.ndir = 1;
-  g.seg[0][0] = GemmSeg{draw, C_mat, C, S, C, 0, 0, 0};
-  RE2NN_CUDA(launch_simt_gemm(g, EpiDAB{alpha, beta, lengths, dalpha, dbeta, L, S, full_pad}, ALoadPlain{}, st));
-  return 0;
+  return label_scores_bwd(dscores, priority_mat, ws, C_mat, C, EpiDAB{alpha, beta, lengths, dalpha, dbeta, L, S, full_pad},
+                          B, nullptr, nullptr, (cudaStream_t)stream, nullptr);
 }
 
 size_t re2nn_token_table_backward_workspace(int rows, int D, int R) {
@@ -978,13 +916,7 @@ int re2nn_token_table_backward(const float* dvtab, const float* V_embed, const f
   RE2NN_CUDA(launch_simt_gemm(g, EpiTokenBwd{dvtab, V_embed, beta_vec, dV_embed, dbeta_prod, dGpre, R, additional_nonlinear},
                               ALoadPlain{}, st));
   if (dbeta_vec) RE2NN_CUDA(colsum_rows(dbeta_prod, rows, R, R, dbeta_vec, 0, st));
-  if (dG) {
-    TnProblem t;
-    memset(&t, 0, sizeof(t));
-    t.P = D; t.Q = R; t.npairs = 1;
-    t.pair[0] = TnPair{E, dGpre, D, R, (size_t)rows};
-    RE2NN_CUDA(run_tn(t, partial, dG, 0, YLoadPlain{}, st));
-  }
+  RE2NN_CUDA(tn(dG, D, R, {{E, dGpre, D, R, (size_t)rows}}, partial, st));
   if (dE) {
     memset(&g, 0, sizeof(g));
     g.M = rows; g.N = D; g.nseg = 1; g.ndir = 1;

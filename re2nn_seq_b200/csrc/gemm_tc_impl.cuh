@@ -19,8 +19,6 @@
 
 #include "gemm_common.cuh"
 
-#define RE2NN_HAVE_TC 1
-
 namespace re2nn {
 
 constexpr int kTcMaxMaps = 16;

@@ -17,9 +17,9 @@
 namespace re2nn {
 
 struct TnPair { const float* X; const float* Y; int ldx, ldy; size_t rows; };
-// Y2 (optional, tensor-core kernel only): the right operand is Y * Y2 element-wise (same layout as pair 0's Y), and
-// with mask_len row m = b * mask_L + t only counts when t < mask_len[b] -- dC = draw^T (alpha * beta) over the valid
-// positions without materialising the product (pad rows of alpha / beta are undefined, possibly NaN).
+// Y2 (optional, single pair): the right operand is Y * Y2 element-wise (same layout as pair 0's Y), and with mask_len
+// row m = b * mask_L + t only counts when t < mask_len[b] -- dC = draw^T (alpha * beta) over the valid positions
+// without materialising the product (pad rows of alpha / beta are undefined, possibly NaN).  Both kernels form it.
 struct TnProblem { int P, Q, npairs; TnPair pair[2]; const float* Y2; const int64_t* mask_len; int mask_L; };
 
 constexpr int kTnLoaderWarps = 8;
@@ -46,7 +46,6 @@ __host__ __device__ inline void tn_split_range(size_t rows, int split, int nspli
   *r1 = b < rows ? b : rows;
 }
 
-#ifdef RE2NN_HAVE_TC
 __global__ void __launch_bounds__(kTnThreads, 1) tn_tc_kernel(const TnProblem prob, float* __restrict__ partial, const int bn,
                                                               const int stages) {
   constexpr int kATile = 128 * 128;                          // one plane of the X^T tile: 128 output rows x 128 bytes
@@ -309,6 +308,5 @@ inline cudaError_t launch_tn_tc(const TnProblem& prob, float* partial, const TnT
   tn_tc_kernel<<<grid, kTnThreads, pl.smem, st>>>(prob, partial, pl.bn, pl.stages);
   return cudaGetLastError();
 }
-#endif
 
 }  // namespace re2nn

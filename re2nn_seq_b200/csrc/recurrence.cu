@@ -393,8 +393,6 @@ static int run_recurrence(const re2nn_recurrence_args& a, cudaStream_t st) {
 
 using namespace re2nn;
 
-extern "C" int re2nn_has_tcgen05(void);
-
 // (alpha * beta) in operand format for the tcgen05 score GEMM; rows past the length are zero.
 // One warp per (sequence, position) row: the row index math happens once per warp, lanes sweep the S columns
 // with 16-byte loads when the row pitch allows it.
@@ -505,9 +503,7 @@ int re2nn_debug_set_tc_timeline(unsigned long long* device_buf) {
 
 int re2nn_debug_set_tc_cta_group(int cta_group) {
   RE2NN_CHECK(cta_group >= 0 && cta_group <= 2, "debug_set_tc_cta_group: expected 0, 1 or 2");
-#ifdef RE2NN_HAVE_TC
   g_tc_force_cg = cta_group;
-#endif
   return 0;
 }
 
@@ -807,12 +803,8 @@ int re2nn_label_scores(const float* alpha, const float* beta, const int64_t* len
 }  // extern "C"
 
 extern "C" int re2nn_has_tcgen05(void) {
-#ifdef RE2NN_HAVE_TC
   int dev = 0, major = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) return 0;
   if (cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev) != cudaSuccess) return 0;
   return major == 10;
-#else
-  return 0;
-#endif
 }

@@ -8,7 +8,7 @@ reference is X.double().T @ Y.double() on the GPU.  Errors are reported two ways
 scale every accumulated product and every rounding of a partial sum is bounded by, so it survives cancellation.
 
 Training level: a shape at which every weight gradient of the backward runs on tcgen05, gradients against the float64
-autograd oracle."""
+autograd oracle, with the GEMMs of every BPTT step on tcgen05 (the default) and on CUDA cores."""
 import numpy as np
 import pytest
 import torch
@@ -415,3 +415,37 @@ def test_training_gradients_on_tensor_core_backward_vs_fp64_oracle(name, capsys)
         assert d < 5e-6, '%s: tcgen05 vs CUDA cores %.3e' % (k, d)
     for k, e in errs[1].items():
         assert e < max(2e-5, errs[0][k] + 5e-6), '%s: %.3e (CUDA-core weight gradients: %.3e)' % (k, e, errs[0][k])
+
+
+# Bounds of the CUDA-core BPTT test, from its measurements on a B200: every gradient within 1.8e-5 of the oracle except
+# hT and wildcard_mat of the farnn = 0 CRF cases (2.4-3.3e-5: the same parameters the fp32 backward is furthest off on
+# in the test above).  Bounds about 1.3-1.4x above that.
+BPTT_CUDA_TOL = 2.5e-5
+BPTT_CUDA_TOL_LOOSE = {'hT': 4.5e-5, 'wildcard_mat': 4.5e-5}
+
+
+@pytest.mark.parametrize('name', list(TRAIN_CASES))
+def test_training_gradients_on_cuda_core_bptt_vs_fp64_oracle(name, capsys):
+    """The same eight training steps with the GEMMs of every BPTT step on the fp32 CUDA-core kernel instead of tcgen05
+    (re2nn_debug_set_backward_tc(0), bench.py --backward-tc 0).  Loss within 1e-5 of the float64 oracle, every trained
+    gradient within BPTT_CUDA_TOL max-norm relative of it (BPTT_CUDA_TOL_LOOSE for hT and wildcard_mat)."""
+    from re2nn_seq_b200 import _lib
+    sf = TRAIN_CASES[name].get('sf', False)
+    m, args, x, lens, lab, dense_v = _train_case(name, 61 + list(TRAIN_CASES).index(name))
+    dev = lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda()   # noqa: E731
+    try:
+        _lib.check(_lib.fn['re2nn_debug_set_backward_tc'](0), 'backward_tc')
+        if sf:
+            loss, _, _ = m(dev(dense_v), dev(lab), dev(lens), True)
+        else:
+            loss, _, _ = m.forward_local(dev(x), dev(lab), dev(lens), train=True)
+        loss.backward()
+        loss_err, errs = oracle_gradient_errors(m, args, x, lab, lens, loss.item(), dense_v=dense_v)
+    finally:
+        _lib.check(_lib.fn['re2nn_debug_set_backward_tc'](1), 'backward_tc')
+    with capsys.disabled():
+        print('\n%s: CUDA-core BPTT: loss %.1e; gradients vs fp64 oracle (max-norm relative): %s'
+              % (name, loss_err, ', '.join('%s %.2e' % kv for kv in sorted(errs.items()))))
+    assert loss_err < 1e-5
+    for k, e in errs.items():
+        assert e < BPTT_CUDA_TOL_LOOSE.get(k, BPTT_CUDA_TOL), '%s: %.3e' % (k, e)

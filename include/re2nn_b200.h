@@ -311,7 +311,8 @@ int re2nn_label_scores_backward(const float* dscores, const float* alpha, const 
  * replaces get_final_score + its L-step loop (model_decompose_single.py:202-205,263-269;
  * model_onehot.py:346-349,417-426).  Optional PriorityLayer (priority.py:20-30) is applied when
  * priority_mat != NULL: scores <- scores @ priority_mat + priority_bias.  Rows past the length are
- * written as 0.  ws: re2nn_label_scores_workspace() bytes. */
+ * written as 0.  ws: re2nn_label_scores_workspace() bytes.  A precision outside RE2NN_PREC_* fails with
+ * "unknown precision" before any CUDA call (so does re2nn_label_scores_ab). */
 size_t re2nn_label_scores_workspace(int B, int L, int S, int C, int precision, int has_priority);
 int re2nn_label_scores(const float* alpha, const float* beta, const int64_t* lengths,
                        int B, int L, int S, const float* C_mat, int C,

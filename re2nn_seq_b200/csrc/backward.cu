@@ -605,7 +605,7 @@ static int grid_for(size_t total) { return (int)std::min<size_t>((total + 255) /
 // One GEMM of a BPTT step: on tcgen05 in 3xTF32 when it has a launch plan (whose tensor maps name the operand-format
 // copies), else on CUDA cores over the fp32 operands of `g`.
 static cudaError_t step_gemm(const GemmProblem& g, const EpiStore2& epi, const TcLaunch* tl, cudaStream_t st) {
-  if (tl) return launch_tc_gemm<RE2NN_PREC_TF32X3>(g, epi, tl, st);
+  if (tl) return launch_tc_gemm<RE2NN_PREC_TF32X3>(epi, tl, st);
   return launch_simt_gemm(g, epi, ALoadPlain{}, st);
 }
 
@@ -618,16 +618,11 @@ static int label_scores_bwd(const float* dscores, const float* priority_mat, flo
                             const float** draw_out) {
   const int M = B * edab.L, S = edab.S;
   const float* draw = dscores;
-  GemmProblem g;
   if (priority_mat) {
-    memset(&g, 0, sizeof(g));
-    g.M = M; g.N = C; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{dscores, priority_mat, C, C, C, 1, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{draw_ws, C, nullptr}, ALoadPlain{}, st));
+    RE2NN_CUDA(launch_simt_gemm(gemm_problem(M, C, GemmSeg{dscores, priority_mat, C, C, C, 1, 0, 0}),
+                                EpiStore{draw_ws, C, nullptr}, ALoadPlain{}, st));
     draw = draw_ws;
   }
-  memset(&g, 0, sizeof(g));
-  g.M = M; g.N = S; g.nseg = 1; g.ndir = 1;
   if (draw_op) {
     constexpr int P = RE2NN_PREC_TF32X3;
     const int ldc = operand_ld(P, C);
@@ -637,13 +632,12 @@ static int label_scores_bwd(const float* dscores, const float* priority_mat, flo
     RE2NN_LAUNCH_CHECK();
     convert_weight_kernel<P><<<(unsigned)((pb + 255) / 256), 256, 0, st>>>(C_mat, S, C, S, 1, cmat_op, ldc, pb, 0);
     RE2NN_LAUNCH_CHECK();
-    g.seg[0][0] = GemmSeg{draw_op, cmat_op, ldc, ldc, C, 1, pa, pb};
     std::unique_ptr<TcLaunch> tl(new TcLaunch);
-    if (int rc = tc_make_launch<P>(g, tl.get())) return rc;
-    RE2NN_CUDA((launch_tc_gemm<P>(g, edab, tl.get(), st)));
+    if (int rc = tc_make_launch<P>(gemm_problem(M, S, GemmSeg{draw_op, cmat_op, ldc, ldc, C, 1, pa, pb}), tl.get()))
+      return rc;
+    RE2NN_CUDA((launch_tc_gemm<P>(edab, tl.get(), st)));
   } else {
-    g.seg[0][0] = GemmSeg{draw, C_mat, C, S, C, 0, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, edab, ALoadPlain{}, st));
+    RE2NN_CUDA(launch_simt_gemm(gemm_problem(M, S, GemmSeg{draw, C_mat, C, S, C, 0, 0, 0}), edab, ALoadPlain{}, st));
   }
   if (draw_out) *draw_out = draw;
   return 0;
@@ -909,20 +903,14 @@ int re2nn_token_table_backward(const float* dvtab, const float* V_embed, const f
   float* dGpre = (float*)w;
   w += align_up((size_t)rows * R * 4, 256);
   float* partial = (float*)w;
-  GemmProblem g;
-  memset(&g, 0, sizeof(g));
-  g.M = rows; g.N = R; g.nseg = 1; g.ndir = 1;
-  g.seg[0][0] = GemmSeg{E, G, D, R, D, 0, 0, 0};
-  RE2NN_CUDA(launch_simt_gemm(g, EpiTokenBwd{dvtab, V_embed, beta_vec, dV_embed, dbeta_prod, dGpre, R, additional_nonlinear},
+  RE2NN_CUDA(launch_simt_gemm(gemm_problem(rows, R, GemmSeg{E, G, D, R, D, 0, 0, 0}),
+                              EpiTokenBwd{dvtab, V_embed, beta_vec, dV_embed, dbeta_prod, dGpre, R, additional_nonlinear},
                               ALoadPlain{}, st));
   if (dbeta_vec) RE2NN_CUDA(colsum_rows(dbeta_prod, rows, R, R, dbeta_vec, 0, st));
   RE2NN_CUDA(tn(dG, D, R, {{E, dGpre, D, R, (size_t)rows}}, partial, st));
-  if (dE) {
-    memset(&g, 0, sizeof(g));
-    g.M = rows; g.N = D; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{dGpre, G, R, R, R, 1, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{dE, D, nullptr}, ALoadPlain{}, st));
-  }
+  if (dE)
+    RE2NN_CUDA(launch_simt_gemm(gemm_problem(rows, D, GemmSeg{dGpre, G, R, R, R, 1, 0, 0}), EpiStore{dE, D, nullptr},
+                                ALoadPlain{}, st));
   return 0;
 }
 

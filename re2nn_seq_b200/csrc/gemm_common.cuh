@@ -22,6 +22,14 @@ struct GemmProblem {
   int M, N, nseg, ndir;
   GemmSeg seg[2][kMaxSeg];
 };
+// One direction, one segment: C[M x N] = A @ B as `s` lays them out.
+inline GemmProblem gemm_problem(int M, int N, const GemmSeg& s) {
+  GemmProblem g;
+  memset(&g, 0, sizeof(g));
+  g.M = M; g.N = N; g.nseg = 1; g.ndir = 1;
+  g.seg[0][0] = s;
+  return g;
+}
 
 // ---- operand formats ---------------------------------------------------------------------------
 // FP32: float, ld = K.   BF16: __nv_bfloat16, ld = roundup(K, 8).   TF32X3: two float planes (hi, lo).

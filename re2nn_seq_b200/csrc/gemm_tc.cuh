@@ -90,6 +90,31 @@ __global__ void convert_weight_kernel(const float* src, int N, int K, int ld_src
   }
 }
 
+// One operand-format copy of a weight: row n + n_off, column k of buf[buf] = src(k, n) (transpose) or src(n, k), src
+// row-major with leading dimension ld_src; the copy's leading dimension is operand_ld(PREC, K).
+struct WeightConv {
+  const float* src;
+  int N, K, ld_src, transpose, buf;
+  size_t plane;
+  int n_off;
+};
+constexpr int kMaxWeightConvs = 8;
+
+// The copies the tensor-core paths make, in launch order (buffer layout: weight_prep_carve); returns how many.
+inline int weight_convs(const re2nn_recurrence_args& a, const WeightPrep& w, WeightConv* out) {
+  const int S = a.S, R = a.R;
+  int n = 0;
+  out[n++] = WeightConv{a.S1, R, S, R, 1, 0, w.pl_g1, 0};     // [R][S] = S1^T
+  out[n++] = WeightConv{a.S2, R, S, R, 1, 1, w.pl_g1, 0};
+  out[n++] = WeightConv{a.S2, S, R, R, 0, 2, w.pl_g2q, 0};    // [S][R] = S2
+  out[n++] = WeightConv{a.S1, S, R, R, 0, 3, w.pl_g2q, 0};
+  out[n++] = WeightConv{a.W, S, S, S, 1, 4, w.pl_ss, 0};      // fwd: B[k=s][n=j] = W[s][j] -> [n][k] = W^T
+  out[n++] = WeightConv{a.W, S, S, S, 0, 5, w.pl_ss, 0};      // bwd: B[k][n] = W[n][k]   -> [n][k] = W
+  if (a.farnn >= 1) out[n++] = WeightConv{a.Wss1, S, S, S, 1, 6, w.pl_gate, 0};
+  if (a.farnn == 2) out[n++] = WeightConv{a.Wss2, S, S, S, 1, 6, w.pl_gate, S};
+  return n;
+}
+
 // operand pointers of the tensor-core formats (the buffers hold the converted copies)
 inline void weight_prep_bind(WeightPrep& w, int farnn) {
   w.g1[0] = w.buf[0]; w.g1[1] = w.buf[1];
@@ -100,7 +125,7 @@ inline void weight_prep_bind(WeightPrep& w, int farnn) {
 
 template <int PREC>
 inline int weight_prep_run(const re2nn_recurrence_args& a, WeightPrep& w, cudaStream_t st) {
-  const int S = a.S, R = a.R;
+  const int S = a.S;
   if (PREC == RE2NN_PREC_FP32) {
     w.g1[0] = a.S1; w.g1[1] = a.S2;
     w.g2q[0] = a.S2; w.g2q[1] = a.S1;
@@ -114,23 +139,15 @@ inline int weight_prep_run(const re2nn_recurrence_args& a, WeightPrep& w, cudaSt
     }
     return 0;
   }
-  auto conv = [&](const float* src, int N, int K, int ld_src, int tr, void* dst, int ldk, size_t plane,
-                  int n_off) -> cudaError_t {
-    size_t total = (size_t)N * ldk;
-    int blocks = (int)((total + 255) / 256);
-    convert_weight_kernel<PREC><<<blocks, 256, 0, st>>>(src, N, K, ld_src, tr, dst, ldk, plane, n_off);
-    return cudaGetLastError();
-  };
-  const size_t pl_g1 = w.pl_g1, pl_g2q = w.pl_g2q, pl_ss = w.pl_ss, pl_gate = w.pl_gate;
-  RE2NN_CUDA(conv(a.S1, R, S, R, 1, w.buf[0], w.ldS, pl_g1, 0));   // [R][S] = S1^T
-  RE2NN_CUDA(conv(a.S2, R, S, R, 1, w.buf[1], w.ldS, pl_g1, 0));
-  RE2NN_CUDA(conv(a.S2, S, R, R, 0, w.buf[2], w.ldR, pl_g2q, 0));  // [S][R] = S2
-  RE2NN_CUDA(conv(a.S1, S, R, R, 0, w.buf[3], w.ldR, pl_g2q, 0));
-  RE2NN_CUDA(conv(a.W, S, S, S, 1, w.buf[4], w.ldS, pl_ss, 0));    // fwd: B[k=s][n=j] = W[s][j] -> [n][k] = W^T
-  RE2NN_CUDA(conv(a.W, S, S, S, 0, w.buf[5], w.ldS, pl_ss, 0));    // bwd: B[k][n] = W[n][k]   -> [n][k] = W
-  if (a.farnn >= 1) {
-    RE2NN_CUDA(conv(a.Wss1, S, S, S, 1, w.buf[6], w.ldS, pl_gate, 0));
-    if (a.farnn == 2) RE2NN_CUDA(conv(a.Wss2, S, S, S, 1, w.buf[6], w.ldS, pl_gate, S));
+  WeightConv convs[kMaxWeightConvs];
+  const int n = weight_convs(a, w, convs);
+  for (int i = 0; i < n; ++i) {
+    const WeightConv& c = convs[i];
+    const int ldk = operand_ld(PREC, c.K);
+    const int blocks = (int)(((size_t)c.N * ldk + 255) / 256);
+    convert_weight_kernel<PREC><<<blocks, 256, 0, st>>>(c.src, c.N, c.K, c.ld_src, c.transpose, w.buf[c.buf], ldk,
+                                                        c.plane, c.n_off);
+    RE2NN_LAUNCH_CHECK();
   }
   weight_prep_bind(w, a.farnn);
   return 0;

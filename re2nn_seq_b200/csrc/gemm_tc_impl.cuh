@@ -33,11 +33,8 @@ struct __align__(64) TcLaunch {
   int cg;   // 1: one CTA per 128 x bn tile; 2: CTA pair per 256 x bn tile (B box rows = bn / 2)
   int launch_id;   // debug trace: index of this launch since tracing was switched on
 };
-typedef TcLaunch TcStepMaps;
 static int g_tc_trace_launches = -1;  // debug: >= 0 while a phase-trace buffer is installed (next launch index)
 static int g_tc_force_cg = 0;        // debug: 0 = cost model picks, 1 / 2 = force the CTA-group size
-static bool g_tc_use_pdl = true;     // programmatic dependent launch between consecutive tcgen05 step kernels
-struct TcRecurrenceMaps { TcLaunch gate, g1[2], g2[2]; };
 
 // ---- host: tensor maps ---------------------------------------------------------------------------------
 typedef CUresult (*PFN_tmapEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -824,11 +821,10 @@ inline cudaError_t launch_tc_bn(const TcLaunch& L, const Epi& epi, cudaStream_t 
     attr[na].val.clusterDim.z = 1;
     ++na;
   }
-  if (g_tc_use_pdl) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
+  // programmatic dependent launch between consecutive tcgen05 step kernels
+  attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[na].val.programmaticStreamSerializationAllowed = 1;
+  ++na;
   cfg.attrs = attr;
   cfg.numAttrs = na;
   if (g_tc_trace_launches >= 0) {
@@ -840,7 +836,7 @@ inline cudaError_t launch_tc_bn(const TcLaunch& L, const Epi& epi, cudaStream_t 
 }
 
 template <int PREC, class Epi>
-inline cudaError_t launch_tc_gemm(const GemmProblem&, const Epi& epi, const TcStepMaps* L, cudaStream_t st) {
+inline cudaError_t launch_tc_gemm(const Epi& epi, const TcLaunch* L, cudaStream_t st) {
   if constexpr (PREC == RE2NN_PREC_FP32) {
     return cudaErrorNotSupported;
   } else {

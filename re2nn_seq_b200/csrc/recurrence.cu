@@ -159,14 +159,188 @@ static std::vector<int> prof_live(int cls) {
 }
 
 template <int PREC, class Epi>
-static cudaError_t launch_gemm(int cls, const GemmProblem& prob, const Epi& epi, const TcStepMaps* maps,
-                               cudaStream_t st) {
+static cudaError_t launch_gemm(int cls, const GemmProblem& prob, const Epi& epi, const TcLaunch* plan, cudaStream_t st) {
   const int pi = prof_begin(cls, st);
   cudaError_t e;
   if (PREC == RE2NN_PREC_FP32) e = launch_simt_gemm(prob, epi, ALoadPlain{}, st);
-  else e = launch_tc_gemm<PREC>(prob, epi, maps, st);
+  else e = launch_tc_gemm<PREC>(epi, plan, st);
   prof_end(pi, st);
   return e;
+}
+
+// How a call runs, decided here only (the argument check and the public queries ask this function too):
+//   resident: inference on a tensor-core precision whose S and R fit the resident kernel -- one launch for all steps;
+//   fused:    otherwise inference without gates on a tensor-core precision, ab_out set, no full_pad -- one direction
+//             at a time, the forward state epilogue writes (alpha * beta) in operand format;
+//   per-step: two or three step-GEMM launches per step (fp32, training, and everything else).
+enum class RecPath { kPerStep, kResident, kFused };
+static RecPath rec_path(const re2nn_recurrence_args& a) {
+  if (a.precision == RE2NN_PREC_FP32 || a.save_for_backward) return RecPath::kPerStep;
+  const int planes = a.precision == RE2NN_PREC_BF16 ? 1 : 2;
+  if (g_resident_on && resident_supported(planes, a.S, a.R, a.precision != RE2NN_PREC_BF16)) return RecPath::kResident;
+  if (a.ab_out != nullptr && a.farnn == 0 && !a.full_pad) return RecPath::kFused;
+  return RecPath::kPerStep;
+}
+
+// Compile-time (NL, FARNN) of the state epilogue EpiH: calls f(EpiSel<NL, FARNN>{}).  A configuration gets its own
+// instantiation where it is common enough to pay for one; -1 reads the value from StepParams at run time.  The
+// resident kernel sizes its epilogue warps by FARNN, so it compiles every FARNN; the fused path runs farnn == 0 only.
+template <int NL_, int FARNN_> struct EpiSel { static constexpr int NL = NL_, FARNN = FARNN_; };
+enum class EpiSet { kTrain, kInfer, kFused, kResident };
+template <EpiSet SET, class F>
+static cudaError_t with_state_epi(int farnn, int nl, F&& f) {
+  constexpr int T = RE2NN_NL_TANH;
+  const bool th = nl == T;
+  if constexpr (SET == EpiSet::kTrain) {
+    if (th && farnn == 0) return f(EpiSel<T, 0>{});
+    if (th && farnn == 2) return f(EpiSel<T, 2>{});
+    return f(EpiSel<-1, -1>{});
+  } else if constexpr (SET == EpiSet::kFused) {
+    return th ? f(EpiSel<T, 0>{}) : f(EpiSel<-1, 0>{});
+  } else if constexpr (SET == EpiSet::kInfer) {
+    if (farnn == 0) return th ? f(EpiSel<T, 0>{}) : f(EpiSel<-1, 0>{});
+    if (th) return farnn == 1 ? f(EpiSel<T, 1>{}) : f(EpiSel<T, 2>{});
+    return f(EpiSel<-1, -1>{});
+  } else {
+    if (farnn == 0) return th ? f(EpiSel<T, 0>{}) : f(EpiSel<-1, 0>{});
+    if (farnn == 1) return th ? f(EpiSel<T, 1>{}) : f(EpiSel<-1, 1>{});
+    return th ? f(EpiSel<T, 2>{}) : f(EpiSel<-1, 2>{});
+  }
+}
+
+// Inference: one resident launch (a CTA pair per 128-row tile runs all steps; recurrence_resident.cuh)
+template <int PREC>
+static int run_resident(const re2nn_recurrence_args& a, const RecWs& w, StepParams p, const GemmProblem& g_gate,
+                        const GemmProblem* g_1, const GemmProblem* g_2, cudaStream_t st) {
+  constexpr int kPlanes = OperandFmt<PREC>::kPlanes;
+  std::unique_ptr<ResidentLaunch> rl(new ResidentLaunch);
+  memset(rl.get(), 0, sizeof(ResidentLaunch));
+  const int bn1 = resident_part(a.R), bn2 = resident_part(a.S);
+  // The TMEM accumulator truncates, so the summation order is part of the result: the parity-grade split formats
+  // keep the order of the per-step path (Q @ S^T first, measured 2-4x closer to fp32 than W first on cfg4);
+  // bf16 starts G2 with Hbar @ W, whose operands do not wait for this step's Q
+  rl->q_first = PREC == RE2NN_PREC_BF16 ? 0 : 1;
+  for (int par = 0; par < 2; ++par) {
+    GemmProblem r2 = g_2[par];
+    if (!rl->q_first)
+      for (int z = 0; z < 2; ++z) {
+        r2.seg[z][0] = g_2[par].seg[z][1];
+        r2.seg[z][1] = g_2[par].seg[z][0];
+      }
+    if (int rc = tc_make_launch<PREC>(g_1[par], &rl->g1[par], bn1)) return rc;
+    if (int rc = tc_make_launch<PREC>(r2, &rl->g2[par], bn2)) return rc;
+  }
+  if (a.farnn >= 1)
+    if (int rc = tc_make_launch<PREC>(g_gate, &rl->gate, bn2)) return rc;
+  rl->steps = a.L;
+  rl->alias_tbuf = resident_alias(kPlanes, rl->q_first != 0) ? 1 : 0;
+  rl->stage_bytes = resident_stage_bytes(kPlanes, a.S, a.R);
+  rl->stages = resident_stages(kPlanes, a.S, a.R, rl->q_first != 0);
+  for (int z = 0; z < 2; ++z) { p.Hbar_cur[z] = w.Hbar[0][z]; p.Hbar_next[z] = w.Hbar[1][z]; p.Z[z] = w.Z[z]; }
+  const int pi = prof_begin(3, st);
+  const cudaError_t e = with_state_epi<EpiSet::kResident>(a.farnn, a.update_nonlinear, [&](auto sel) {
+    using E = decltype(sel);
+    return launch_resident<PREC, E::NL, E::FARNN>(*rl, p, a.B, st);
+  });
+  prof_end(pi, st);
+  RE2NN_CUDA(e);
+  return 0;
+}
+
+// Fused label-score operand (ab_out): the backward direction first (beta complete), then the forward direction
+// whose state epilogue writes alpha * beta in operand format -- alpha itself is never materialised and the
+// (alpha, beta) re-read of re2nn_label_scores disappears.  Single-direction launches (ndir = 1, dir_base = z).
+template <int PREC>
+static int run_fused(const re2nn_recurrence_args& a, const RecWs& w, StepParams p, const GemmProblem* g_1,
+                     const GemmProblem* g_2, cudaStream_t st) {
+  p.AB = a.ab_out; p.ldab = p.ldh; p.ab_plane = (size_t)a.B * a.L * p.ldh; p.beta_in = a.beta;
+  for (int z = 0; z < 2; ++z) { p.Z[z] = w.Z[z]; p.Rg[z] = nullptr; }
+  std::unique_ptr<TcLaunch[]> plan(new TcLaunch[8]);       // [z][par][g1 | g2]
+  GemmProblem g1d[2][2], g2d[2][2];
+  for (int z = 0; z < 2; ++z)
+    for (int par = 0; par < 2; ++par) {
+      g1d[z][par] = g_1[par]; g1d[z][par].ndir = 1; g1d[z][par].seg[0][0] = g_1[par].seg[z][0];
+      g2d[z][par] = g_2[par]; g2d[z][par].ndir = 1;
+      g2d[z][par].seg[0][0] = g_2[par].seg[z][0]; g2d[z][par].seg[0][1] = g_2[par].seg[z][1];
+      if (int rc = tc_make_launch<PREC>(g1d[z][par], &plan[(z * 2 + par) * 2])) return rc;
+      if (int rc = tc_make_launch<PREC>(g2d[z][par], &plan[(z * 2 + par) * 2 + 1])) return rc;
+    }
+  for (int zi = 0; zi < 2; ++zi) {
+    const int z = 1 - zi;                                    // backward direction first
+    p.dir_base = z;
+    for (int k = 0; k < a.L; ++k) {
+      p.k = k;
+      const int par = k & 1;
+      for (int zz = 0; zz < 2; ++zz) { p.Hbar_cur[zz] = w.Hbar[par][zz]; p.Hbar_next[zz] = w.Hbar[par ^ 1][zz]; }
+      RE2NN_CUDA((launch_gemm<PREC>(1, g1d[z][par], EpiQ<PREC>{p}, &plan[(z * 2 + par) * 2], st)));
+      const TcLaunch* p2 = &plan[(z * 2 + par) * 2 + 1];
+      RE2NN_CUDA(with_state_epi<EpiSet::kFused>(a.farnn, a.update_nonlinear, [&](auto sel) {
+        using E = decltype(sel);
+        if (z == 1) return launch_gemm<PREC>(2, g2d[z][par], EpiH<PREC, E::NL, E::FARNN>{p}, p2, st);
+        return launch_gemm<PREC>(2, g2d[z][par], EpiH<PREC, E::NL, E::FARNN, false, true>{p}, p2, st);
+      }));
+    }
+  }
+  return 0;
+}
+
+// One launch per step GEMM: gate (farnn >= 1), G1, G2.  TRAIN: the epilogues also write the save slabs.
+template <int PREC, bool TRAIN>
+static int run_steps(const re2nn_recurrence_args& a, const RecWs& w, StepParams p, const GemmProblem& g_gate,
+                     const GemmProblem* g_1, const GemmProblem* g_2, cudaStream_t st) {
+  const int B = a.B, S = a.S, R = a.R, L = a.L;
+  std::unique_ptr<TcLaunch[]> plan;      // tcgen05: [gate, g1[0], g1[1], g2[0], g2[1]]; none on CUDA cores
+  if constexpr (PREC != RE2NN_PREC_FP32) {
+    plan.reset(new TcLaunch[5]);
+    if (a.farnn >= 1)
+      if (int rc = tc_make_launch<PREC>(g_gate, &plan[0])) return rc;
+    for (int par = 0; par < 2; ++par) {
+      if (int rc = tc_make_launch<PREC>(g_1[par], &plan[1 + par])) return rc;
+      if (int rc = tc_make_launch<PREC>(g_2[par], &plan[3 + par])) return rc;
+    }
+  }
+  auto plan_of = [&](int i) -> const TcLaunch* { return plan ? &plan[i] : nullptr; };
+  for (int k = 0; k < L; ++k) {
+    p.k = k;
+    const int par = k & 1;
+    GemmProblem gg = g_gate, g1 = g_1[par], g2 = g_2[par];
+    for (int z = 0; z < 2; ++z) {
+      p.Hbar_cur[z] = w.Hbar[par][z];
+      p.Hbar_next[z] = w.Hbar[par ^ 1][z];
+      p.Z[z] = w.Z[z];
+      p.Rg[z] = nullptr;
+      if constexpr (TRAIN) {
+        const size_t sS = (size_t)B * S, sR = (size_t)B * R;
+        float* hb_k = a.hbar_save + ((size_t)z * (L + 1) + k) * sS;
+        float* hs_k = a.hst_save + ((size_t)z * (L + 1) + k) * sS;
+        p.HstNext[z] = hs_k + sS;
+        p.Usave[z] = a.u_save + ((size_t)z * L + k) * sR;
+        p.Asave[z] = a.a_save + ((size_t)z * L + k) * sS;
+        if (a.farnn >= 1) p.Z[z] = a.zsave + ((size_t)z * L + k) * sS;
+        p.Rg[z] = a.farnn == 2 ? a.rsave + ((size_t)z * L + k) * sS : nullptr;
+        if (PREC == RE2NN_PREC_FP32) {
+          // fp32: the operands themselves live in the step-major save slabs instead of the ping-pong buffers
+          p.Hbar_cur[z] = hb_k;
+          p.Hbar_next[z] = hb_k + sS;
+          p.Hst[z] = hs_k + sS;
+          gg.seg[z][0].A = hs_k;
+          g1.seg[z][0].A = hb_k;
+          g2.seg[z][1].A = hb_k;
+        } else {
+          // tensor cores: operands stay in their (ping-pong) operand-format buffers, the epilogues add fp32 copies
+          p.HbarSaveNext[z] = hb_k + sS;
+          p.HbarSaveCur[z] = hb_k;
+        }
+      }
+    }
+    if (a.farnn >= 1) RE2NN_CUDA((launch_gemm<PREC>(0, gg, EpiGate<PREC, TRAIN>{p}, plan_of(0), st)));
+    RE2NN_CUDA((launch_gemm<PREC>(1, g1, EpiQ<PREC, TRAIN>{p}, plan_of(1 + par), st)));
+    RE2NN_CUDA(with_state_epi<TRAIN ? EpiSet::kTrain : EpiSet::kInfer>(a.farnn, a.update_nonlinear, [&](auto sel) {
+      using E = decltype(sel);
+      return launch_gemm<PREC>(2, g2, EpiH<PREC, E::NL, E::FARNN, TRAIN>{p}, plan_of(3 + par), st);
+    }));
+  }
+  return 0;
 }
 
 template <int PREC>
@@ -224,169 +398,30 @@ static int run_recurrence(const re2nn_recurrence_args& a, cudaStream_t st) {
   for (int z = 0; z < 2; ++z) { p.Q[z] = w.Q[z]; p.Hst[z] = w.Hst[z]; p.H[z] = w.H[z]; }
 
   if constexpr (PREC != RE2NN_PREC_FP32) {
-    // Inference: one resident launch (a CTA pair per 128-row tile runs all steps; recurrence_resident.cuh)
-    if (g_resident_on && !a.save_for_backward &&
-        resident_supported(OperandFmt<PREC>::kPlanes, S, R, PREC != RE2NN_PREC_BF16)) {
-      std::unique_ptr<ResidentLaunch> rl(new ResidentLaunch);
-      memset(rl.get(), 0, sizeof(ResidentLaunch));
-      const int bn1 = resident_part(R), bn2 = resident_part(S);
-      // The TMEM accumulator truncates, so the summation order is part of the result: the parity-grade split formats
-      // keep the order of the per-step path (Q @ S^T first, measured 2-4x closer to fp32 than W first on cfg4);
-      // bf16 starts G2 with Hbar @ W, whose operands do not wait for this step's Q
-      rl->q_first = PREC == RE2NN_PREC_BF16 ? 0 : 1;
-      for (int par = 0; par < 2; ++par) {
-        GemmProblem r2 = g_2[par];
-        if (!rl->q_first)
-          for (int z = 0; z < 2; ++z) {
-            r2.seg[z][0] = g_2[par].seg[z][1];
-            r2.seg[z][1] = g_2[par].seg[z][0];
-          }
-        if (int rc = tc_make_launch<PREC>(g_1[par], &rl->g1[par], bn1)) return rc;
-        if (int rc = tc_make_launch<PREC>(r2, &rl->g2[par], bn2)) return rc;
-      }
-      if (a.farnn >= 1)
-        if (int rc = tc_make_launch<PREC>(g_gate, &rl->gate, bn2)) return rc;
-      rl->steps = L;
-      rl->alias_tbuf = resident_alias(OperandFmt<PREC>::kPlanes, rl->q_first != 0) ? 1 : 0;
-      rl->stage_bytes = resident_stage_bytes(OperandFmt<PREC>::kPlanes, S, R);
-      rl->stages = resident_stages(OperandFmt<PREC>::kPlanes, S, R, rl->q_first != 0);
-      for (int z = 0; z < 2; ++z) { p.Hbar_cur[z] = w.Hbar[0][z]; p.Hbar_next[z] = w.Hbar[1][z]; p.Z[z] = w.Z[z]; }
-      const int pi = prof_begin(3, st);
-      const bool th = a.update_nonlinear == RE2NN_NL_TANH;
-      cudaError_t e;
-      if (a.farnn == 0) e = th ? launch_resident<PREC, RE2NN_NL_TANH, 0>(*rl, p, B, st) : launch_resident<PREC, -1, 0>(*rl, p, B, st);
-      else if (a.farnn == 1) e = th ? launch_resident<PREC, RE2NN_NL_TANH, 1>(*rl, p, B, st) : launch_resident<PREC, -1, 1>(*rl, p, B, st);
-      else e = th ? launch_resident<PREC, RE2NN_NL_TANH, 2>(*rl, p, B, st) : launch_resident<PREC, -1, 2>(*rl, p, B, st);
-      prof_end(pi, st);
-      RE2NN_CUDA(e);
-      return 0;
+    switch (rec_path(a)) {
+      case RecPath::kResident: return run_resident<PREC>(a, w, p, g_gate, g_1, g_2, st);
+      case RecPath::kFused: return run_fused<PREC>(a, w, p, g_1, g_2, st);
+      case RecPath::kPerStep: break;
     }
   }
+  if (a.save_for_backward) return run_steps<PREC, true>(a, w, p, g_gate, g_1, g_2, st);
+  return run_steps<PREC, false>(a, w, p, g_gate, g_1, g_2, st);
+}
 
-  if constexpr (PREC != RE2NN_PREC_FP32) {
-    // Fused label-score operand (ab_out): the backward direction first (beta complete), then the forward direction
-    // whose state epilogue writes alpha * beta in operand format -- alpha itself is never materialised and the
-    // (alpha, beta) re-read of re2nn_label_scores disappears.  Single-direction launches (ndir = 1, dir_base = z).
-    if (a.ab_out != nullptr && !a.save_for_backward && a.farnn == 0 && !a.full_pad) {
-      p.AB = a.ab_out; p.ldab = ldh; p.ab_plane = (size_t)B * L * ldh; p.beta_in = a.beta;
-      for (int z = 0; z < 2; ++z) { p.Z[z] = w.Z[z]; p.Rg[z] = nullptr; }
-      std::unique_ptr<TcLaunch[]> maps(new TcLaunch[8]);       // [z][par][g1 | g2]
-      GemmProblem g1d[2][2], g2d[2][2];
-      for (int z = 0; z < 2; ++z)
-        for (int par = 0; par < 2; ++par) {
-          g1d[z][par] = g_1[par]; g1d[z][par].ndir = 1; g1d[z][par].seg[0][0] = g_1[par].seg[z][0];
-          g2d[z][par] = g_2[par]; g2d[z][par].ndir = 1;
-          g2d[z][par].seg[0][0] = g_2[par].seg[z][0]; g2d[z][par].seg[0][1] = g_2[par].seg[z][1];
-          if (int rc = tc_make_launch<PREC>(g1d[z][par], &maps[(z * 2 + par) * 2])) return rc;
-          if (int rc = tc_make_launch<PREC>(g2d[z][par], &maps[(z * 2 + par) * 2 + 1])) return rc;
-        }
-      const bool th = a.update_nonlinear == RE2NN_NL_TANH;
-      for (int zi = 0; zi < 2; ++zi) {
-        const int z = 1 - zi;                                    // backward direction first
-        p.dir_base = z;
-        for (int k = 0; k < L; ++k) {
-          p.k = k;
-          const int par = k & 1;
-          for (int zz = 0; zz < 2; ++zz) { p.Hbar_cur[zz] = w.Hbar[par][zz]; p.Hbar_next[zz] = w.Hbar[par ^ 1][zz]; }
-          RE2NN_CUDA((launch_gemm<PREC>(1, g1d[z][par], EpiQ<PREC>{p}, &maps[(z * 2 + par) * 2], st)));
-          const TcLaunch* m2 = &maps[(z * 2 + par) * 2 + 1];
-          cudaError_t e;
-          if (z == 1) e = th ? launch_gemm<PREC>(2, g2d[z][par], EpiH<PREC, RE2NN_NL_TANH, 0>{p}, m2, st)
-                             : launch_gemm<PREC>(2, g2d[z][par], EpiH<PREC, -1, 0>{p}, m2, st);
-          else e = th ? launch_gemm<PREC>(2, g2d[z][par], EpiH<PREC, RE2NN_NL_TANH, 0, false, true>{p}, m2, st)
-                      : launch_gemm<PREC>(2, g2d[z][par], EpiH<PREC, -1, 0, false, true>{p}, m2, st);
-          RE2NN_CUDA(e);
-        }
-      }
-      return 0;
-    }
+// Calls f(std::integral_constant<int, PREC>{}) for a RE2NN_PREC_* value.  Any other value fails with "unknown
+// precision" before a CUDA call.  check_tc: the tensor-core precisions first need an sm_100 device.
+template <class F>
+static int with_precision(const char* who, int precision, bool check_tc, F&& f) {
+  if (precision < RE2NN_PREC_FP32 || precision > RE2NN_PREC_FP16X3)
+    return set_error("%s: unknown precision %d", who, precision);
+  RE2NN_CHECK(!check_tc || precision == RE2NN_PREC_FP32 || re2nn_has_tcgen05(), "%s: tcgen05 path needs an sm_100 device",
+              who);
+  switch (precision) {
+    case RE2NN_PREC_FP32: return f(std::integral_constant<int, RE2NN_PREC_FP32>{});
+    case RE2NN_PREC_BF16: return f(std::integral_constant<int, RE2NN_PREC_BF16>{});
+    case RE2NN_PREC_TF32X3: return f(std::integral_constant<int, RE2NN_PREC_TF32X3>{});
+    default: return f(std::integral_constant<int, RE2NN_PREC_FP16X3>{});
   }
-
-  TcRecurrenceMaps* tm = nullptr;
-  std::unique_ptr<TcRecurrenceMaps> tm_hold;
-  if constexpr (PREC != RE2NN_PREC_FP32) {
-    tm_hold.reset(new TcRecurrenceMaps);
-    tm = tm_hold.get();
-    if (a.farnn >= 1)
-      if (int rc = tc_make_launch<PREC>(g_gate, &tm->gate)) return rc;
-    for (int par = 0; par < 2; ++par) {
-      if (int rc = tc_make_launch<PREC>(g_1[par], &tm->g1[par])) return rc;
-      if (int rc = tc_make_launch<PREC>(g_2[par], &tm->g2[par])) return rc;
-    }
-  }
-
-
-  const bool saving = a.save_for_backward != 0;
-  for (int k = 0; k < L; ++k) {
-    p.k = k;
-    const int par = k & 1;
-    GemmProblem gg = g_gate, g1 = g_1[par], g2 = g_2[par];
-    for (int z = 0; z < 2; ++z) {
-      p.Hbar_cur[z] = w.Hbar[par][z];
-      p.Hbar_next[z] = w.Hbar[par ^ 1][z];
-      p.Z[z] = w.Z[z];
-      p.Rg[z] = nullptr;
-      if (saving) {
-        const size_t sS = (size_t)B * S, sR = (size_t)B * R;
-        float* hb_k = a.hbar_save + ((size_t)z * (L + 1) + k) * sS;
-        float* hs_k = a.hst_save + ((size_t)z * (L + 1) + k) * sS;
-        p.HstNext[z] = hs_k + sS;
-        p.Usave[z] = a.u_save + ((size_t)z * L + k) * sR;
-        p.Asave[z] = a.a_save + ((size_t)z * L + k) * sS;
-        if (a.farnn >= 1) p.Z[z] = a.zsave + ((size_t)z * L + k) * sS;
-        p.Rg[z] = a.farnn == 2 ? a.rsave + ((size_t)z * L + k) * sS : nullptr;
-        if (PREC == RE2NN_PREC_FP32) {
-          // fp32: the operands themselves live in the step-major save slabs instead of the ping-pong buffers
-          p.Hbar_cur[z] = hb_k;
-          p.Hbar_next[z] = hb_k + sS;
-          p.Hst[z] = hs_k + sS;
-          gg.seg[z][0].A = hs_k;
-          g1.seg[z][0].A = hb_k;
-          g2.seg[z][1].A = hb_k;
-        } else {
-          // tensor cores: operands stay in their (ping-pong) operand-format buffers, the epilogues add fp32 copies
-          p.HbarSaveNext[z] = hb_k + sS;
-          p.HbarSaveCur[z] = hb_k;
-        }
-      }
-    }
-    if (saving) {   // training: generic functors with the save stores compiled in
-      if (a.farnn >= 1)
-        RE2NN_CUDA((launch_gemm<PREC>(0, gg, EpiGate<PREC, true>{p}, tm ? &tm->gate : nullptr, st)));
-      RE2NN_CUDA((launch_gemm<PREC>(1, g1, EpiQ<PREC, true>{p}, tm ? &tm->g1[par] : nullptr, st)));
-      {   // compile-time specialisations of the common training configurations (generic functor otherwise)
-        const TcStepMaps* m2 = tm ? &tm->g2[par] : nullptr;
-        cudaError_t e;
-        if (a.farnn == 0 && a.update_nonlinear == RE2NN_NL_TANH)
-          e = launch_gemm<PREC>(2, g2, EpiH<PREC, RE2NN_NL_TANH, 0, true>{p}, m2, st);
-        else if (a.farnn == 2 && a.update_nonlinear == RE2NN_NL_TANH)
-          e = launch_gemm<PREC>(2, g2, EpiH<PREC, RE2NN_NL_TANH, 2, true>{p}, m2, st);
-        else
-          e = launch_gemm<PREC>(2, g2, EpiH<PREC, -1, -1, true>{p}, m2, st);
-        RE2NN_CUDA(e);
-      }
-      continue;
-    }
-    if (a.farnn >= 1)
-      RE2NN_CUDA((launch_gemm<PREC>(0, gg, EpiGate<PREC>{p}, tm ? &tm->gate : nullptr, st)));
-    RE2NN_CUDA((launch_gemm<PREC>(1, g1, EpiQ<PREC>{p}, tm ? &tm->g1[par] : nullptr, st)));
-    {   // compile-time specialisations of the hot configurations; everything else takes the generic functor
-      const TcStepMaps* m2 = tm ? &tm->g2[par] : nullptr;
-      cudaError_t e;
-      if (a.farnn == 0 && a.update_nonlinear == RE2NN_NL_TANH)
-        e = launch_gemm<PREC>(2, g2, EpiH<PREC, RE2NN_NL_TANH, 0>{p}, m2, st);
-      else if (a.farnn == 0)
-        e = launch_gemm<PREC>(2, g2, EpiH<PREC, -1, 0>{p}, m2, st);
-      else if (a.farnn == 2 && a.update_nonlinear == RE2NN_NL_TANH)
-        e = launch_gemm<PREC>(2, g2, EpiH<PREC, RE2NN_NL_TANH, 2>{p}, m2, st);
-      else if (a.farnn == 1 && a.update_nonlinear == RE2NN_NL_TANH)
-        e = launch_gemm<PREC>(2, g2, EpiH<PREC, RE2NN_NL_TANH, 1>{p}, m2, st);
-      else
-        e = launch_gemm<PREC>(2, g2, EpiH<PREC, -1, -1>{p}, m2, st);
-      RE2NN_CUDA(e);
-    }
-  }
-  return 0;
 }
 
 }  // namespace re2nn
@@ -423,65 +458,67 @@ __global__ void __launch_bounds__(256) ab_operand_kernel(const float* __restrict
   }
 }
 
+// fp32 row-major [N x K] -> K-major PREC operand (leading dimension operand_ld(PREC, K)) at dst
 template <int PREC>
-static int label_scores_tc(const float* alpha, const float* beta, const int64_t* lengths, int B, int L, int S,
-                           const float* C_mat, int C, int full_pad, float* out, char* ws, cudaStream_t st) {
-  const int ld = operand_ld(PREC, S);
-  const size_t M = (size_t)B * L;
-  void* Aop = ws;
-  void* Bop = ws + operand_bytes(PREC, M, S);
-  const size_t pa = M * ld, pb = (size_t)C * ld;
-  {
-    ab_operand_kernel<PREC><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(alpha, beta, lengths, B, L, S, ld, full_pad, Aop, pa);
-    RE2NN_LAUNCH_CHECK();
-    convert_weight_kernel<PREC><<<(unsigned)(((size_t)C * ld + 255) / 256), 256, 0, st>>>(C_mat, C, S, S, 0, Bop, ld, pb, 0);
-    RE2NN_LAUNCH_CHECK();
-  }
-  GemmProblem g;
-  memset(&g, 0, sizeof(g));
-  g.M = (int)M; g.N = C; g.nseg = 1; g.ndir = 1;
-  g.seg[0][0] = GemmSeg{Aop, Bop, ld, ld, S, 1, pa, pb};
-  TcLaunch Lc;
-  if (int rc = tc_make_launch<PREC>(g, &Lc)) return rc;
-  RE2NN_CUDA((launch_tc_gemm<PREC>(g, EpiStore{out, C, nullptr}, &Lc, st)));
-  return 0;
-}
-
-template <int PREC>
-static int label_scores_ab_tc(const void* ab, size_t M, int S, const float* C_mat, int C, float* out, char* ws, cudaStream_t st) {
-  const int ld = operand_ld(PREC, S);
-  void* Bop = ws;
-  const size_t pa = M * ld, pb = (size_t)C * ld;
-  convert_weight_kernel<PREC><<<(unsigned)(((size_t)C * ld + 255) / 256), 256, 0, st>>>(C_mat, C, S, S, 0, Bop, ld, pb, 0);
-  RE2NN_LAUNCH_CHECK();
-  GemmProblem g;
-  memset(&g, 0, sizeof(g));
-  g.M = (int)M; g.N = C; g.nseg = 1; g.ndir = 1;
-  g.seg[0][0] = GemmSeg{ab, Bop, ld, ld, S, 1, pa, pb};
-  TcLaunch Lc;
-  if (int rc = tc_make_launch<PREC>(g, &Lc)) return rc;
-  RE2NN_CUDA((launch_tc_gemm<PREC>(g, EpiStore{out, C, nullptr}, &Lc, st)));
-  return 0;
-}
-
-template <int PREC>
-static int gemm_nt_tc(const float* A, const float* B, int M, int N, int K, float* C, void* ws, cudaStream_t st) {
+static cudaError_t to_operand(const float* src, size_t N, int K, void* dst, cudaStream_t st) {
   const int ld = operand_ld(PREC, K);
-  void* Ao = ws;
-  void* Bo = (char*)ws + operand_bytes(PREC, M, K);
-  const size_t pa = (size_t)M * ld, pb = (size_t)N * ld;
-  convert_weight_kernel<PREC><<<(unsigned)(((size_t)M * ld + 255) / 256), 256, 0, st>>>(A, M, K, K, 0, Ao, ld, pa, 0);
-  RE2NN_LAUNCH_CHECK();
-  convert_weight_kernel<PREC><<<(unsigned)(((size_t)N * ld + 255) / 256), 256, 0, st>>>(B, N, K, K, 0, Bo, ld, pb, 0);
-  RE2NN_LAUNCH_CHECK();
-  GemmProblem g;
-  memset(&g, 0, sizeof(g));
-  g.M = M; g.N = N; g.nseg = 1; g.ndir = 1;
-  g.seg[0][0] = GemmSeg{Ao, Bo, ld, ld, K, 1, pa, pb};
-  TcLaunch L;
-  if (int rc = tc_make_launch<PREC>(g, &L)) return rc;
-  RE2NN_CUDA((launch_tc_gemm<PREC>(g, EpiStore{C, N, nullptr}, &L, st)));
+  convert_weight_kernel<PREC><<<(unsigned)((N * ld + 255) / 256), 256, 0, st>>>(src, (int)N, K, K, 0, dst, ld, N * ld, 0);
+  return cudaGetLastError();
+}
+
+// C[M x N] = A_op @ B_op^T on tcgen05, both operands K-major PREC operands with leading dimension operand_ld(PREC, K)
+template <int PREC>
+static int gemm_nt_op(const void* A, const void* B, size_t M, int N, int K, float* C, cudaStream_t st) {
+  const int ld = operand_ld(PREC, K);
+  TcLaunch plan;
+  if (int rc = tc_make_launch<PREC>(gemm_problem((int)M, N, GemmSeg{A, B, ld, ld, K, 1, M * ld, (size_t)N * ld}), &plan))
+    return rc;
+  RE2NN_CUDA((launch_tc_gemm<PREC>(EpiStore{C, N, nullptr}, &plan, st)));
   return 0;
+}
+
+// Label-score workspace: the raw scores ahead of a priority layer, then the operand-format copies of (alpha * beta)
+// (unless the caller has them: ab_given) and of C_mat.
+static size_t label_scores_bytes(int B, int L, int S, int C, int precision, bool has_priority, bool ab_given) {
+  const size_t M = (size_t)B * L;
+  size_t need = 256;
+  if (has_priority) need += align_up(M * C * 4, 256);
+  if (precision != RE2NN_PREC_FP32) need += operand_bytes(precision, ab_given ? 0 : M, S) + operand_bytes(precision, C, S);
+  return need;
+}
+
+// scores = (alpha * beta) @ C^T [@ P + b], or from the fused operand `ab` when it is given (tensor-core precisions).
+static int label_scores(const char* who, const void* ab, const float* alpha, const float* beta, const int64_t* lengths,
+                        int B, int L, int S, const float* C_mat, int C, const float* priority_mat,
+                        const float* priority_bias, int full_pad, int precision, float* scores, void* ws,
+                        size_t ws_bytes, cudaStream_t st) {
+  return with_precision(who, precision, true, [&](auto prec) -> int {
+    constexpr int PREC = decltype(prec)::value;
+    const size_t M = (size_t)B * L;
+    const size_t need = label_scores_bytes(B, L, S, C, PREC, priority_mat != nullptr, ab != nullptr);
+    RE2NN_CHECK(need <= 256 || (ws && ws_bytes >= need), "%s: workspace too small", who);
+    float* raw = priority_mat ? (float*)ws : scores;       // the priority layer's input, at the head of the workspace
+    char* wp = (char*)ws + (priority_mat ? align_up(M * C * 4, 256) : 0);
+    if constexpr (PREC == RE2NN_PREC_FP32) {
+      RE2NN_CUDA(launch_simt_gemm(gemm_problem((int)M, C, GemmSeg{alpha, C_mat, S, S, S, 1, 0, 0}), EpiStore{raw, C, nullptr},
+                                  ALoadAlphaBeta{alpha, beta, lengths, L, full_pad}, st));
+    } else {
+      if (!ab) {
+        const int ld = operand_ld(PREC, S);
+        ab_operand_kernel<PREC><<<(unsigned)((M + 7) / 8), 256, 0, st>>>(alpha, beta, lengths, B, L, S, ld, full_pad, wp,
+                                                                          M * ld);
+        RE2NN_LAUNCH_CHECK();
+        ab = wp;
+        wp += operand_bytes(PREC, M, S);
+      }
+      RE2NN_CUDA(to_operand<PREC>(C_mat, C, S, wp, st));
+      if (int rc = gemm_nt_op<PREC>(ab, wp, M, C, S, raw, st)) return rc;
+    }
+    if (priority_mat)
+      RE2NN_CUDA(launch_simt_gemm(gemm_problem((int)M, C, GemmSeg{raw, priority_mat, C, C, C, 0, 0, 0}),
+                                  EpiStore{scores, C, priority_bias}, ALoadPlain{}, st));
+    return 0;
+  });
 }
 
 extern "C" {
@@ -577,26 +614,16 @@ size_t re2nn_decompose_recurrence_workspace(const re2nn_recurrence_args* a) {
   return carve(*a, nullptr, nullptr);
 }
 
-// does this call take the resident single-launch path?  (mirrors the test in run_recurrence)
-static bool takes_resident_path(const re2nn_recurrence_args& a) {
-  if (a.precision == RE2NN_PREC_FP32 || !g_resident_on || a.save_for_backward) return false;
-  const int planes = a.precision == RE2NN_PREC_BF16 ? 1 : 2;
-  return resident_supported(planes, a.S, a.R, a.precision != RE2NN_PREC_BF16);
-}
-
-// does a call with ab_out set write the fused (alpha * beta) operand?  (mirrors the test in run_recurrence)
-static bool decompose_fuses(const re2nn_recurrence_args& a) {
-  return a.precision != RE2NN_PREC_FP32 && !a.save_for_backward && a.farnn == 0 && !a.full_pad && !takes_resident_path(a);
-}
-
 int re2nn_decompose_recurrence_fuses(const re2nn_recurrence_args* a) {
   if (!a) return 0;
-  return decompose_fuses(*a) ? 1 : 0;
+  re2nn_recurrence_args q = *a;
+  q.ab_out = &q;                 // as if the caller asked for the operand
+  return rec_path(q) == RecPath::kFused ? 1 : 0;
 }
 
 int re2nn_decompose_recurrence_resident(const re2nn_recurrence_args* a) {
   if (!a) return 0;
-  return takes_resident_path(*a) ? 1 : 0;
+  return rec_path(*a) == RecPath::kResident ? 1 : 0;
 }
 
 size_t re2nn_decompose_weight_prep_bytes(const re2nn_recurrence_args* a) {
@@ -609,25 +636,29 @@ int re2nn_decompose_weight_prep(const re2nn_recurrence_args* a, void* out, void*
   RE2NN_CHECK(a->precision != RE2NN_PREC_FP32, "decompose_weight_prep: the fp32 path uses the parameters as they are");
   RE2NN_CHECK(a->farnn == 0 || a->Wss1, "decompose_weight_prep: farnn>=1 needs Wss1");
   RE2NN_CHECK(a->farnn < 2 || a->Wss2, "decompose_weight_prep: farnn==2 needs Wss2");
-  WeightPrep wp;
-  weight_prep_carve(a->precision, a->S, a->R, a->farnn, (char*)out, &wp);
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (a->precision) {
-    case RE2NN_PREC_BF16: return weight_prep_run<RE2NN_PREC_BF16>(*a, wp, st);
-    case RE2NN_PREC_TF32X3: return weight_prep_run<RE2NN_PREC_TF32X3>(*a, wp, st);
-    case RE2NN_PREC_FP16X3: return weight_prep_run<RE2NN_PREC_FP16X3>(*a, wp, st);
-    default: return set_error("decompose_weight_prep: unknown precision %d", a->precision);
-  }
+  // no device check: the conversion kernels run on any GPU
+  return with_precision("decompose_weight_prep", a->precision, false, [&](auto prec) -> int {
+    WeightPrep wp;
+    weight_prep_carve(prec, a->S, a->R, a->farnn, (char*)out, &wp);
+    return weight_prep_run<decltype(prec)::value>(*a, wp, (cudaStream_t)stream);
+  });
 }
 
 int re2nn_decompose_recurrence_launches(const re2nn_recurrence_args* a) {
   if (!a) return -1;
   int n = 2;                                                     // tile_last + rec_init
-  if (a->precision == RE2NN_PREC_FP32) n += a->farnn == 2 ? 1 : 0;   // [Wss1 | Wss2] concat
-  else if (a->wprep == nullptr) n += 6 + a->farnn;               // operand-format copies of the weights
-  if (a->ab_out && decompose_fuses(*a)) n += a->L * 4;          // single-direction launches, two directions
-  else n += takes_resident_path(*a) ? 1 : a->L * (2 + (a->farnn >= 1 ? 1 : 0));
-  return n;
+  if (a->precision == RE2NN_PREC_FP32) {
+    n += a->farnn == 2 ? 1 : 0;                                  // [Wss1 | Wss2] concat
+  } else if (a->wprep == nullptr) {
+    WeightConv convs[kMaxWeightConvs];                           // operand-format copies of the weights
+    n += weight_convs(*a, WeightPrep{}, convs);
+  }
+  switch (rec_path(*a)) {
+    case RecPath::kResident: return n + 1;
+    case RecPath::kFused: return n + a->L * 4;                  // single-direction launches, two directions
+    case RecPath::kPerStep: break;
+  }
+  return n + a->L * (2 + (a->farnn >= 1 ? 1 : 0));
 }
 
 int re2nn_decompose_recurrence(const re2nn_recurrence_args* a, void* stream) {
@@ -640,7 +671,7 @@ int re2nn_decompose_recurrence(const re2nn_recurrence_args* a, void* stream) {
               "decompose_recurrence: unsupported update_nonlinear %d", a->update_nonlinear);
   RE2NN_CHECK(a->v_mode == RE2NN_V_DENSE || a->x != nullptr, "decompose_recurrence: token mode needs x");
   RE2NN_CHECK(a->lengths && a->vtab && a->S1 && a->S2 && a->W && a->o && a->h0 && a->hT && a->beta &&
-                  (a->alpha || (a->ab_out && decompose_fuses(*a))),
+                  (a->alpha || rec_path(*a) == RecPath::kFused),
               "decompose_recurrence: null tensor");
   RE2NN_CHECK(a->farnn == 0 || (a->gtab && a->Wss1), "decompose_recurrence: farnn>=1 needs gtab and Wss1");
   RE2NN_CHECK(a->farnn < 2 || a->Wss2, "decompose_recurrence: farnn==2 needs Wss2");
@@ -650,20 +681,9 @@ int re2nn_decompose_recurrence(const re2nn_recurrence_args* a, void* stream) {
     RE2NN_CHECK(a->farnn == 0 || a->zsave, "decompose_recurrence: farnn>=1 training needs zsave");
     RE2NN_CHECK(a->farnn < 2 || a->rsave, "decompose_recurrence: farnn==2 training needs rsave");
   }
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (a->precision) {
-    case RE2NN_PREC_FP32: return run_recurrence<RE2NN_PREC_FP32>(*a, st);
-    case RE2NN_PREC_BF16:
-      RE2NN_CHECK(re2nn_has_tcgen05(), "decompose_recurrence: tcgen05 path needs an sm_100 device");
-      return run_recurrence<RE2NN_PREC_BF16>(*a, st);
-    case RE2NN_PREC_TF32X3:
-      RE2NN_CHECK(re2nn_has_tcgen05(), "decompose_recurrence: tcgen05 path needs an sm_100 device");
-      return run_recurrence<RE2NN_PREC_TF32X3>(*a, st);
-    case RE2NN_PREC_FP16X3:
-      RE2NN_CHECK(re2nn_has_tcgen05(), "decompose_recurrence: tcgen05 path needs an sm_100 device");
-      return run_recurrence<RE2NN_PREC_FP16X3>(*a, st);
-    default: return set_error("decompose_recurrence: unknown precision %d", a->precision);
-  }
+  return with_precision("decompose_recurrence", a->precision, true, [&](auto prec) -> int {
+    return run_recurrence<decltype(prec)::value>(*a, (cudaStream_t)stream);
+  });
 }
 
 size_t re2nn_gemm_nt_workspace(int precision, int M, int N, int K) {
@@ -675,32 +695,28 @@ int re2nn_gemm_nt(int precision, const float* A, const float* B, int M, int N, i
                   size_t ws_bytes, void* stream) {
   RE2NN_CHECK(A && B && C && M > 0 && N > 0 && K > 0, "gemm_nt: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
-  if (precision == RE2NN_PREC_FP32) {
-    GemmProblem g;
-    memset(&g, 0, sizeof(g));
-    g.M = M; g.N = N; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{A, B, K, K, K, 1, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{C, N, nullptr}, ALoadPlain{}, st));
-    return 0;
-  }
-  RE2NN_CHECK(re2nn_has_tcgen05(), "gemm_nt: tcgen05 path needs an sm_100 device");
-  RE2NN_CHECK(ws && ws_bytes >= re2nn_gemm_nt_workspace(precision, M, N, K), "gemm_nt: workspace too small");
-  if (precision == RE2NN_PREC_BF16) return gemm_nt_tc<RE2NN_PREC_BF16>(A, B, M, N, K, C, ws, st);
-  if (precision == RE2NN_PREC_TF32X3) return gemm_nt_tc<RE2NN_PREC_TF32X3>(A, B, M, N, K, C, ws, st);
-  if (precision == RE2NN_PREC_FP16X3) return gemm_nt_tc<RE2NN_PREC_FP16X3>(A, B, M, N, K, C, ws, st);
-  return set_error("gemm_nt: unknown precision %d", precision);
+  return with_precision("gemm_nt", precision, true, [&](auto prec) -> int {
+    constexpr int PREC = decltype(prec)::value;
+    if constexpr (PREC == RE2NN_PREC_FP32) {
+      RE2NN_CUDA(launch_simt_gemm(gemm_problem(M, N, GemmSeg{A, B, K, K, K, 1, 0, 0}), EpiStore{C, N, nullptr},
+                                  ALoadPlain{}, st));
+      return 0;
+    } else {
+      RE2NN_CHECK(ws && ws_bytes >= re2nn_gemm_nt_workspace(precision, M, N, K), "gemm_nt: workspace too small");
+      void* Bo = (char*)ws + operand_bytes(PREC, M, K);
+      RE2NN_CUDA(to_operand<PREC>(A, M, K, ws, st));
+      RE2NN_CUDA(to_operand<PREC>(B, N, K, Bo, st));
+      return gemm_nt_op<PREC>(ws, Bo, M, N, K, C, st);
+    }
+  });
 }
 
 int re2nn_token_table(const float* V_embed, const float* E, const float* G, const float* beta_vec, int rows, int D,
                       int R, int additional_nonlinear, float* table, void* stream) {
   RE2NN_CHECK(V_embed && E && G && beta_vec && table, "token_table: null tensor");
   RE2NN_CHECK(rows > 0 && D > 0 && R > 0, "token_table: bad dims");
-  GemmProblem g;
-  memset(&g, 0, sizeof(g));
-  g.M = rows; g.N = R; g.nseg = 1; g.ndir = 1;
-  g.seg[0][0] = GemmSeg{E, G, D, R, D, 0, 0, 0};
   EpiTokenTable epi{table, V_embed, beta_vec, R, additional_nonlinear};
-  RE2NN_CUDA(launch_simt_gemm(g, epi, ALoadPlain{}, (cudaStream_t)stream));
+  RE2NN_CUDA(launch_simt_gemm(gemm_problem(rows, R, GemmSeg{E, G, D, R, D, 0, 0, 0}), epi, ALoadPlain{}, (cudaStream_t)stream));
   return 0;
 }
 
@@ -710,10 +726,7 @@ int re2nn_gate_table(const float* vtab, int rows, int R, int S, int farnn, const
   RE2NN_CHECK(vtab && Wrs1 && bs1 && gate && (farnn == 1 || (Wrs2 && bs2)), "gate_table: null tensor");
   const int ldg = S * farnn;
   for (int gi = 0; gi < farnn; ++gi) {
-    GemmProblem g;
-    memset(&g, 0, sizeof(g));
-    g.M = rows; g.N = S; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{vtab, gi == 0 ? Wrs1 : Wrs2, R, S, R, 0, 0, 0};
+    const GemmProblem g = gemm_problem(rows, S, GemmSeg{vtab, gi == 0 ? Wrs1 : Wrs2, R, S, R, 0, 0, 0});
     EpiStore epi{gate + (size_t)gi * S, ldg, gi == 0 ? bs1 : bs2};
     RE2NN_CUDA(launch_simt_gemm(g, epi, ALoadPlain{}, (cudaStream_t)stream));
   }
@@ -730,74 +743,20 @@ int re2nn_label_scores_ab(const void* ab, int B, int L, int S, const float* C_ma
                           void* stream) {
   RE2NN_CHECK(ab && C_mat && scores && B > 0 && L > 0 && S > 0 && C > 0, "label_scores_ab: bad arguments");
   RE2NN_CHECK(precision != RE2NN_PREC_FP32, "label_scores_ab: the fused operand exists for the tensor-core precisions only");
-  RE2NN_CHECK(re2nn_has_tcgen05(), "label_scores_ab: tcgen05 path needs an sm_100 device");
-  const size_t need = 256 + (priority_mat ? align_up((size_t)B * L * C * 4, 256) : 0) + operand_bytes(precision, C, S);
-  RE2NN_CHECK(ws && ws_bytes >= need, "label_scores_ab: workspace too small");
-  cudaStream_t st = (cudaStream_t)stream;
-  char* wp = (char*)ws;
-  float* raw = scores;
-  if (priority_mat) {
-    raw = (float*)wp;
-    wp += align_up((size_t)B * L * C * 4, 256);
-  }
-  const size_t M = (size_t)B * L;
-  int rc = precision == RE2NN_PREC_BF16 ? label_scores_ab_tc<RE2NN_PREC_BF16>(ab, M, S, C_mat, C, raw, wp, st)
-           : precision == RE2NN_PREC_FP16X3 ? label_scores_ab_tc<RE2NN_PREC_FP16X3>(ab, M, S, C_mat, C, raw, wp, st)
-                                            : label_scores_ab_tc<RE2NN_PREC_TF32X3>(ab, M, S, C_mat, C, raw, wp, st);
-  if (rc) return rc;
-  if (priority_mat) {
-    GemmProblem g;
-    memset(&g, 0, sizeof(g));
-    g.M = B * L; g.N = C; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{raw, priority_mat, C, C, C, 0, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{scores, C, priority_bias}, ALoadPlain{}, st));
-  }
-  return 0;
+  return label_scores("label_scores_ab", ab, nullptr, nullptr, nullptr, B, L, S, C_mat, C, priority_mat, priority_bias, 0,
+                      precision, scores, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 size_t re2nn_label_scores_workspace(int B, int L, int S, int C, int precision, int has_priority) {
-  size_t need = 256;
-  if (has_priority) need += align_up((size_t)B * L * C * 4, 256);
-  if (precision != RE2NN_PREC_FP32) need += operand_bytes(precision, (size_t)B * L, S) + operand_bytes(precision, C, S);
-  return need;
+  return label_scores_bytes(B, L, S, C, precision, has_priority != 0, false);
 }
 
 int re2nn_label_scores(const float* alpha, const float* beta, const int64_t* lengths, int B, int L, int S,
                        const float* C_mat, int C, const float* priority_mat, const float* priority_bias, int full_pad,
                        int precision, float* scores, void* ws, size_t ws_bytes, void* stream) {
   RE2NN_CHECK(alpha && beta && lengths && C_mat && scores, "label_scores: null tensor");
-  const size_t need = re2nn_label_scores_workspace(B, L, S, C, precision, priority_mat != nullptr);
-  RE2NN_CHECK(need <= 256 || (ws && ws_bytes >= need), "label_scores: workspace too small");
-  cudaStream_t st = (cudaStream_t)stream;
-  char* wp = (char*)ws;
-  float* raw = scores;
-  if (priority_mat) {
-    raw = (float*)wp;
-    wp += align_up((size_t)B * L * C * 4, 256);
-  }
-  if (precision == RE2NN_PREC_FP32) {
-    GemmProblem g;
-    memset(&g, 0, sizeof(g));
-    g.M = B * L; g.N = C; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{alpha, C_mat, S, S, S, 1, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{raw, C, nullptr}, ALoadAlphaBeta{alpha, beta, lengths, L, full_pad}, st));
-  } else {
-    RE2NN_CHECK(re2nn_has_tcgen05(), "label_scores: tcgen05 path needs an sm_100 device");
-    int rc = precision == RE2NN_PREC_BF16
-                 ? label_scores_tc<RE2NN_PREC_BF16>(alpha, beta, lengths, B, L, S, C_mat, C, full_pad, raw, wp, st)
-                 : precision == RE2NN_PREC_FP16X3
-                       ? label_scores_tc<RE2NN_PREC_FP16X3>(alpha, beta, lengths, B, L, S, C_mat, C, full_pad, raw, wp, st)
-                       : label_scores_tc<RE2NN_PREC_TF32X3>(alpha, beta, lengths, B, L, S, C_mat, C, full_pad, raw, wp, st);
-    if (rc) return rc;
-  }
-  if (priority_mat) {
-    GemmProblem g;
-    memset(&g, 0, sizeof(g));
-    g.M = B * L; g.N = C; g.nseg = 1; g.ndir = 1;
-    g.seg[0][0] = GemmSeg{raw, priority_mat, C, C, C, 0, 0, 0};
-    RE2NN_CUDA(launch_simt_gemm(g, EpiStore{scores, C, priority_bias}, ALoadPlain{}, st));
-  }
-  return 0;
+  return label_scores("label_scores", nullptr, alpha, beta, lengths, B, L, S, C_mat, C, priority_mat, priority_bias,
+                      full_pad, precision, scores, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -56,6 +56,20 @@ def require_cuda():
         raise RuntimeError("re2nn_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
 
 
+def _rec_args(S, R, farnn, precision, B=0, L=0, Lpad=None, x=None, update_nonlinear=None, v_mode=V_TOKEN,
+              full_pad=False, save_for_backward=False, sigmoid_exponent=0.0):
+    """RecurrenceArgs with the shape and configuration fields set; the tensor pointers are left to the caller.
+    Lpad defaults to the row stride of x (L without x)."""
+    a = RecurrenceArgs()
+    a.B, a.L, a.S, a.R = B, L, S, R
+    a.Lpad = Lpad if Lpad is not None else (x.shape[1] if x is not None else L)
+    a.farnn, a.precision = farnn, PREC[precision]
+    a.update_nonlinear = NL[update_nonlinear] if update_nonlinear is not None else 0
+    a.v_mode, a.full_pad, a.save_for_backward = v_mode, int(full_pad), int(save_for_backward)
+    a.sigmoid_exponent = float(sigmoid_exponent)
+    return a
+
+
 def token_table(V_embed, E, G, beta_vec, additional_nonlinear):
     rows, R = V_embed.shape
     D = E.shape[1]
@@ -99,12 +113,8 @@ def decompose_recurrence(x, lengths, L, vtab, gtab, S1, S2, W, o, h0, hT, Wss1, 
     B = lengths.shape[0]
     S, R = S1.shape
     dev = S1.device
-    a = RecurrenceArgs()
-    a.B, a.L, a.S, a.R = B, L, S, R
-    a.Lpad = Lpad if Lpad is not None else (x.shape[1] if x is not None else L)
-    a.farnn, a.update_nonlinear, a.precision = farnn, NL[update_nonlinear], PREC[precision]
-    a.v_mode, a.full_pad, a.save_for_backward = v_mode, int(full_pad), int(save_for_backward)
-    a.sigmoid_exponent = float(sigmoid_exponent)
+    a = _rec_args(S, R, farnn, precision, B, L, Lpad, x, update_nonlinear, v_mode, full_pad, save_for_backward,
+                  sigmoid_exponent)
     # pad rows are never read downstream (label_scores masks them), so no zero-fill is needed
     alloc = torch.zeros if zero_fill else torch.empty
     alpha = alloc((B, L, S), dtype=torch.float32, device=dev)
@@ -156,8 +166,7 @@ def weight_prep(S1, S2, W, Wss1, Wss2, farnn, precision):
     """Operand-format copies of the recurrence weights for `wprep` (tensor-core precisions): 6-8 conversion launches
     once per parameter version instead of once per call."""
     S, R = S1.shape
-    a = RecurrenceArgs()
-    a.S, a.R, a.farnn, a.precision = S, R, farnn, PREC[precision]
+    a = _rec_args(S, R, farnn, precision)
     a.S1, a.S2, a.W = _f32(S1), _f32(S2), _f32(W)
     a.Wss1 = _f32(Wss1) if Wss1 is not None else None
     a.Wss2 = _f32(Wss2) if Wss2 is not None else None
@@ -177,11 +186,7 @@ def decompose_recurrence_fused(x, lengths, L, vtab, S1, S2, W, o, h0, hT, update
     B = lengths.shape[0]
     S, R = S1.shape
     dev = S1.device
-    a = RecurrenceArgs()
-    a.B, a.L, a.S, a.R = B, L, S, R
-    a.Lpad = Lpad if Lpad is not None else (x.shape[1] if x is not None else L)
-    a.farnn, a.update_nonlinear, a.precision = 0, NL[update_nonlinear], PREC[precision]
-    a.v_mode, a.full_pad, a.save_for_backward = v_mode, 0, 0
+    a = _rec_args(S, R, 0, precision, B, L, Lpad, x, update_nonlinear, v_mode)
     if not fn['re2nn_decompose_recurrence_fuses'](C.byref(a)):
         return None
     nbytes = fn['re2nn_label_scores_ab_bytes'](B, L, S, PREC[precision])
@@ -220,9 +225,7 @@ def label_scores_ab(ab, B, L, S, C_mat, priority_mat=None, priority_bias=None, p
 
 def recurrence_fuses(S, R, farnn, precision):
     """Would an inference call of this shape write the fused (alpha * beta) operand when asked to?"""
-    a = RecurrenceArgs()
-    a.S, a.R, a.farnn, a.precision, a.save_for_backward, a.full_pad = S, R, farnn, PREC[precision], 0, 0
-    return bool(fn['re2nn_decompose_recurrence_fuses'](C.byref(a)))
+    return bool(fn['re2nn_decompose_recurrence_fuses'](C.byref(_rec_args(S, R, farnn, precision))))
 
 
 def onehot_recurrence(x, lengths, L, language, W, o, h0, hT, update_nonlinear, max_semiring=False, full_pad=False,
@@ -318,9 +321,7 @@ def profile_enable(on):
 
 def recurrence_is_resident(S, R, farnn, precision):
     """Would an inference call of this shape run all steps in the resident kernel?"""
-    a = RecurrenceArgs()
-    a.S, a.R, a.farnn, a.precision, a.save_for_backward = S, R, farnn, PREC[precision], 0
-    return bool(fn['re2nn_decompose_recurrence_resident'](C.byref(a)))
+    return bool(fn['re2nn_decompose_recurrence_resident'](C.byref(_rec_args(S, R, farnn, precision))))
 
 
 def profile_read():

@@ -31,6 +31,23 @@ def test_version_and_error_channel():
     assert b'null args' in _lib.fn['re2nn_last_error']()
     assert _lib.fn['re2nn_debug_set_viterbi_seqs'](4) != 0
     assert b'expected 0, 1 or 2' in _lib.fn['re2nn_last_error']()
+    # a precision outside the enum is refused before anything is launched or sized from it (dummy pointers, ample ws)
+    bad, p, ws = 7, ctypes.c_void_p(0x1000), 1 << 40
+    a = _lib.RecurrenceArgs()
+    a.B, a.Lpad, a.L, a.S, a.R, a.precision = 4, 8, 8, 32, 16, bad
+    for f in ('x', 'lengths', 'vtab', 'S1', 'S2', 'W', 'o', 'h0', 'hT', 'alpha', 'beta', 'ws'):
+        setattr(a, f, p)
+    a.ws_bytes = ws
+    calls = {
+        're2nn_label_scores': lambda f: f(p, p, p, 4, 8, 32, p, 5, None, None, 0, bad, p, p, ws, None),
+        're2nn_label_scores_ab': lambda f: f(p, 4, 8, 32, p, 5, None, None, bad, p, p, ws, None),
+        're2nn_gemm_nt': lambda f: f(bad, p, p, 16, 16, 16, p, p, ws, None),
+        're2nn_decompose_weight_prep': lambda f: f(ctypes.byref(a), p, None),
+        're2nn_decompose_recurrence': lambda f: f(ctypes.byref(a), None),
+    }
+    for name, call in calls.items():
+        assert call(_lib.fn[name]) != 0, name
+        assert b'unknown precision' in _lib.fn['re2nn_last_error'](), (name, _lib.fn['re2nn_last_error']())
 
 
 def test_no_oracle_in_product():

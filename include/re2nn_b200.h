@@ -369,7 +369,8 @@ int re2nn_debug_set_viterbi_seqs(int ns);
 /* ---- CRF negative log-likelihood ---------------------------------------------------------------------
  * replaces CRF.neg_log_likelihood_loss = _calculate_PZ - _score_sentence (baselines/crf.py:48-99,
  * 202-260).  per_seq[b] = logZ_b - gold_b ; *loss = sum_b per_seq[b] (deterministic reduction).
- * part_save (B x L x T, may be NULL) keeps the forward partitions for re2nn_crf_nll_backward. */
+ * part_save (B x L x T, may be NULL) keeps the forward partitions for re2nn_crf_nll_backward.
+ * tags may be NULL: the gold score is skipped and per_seq[b] = logZ_b (0 for an empty sequence). */
 int re2nn_crf_nll(const float* feats, const float* transitions, const int64_t* lengths,
                   const int64_t* tags, int B, int L, int Ltags, int T, float* per_seq, float* loss,
                   float* part_save, void* stream);
@@ -380,6 +381,27 @@ int re2nn_crf_nll(const float* feats, const float* transitions, const int64_t* l
 int re2nn_crf_nll_backward(const float* feats, const float* transitions, const int64_t* lengths,
                            const int64_t* tags, const float* part_save, const float* gscale,
                            int B, int L, int Ltags, int T, float* dfeats, float* dtrans, void* stream);
+
+/* ---- CRF N-best decoding and tag marginals ---------------------------------------------------------------
+ * no counterpart in the reference's cut-down crf.py; NCRF++'s CRF._viterbi_decode_nbest returns the same K-lists.
+ * Tags run over all T columns (START / STOP included) as in re2nn_crf_viterbi, and a path is scored with its
+ * expressions: part_0[j] = feat_0[j] + trans[T-2][j], then (feat_t[j] + trans[i][j]) + part_{t-1}[i], then
+ * part_{n-1}[i] + trans[i][T-1].
+ * re2nn_crf_nbest: the K (1..16) highest-scoring distinct tag sequences of every sequence in descending score order;
+ * equal scores are ordered by the reversed sequence (y_{n-1}, ..., y_0) ascending, so rank 0 is re2nn_crf_viterbi's
+ * path.  paths B x L x K (int64): tags at valid positions, 0 at pads, -1 at every valid position of a rank that does
+ * not exist (fewer than K sequences, or only -inf ones); scores B x K, -inf for such ranks.  A sequence of length 0
+ * has an all-zero row and scores -inf; lengths are clamped to L.  ws: re2nn_crf_nbest_workspace() bytes (the 16-bit
+ * back-pointers).  K outside [1, 16], T > 4096 or T * K > 25600 fail before any CUDA call. */
+size_t re2nn_crf_nbest_workspace(int B, int L, int T, int K);
+int re2nn_crf_nbest(const float* feats, const float* transitions, const int64_t* lengths, int B, int L, int T, int K,
+                    int64_t* paths, float* scores, void* ws, size_t ws_bytes, void* stream);
+/* re2nn_crf_marginals: marginals[b,t,j] = P(y_t = j | x) (B x L x T, 0 at pads; rows sum to 1) and log_z[b] = log Z_b
+ * (0 for an empty sequence, as re2nn_crf_nll gives), by the forward sweep of re2nn_crf_nll and a backward sweep
+ * without the pairwise accumulators of re2nn_crf_nll_backward, so no tag-set limit of its own.
+ * part_ws: B*L*T fp32 scratch (the forward partitions). */
+int re2nn_crf_marginals(const float* feats, const float* transitions, const int64_t* lengths, int B, int L, int T,
+                        float* marginals, float* log_z, float* part_ws, void* stream);
 
 /* ---- cross entropy over valid positions -----------------------------------------------------------------
  * nn.CrossEntropyLoss() mean over the N valid tokens (model_decompose.py:80, :289).

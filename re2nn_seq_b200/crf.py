@@ -63,5 +63,26 @@ class CRF(nn.Module):
             _, padded = ops.crf_viterbi(feats, self.transitions.detach(), lengths, want_padded=True)
         return None, padded
 
+    def _viterbi_decode_nbest(self, feats, mask, nbest, lengths=None):
+        """NCRF++'s N-best decode -> (path_score B x K, decode_idx B x L x K): the K best distinct tag sequences, best
+        first (rank 0 is _viterbi_decode's path).  path_score is NCRF++'s softmax over the K returned path scores; a
+        rank that does not exist (fewer than K sequences) scores 0 and decodes to -1 at valid positions."""
+        assert feats.size(2) == self.tagset_size + 2
+        with torch.no_grad():
+            feats = self._prep(feats.detach())
+            lengths = (self._lengths(mask) if lengths is None else lengths).to(feats.device).contiguous()
+            decode_idx, scores = ops.crf_nbest(feats, self.transitions.detach(), lengths, nbest)
+            path_score = torch.softmax(scores, 1)       # missing ranks (-inf) get 0; a row without any sequence NaN:
+            path_score = torch.where(torch.isfinite(scores), path_score, torch.zeros_like(path_score))
+        return path_score, decode_idx
+
+    def marginals(self, feats, mask, lengths=None):
+        """Per-token posteriors P(y_t = j | x) (B x L x T, zero at pads) and log Z (B)."""
+        assert feats.size(2) == self.tagset_size + 2
+        with torch.no_grad():
+            feats = self._prep(feats.detach())
+            lengths = (self._lengths(mask) if lengths is None else lengths).to(feats.device).contiguous()
+            return ops.crf_marginals(feats, self.transitions.detach(), lengths)
+
     def forward(self, feats, mask):
         return self._viterbi_decode(feats, mask)

@@ -15,6 +15,9 @@
 //                            (re2nn_debug_set_crf_backward_split(0): 3-111 crf_nll_backward_exp_kernel)
 //   re2nn_crf_viterbi        3-160 crf_viterbi_kernel<cdiv(T, 32), NS> (NS = 2 for large batches, else 1),
 //                            161-216 crf_viterbi_kernel<0, 1>, >= 217 crf_viterbi_global_kernel
+//   re2nn_crf_nbest          crf_nbest_kernel<KM> (KM = K rounded up to a power of two), transitions in shared memory
+//                            while they fit next to one sequence's lists; T <= 4096 and T * K <= 25600, else an error
+//   re2nn_crf_marginals      re2nn_crf_nll without tags, then 3-153 crf_marginal_kernel<true>, >= 154 <false>
 #include <algorithm>
 
 #include "common.cuh"
@@ -302,10 +305,14 @@ __device__ __forceinline__ float crf_log_z(const float* tr, const float* part, i
   return m + logf(s);
 }
 
-// per_seq = logZ - (score of the gold path of the n tags tg), one warp
+// per_seq = logZ - (score of the gold path of the n tags tg), one warp; without tags (tg == NULL) per_seq = logZ
 __device__ __forceinline__ void crf_store_nll(const float* tr, const float* part, const float* fb, const int64_t* tg,
                                               int n, int T, int lane, float* per_seq) {
   const float logZ = crf_log_z(tr, part, T, lane);
+  if (!tg) {
+    if (lane == 0) *per_seq = logZ;
+    return;
+  }
   float g = 0.f;
   for (int t = lane; t < n; t += 32) {
     int cur = (int)tg[t];
@@ -425,7 +432,7 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_kernel(
     __syncwarp();
     float* tmp = pa; pa = pb; pb = tmp;
   }
-  crf_store_nll(tr, pa, fb, tags + (size_t)b * Ltags, n, T, lane, per_seq + b);
+  crf_store_nll(tr, pa, fb, tags ? tags + (size_t)b * Ltags : nullptr, n, T, lane, per_seq + b);
 }
 
 // Same log-partition in the scaled exponential domain: with M = max_i part[i] and cmax[j] = max_i trans[i][j]
@@ -512,7 +519,7 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
     __syncwarp();
     float* tmp = pa; pa = pb; pb = tmp;
   }
-  crf_store_nll(tr, pa, fb, tags + (size_t)b * Ltags, n, T, lane, per_seq + b);
+  crf_store_nll(tr, pa, fb, tags ? tags + (size_t)b * Ltags : nullptr, n, T, lane, per_seq + b);
 }
 
 // CRF backward: marginals by the backward recursion, reusing the saved forward partitions.
@@ -816,6 +823,256 @@ __global__ void crf_nll_backward_exp3_kernel(
   crf_fold_dtrans(s_dtr, nseq, T, Tq, dtrans);
 }
 
+// ---- N-best Viterbi (NCRF++ CRF._viterbi_decode_nbest) -----------------------------------------------------------
+// List Viterbi, one warp per sequence.  The entry of rank r at (t, j) is the r-th best prefix ending in tag j at t,
+// scored with the Viterbi sweep's own expressions -- (feat_t[j] + trans[i][j]) + part_{t-1}[i, r'], and at the end
+// part_{n-1}[i, r'] + trans[i][STOP] -- and ranked by value, then by smaller source tag i, then by smaller source rank r'.
+// For K = 1 that is the first-maximal-index rule of the Viterbi kernels, so rank 0 is their path.  A back-pointer is the
+// key i * 16 + r' (16 bits for T <= 4096), so "smaller key" is the tie rule.  -inf candidates are missing.
+// Selection: every source list is sorted and adding feat + trans is monotone, so ranks r' = 0, 1, ... are scanned over
+// all sources; once a whole rank inserts nothing, no later rank can (each of its candidates is at most the rejected
+// one of the same source, with a larger key).
+constexpr int kNbestMax = 16;
+constexpr int kNbestMaxT = 4096;
+
+// candidate (v, key) ranks above (w, kw)
+__device__ __forceinline__ bool nbest_above(float v, int key, float w, int kw) { return v > w || (v == w && key < kw); }
+
+// Sorted list in registers: KM slots (a power of two >= K), the first K are exact; (tv, tk) is entry K-1, the bar a
+// candidate has to clear.
+template <int KM>
+struct NbestList {
+  float v[KM];
+  int key[KM];
+  float tv;
+  int tk;
+  __device__ __forceinline__ void clear() {
+#pragma unroll
+    for (int k = 0; k < KM; ++k) {
+      v[k] = -INFINITY;
+      key[k] = 0x7fffffff;
+    }
+    tv = -INFINITY;
+    tk = 0x7fffffff;
+  }
+  // inserts (c, ck) if it ranks above entry K-1; returns whether it did
+  __device__ __forceinline__ bool push(float c, int ck, int K) {
+    if (c == -INFINITY || !nbest_above(c, ck, tv, tk)) return false;
+#pragma unroll
+    for (int k = KM - 1; k > 0; --k) {
+      const bool prev = nbest_above(c, ck, v[k - 1], key[k - 1]);
+      const bool here = nbest_above(c, ck, v[k], key[k]);
+      v[k] = prev ? v[k - 1] : (here ? c : v[k]);
+      key[k] = prev ? key[k - 1] : (here ? ck : key[k]);
+    }
+    if (nbest_above(c, ck, v[0], key[0])) {
+      v[0] = c;
+      key[0] = ck;
+    }
+#pragma unroll
+    for (int k = 0; k < KM; ++k)
+      if (k == K - 1) {
+        tv = v[k];
+        tk = key[k];
+      }
+    return true;
+  }
+  __device__ __forceinline__ void pop() {
+#pragma unroll
+    for (int k = 0; k + 1 < KM; ++k) {
+      v[k] = v[k + 1];
+      key[k] = key[k + 1];
+    }
+    v[KM - 1] = -INFINITY;
+    key[KM - 1] = 0x7fffffff;
+  }
+};
+
+// dynamic smem: [trans T*T, row-major, when it fits] | per warp two K x T lists (rank-major: lanes own target tags, the
+// source-tag loop reads one broadcast word).  bp: B x L x K x T back-pointers (position 0 unused).  paths B x L x K:
+// tags at valid positions (-1 for a missing rank), 0 at pads; scores B x K (-inf for a missing rank).
+template <int KM>
+__global__ void __launch_bounds__(kCrfWarps * 32) crf_nbest_kernel(
+    const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len, int B, int L,
+    int T, int K, int tr_smem, int64_t* __restrict__ paths, float* __restrict__ scores, uint16_t* __restrict__ bp) {
+  extern __shared__ __align__(16) float smem[];
+  const int nw = blockDim.x >> 5;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (tr_smem) {
+    for (int e = threadIdx.x; e < T * T; e += blockDim.x) smem[e] = trans_g[e];
+    __syncthreads();
+  }
+  const RowMajorTrans tr{tr_smem ? smem : trans_g, T};
+  const int b = blockIdx.x * nw + warp;
+  if (b >= B) return;
+  const int n = min((int)len[b], L);
+  int64_t* pth = paths + (size_t)b * L * K;
+  if (n <= 0) {
+    for (int e = lane; e < L * K; e += 32) pth[e] = 0;
+    if (lane < K) scores[(size_t)b * K + lane] = -INFINITY;
+    return;
+  }
+  float* pa = smem + (tr_smem ? (size_t)T * T : 0) + (size_t)warp * 2 * K * T;   // lists of position t-1
+  float* pb = pa + (size_t)K * T;                                                 // lists of position t
+  const float* fb = feats + (size_t)b * L * T;
+  uint16_t* bpb = bp + (size_t)b * L * K * T;
+  for (int j = lane; j < T; j += 32) {
+    pa[j] = viterbi_start(tr, fb, j, T, -1, 0.f);
+    for (int r = 1; r < K; ++r) pa[r * T + j] = -INFINITY;
+  }
+  __syncwarp();
+  for (int t = 1; t < n; ++t) {
+    const float* ft = fb + (size_t)t * T;
+    uint16_t* bpt = bpb + (size_t)t * K * T;
+    for (int j0 = 0; j0 < T; j0 += 32) {          // warp-uniform, so that the rank scan can vote
+      const int j = j0 + lane;
+      const bool has = j < T;
+      const float f = has ? __ldg(ft + j) : 0.f;
+      NbestList<KM> lst;
+      lst.clear();
+      bool go = has;
+      for (int r = 0; r < K && __any_sync(0xffffffffu, go); ++r) {
+        if (go) {
+          const float* pr = pa + r * T;
+          bool ins = false;
+          for (int i = 0; i < T; ++i) ins |= lst.push((f + tr(i, j)) + pr[i], i * kNbestMax + r, K);
+          go = ins;
+        }
+      }
+      if (has) {
+#pragma unroll
+        for (int k = 0; k < KM; ++k)
+          if (k < K) {
+            pb[k * T + j] = lst.v[k];
+            bpt[k * T + j] = (uint16_t)lst.key[k];
+          }
+      }
+    }
+    __syncwarp();      // lists and back-pointers of position t are complete
+    float* tmp = pa; pa = pb; pb = tmp;
+  }
+  // STOP: every lane ranks the candidates of its own source tags (a source's ranks stop at the first one that does
+  // not enter), then K rounds of a warp arg-max merge the 32 lists; lane k keeps the final entry of rank k
+  NbestList<KM> lst;
+  lst.clear();
+  for (int i = lane; i < T; i += 32) {
+    const float s = tr(i, T - 1);
+    for (int r = 0; r < K; ++r)
+      if (!lst.push(pa[r * T + i] + s, i * kNbestMax + r, K)) break;
+  }
+  float fv = -INFINITY;
+  int fk = 0;
+  for (int k = 0; k < K; ++k) {
+    float v = lst.v[0];
+    int key = lst.key[0];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, v, o);
+      const int ok = __shfl_xor_sync(0xffffffffu, key, o);
+      if (nbest_above(ov, ok, v, key)) {
+        v = ov;
+        key = ok;
+      }
+    }
+    if (lane == k) {
+      fv = v;
+      fk = key;
+    }
+    if (v != -INFINITY && key == lst.key[0]) lst.pop();     // keys are distinct: exactly one lane pops
+  }
+  if (lane < K) {
+    scores[(size_t)b * K + lane] = fv;
+    if (fv == -INFINITY) {
+      for (int t = 0; t < n; ++t) pth[(size_t)t * K + lane] = -1;
+    } else {
+      int j = fk / kNbestMax, r = fk % kNbestMax;
+      for (int t = n - 1; t >= 0; --t) {
+        pth[(size_t)t * K + lane] = j;
+        if (t > 0) {
+          const int key = bpb[(size_t)t * K * T + r * T + j];
+          j = key / kNbestMax;
+          r = key % kNbestMax;
+        }
+      }
+    }
+  }
+  for (int e = n * K + lane; e < L * K; e += 32) pth[e] = 0;
+}
+
+// ---- tag marginals --------------------------------------------------------------------------------------------------
+// exact log-domain LSE_j((tri[j] + feat_t[j]) + beta[j]) of row i (the expressions of crf_backward_row_exact)
+__device__ __forceinline__ float crf_row_lse(const float* tri, const float* ft, const float* beta, int T) {
+  float mx = -INFINITY;
+  for (int j = 0; j < T; ++j) mx = fmaxf(mx, (tri[j] + __ldg(ft + j)) + beta[j]);
+  float sm = 0.f;
+  for (int j = 0; j < T; ++j) sm += expf(((tri[j] + __ldg(ft + j)) + beta[j]) - mx);
+  return mx + logf(sm);
+}
+
+// marg[b,t,j] = P(y_t = j | x) = exp(part_t[j] + beta_t[j] - logZ) by the backward (beta) sweep alone, one warp per
+// sequence, from the forward partitions re2nn_crf_nll saved.  Without the pairwise T x T accumulators of the training
+// backward (which hold it to seven sequences per SM and T <= 225), a CTA holds eight sequences and the tag set is not
+// limited by them.  EXP: the scaled-exponential rows of crf_nll_backward_exp_kernel (lanes own rows of the table
+// exp(trans[i][j] - rmax[i]), odd pitch: conflict-free), an underflowing row is evaluated exactly in the log domain;
+// otherwise (tables beyond shared memory) every row is evaluated in the log domain from the global transition matrix.
+// dynamic smem: (EXP: trans T*T | table T*Tq | rmax Tp) | per warp beta a / b, W (3 * Tp)
+template <bool EXP>
+__global__ void __launch_bounds__(kCrfWarps * 32) crf_marginal_kernel(
+    const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len,
+    const float* __restrict__ part_save, int B, int L, int T, float* __restrict__ marg, float* __restrict__ log_z) {
+  extern __shared__ float smem[];
+  const int nw = blockDim.x >> 5;
+  const int Tp = (T + 31) & ~31, Tq = T | 1;
+  float* tr = smem;
+  float* te = tr + (EXP ? T * T : 0);
+  float* rmax = te + (EXP ? T * Tq : 0);
+  float* s_vec = rmax + (EXP ? Tp : 0);
+  if (EXP) crf_exp_row_table(trans_g, T, Tp, Tq, tr, te, rmax);
+  const float* trr = EXP ? tr : trans_g;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.x * nw + warp;
+  if (b >= B) return;
+  const int n = min((int)len[b], L);
+  float* mb = marg + (size_t)b * L * T;
+  crf_zero_rows(mb, max(n, 0), L, T, lane, 32);
+  if (n <= 0) {      // log Z of an empty sequence is 0, as re2nn_crf_nll has it
+    if (lane == 0) log_z[b] = 0.f;
+    return;
+  }
+  float* ba = s_vec + warp * 3 * Tp;   // beta_t
+  float* bb = ba + Tp;                 // beta_{t-1}
+  float* W = bb + Tp;
+  const float* fb = feats + (size_t)b * L * T;
+  const float* ps = part_save + (size_t)b * L * T;
+  const float logZ = crf_log_z(trr, ps + (size_t)(n - 1) * T, T, lane);
+  if (lane == 0) log_z[b] = logZ;
+  for (int i = lane; i < T; i += 32) ba[i] = trr[i * T + (T - 1)];   // beta_{n-1}[i] = trans[i][STOP]
+  __syncwarp();
+  for (int t = n - 1;; --t) {
+    const float* pt = ps + (size_t)t * T;
+    for (int j = lane; j < T; j += 32) mb[(size_t)t * T + j] = expf(pt[j] + ba[j] - logZ);
+    if (t == 0) break;
+    const float* ft = fb + (size_t)t * T;
+    if (EXP) {
+      float Mw = -INFINITY;
+      for (int j = lane; j < T; j += 32) Mw = fmaxf(Mw, __ldg(ft + j) + ba[j]);
+      Mw = warp_max(Mw);
+      for (int j = lane; j < T; j += 32) W[j] = expf((__ldg(ft + j) + ba[j]) - Mw);
+      __syncwarp();
+      for (int i = lane; i < T; i += 32) {
+        const float* tei = te + i * Tq;
+        float S = 0.f;
+        for (int j = 0; j < T; ++j) S = fmaf(tei[j], W[j], S);
+        bb[i] = S > 1e-30f ? (rmax[i] + Mw) + logf(S) : crf_row_lse(tr + i * T, ft, ba, T);
+      }
+    } else {
+      for (int i = lane; i < T; i += 32) bb[i] = crf_row_lse(trans_g + (size_t)i * T, ft, ba, T);
+    }
+    __syncwarp();
+    float* tmp = ba; ba = bb; bb = tmp;
+  }
+}
+
 // deterministic sum of n floats (double accumulation), scaled
 __global__ void __launch_bounds__(1024) reduce_sum_kernel(const float* __restrict__ v, size_t n, double scale,
                                                           float* __restrict__ out) {
@@ -1089,7 +1346,7 @@ int re2nn_debug_set_viterbi_seqs(int ns) {
 
 int re2nn_crf_nll(const float* feats, const float* transitions, const int64_t* lengths, const int64_t* tags, int B,
                   int L, int Ltags, int T, float* per_seq, float* loss, float* part_save, void* stream) {
-  RE2NN_CHECK(feats && transitions && lengths && tags && per_seq, "crf_nll: null tensor");
+  RE2NN_CHECK(feats && transitions && lengths && per_seq, "crf_nll: null tensor");
   RE2NN_CHECK(B > 0 && L > 0 && T >= 3, "crf_nll: bad dims");
   using Kernel = decltype(&crf_nll_kernel<true>);
   static const Kernel kernels[7] = {crf_nll_exp_kernel<1>, crf_nll_exp_kernel<2>, crf_nll_exp_kernel<3>,
@@ -1167,6 +1424,56 @@ int re2nn_crf_nll_backward(const float* feats, const float* transitions, const i
   RE2NN_CUDA(cudaMemsetAsync(dtrans, 0, tr_bytes, st));
   return crf_launch(kernels[k], configured[k], cdiv(B, nseq), block, smem, st, feats, transitions, lengths, tags,
                     part_save, gscale, B, L, Ltags, T, dfeats, dtrans);
+}
+
+size_t re2nn_crf_nbest_workspace(int B, int L, int T, int K) {
+  if (B <= 0 || L <= 0 || T <= 0 || K <= 0) return 0;
+  return (size_t)B * L * T * K * sizeof(uint16_t);
+}
+
+int re2nn_crf_nbest(const float* feats, const float* transitions, const int64_t* lengths, int B, int L, int T, int K,
+                    int64_t* paths, float* scores, void* ws, size_t ws_bytes, void* stream) {
+  RE2NN_CHECK(B > 0 && L > 0 && T >= 3, "crf_nbest: bad dims B=%d L=%d T=%d", B, L, T);
+  RE2NN_CHECK(K >= 1 && K <= kNbestMax, "crf_nbest: nbest K = %d outside [1, %d]", K, kNbestMax);
+  const size_t lists = (size_t)2 * K * T * sizeof(float);     // one sequence's two K-lists
+  RE2NN_CHECK(T <= kNbestMaxT && lists <= kSmemLimit,
+              "crf_nbest: T x K = %d x %d too large (limit: T <= %d and T * K <= %d, one sequence's K-lists in shared "
+              "memory)", T, K, kNbestMaxT, (int)(kSmemLimit / (2 * sizeof(float))));
+  RE2NN_CHECK(feats && transitions && lengths && paths && scores && ws, "crf_nbest: null tensor");
+  const size_t need = re2nn_crf_nbest_workspace(B, L, T, K);
+  RE2NN_CHECK(ws_bytes >= need, "crf_nbest: workspace too small (%zu < %zu bytes)", ws_bytes, need);
+  using Kernel = decltype(&crf_nbest_kernel<1>);
+  static const Kernel kernels[5] = {crf_nbest_kernel<1>, crf_nbest_kernel<2>, crf_nbest_kernel<4>, crf_nbest_kernel<8>,
+                                    crf_nbest_kernel<16>};
+  static int configured[5][kMaxDevices];
+  const int km = K <= 1 ? 0 : K <= 2 ? 1 : K <= 4 ? 2 : K <= 8 ? 3 : 4;
+  const size_t tr_bytes = (size_t)T * T * sizeof(float);
+  const bool ts = tr_bytes + lists <= kSmemLimit;          // transitions in shared memory as long as one warp still fits
+  const int nw = (int)std::min<size_t>(kCrfWarps, (kSmemLimit - (ts ? tr_bytes : 0)) / lists);
+  const size_t smem = (ts ? tr_bytes : 0) + nw * lists;
+  return crf_launch(kernels[km], configured[km], cdiv(B, nw), nw * 32, smem, (cudaStream_t)stream, feats, transitions,
+                    lengths, B, L, T, K, ts ? 1 : 0, paths, scores, (uint16_t*)ws);
+}
+
+int re2nn_crf_marginals(const float* feats, const float* transitions, const int64_t* lengths, int B, int L, int T,
+                        float* marginals, float* log_z, float* part_ws, void* stream) {
+  RE2NN_CHECK(feats && transitions && lengths && marginals && log_z && part_ws, "crf_marginals: null tensor");
+  RE2NN_CHECK(B > 0 && L > 0 && T >= 3, "crf_marginals: bad dims B=%d L=%d T=%d", B, L, T);
+  using Kernel = decltype(&crf_marginal_kernel<true>);
+  static const Kernel kernels[2] = {crf_marginal_kernel<true>, crf_marginal_kernel<false>};
+  static int configured[2][kMaxDevices];
+  const int Tp = (T + 31) & ~31, Tq = T | 1;
+  const size_t per_warp = (size_t)3 * Tp * sizeof(float);
+  const size_t exp_smem = ((size_t)T * T + (size_t)T * Tq + Tp) * sizeof(float) + kCrfWarps * per_warp;
+  const int k = exp_smem <= kSmemLimit ? 0 : 1;
+  const int nw = k == 0 ? kCrfWarps : (int)std::min<size_t>(kCrfWarps, kSmemLimit / per_warp);
+  RE2NN_CHECK(nw >= 1, "crf_marginals: tag set too large (T=%d)", T);
+  const size_t smem = k == 0 ? exp_smem : nw * per_warp;
+  // forward partitions (and log Z) from the loss kernels' sweep, without a gold score
+  if (int rc = re2nn_crf_nll(feats, transitions, lengths, nullptr, B, L, 0, T, log_z, nullptr, part_ws, stream))
+    return rc;
+  return crf_launch(kernels[k], configured[k], cdiv(B, nw), nw * 32, smem, (cudaStream_t)stream, feats, transitions,
+                    lengths, (const float*)part_ws, B, L, T, marginals, log_z);
 }
 
 int re2nn_argmax_decode(const float* scores, const int64_t* lengths, const int64_t* offsets, int B, int L, int C,

@@ -6,7 +6,7 @@
 // carrying re2nn_last_error().  The op set is the one SURVEY.md section 8b proposes for the reference's modules
 // (farnn/model_decompose_single.py:207-304, farnn/model_onehot.py:351-428, baselines/crf.py:48-260):
 //   re2nn::ifst_decompose_forward, re2nn::ifst_onehot_forward, re2nn::label_scores, re2nn::argmax_decode,
-//   re2nn::crf_viterbi, re2nn::crf_nll, re2nn::crf_nll_backward.
+//   re2nn::crf_viterbi, re2nn::crf_nll, re2nn::crf_nll_backward; beyond it re2nn::crf_nbest, re2nn::crf_marginals.
 // Built by re2nn_seq_b200/build.py into re2nn_seq_b200/libre2nn_torch.so (links libre2nn_b200.so, rpath $ORIGIN).
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
@@ -177,6 +177,32 @@ std::tuple<Tensor, Tensor> crf_nll_backward(const Tensor& feats, const Tensor& t
   return {dfeats, dtrans};
 }
 
+// NCRF++ CRF._viterbi_decode_nbest -> (paths B x L x K int64, scores B x K)
+std::tuple<Tensor, Tensor> crf_nbest(const Tensor& feats, const Tensor& transitions, const Tensor& lengths, int64_t nbest) {
+  c10::cuda::CUDAGuard guard(feats.device());
+  const int64_t B = feats.size(0), L = feats.size(1), T = feats.size(2);
+  Tensor paths = at::empty({B, L, nbest}, feats.options().dtype(at::kLong));
+  Tensor scores = at::empty({B, nbest}, feats.options());
+  const size_t need = re2nn_crf_nbest_workspace((int)B, (int)L, (int)T, (int)nbest);
+  Tensor ws = bytes(need, feats);
+  fail(re2nn_crf_nbest(f32(feats, "feats"), f32(transitions, "transitions"), i64(lengths, "lengths"), (int)B, (int)L, (int)T,
+                       (int)nbest, paths.data_ptr<int64_t>(), scores.data_ptr<float>(), ws.data_ptr(), need, stream()),
+       "crf_nbest");
+  return {paths, scores};
+}
+
+// tag marginals P(y_t = j | x) -> (marginals B x L x T, log Z B)
+std::tuple<Tensor, Tensor> crf_marginals(const Tensor& feats, const Tensor& transitions, const Tensor& lengths) {
+  c10::cuda::CUDAGuard guard(feats.device());
+  const int64_t B = feats.size(0), L = feats.size(1), T = feats.size(2);
+  Tensor marg = at::empty({B, L, T}, feats.options()), log_z = at::empty({B}, feats.options());
+  Tensor part = at::empty({B, L, T}, feats.options());
+  fail(re2nn_crf_marginals(f32(feats, "feats"), f32(transitions, "transitions"), i64(lengths, "lengths"), (int)B, (int)L,
+                           (int)T, marg.data_ptr<float>(), log_z.data_ptr<float>(), part.data_ptr<float>(), stream()),
+       "crf_marginals");
+  return {marg, log_z};
+}
+
 int64_t abi_version() { return re2nn_abi_version(); }
 
 }  // namespace
@@ -196,6 +222,8 @@ TORCH_LIBRARY(re2nn, m) {
   m.def("crf_nll(Tensor feats, Tensor transitions, Tensor lengths, Tensor tags, bool save) -> (Tensor, Tensor, Tensor)");
   m.def("crf_nll_backward(Tensor feats, Tensor transitions, Tensor lengths, Tensor tags, Tensor part, Tensor gscale) -> "
         "(Tensor, Tensor)");
+  m.def("crf_nbest(Tensor feats, Tensor transitions, Tensor lengths, int nbest) -> (Tensor paths, Tensor scores)");
+  m.def("crf_marginals(Tensor feats, Tensor transitions, Tensor lengths) -> (Tensor marginals, Tensor log_z)");
   m.def("abi_version() -> int", &abi_version);
 }
 
@@ -207,4 +235,6 @@ TORCH_LIBRARY_IMPL(re2nn, CUDA, m) {
   m.impl("crf_viterbi", &crf_viterbi);
   m.impl("crf_nll", &crf_nll);
   m.impl("crf_nll_backward", &crf_nll_backward);
+  m.impl("crf_nbest", &crf_nbest);
+  m.impl("crf_marginals", &crf_marginals);
 }

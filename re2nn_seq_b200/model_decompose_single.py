@@ -157,6 +157,32 @@ class _DecomposeBase(nn.Module):
                                             threshold=self.args.threshold, o_idx=self.o_idx, flat_out=_flat_out)
         return flat
 
+    def forward_nbest(self, input, lengths, nbest=1):
+        """N-best CRF decoding with confidences -> (pred B x L x K int64, seq_prob B x K, marginals B x L x C).
+        pred[..., 0] is what forward_local decodes (padded, in the caller's order; -1 marks a rank with no sequence,
+        pads are 0), seq_prob[:, k] = P(path k | x) and marginals[b, t, c] = P(y_t = c | x), zero at pads.  Under CE1
+        decode's clamp of column C-3 to the threshold applies to both, and tag C-3 is reported as o_idx in pred.
+        Eager (no graph capture), no gradient."""
+        if not self.use_crf:
+            raise NotImplementedError("forward_nbest needs a CRF head (use_crf=1); %s decodes per position"
+                                      % type(self).__name__)
+        with torch.no_grad():
+            dev = self._device()
+            lengths = lengths.to(dev).contiguous()
+            sc = self.forward_scores(input, lengths).detach().contiguous()
+            ce1 = self.args.local_loss_func == 'CE1'
+            if ce1:
+                sc = sc.clone()
+                sc[:, :, self.C - 3] = torch.minimum(sc[:, :, self.C - 3], sc.new_tensor(self.args.threshold))
+            trans = self.crf.transitions.detach()
+            pred, score = ops.crf_nbest(sc, trans, lengths, nbest)
+            marg, log_z = ops.crf_marginals(sc, trans, lengths)
+            if ce1:
+                valid = get_length_mask(lengths, sc.shape[1])[:, :, None]
+                pred = torch.where(valid & (pred == self.C - 3), torch.full_like(pred, self.o_idx), pred)
+            seq_prob = torch.exp(score - log_z[:, None])
+        return pred, seq_prob, marg
+
     # ---- loss + decode tail shared by forward_local / forward (model_decompose_single.py:271-304) ---
     def _length_order(self, lengths, re_tags, L=None):
         """Process sequences longest-first so 128-row tiles finish together and are skipped once all their rows

@@ -296,6 +296,25 @@ def crf_nll_backward(feats, transitions, lengths, tags, part, gscale):
     return dfeats, dtrans
 
 
+def crf_nbest(feats, transitions, lengths, nbest):
+    """K-best Viterbi -> (paths B x L x K int64, scores B x K): rank 0 is crf_viterbi's path; a missing rank has
+    score -inf and path -1 at valid positions; pads hold 0."""
+    for t in (feats, transitions, lengths):
+        _p(t)
+    paths, scores = tops.crf_nbest(feats, transitions, lengths, int(nbest))
+    _count(1)
+    return paths, scores
+
+
+def crf_marginals(feats, transitions, lengths):
+    """Tag marginals -> (P(y_t = j | x) B x L x T, zero at pads; log Z B)."""
+    for t in (feats, transitions, lengths):
+        _p(t)
+    marg, log_z = tops.crf_marginals(feats, transitions, lengths)
+    _count(2)
+    return marg, log_z
+
+
 def ce_loss(scores, lengths, labels, n_total):
     B, L, Cn = scores.shape
     per_pos = torch.empty((B * L,), dtype=torch.float32, device=scores.device)

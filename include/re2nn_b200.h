@@ -382,6 +382,28 @@ int re2nn_crf_nll_backward(const float* feats, const float* transitions, const i
                            const int64_t* tags, const float* part_save, const float* gscale,
                            int B, int L, int Ltags, int T, float* dfeats, float* dtrans, void* stream);
 
+/* ---- CRF partial-annotation loss --------------------------------------------------------------------------
+ * no counterpart in the reference; the partial-label likelihood of Tsuboi et al. (COLING 2008).  allowed is a
+ * B x L x T byte mask (bool / uint8, nonzero = allowed; T = tagset+2, START / STOP columns included): position t of
+ * sequence b may only take the tags j with allowed[b,t,j] set; positions at or past the (clamped) length are ignored.
+ * per_seq[b] = logZ_b - logZ^A_b, where logZ^A is logZ over only the paths that satisfy the mask, with the path score
+ * of re2nn_crf_nll; *loss = sum_b per_seq[b] (loss may be NULL).  A one-hot mask of the gold tags gives the
+ * re2nn_crf_nll loss, an all-true mask gives exactly 0 (the two partitions are the same float operations), an empty
+ * sequence 0.  Every valid position needs at least one allowed tag (else log Z^A is -inf); callers check that.
+ * part_save / part_save_allowed (B x L x T each, both or neither) keep the free and the constrained forward partitions
+ * for the backward.  Same tag-set range as re2nn_crf_nll. */
+int re2nn_crf_partial_nll(const float* feats, const float* transitions, const int64_t* lengths, const uint8_t* allowed,
+                          int B, int L, int T, float* per_seq, float* loss, float* part_save, float* part_save_allowed,
+                          void* stream);
+
+/* d loss / d feats = gs * (P(y_t=j) - P_A(y_t=j)) (zero at pads) and d loss / d transitions = gs * sum_t
+ * (P(y_{t-1}=i, y_t=j) - P_A(...)) (START row and STOP column included), scaled by *gscale, from one sweep over both
+ * lattices.  An all-true mask gives exactly zero.  T <= 225, as re2nn_crf_nll_backward ("tag set too large"). */
+int re2nn_crf_partial_nll_backward(const float* feats, const float* transitions, const int64_t* lengths,
+                                   const uint8_t* allowed, const float* part_save, const float* part_save_allowed,
+                                   const float* gscale, int B, int L, int T, float* dfeats, float* dtrans,
+                                   void* stream);
+
 /* ---- CRF N-best decoding and tag marginals ---------------------------------------------------------------
  * no counterpart in the reference's cut-down crf.py; NCRF++'s CRF._viterbi_decode_nbest returns the same K-lists.
  * Tags run over all T columns (START / STOP included) as in re2nn_crf_viterbi, and a path is scored with its

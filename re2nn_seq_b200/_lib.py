@@ -145,6 +145,8 @@ SYMBOLS = {
     're2nn_crf_viterbi': (C.c_int, [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, f32, i64, vp, vp, vp, vp]),
     're2nn_crf_nll': (C.c_int, [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp]),
     're2nn_crf_nll_backward': (C.c_int, [vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
+    're2nn_crf_partial_nll': (C.c_int, [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, vp]),
+    're2nn_crf_partial_nll_backward': (C.c_int, [vp, vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, vp]),
     're2nn_crf_nbest_workspace': (sz, [C.c_int, C.c_int, C.c_int, C.c_int]),
     're2nn_crf_nbest': (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, sz, vp]),
     're2nn_crf_marginals': (C.c_int, [vp, vp, vp, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp]),

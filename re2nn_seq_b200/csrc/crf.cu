@@ -18,6 +18,12 @@
 //   re2nn_crf_nbest          crf_nbest_kernel<KM> (KM = K rounded up to a power of two), transitions in shared memory
 //                            while they fit next to one sequence's lists; T <= 4096 and T * K <= 25600, else an error
 //   re2nn_crf_marginals      re2nn_crf_nll without tags, then 3-153 crf_marginal_kernel<true>, >= 154 <false>
+//   re2nn_crf_partial_nll    the ranges of re2nn_crf_nll with PARTIAL = true: crf_nll_exp_kernel<NJ, true>,
+//                            crf_nll_kernel<TS, true> (>= 219: fewer than eight warps once four partitions of each do not
+//                            fit kSmemAll)
+//   re2nn_crf_partial_nll_backward  the ranges and split switch of re2nn_crf_nll_backward with PARTIAL = true (three more
+//                            Tp vectors per sequence, two in the log domain; sized against kSmemAll); >= 226 error
+//   constrained decoding     re2nn_crf_viterbi on the scores with -inf in the disallowed cells (every step is a max)
 #include <algorithm>
 
 #include "common.cuh"
@@ -326,6 +332,14 @@ __device__ __forceinline__ void crf_store_nll(const float* tr, const float* part
   }
 }
 
+// per_seq = logZ - logZ^A: the partial-annotation loss from the free and the constrained last partitions, one warp
+__device__ __forceinline__ void crf_store_partial(const float* tr, const float* part, const float* part_a, int T,
+                                                  int lane, float* per_seq) {
+  const float logZ = crf_log_z(tr, part, T, lane);
+  const float logZa = crf_log_z(tr, part_a, T, lane);
+  if (lane == 0) *per_seq = logZ - logZa;
+}
+
 // exact log-domain LSE_i((f + trans[i][j]) + part[i]) of column j
 __device__ __forceinline__ float crf_column_lse(const float* tr, const float* part, float f, int j, int T) {
   float m = -INFINITY;
@@ -348,6 +362,44 @@ __device__ __forceinline__ float crf_backward_row_exact(const float* tri, const 
     dwi[j] += gs * expf(pi + e);
   }
   return mx + logf(sm);
+}
+
+// exact log-domain LSE_j((tri[j] + feat_t[j]) + beta[j]) of row i (the expressions of crf_backward_row_exact)
+__device__ __forceinline__ float crf_row_lse(const float* tri, const float* ft, const float* beta, int T) {
+  float mx = -INFINITY;
+  for (int j = 0; j < T; ++j) mx = fmaxf(mx, (tri[j] + __ldg(ft + j)) + beta[j]);
+  float sm = 0.f;
+  for (int j = 0; j < T; ++j) sm += expf(((tri[j] + __ldg(ft + j)) + beta[j]) - mx);
+  return mx + logf(sm);
+}
+
+// Backward row i of the partial-annotation loss, general form: dwi[j] += P(i,j) - P_A(i,j), each pairwise marginal
+// (times gs) a rounded value of its own lattice.  A lattice whose row sum did not underflow (fe / fa) uses the
+// scaled-exponential form __fmul_rn(A * table[i][j], W_j); otherwise the exact form gs * exp(pi + e_ij),
+// e_ij = (trans[i][j] + feat_t[j]) + beta_t[j].  The products are rounded before they are subtracted (no FMA
+// contraction), so two identical lattices add exact zeros.  A tag i masked at t-1 has pia = -inf and adds no P_A.
+// The log-domain kernel passes fe = fa = false (tei, W, WA unused).
+__device__ __forceinline__ void crf_partial_row_pairs(const float* tri, const float* tei, const float* ft,
+                                                      const float* ba, const float* ca, const float* W,
+                                                      const float* WA, float A, float AA, float pi, float pia,
+                                                      bool fe, bool fa, float gs, float* dwi, int T) {
+  for (int j = 0; j < T; ++j) {
+    const float f = __ldg(ft + j);
+    const float p = fe ? __fmul_rn(A * tei[j], W[j]) : __fmul_rn(gs, expf(pi + ((tri[j] + f) + ba[j])));
+    const float q = fa ? __fmul_rn(AA * tei[j], WA[j]) : __fmul_rn(gs, expf(pia + ((tri[j] + f) + ca[j])));
+    dwi[j] += p - q;
+  }
+}
+
+// Lanes 8-13 of the partial backward's prefetch: the constrained partition row t-2 (four 128-byte lines) and the mask
+// row t-1 (T bytes, two lines) of the next step into L1
+__device__ __forceinline__ void crf_prefetch_partial(const float* qs, const uint8_t* ab, int t, int T, int lane) {
+  const int part = (lane & 3) * 32;
+  if (lane < 12) {
+    if (part < T) asm volatile("prefetch.global.L1 [%0];" ::"l"(qs + (size_t)(t >= 2 ? t - 2 : 0) * T + part));
+  } else if ((lane - 12) * 128 < T) {
+    asm volatile("prefetch.global.L1 [%0];" ::"l"(ab + (size_t)(t - 1) * T + (lane - 12) * 128));
+  }
 }
 
 // Shared-memory tables of the scaled-exponential backward kernels, built by the whole CTA: tr = trans_g (T x T),
@@ -389,13 +441,19 @@ __device__ __forceinline__ void crf_fold_dtrans(const float* s_dtr, int nacc, in
 }
 
 // log-partition + gold score.  per_seq[b] = logZ_b - gold_b.   (crf.py:48-99, 202-251)
-template <bool TS>
+// PARTIAL: the partial-annotation loss per_seq[b] = logZ_b - logZ^A_b instead of the gold score.  The same sweep carries
+// a second partition over only the paths that keep every position t on a tag j with allowed[b, t, j] set: a masked
+// tag's constrained partition is exactly -inf (never computed), an allowed one is evaluated with the free partition's
+// own expressions, so an all-true mask reproduces the free partitions bit for bit and per_seq = 0.  part_save_allowed
+// keeps the constrained history next to part_save.
+template <bool TS, bool PARTIAL>
 __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_kernel(
     const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len,
     const int64_t* __restrict__ tags, int B, int L, int Ltags, int T, float* __restrict__ per_seq,
-    float* __restrict__ part_save) {
+    float* __restrict__ part_save, const uint8_t* __restrict__ allowed, float* __restrict__ part_save_allowed) {
   extern __shared__ float smem[];
   const int Tp = (T + 31) & ~31;
+  const int nw = PARTIAL ? blockDim.x >> 5 : kCrfWarps;   // the partial loss runs fewer warps once four vectors are large
   float* s_trans = smem;
   float* s_part = smem + (TS ? T * T : 0);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -404,22 +462,31 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_kernel(
     __syncthreads();
   }
   const float* tr = TS ? s_trans : trans_g;
-  const int b = blockIdx.x * kCrfWarps + warp;
+  const int b = blockIdx.x * nw + warp;
   if (b >= B) return;
   const int n = min((int)len[b], L);      // lengths past the row are clamped
   if (n <= 0) {                           // an empty sequence contributes nothing (the reference cannot express it)
     if (lane == 0) per_seq[b] = 0.f;
     return;
   }
-  float* pa = s_part + warp * 2 * Tp;
+  float* pa = s_part + warp * (PARTIAL ? 4 : 2) * Tp;
   float* pb = pa + Tp;
+  float* qa = pb + Tp;                    // constrained partitions (PARTIAL)
+  float* qb = qa + Tp;
   const float* fb = feats + (size_t)b * L * T;
   float* ps = part_save ? part_save + (size_t)b * L * T : nullptr;
+  const uint8_t* ab = PARTIAL ? allowed + (size_t)b * L * T : nullptr;
+  float* qs = PARTIAL && part_save_allowed ? part_save_allowed + (size_t)b * L * T : nullptr;
 
   for (int j = lane; j < T; j += 32) {
     float v = __ldg(fb + j) + tr[(T - 2) * T + j];
     pa[j] = v;
     if (ps) ps[j] = v;
+    if (PARTIAL) {
+      const float w = __ldg(ab + j) ? v : -INFINITY;
+      qa[j] = w;
+      if (qs) qs[j] = w;
+    }
   }
   __syncwarp();
   for (int t = 1; t < n; ++t) {
@@ -428,11 +495,20 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_kernel(
       const float v = crf_column_lse(tr, pa, __ldg(ft + j), j, T);
       pb[j] = v;
       if (ps) ps[(size_t)t * T + j] = v;
+      if (PARTIAL) {
+        const float w = __ldg(ab + (size_t)t * T + j) ? crf_column_lse(tr, qa, __ldg(ft + j), j, T) : -INFINITY;
+        qb[j] = w;
+        if (qs) qs[(size_t)t * T + j] = w;
+      }
     }
     __syncwarp();
     float* tmp = pa; pa = pb; pb = tmp;
+    tmp = qa; qa = qb; qb = tmp;
   }
-  crf_store_nll(tr, pa, fb, tags ? tags + (size_t)b * Ltags : nullptr, n, T, lane, per_seq + b);
+  if (PARTIAL)
+    crf_store_partial(tr, pa, qa, T, lane, per_seq + b);
+  else
+    crf_store_nll(tr, pa, fb, tags ? tags + (size_t)b * Ltags : nullptr, n, T, lane, per_seq + b);
 }
 
 // Same log-partition in the scaled exponential domain: with M = max_i part[i] and cmax[j] = max_i trans[i][j]
@@ -441,12 +517,14 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_kernel(
 // per (t, j); this one ~100).  exp(trans - cmax) is tabulated once per CTA.  A column whose sum underflows (only
 // reachable from states that are e^-87 below the best one, e.g. hard-constrained transitions) falls back to the
 // exact two-pass form for that (t, j), so the result stays within fp32 rounding of the log-domain kernel.
-// dynamic smem: trans T*T | exp table T*T | cmax Tp | per warp: part a, part b, E (3 * Tp)
-template <int NJ>
+// PARTIAL: the constrained partition of crf_nll_kernel<., true> rides along with its own maximum, E vector and column
+// sums over the same exp(trans - cmax) table, operation for operation as the free one.
+// dynamic smem: trans T*T | exp table T*T | cmax Tp | per warp: part a, part b, E (3 * Tp) [, constrained a, b, E]
+template <int NJ, bool PARTIAL>
 __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
     const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len,
     const int64_t* __restrict__ tags, int B, int L, int Ltags, int T, float* __restrict__ per_seq,
-    float* __restrict__ part_save) {
+    float* __restrict__ part_save, const uint8_t* __restrict__ allowed, float* __restrict__ part_save_allowed) {
   extern __shared__ float smem[];
   const int Tp = (T + 31) & ~31;
   float* tr = smem;
@@ -472,31 +550,46 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
     if (lane == 0) per_seq[b] = 0.f;
     return;
   }
-  float* pa = s_part + warp * 3 * Tp;
+  float* pa = s_part + warp * (PARTIAL ? 6 : 3) * Tp;
   float* pb = pa + Tp;
   float* E = pb + Tp;
+  float* qa = E + Tp;                     // constrained partitions and their E vector (PARTIAL)
+  float* qb = qa + Tp;
+  float* EA = qb + Tp;
   const float* fb = feats + (size_t)b * L * T;
   float* ps = part_save ? part_save + (size_t)b * L * T : nullptr;
+  const uint8_t* ab = PARTIAL ? allowed + (size_t)b * L * T : nullptr;
+  float* qs = PARTIAL && part_save_allowed ? part_save_allowed + (size_t)b * L * T : nullptr;
 
   for (int j = lane; j < Tp; j += 32) {
-    float v = -INFINITY;
+    float v = -INFINITY, w = -INFINITY;
     if (j < T) {
       v = __ldg(fb + j) + tr[(T - 2) * T + j];
       if (ps) ps[j] = v;
+      if (PARTIAL) {
+        w = __ldg(ab + j) ? v : -INFINITY;
+        if (qs) qs[j] = w;
+      }
     }
     pa[j] = v;
+    if (PARTIAL) qa[j] = w;
   }
   __syncwarp();
   for (int t = 1; t < n; ++t) {
     const float* ft = fb + (size_t)t * T;
-    float M = -INFINITY;
+    float M = -INFINITY, MA = -INFINITY;
     for (int i = lane; i < T; i += 32) M = fmaxf(M, pa[i]);
     M = warp_max(M);
     for (int i = lane; i < Tp; i += 32) E[i] = i < T ? expf(pa[i] - M) : 0.f;
+    if (PARTIAL) {
+      for (int i = lane; i < T; i += 32) MA = fmaxf(MA, qa[i]);
+      MA = warp_max(MA);
+      for (int i = lane; i < Tp; i += 32) EA[i] = i < T ? expf(qa[i] - MA) : 0.f;
+    }
     __syncwarp();
-    float acc[NJ];
+    float acc[NJ], accA[NJ];
 #pragma unroll
-    for (int q = 0; q < NJ; ++q) acc[q] = 0.f;
+    for (int q = 0; q < NJ; ++q) acc[q] = accA[q] = 0.f;
     // lanes whose last slot falls past T read (and ignore) the following shared-memory words
 #pragma unroll 5
     for (int i = 0; i < T; ++i) {
@@ -504,6 +597,11 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
       const float* tei = te + i * T + lane;
 #pragma unroll
       for (int q = 0; q < NJ; ++q) acc[q] = fmaf(e, tei[32 * q], acc[q]);
+      if (PARTIAL) {
+        const float ea = EA[i];
+#pragma unroll
+        for (int q = 0; q < NJ; ++q) accA[q] = fmaf(ea, tei[32 * q], accA[q]);
+      }
     }
 #pragma unroll
     for (int q = 0; q < NJ; ++q) {
@@ -514,12 +612,23 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
         const float v = acc[q] > 1e-30f ? ((M + cmax[j]) + f) + logf(acc[q]) : crf_column_lse(tr, pa, f, j, T);
         pb[j] = v;
         if (ps) ps[(size_t)t * T + j] = v;
+        if (PARTIAL) {
+          float w = -INFINITY;
+          if (__ldg(ab + (size_t)t * T + j))
+            w = accA[q] > 1e-30f ? ((MA + cmax[j]) + f) + logf(accA[q]) : crf_column_lse(tr, qa, f, j, T);
+          qb[j] = w;
+          if (qs) qs[(size_t)t * T + j] = w;
+        }
       }
     }
     __syncwarp();
     float* tmp = pa; pa = pb; pb = tmp;
+    tmp = qa; qa = qb; qb = tmp;
   }
-  crf_store_nll(tr, pa, fb, tags ? tags + (size_t)b * Ltags : nullptr, n, T, lane, per_seq + b);
+  if (PARTIAL)
+    crf_store_partial(tr, pa, qa, T, lane, per_seq + b);
+  else
+    crf_store_nll(tr, pa, fb, tags ? tags + (size_t)b * Ltags : nullptr, n, T, lane, per_seq + b);
 }
 
 // CRF backward: marginals by the backward recursion, reusing the saved forward partitions.
@@ -527,18 +636,23 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nll_exp_kernel(
 // Every warp owns a private T x T accumulator in shared memory (row pitch padded to an odd number of words:
 // lanes own rows, so the pitch decides the bank) => plain read-modify-write, no shared atomics; the CTA folds
 // its warps' copies together and issues one global atomicAdd per element.
-template <bool TS>
+// PARTIAL (gradient of the partial-annotation loss): the same sweep runs the constrained beta recursion next to the free
+// one, over the constrained partitions part_save_allowed, and writes P - P_A in place of P - [gold]:
+//   dfeats[b,t,j] = gs * (P(y_t=j) - P_A(y_t=j));  dtrans[i,j] += gs * sum_t (P(y_{t-1}=i,y_t=j) - P_A(...)).
+// The constrained beta of a tag masked at its position is -inf (never computed).
+template <bool TS, bool PARTIAL>
 __global__ void crf_nll_backward_kernel(
     const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len,
     const int64_t* __restrict__ tags, const float* __restrict__ part_save, const float* __restrict__ gscale, int B,
-    int L, int Ltags, int T, float* __restrict__ dfeats, float* __restrict__ dtrans) {
+    int L, int Ltags, int T, float* __restrict__ dfeats, float* __restrict__ dtrans, const uint8_t* __restrict__ allowed,
+    const float* __restrict__ part_save_allowed) {
   extern __shared__ float smem[];
   const int nw = blockDim.x >> 5;
   const int Tp = (T + 31) & ~31;
   const int Tq = T | 1;                          // odd pitch of the private accumulators
   float* s_trans = smem;                         // T*T (if TS)
   float* s_dtr = smem + (TS ? T * T : 0);        // nw * T * Tq
-  float* s_beta = s_dtr + (size_t)nw * T * Tq;   // nw * 2 * Tp
+  float* s_beta = s_dtr + (size_t)nw * T * Tq;   // nw * 2 * Tp (PARTIAL: nw * 4 * Tp)
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (TS)
     for (int i = threadIdx.x; i < T * T; i += blockDim.x) s_trans[i] = trans_g[i];
@@ -551,20 +665,29 @@ __global__ void crf_nll_backward_kernel(
   const int n = b < B ? min((int)len[b], L) : 0;
   float* df = dfeats + (size_t)b * L * T;
   if (n > 0) {
-    float* ba = s_beta + warp * 2 * Tp;   // beta_t
-    float* bb = ba + Tp;                  // beta_{t-1}
+    float* ba = s_beta + warp * (PARTIAL ? 4 : 2) * Tp;   // beta_t
+    float* bb = ba + Tp;                                  // beta_{t-1}
+    float* ca = bb + Tp;                                  // constrained beta_t, beta_{t-1} (PARTIAL)
+    float* cb = ca + Tp;
     const float* fb = feats + (size_t)b * L * T;
     const float* ps = part_save + (size_t)b * L * T;
-    const int64_t* tg = tags + (size_t)b * Ltags;
+    const int64_t* tg = PARTIAL ? nullptr : tags + (size_t)b * Ltags;
+    const float* qs = PARTIAL ? part_save_allowed + (size_t)b * L * T : nullptr;
+    const uint8_t* ab = PARTIAL ? allowed + (size_t)b * L * T : nullptr;
     const float logZ = crf_log_z(tr, ps + (size_t)(n - 1) * T, T, lane);
-    for (int i = lane; i < T; i += 32) ba[i] = tr[i * T + (T - 1)];   // beta_{n-1}[i] = trans[i][STOP]
+    const float logZa = PARTIAL ? crf_log_z(tr, qs + (size_t)(n - 1) * T, T, lane) : 0.f;
+    for (int i = lane; i < T; i += 32) {
+      ba[i] = tr[i * T + (T - 1)];   // beta_{n-1}[i] = trans[i][STOP]
+      if (PARTIAL) ca[i] = __ldg(ab + (size_t)(n - 1) * T + i) ? ba[i] : -INFINITY;
+    }
     __syncwarp();
     for (int t = n - 1; t >= 0; --t) {
       const float* pt = ps + (size_t)t * T;
-      const int gold = (int)tg[t];
+      const int gold = PARTIAL ? 0 : (int)tg[t];
       // unary marginal at t  (+ STOP column / START row of dtrans); lane owns j => distinct addresses
       for (int j = lane; j < T; j += 32) {
-        const float d = gs * (expf(pt[j] + ba[j] - logZ) - (j == gold ? 1.f : 0.f));
+        const float sub = PARTIAL ? expf(qs[(size_t)t * T + j] + ca[j] - logZa) : (j == gold ? 1.f : 0.f);
+        const float d = gs * (expf(pt[j] + ba[j] - logZ) - sub);
         df[(size_t)t * T + j] = d;
         if (t == n - 1) dw[j * Tq + (T - 1)] += d;
       }
@@ -576,14 +699,27 @@ __global__ void crf_nll_backward_kernel(
       // pairwise marginals (t-1 -> t) and beta_{t-1}; lane owns source rows i
       const float* pp = ps + (size_t)(t - 1) * T;
       const float* ft = fb + (size_t)t * T;
-      const int gprev = (int)tg[t - 1];
-      for (int i = lane; i < T; i += 32) {
-        float* dwi = dw + i * Tq;
-        bb[i] = crf_backward_row_exact(tr + i * T, ft, ba, pp[i] - logZ, gs, dwi, T);
-        if (i == gprev) dwi[gold] -= gs;
+      if (PARTIAL) {
+        const float* qp = qs + (size_t)(t - 1) * T;
+        for (int i = lane; i < T; i += 32) {
+          const float* tri = tr + i * T;
+          const bool ai = __ldg(ab + (size_t)(t - 1) * T + i) != 0;
+          crf_partial_row_pairs(tri, nullptr, ft, ba, ca, nullptr, nullptr, 0.f, 0.f, pp[i] - logZ,
+                                ai ? qp[i] - logZa : -INFINITY, false, false, gs, dw + i * Tq, T);
+          bb[i] = crf_row_lse(tri, ft, ba, T);
+          cb[i] = ai ? crf_row_lse(tri, ft, ca, T) : -INFINITY;
+        }
+      } else {
+        const int gprev = (int)tg[t - 1];
+        for (int i = lane; i < T; i += 32) {
+          float* dwi = dw + i * Tq;
+          bb[i] = crf_backward_row_exact(tr + i * T, ft, ba, pp[i] - logZ, gs, dwi, T);
+          if (i == gprev) dwi[gold] -= gs;
+        }
       }
       __syncwarp();
       float* tmp = ba; ba = bb; bb = tmp;
+      tmp = ca; ca = cb; cb = tmp;
     }
   }
   if (b < B) crf_zero_rows(df, max(n, 0), L, T, lane, 32);
@@ -596,11 +732,16 @@ __global__ void crf_nll_backward_kernel(
 //   P(y_{t-1}=i,y_t=j) = exp(part_{t-1}[i] - logZ + rmax[i] + Mw) * table[i][j] * W_j
 // i.e. T exps, T logs and 2 T*T multiply-adds per step instead of 3 T*T exps.  A row whose S_i underflows is
 // evaluated exactly in the log domain (same formulas as crf_nll_backward_kernel).
+// PARTIAL: the constrained lattice of crf_nll_backward_kernel<., true> with its own beta, Mw and W vectors over the same
+// table; a row's two pairwise terms are rounded products subtracted before they reach the accumulator.
 // dynamic smem: trans T*T | table T*T | rmax Tp | per warp: dtrans accumulator T*Tq, beta a / b, W (3 * Tp)
+//               [, constrained beta a / b, W (3 * Tp)]
+template <bool PARTIAL>
 __global__ void crf_nll_backward_exp_kernel(
     const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len,
     const int64_t* __restrict__ tags, const float* __restrict__ part_save, const float* __restrict__ gscale, int B,
-    int L, int Ltags, int T, float* __restrict__ dfeats, float* __restrict__ dtrans) {
+    int L, int Ltags, int T, float* __restrict__ dfeats, float* __restrict__ dtrans, const uint8_t* __restrict__ allowed,
+    const float* __restrict__ part_save_allowed) {
   extern __shared__ float smem[];
   const int nw = blockDim.x >> 5;
   const int Tp = (T + 31) & ~31;
@@ -619,28 +760,40 @@ __global__ void crf_nll_backward_exp_kernel(
   const int n = b < B ? min((int)len[b], L) : 0;
   float* df = dfeats + (size_t)b * L * T;
   if (n > 0) {
-    float* ba = s_vec + warp * 3 * Tp;   // beta_t
-    float* bb = ba + Tp;                 // beta_{t-1}
+    float* ba = s_vec + warp * (PARTIAL ? 6 : 3) * Tp;   // beta_t
+    float* bb = ba + Tp;                                 // beta_{t-1}
     float* W = bb + Tp;
+    float* ca = W + Tp;                                  // constrained beta_t, beta_{t-1}, W (PARTIAL)
+    float* cb = ca + Tp;
+    float* WA = cb + Tp;
     const float* fb = feats + (size_t)b * L * T;
     const float* ps = part_save + (size_t)b * L * T;
-    const int64_t* tg = tags + (size_t)b * Ltags;
+    const int64_t* tg = PARTIAL ? nullptr : tags + (size_t)b * Ltags;
+    const float* qs = PARTIAL ? part_save_allowed + (size_t)b * L * T : nullptr;
+    const uint8_t* ab = PARTIAL ? allowed + (size_t)b * L * T : nullptr;
     const float logZ = crf_log_z(tr, ps + (size_t)(n - 1) * T, T, lane);
-    for (int i = lane; i < T; i += 32) ba[i] = tr[i * T + (T - 1)];
+    const float logZa = PARTIAL ? crf_log_z(tr, qs + (size_t)(n - 1) * T, T, lane) : 0.f;
+    for (int i = lane; i < T; i += 32) {
+      ba[i] = tr[i * T + (T - 1)];
+      if (PARTIAL) ca[i] = __ldg(ab + (size_t)(n - 1) * T + i) ? ba[i] : -INFINITY;
+    }
     __syncwarp();
     for (int t = n - 1; t >= 0; --t) {
       // The sweep is one dependent chain per sequence and every step used to pay three or four HBM round trips in
       // sequence (partition row, feature row, tags: nobody has touched them since the forward pass).  Pull the rows of
-      // the NEXT step into L1 now; they arrive while this step's T x T loops run.
+      // the NEXT step into L1 now; they arrive while this step's T x T loops run (PARTIAL: the constrained partition
+      // row and the mask row too).
       if (t >= 1 && lane < 8) {
         const int part = (lane & 3) * 32;                       // a row is T floats: up to four 128-byte lines
         const float* row = lane < 4 ? fb + (size_t)(t - 1) * T : ps + (size_t)(t >= 2 ? t - 2 : 0) * T;
         if (part < T) asm volatile("prefetch.global.L1 [%0];" ::"l"(row + part));
       }
+      if (PARTIAL && t >= 1 && lane >= 8 && lane < 14) crf_prefetch_partial(qs, ab, t, T, lane);
       const float* pt = ps + (size_t)t * T;
-      const int gold = (int)tg[t];
+      const int gold = PARTIAL ? 0 : (int)tg[t];
       for (int j = lane; j < T; j += 32) {
-        const float d = gs * (expf(pt[j] + ba[j] - logZ) - (j == gold ? 1.f : 0.f));
+        const float sub = PARTIAL ? expf(qs[(size_t)t * T + j] + ca[j] - logZa) : (j == gold ? 1.f : 0.f);
+        const float d = gs * (expf(pt[j] + ba[j] - logZ) - sub);
         df[(size_t)t * T + j] = d;
         if (t == n - 1) dw[j * Tq + (T - 1)] += d;
       }
@@ -651,12 +804,45 @@ __global__ void crf_nll_backward_exp_kernel(
       }
       const float* pp = ps + (size_t)(t - 1) * T;
       const float* ft = fb + (size_t)t * T;
-      const int gprev = (int)tg[t - 1];
+      const int gprev = PARTIAL ? 0 : (int)tg[t - 1];
       // W_j = exp(feat_t[j] + beta_t[j] - Mw)
       float Mw = -INFINITY;
       for (int j = lane; j < T; j += 32) Mw = fmaxf(Mw, __ldg(ft + j) + ba[j]);
       Mw = warp_max(Mw);
       for (int j = lane; j < T; j += 32) W[j] = expf((__ldg(ft + j) + ba[j]) - Mw);
+      if (PARTIAL) {
+        float MwA = -INFINITY;
+        for (int j = lane; j < T; j += 32) MwA = fmaxf(MwA, __ldg(ft + j) + ca[j]);
+        MwA = warp_max(MwA);
+        for (int j = lane; j < T; j += 32) WA[j] = expf((__ldg(ft + j) + ca[j]) - MwA);
+        __syncwarp();
+        const float* qp = qs + (size_t)(t - 1) * T;
+        for (int i = lane; i < T; i += 32) {
+          const float* tei = te + i * T;
+          float* dwi = dw + i * Tq;
+          const bool ai = __ldg(ab + (size_t)(t - 1) * T + i) != 0;
+          float S = 0.f, SA = 0.f;
+          for (int j = 0; j < T; ++j) S = fmaf(tei[j], W[j], S);
+          if (ai)
+            for (int j = 0; j < T; ++j) SA = fmaf(tei[j], WA[j], SA);
+          const bool fe = S > 1e-30f, fa = SA > 1e-30f;
+          const float pi = pp[i] - logZ, pia = ai ? qp[i] - logZa : -INFINITY;
+          const float A = gs * expf((pi + rmax[i]) + Mw);
+          const float AA = ai ? gs * expf((pia + rmax[i]) + MwA) : 0.f;
+          if (fe && (fa || !ai)) {
+#pragma unroll 4
+            for (int j = 0; j < T; ++j) dwi[j] += __fmul_rn(A * tei[j], W[j]) - __fmul_rn(AA * tei[j], WA[j]);
+          } else {
+            crf_partial_row_pairs(tr + i * T, tei, ft, ba, ca, W, WA, A, AA, pi, pia, fe, fa, gs, dwi, T);
+          }
+          bb[i] = fe ? (rmax[i] + Mw) + logf(S) : crf_row_lse(tr + i * T, ft, ba, T);
+          cb[i] = !ai ? -INFINITY : fa ? (rmax[i] + MwA) + logf(SA) : crf_row_lse(tr + i * T, ft, ca, T);
+        }
+        __syncwarp();
+        float* tmp = ba; ba = bb; bb = tmp;
+        tmp = ca; ca = cb; cb = tmp;
+        continue;
+      }
       __syncwarp();
       for (int i = lane; i < T; i += 32) {
         const float* tei = te + i * T;
@@ -693,11 +879,15 @@ __global__ void crf_nll_backward_exp_kernel(
 // sequence meet at a named barrier twice per step (W complete; beta_{t-1} complete).  The sweep is latency-bound --
 // one dependent chain per sequence, seven sequences per SM because of the T x T accumulators -- so the step latency is
 // the kernel time.  Same arithmetic per element and the same left-to-right row sums as crf_nll_backward_exp_kernel.
+// PARTIAL: the constrained lattice as in crf_nll_backward_exp_kernel<true>, with the same float4 row sums.
 // dynamic smem: trans T*T | table T*T | rmax Tp | per SEQUENCE: dtrans accumulator T*Tq, beta a / b, W (3 * Tp)
+//               [, constrained beta a / b, W (3 * Tp)]
+template <bool PARTIAL>
 __global__ void crf_nll_backward_exp3_kernel(
     const float* __restrict__ feats, const float* __restrict__ trans_g, const int64_t* __restrict__ len,
     const int64_t* __restrict__ tags, const float* __restrict__ part_save, const float* __restrict__ gscale, int B,
-    int L, int Ltags, int T, float* __restrict__ dfeats, float* __restrict__ dtrans) {
+    int L, int Ltags, int T, float* __restrict__ dfeats, float* __restrict__ dtrans, const uint8_t* __restrict__ allowed,
+    const float* __restrict__ part_save_allowed) {
   extern __shared__ float smem[];
   const int nseq = (blockDim.x >> 5) / 3;
   const int Tp = (T + 31) & ~31;
@@ -709,7 +899,7 @@ __global__ void crf_nll_backward_exp3_kernel(
   float* s_vec = s_dtr + (size_t)nseq * T * Tq;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int i = threadIdx.x; i < nseq * T * Tq; i += blockDim.x) s_dtr[i] = 0.f;
-  for (int i = threadIdx.x; i < nseq * 3 * Tp; i += blockDim.x) s_vec[i] = 0.f;   // W pad entries stay 0
+  for (int i = threadIdx.x; i < nseq * (PARTIAL ? 6 : 3) * Tp; i += blockDim.x) s_vec[i] = 0.f;   // W pad entries stay 0
   crf_exp_row_table(trans_g, T, Tp, Tq, tr, te, rmax);      // pad columns of the table contribute exact zeros
   const float gs = gscale ? *gscale : 1.f;
   const int seq = warp / 3, part = warp - seq * 3;
@@ -722,14 +912,23 @@ __global__ void crf_nll_backward_exp3_kernel(
   const int n = b < B ? min((int)len[b], L) : 0;
   float* df = dfeats + (size_t)b * L * T;
   if (n > 0) {       // uniform over the three warps of a sequence
-    float* ba = s_vec + seq * 3 * Tp;    // beta_t
-    float* bb = ba + Tp;                 // beta_{t-1}
+    float* ba = s_vec + seq * (PARTIAL ? 6 : 3) * Tp;   // beta_t
+    float* bb = ba + Tp;                                // beta_{t-1}
     float* W = bb + Tp;
+    float* ca = W + Tp;                                 // constrained beta_t, beta_{t-1}, W (PARTIAL)
+    float* cb = ca + Tp;
+    float* WA = cb + Tp;
     const float* fb = feats + (size_t)b * L * T;
     const float* ps = part_save + (size_t)b * L * T;
-    const int64_t* tg = tags + (size_t)b * Ltags;
+    const int64_t* tg = PARTIAL ? nullptr : tags + (size_t)b * Ltags;
+    const float* qs = PARTIAL ? part_save_allowed + (size_t)b * L * T : nullptr;
+    const uint8_t* ab = PARTIAL ? allowed + (size_t)b * L * T : nullptr;
     const float logZ = crf_log_z(tr, ps + (size_t)(n - 1) * T, T, lane);   // every warp for itself, same result
-    if (has) ba[own] = tr[own * T + (T - 1)];
+    const float logZa = PARTIAL ? crf_log_z(tr, qs + (size_t)(n - 1) * T, T, lane) : 0.f;
+    if (has) {
+      ba[own] = tr[own * T + (T - 1)];
+      if (PARTIAL) ca[own] = __ldg(ab + (size_t)(n - 1) * T + own) ? ba[own] : -INFINITY;
+    }
     seq_sync();
     const float4* tei4 = reinterpret_cast<const float4*>(te + (has ? own : 0) * Tq);
     float* dwi = dw + (has ? own : 0) * Tq;
@@ -740,6 +939,7 @@ __global__ void crf_nll_backward_exp3_kernel(
         const float* row = lane < 4 ? fb + (size_t)(t - 1) * T : ps + (size_t)(t >= 2 ? t - 2 : 0) * T;
         if (seg < T) asm volatile("prefetch.global.L1 [%0];" ::"l"(row + seg));
       }
+      if (PARTIAL && t >= 1 && part == 0 && lane >= 8 && lane < 14) crf_prefetch_partial(qs, ab, t, T, lane);
       // every global value of the step is requested here, ahead of the barriers (the compiler cannot move a load
       // above a bar.sync): partition rows t and t-1, feature row t, the two tags
       const float* pt = ps + (size_t)t * T;
@@ -750,11 +950,16 @@ __global__ void crf_nll_backward_exp3_kernel(
       float ftm[3];
 #pragma unroll
       for (int q = 0; q < 3; ++q) ftm[q] = lane + 32 * q < T ? __ldg(ft + lane + 32 * q) : 0.f;
-      const int gold = (int)tg[t];
-      const int gprev = (int)tg[t >= 1 ? t - 1 : 0];
+      const int gold = PARTIAL ? 0 : (int)tg[t];
+      const int gprev = PARTIAL ? 0 : (int)tg[t >= 1 ? t - 1 : 0];
+      // PARTIAL: constrained partition rows t and t-1 and whether tag `own` is allowed at t-1
+      const float qtv = PARTIAL ? qs[(size_t)t * T + oc] : 0.f;
+      const float qpv = PARTIAL ? qs[(size_t)(t >= 1 ? t - 1 : 0) * T + oc] : 0.f;
+      const bool ai = PARTIAL && has && __ldg(ab + (size_t)(t >= 1 ? t - 1 : 0) * T + oc) != 0;
       float d = 0.f;
       if (has) {
-        d = gs * (expf(ptv + ba[own] - logZ) - (own == gold ? 1.f : 0.f));
+        const float sub = PARTIAL ? expf(qtv + ca[own] - logZa) : (own == gold ? 1.f : 0.f);
+        d = gs * (expf(ptv + ba[own] - logZ) - sub);
         df[(size_t)t * T + own] = d;
         if (t == n - 1) dwi[T - 1] += d;
       }
@@ -773,8 +978,61 @@ __global__ void crf_nll_backward_exp3_kernel(
         if (lane + 32 * q < T) Mw = fmaxf(Mw, ftm[q] + ba[lane + 32 * q]);
       Mw = warp_max(Mw);
       if (has) W[own] = expf((ftv + ba[own]) - Mw);
+      float MwA = -INFINITY;
+      if (PARTIAL) {
+#pragma unroll
+        for (int q = 0; q < 3; ++q)
+          if (lane + 32 * q < T) MwA = fmaxf(MwA, ftm[q] + ca[lane + 32 * q]);
+        MwA = warp_max(MwA);
+        if (has) WA[own] = expf((ftv + ca[own]) - MwA);
+      }
       seq_sync();
-      if (has) {
+      if (PARTIAL && has) {
+        const float4* W4 = reinterpret_cast<const float4*>(W);
+        const float4* WA4 = reinterpret_cast<const float4*>(WA);
+        float4* dwi4 = reinterpret_cast<float4*>(dwi);
+        const int n4 = Tq >> 2;
+        float S = 0.f, SA = 0.f;
+#pragma unroll 4
+        for (int j = 0; j < n4; ++j) {
+          const float4 t = tei4[j], w = W4[j];
+          S = fmaf(t.x, w.x, S);
+          S = fmaf(t.y, w.y, S);
+          S = fmaf(t.z, w.z, S);
+          S = fmaf(t.w, w.w, S);
+        }
+        if (ai) {
+#pragma unroll 4
+          for (int j = 0; j < n4; ++j) {
+            const float4 t = tei4[j], w = WA4[j];
+            SA = fmaf(t.x, w.x, SA);
+            SA = fmaf(t.y, w.y, SA);
+            SA = fmaf(t.z, w.z, SA);
+            SA = fmaf(t.w, w.w, SA);
+          }
+        }
+        const bool fe = S > 1e-30f, fa = SA > 1e-30f;
+        const float pi = ppv - logZ, pia = ai ? qpv - logZa : -INFINITY;
+        const float A = gs * expf((pi + rmax[own]) + Mw);
+        const float AA = ai ? gs * expf((pia + rmax[own]) + MwA) : 0.f;
+        if (fe && (fa || !ai)) {
+#pragma unroll 2
+          for (int j = 0; j < n4; ++j) {
+            const float4 t0 = tei4[j], w0 = W4[j], v0 = WA4[j];
+            float4 d0 = dwi4[j];
+            d0.x += __fmul_rn(A * t0.x, w0.x) - __fmul_rn(AA * t0.x, v0.x);
+            d0.y += __fmul_rn(A * t0.y, w0.y) - __fmul_rn(AA * t0.y, v0.y);
+            d0.z += __fmul_rn(A * t0.z, w0.z) - __fmul_rn(AA * t0.z, v0.z);
+            d0.w += __fmul_rn(A * t0.w, w0.w) - __fmul_rn(AA * t0.w, v0.w);
+            dwi4[j] = d0;
+          }
+        } else {
+          crf_partial_row_pairs(tr + own * T, te + own * Tq, ft, ba, ca, W, WA, A, AA, pi, pia, fe, fa, gs, dwi, T);
+        }
+        bb[own] = fe ? (rmax[own] + Mw) + logf(S) : crf_row_lse(tr + own * T, ft, ba, T);
+        cb[own] = !ai ? -INFINITY : fa ? (rmax[own] + MwA) + logf(SA) : crf_row_lse(tr + own * T, ft, ca, T);
+      }
+      if (!PARTIAL && has) {
         // four tag pairs per shared-memory instruction (the sweep issues ~2.5 loads per FMA otherwise); the row sum keeps
         // its left-to-right order, the pad columns add exact zeros
         const float4* W4 = reinterpret_cast<const float4*>(W);
@@ -817,6 +1075,7 @@ __global__ void crf_nll_backward_exp3_kernel(
       }
       seq_sync();                          // beta_{t-1} complete, nobody reads beta_t / W any more
       float* tmp = ba; ba = bb; bb = tmp;
+      tmp = ca; ca = cb; cb = tmp;
     }
   }
   if (b < B) crf_zero_rows(df, max(n, 0), L, T, tid96, 96);
@@ -1000,14 +1259,6 @@ __global__ void __launch_bounds__(kCrfWarps * 32) crf_nbest_kernel(
 }
 
 // ---- tag marginals --------------------------------------------------------------------------------------------------
-// exact log-domain LSE_j((tri[j] + feat_t[j]) + beta[j]) of row i (the expressions of crf_backward_row_exact)
-__device__ __forceinline__ float crf_row_lse(const float* tri, const float* ft, const float* beta, int T) {
-  float mx = -INFINITY;
-  for (int j = 0; j < T; ++j) mx = fmaxf(mx, (tri[j] + __ldg(ft + j)) + beta[j]);
-  float sm = 0.f;
-  for (int j = 0; j < T; ++j) sm += expf(((tri[j] + __ldg(ft + j)) + beta[j]) - mx);
-  return mx + logf(sm);
-}
 
 // marg[b,t,j] = P(y_t = j | x) = exp(part_t[j] + beta_t[j] - logZ) by the backward (beta) sweep alone, one warp per
 // sequence, from the forward partitions re2nn_crf_nll saved.  Without the pairwise T x T accumulators of the training
@@ -1256,6 +1507,7 @@ __global__ void __launch_bounds__(1024) length_order_kernel(const int64_t* __res
 }
 
 static const size_t kSmemLimit = 200 * 1024;
+static const size_t kSmemAll = 226 * 1024;   // what one CTA may take when it is alone on its SM
 static bool g_crf_bwd_split = true;      // CRF backward: three warps per sequence when T <= 96 (re2nn_debug_set_crf_backward_split)
 static int g_viterbi_ns = 0;             // sequences per Viterbi warp, 0 = by batch size (re2nn_debug_set_viterbi_seqs)
 
@@ -1267,6 +1519,108 @@ static int crf_launch(Kernel kernel, int (&configured)[kMaxDevices], int grid, i
   kernel<<<grid, block, smem, st>>>(args...);
   RE2NN_LAUNCH_CHECK();
   return 0;
+}
+
+// re2nn_crf_nll (PARTIAL = false) and re2nn_crf_partial_nll (true): kernel by tag-set width, then the loss sum.  The
+// partial loss takes the same kernel at every T; its second lattice adds three (scaled-exponential) or two
+// (log-domain) Tp vectors per warp, up to kSmemAll, and the global-transition kernel runs fewer warps once eight do not
+// fit.
+template <bool PARTIAL>
+static int crf_nll_run(const float* feats, const float* transitions, const int64_t* lengths, const int64_t* tags,
+                       const uint8_t* allowed, int B, int L, int Ltags, int T, float* per_seq, float* loss,
+                       float* part_save, float* part_save_allowed, cudaStream_t st) {
+  using Kernel = decltype(&crf_nll_kernel<true, PARTIAL>);
+  static const Kernel kernels[7] = {crf_nll_exp_kernel<1, PARTIAL>, crf_nll_exp_kernel<2, PARTIAL>,
+                                    crf_nll_exp_kernel<3, PARTIAL>, crf_nll_exp_kernel<4, PARTIAL>,
+                                    crf_nll_exp_kernel<5, PARTIAL>, crf_nll_kernel<true, PARTIAL>,
+                                    crf_nll_kernel<false, PARTIAL>};
+  static int configured[7][kMaxDevices];
+  const int Tp = (T + 31) & ~31;
+  const size_t part = (size_t)kCrfWarps * 2 * Tp * 4;
+  const size_t with_tr = part + (size_t)T * T * 4;
+  const size_t exp_smem = ((size_t)2 * T * T + kCrfOverrun + Tp + (size_t)kCrfWarps * 3 * Tp) * 4;
+  int k;           // exp<cdiv(T, 32)>, then the log-domain kernel with / without the transitions in shared memory
+  size_t smem;
+  if (exp_smem <= kSmemLimit && T <= 160) {
+    k = cdiv(T, 32) - 1;
+    smem = exp_smem;
+  } else if (with_tr <= kSmemLimit) {
+    k = 5;
+    smem = with_tr;
+  } else {
+    k = 6;
+    smem = part;
+  }
+  int nw = kCrfWarps;
+  if (PARTIAL) {
+    if (k < 6) {
+      smem += (size_t)kCrfWarps * (k < 5 ? 3 : 2) * Tp * 4;
+    } else {
+      nw = (int)std::min<size_t>(kCrfWarps, kSmemAll / ((size_t)4 * Tp * 4));
+      RE2NN_CHECK(nw >= 1, "crf_partial_nll: tag set too large (T=%d)", T);
+      smem = (size_t)nw * 4 * Tp * 4;
+    }
+  }
+  if (int rc = crf_launch(kernels[k], configured[k], cdiv(B, nw), nw * 32, smem, st, feats, transitions, lengths, tags,
+                          B, L, Ltags, T, per_seq, part_save, allowed, part_save_allowed))
+    return rc;
+  if (loss) {
+    reduce_sum_kernel<<<1, 1024, 0, st>>>(per_seq, (size_t)B, 1.0, loss);
+    RE2NN_LAUNCH_CHECK();
+  }
+  return 0;
+}
+
+// re2nn_crf_nll_backward (PARTIAL = false) and re2nn_crf_partial_nll_backward (true).  The kernel and the T <= 225
+// limit follow from the supervised sizes; the partial gradient then sizes its CTAs with its second lattice's vectors
+// (three Tp per sequence, two in the log domain) against kSmemAll.  At T = 75 that is still seven sequences per CTA.
+template <bool PARTIAL>
+static int crf_nll_backward_run(const float* feats, const float* transitions, const int64_t* lengths,
+                                const int64_t* tags, const uint8_t* allowed, const float* part_save,
+                                const float* part_save_allowed, const float* gscale, int B, int L, int Ltags, int T,
+                                float* dfeats, float* dtrans, cudaStream_t st) {
+  using Kernel = decltype(&crf_nll_backward_exp_kernel<PARTIAL>);
+  static const Kernel kernels[4] = {crf_nll_backward_exp3_kernel<PARTIAL>, crf_nll_backward_exp_kernel<PARTIAL>,
+                                    crf_nll_backward_kernel<true, PARTIAL>, crf_nll_backward_kernel<false, PARTIAL>};
+  static int configured[4][kMaxDevices];
+  const int Tp = (T + 31) & ~31, Tq = T | 1;
+  const size_t tr_bytes = (size_t)T * T * 4;
+  // one CTA per SM either way (the per-sequence accumulators fill the shared memory): the scaled-exponential kernels
+  // take everything the SM has, so that e.g. B = 1024 at T = 74 is 147 CTAs of seven sequences = ONE wave instead of
+  // 171 CTAs of six = two
+  const size_t smem_all = kSmemAll;
+  const size_t extra = (size_t)(PARTIAL ? 3 : 0) * Tp * 4;     // the constrained lattice's vectors per sequence
+  const size_t pw = ((size_t)T * Tq + 3 * Tp) * 4;             // per sequence of the scaled-exponential kernels
+  const size_t fixed = 2 * tr_bytes + (size_t)Tp * 4;
+  int k, nseq, block;       // kernel, sequences per CTA, threads per CTA
+  size_t smem;
+  if (fixed + 2 * pw <= kSmemLimit && T <= 96 && g_crf_bwd_split) {   // three warps per sequence
+    const int Tv = (T + 3) & ~3;                                         // 16-byte rows of the table and accumulators
+    const size_t fixed3 = ((((size_t)T * T + 3) & ~(size_t)3) + (size_t)T * Tv + Tp) * 4;
+    const size_t pw3 = ((size_t)T * Tv + 3 * Tp) * 4 + extra;
+    k = 0;
+    nseq = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed3) / pw3);
+    block = nseq * 96;
+    smem = fixed3 + nseq * pw3;
+  } else if (fixed + 2 * pw <= kSmemLimit) {        // transitions + table + at least two accumulators fit
+    k = 1;
+    nseq = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed) / (pw + extra));
+    block = nseq * 32;
+    smem = fixed + nseq * (pw + extra);
+  } else {   // log domain: as many warps as the accumulators allow, transitions in shared memory when they still fit
+    const size_t per_warp = ((size_t)T * Tq + 2 * Tp) * 4;
+    const bool ts = tr_bytes + per_warp <= kSmemLimit;
+    nseq = (int)std::min<size_t>(kCrfWarps, (kSmemLimit - (ts ? tr_bytes : 0)) / per_warp);
+    RE2NN_CHECK(nseq >= 1, "%s: tag set too large (T=%d)", PARTIAL ? "crf_partial_nll_backward" : "crf_nll_backward", T);
+    k = ts ? 2 : 3;
+    if (PARTIAL)
+      nseq = (int)std::min<size_t>(kCrfWarps, (smem_all - (ts ? tr_bytes : 0)) / (per_warp + 2 * Tp * 4));
+    block = nseq * 32;
+    smem = (ts ? tr_bytes : 0) + nseq * (per_warp + (PARTIAL ? 2 * Tp * 4 : 0));
+  }
+  RE2NN_CUDA(cudaMemsetAsync(dtrans, 0, tr_bytes, st));
+  return crf_launch(kernels[k], configured[k], cdiv(B, nseq), block, smem, st, feats, transitions, lengths, tags,
+                    part_save, gscale, B, L, Ltags, T, dfeats, dtrans, allowed, part_save_allowed);
 }
 
 }  // namespace re2nn
@@ -1348,82 +1702,37 @@ int re2nn_crf_nll(const float* feats, const float* transitions, const int64_t* l
                   int L, int Ltags, int T, float* per_seq, float* loss, float* part_save, void* stream) {
   RE2NN_CHECK(feats && transitions && lengths && per_seq, "crf_nll: null tensor");
   RE2NN_CHECK(B > 0 && L > 0 && T >= 3, "crf_nll: bad dims");
-  using Kernel = decltype(&crf_nll_kernel<true>);
-  static const Kernel kernels[7] = {crf_nll_exp_kernel<1>, crf_nll_exp_kernel<2>, crf_nll_exp_kernel<3>,
-                                    crf_nll_exp_kernel<4>, crf_nll_exp_kernel<5>, crf_nll_kernel<true>,
-                                    crf_nll_kernel<false>};
-  static int configured[7][kMaxDevices];
-  const int Tp = (T + 31) & ~31;
-  const size_t part = (size_t)kCrfWarps * 2 * Tp * 4;
-  const size_t with_tr = part + (size_t)T * T * 4;
-  const size_t exp_smem = ((size_t)2 * T * T + kCrfOverrun + Tp + (size_t)kCrfWarps * 3 * Tp) * 4;
-  int k;           // exp<cdiv(T, 32)>, then the log-domain kernel with / without the transitions in shared memory
-  size_t smem;
-  if (exp_smem <= kSmemLimit && T <= 160) {
-    k = cdiv(T, 32) - 1;
-    smem = exp_smem;
-  } else if (with_tr <= kSmemLimit) {
-    k = 5;
-    smem = with_tr;
-  } else {
-    k = 6;
-    smem = part;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  if (int rc = crf_launch(kernels[k], configured[k], cdiv(B, kCrfWarps), kCrfWarps * 32, smem, st, feats, transitions,
-                          lengths, tags, B, L, Ltags, T, per_seq, part_save))
-    return rc;
-  if (loss) {
-    reduce_sum_kernel<<<1, 1024, 0, st>>>(per_seq, (size_t)B, 1.0, loss);
-    RE2NN_LAUNCH_CHECK();
-  }
-  return 0;
+  return crf_nll_run<false>(feats, transitions, lengths, tags, nullptr, B, L, Ltags, T, per_seq, loss, part_save,
+                            nullptr, (cudaStream_t)stream);
 }
 
 int re2nn_crf_nll_backward(const float* feats, const float* transitions, const int64_t* lengths, const int64_t* tags,
                            const float* part_save, const float* gscale, int B, int L, int Ltags, int T, float* dfeats,
                            float* dtrans, void* stream) {
   RE2NN_CHECK(feats && transitions && lengths && tags && part_save && dfeats && dtrans, "crf_nll_backward: null tensor");
-  using Kernel = decltype(&crf_nll_backward_exp_kernel);
-  static const Kernel kernels[4] = {crf_nll_backward_exp3_kernel, crf_nll_backward_exp_kernel,
-                                    crf_nll_backward_kernel<true>, crf_nll_backward_kernel<false>};
-  static int configured[4][kMaxDevices];
-  const int Tp = (T + 31) & ~31, Tq = T | 1;
-  const size_t tr_bytes = (size_t)T * T * 4;
-  // one CTA per SM either way (the per-sequence accumulators fill the shared memory): the scaled-exponential kernels
-  // take everything the SM has, so that e.g. B = 1024 at T = 74 is 147 CTAs of seven sequences = ONE wave instead of
-  // 171 CTAs of six = two
-  const size_t smem_all = 226 * 1024;
-  const size_t pw = ((size_t)T * Tq + 3 * Tp) * 4;             // per sequence of the scaled-exponential kernels
-  const size_t fixed = 2 * tr_bytes + (size_t)Tp * 4;
-  int k, nseq, block;       // kernel, sequences per CTA, threads per CTA
-  size_t smem;
-  if (fixed + 2 * pw <= kSmemLimit && T <= 96 && g_crf_bwd_split) {   // three warps per sequence
-    const int Tv = (T + 3) & ~3;                                         // 16-byte rows of the table and accumulators
-    const size_t fixed3 = ((((size_t)T * T + 3) & ~(size_t)3) + (size_t)T * Tv + Tp) * 4;
-    const size_t pw3 = ((size_t)T * Tv + 3 * Tp) * 4;
-    k = 0;
-    nseq = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed3) / pw3);
-    block = nseq * 96;
-    smem = fixed3 + nseq * pw3;
-  } else if (fixed + 2 * pw <= kSmemLimit) {        // transitions + table + at least two accumulators fit
-    k = 1;
-    nseq = (int)std::min<size_t>(kCrfWarps, (smem_all - fixed) / pw);
-    block = nseq * 32;
-    smem = fixed + nseq * pw;
-  } else {   // log domain: as many warps as the accumulators allow, transitions in shared memory when they still fit
-    const size_t per_warp = ((size_t)T * Tq + 2 * Tp) * 4;
-    const bool ts = tr_bytes + per_warp <= kSmemLimit;
-    nseq = (int)std::min<size_t>(kCrfWarps, (kSmemLimit - (ts ? tr_bytes : 0)) / per_warp);
-    RE2NN_CHECK(nseq >= 1, "crf_nll_backward: tag set too large (T=%d)", T);
-    k = ts ? 2 : 3;
-    block = nseq * 32;
-    smem = (ts ? tr_bytes : 0) + nseq * per_warp;
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  RE2NN_CUDA(cudaMemsetAsync(dtrans, 0, tr_bytes, st));
-  return crf_launch(kernels[k], configured[k], cdiv(B, nseq), block, smem, st, feats, transitions, lengths, tags,
-                    part_save, gscale, B, L, Ltags, T, dfeats, dtrans);
+  return crf_nll_backward_run<false>(feats, transitions, lengths, tags, nullptr, part_save, nullptr, gscale, B, L, Ltags,
+                                     T, dfeats, dtrans, (cudaStream_t)stream);
+}
+
+int re2nn_crf_partial_nll(const float* feats, const float* transitions, const int64_t* lengths, const uint8_t* allowed,
+                          int B, int L, int T, float* per_seq, float* loss, float* part_save, float* part_save_allowed,
+                          void* stream) {
+  RE2NN_CHECK(feats && transitions && lengths && allowed && per_seq, "crf_partial_nll: null tensor");
+  RE2NN_CHECK(!part_save == !part_save_allowed, "crf_partial_nll: part_save and part_save_allowed go together");
+  RE2NN_CHECK(B > 0 && L > 0 && T >= 3, "crf_partial_nll: bad dims B=%d L=%d T=%d", B, L, T);
+  return crf_nll_run<true>(feats, transitions, lengths, nullptr, allowed, B, L, 0, T, per_seq, loss, part_save,
+                           part_save_allowed, (cudaStream_t)stream);
+}
+
+int re2nn_crf_partial_nll_backward(const float* feats, const float* transitions, const int64_t* lengths,
+                                   const uint8_t* allowed, const float* part_save, const float* part_save_allowed,
+                                   const float* gscale, int B, int L, int T, float* dfeats, float* dtrans,
+                                   void* stream) {
+  RE2NN_CHECK(feats && transitions && lengths && allowed && part_save && part_save_allowed && dfeats && dtrans,
+              "crf_partial_nll_backward: null tensor");
+  RE2NN_CHECK(B > 0 && L > 0 && T >= 3, "crf_partial_nll_backward: bad dims B=%d L=%d T=%d", B, L, T);
+  return crf_nll_backward_run<true>(feats, transitions, lengths, nullptr, allowed, part_save, part_save_allowed, gscale,
+                                    B, L, 0, T, dfeats, dtrans, (cudaStream_t)stream);
 }
 
 size_t re2nn_crf_nbest_workspace(int B, int L, int T, int K) {

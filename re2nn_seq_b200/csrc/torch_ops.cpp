@@ -6,7 +6,8 @@
 // carrying re2nn_last_error().  The op set is the one SURVEY.md section 8b proposes for the reference's modules
 // (farnn/model_decompose_single.py:207-304, farnn/model_onehot.py:351-428, baselines/crf.py:48-260):
 //   re2nn::ifst_decompose_forward, re2nn::ifst_onehot_forward, re2nn::label_scores, re2nn::argmax_decode,
-//   re2nn::crf_viterbi, re2nn::crf_nll, re2nn::crf_nll_backward; beyond it re2nn::crf_nbest, re2nn::crf_marginals.
+//   re2nn::crf_viterbi, re2nn::crf_nll, re2nn::crf_nll_backward; beyond it re2nn::crf_nbest, re2nn::crf_marginals,
+//   re2nn::crf_partial_nll, re2nn::crf_partial_nll_backward.
 // Built by re2nn_seq_b200/build.py into re2nn_seq_b200/libre2nn_torch.so (links libre2nn_b200.so, rpath $ORIGIN).
 #include <ATen/cuda/CUDAContext.h>
 #include <c10/cuda/CUDAGuard.h>
@@ -177,6 +178,45 @@ std::tuple<Tensor, Tensor> crf_nll_backward(const Tensor& feats, const Tensor& t
   return {dfeats, dtrans};
 }
 
+// allowed-tag mask B x L x T: bool or uint8, one byte per tag
+const uint8_t* mask8(const Tensor& t, const Tensor& feats) {
+  TORCH_CHECK(t.is_cuda(), "re2nn_b200: allowed must be a CUDA tensor (there is no CPU path)");
+  TORCH_CHECK(t.is_contiguous(), "re2nn_b200: allowed must be contiguous");
+  TORCH_CHECK(t.scalar_type() == at::kBool || t.scalar_type() == at::kByte, "re2nn_b200: allowed must be bool or uint8");
+  TORCH_CHECK(t.sizes() == feats.sizes(), "re2nn_b200: allowed must have the shape of feats (B x L x T)");
+  return reinterpret_cast<const uint8_t*>(t.data_ptr());
+}
+
+// partial-annotation loss -> (loss scalar, per-sequence B, free and constrained partitions B x L x T each, or empty)
+std::tuple<Tensor, Tensor, Tensor, Tensor> crf_partial_nll(const Tensor& feats, const Tensor& transitions,
+                                                           const Tensor& lengths, const Tensor& allowed, bool save) {
+  c10::cuda::CUDAGuard guard(feats.device());
+  const int64_t B = feats.size(0), L = feats.size(1), T = feats.size(2);
+  Tensor per_seq = at::empty({B}, feats.options()), loss = at::empty({}, feats.options());
+  Tensor part = save ? at::empty({B, L, T}, feats.options()) : at::empty({0}, feats.options());
+  Tensor part_a = save ? at::empty({B, L, T}, feats.options()) : at::empty({0}, feats.options());
+  fail(re2nn_crf_partial_nll(f32(feats, "feats"), f32(transitions, "transitions"), i64(lengths, "lengths"),
+                             mask8(allowed, feats), (int)B, (int)L, (int)T, per_seq.data_ptr<float>(),
+                             loss.data_ptr<float>(), save ? part.data_ptr<float>() : nullptr,
+                             save ? part_a.data_ptr<float>() : nullptr, stream()),
+       "crf_partial_nll");
+  return {loss, per_seq, part, part_a};
+}
+
+std::tuple<Tensor, Tensor> crf_partial_nll_backward(const Tensor& feats, const Tensor& transitions, const Tensor& lengths,
+                                                    const Tensor& allowed, const Tensor& part, const Tensor& part_allowed,
+                                                    const Tensor& gscale) {
+  c10::cuda::CUDAGuard guard(feats.device());
+  const int64_t B = feats.size(0), L = feats.size(1), T = feats.size(2);
+  Tensor dfeats = at::empty_like(feats), dtrans = at::empty({T, T}, feats.options());
+  fail(re2nn_crf_partial_nll_backward(f32(feats, "feats"), f32(transitions, "transitions"), i64(lengths, "lengths"),
+                                      mask8(allowed, feats), f32(part, "part"), f32(part_allowed, "part_allowed"),
+                                      f32(gscale, "gscale"), (int)B, (int)L, (int)T, dfeats.data_ptr<float>(),
+                                      dtrans.data_ptr<float>(), stream()),
+       "crf_partial_nll_backward");
+  return {dfeats, dtrans};
+}
+
 // NCRF++ CRF._viterbi_decode_nbest -> (paths B x L x K int64, scores B x K)
 std::tuple<Tensor, Tensor> crf_nbest(const Tensor& feats, const Tensor& transitions, const Tensor& lengths, int64_t nbest) {
   c10::cuda::CUDAGuard guard(feats.device());
@@ -222,6 +262,10 @@ TORCH_LIBRARY(re2nn, m) {
   m.def("crf_nll(Tensor feats, Tensor transitions, Tensor lengths, Tensor tags, bool save) -> (Tensor, Tensor, Tensor)");
   m.def("crf_nll_backward(Tensor feats, Tensor transitions, Tensor lengths, Tensor tags, Tensor part, Tensor gscale) -> "
         "(Tensor, Tensor)");
+  m.def("crf_partial_nll(Tensor feats, Tensor transitions, Tensor lengths, Tensor allowed, bool save) -> "
+        "(Tensor, Tensor, Tensor, Tensor)");
+  m.def("crf_partial_nll_backward(Tensor feats, Tensor transitions, Tensor lengths, Tensor allowed, Tensor part, "
+        "Tensor part_allowed, Tensor gscale) -> (Tensor, Tensor)");
   m.def("crf_nbest(Tensor feats, Tensor transitions, Tensor lengths, int nbest) -> (Tensor paths, Tensor scores)");
   m.def("crf_marginals(Tensor feats, Tensor transitions, Tensor lengths) -> (Tensor marginals, Tensor log_z)");
   m.def("abi_version() -> int", &abi_version);
@@ -235,6 +279,8 @@ TORCH_LIBRARY_IMPL(re2nn, CUDA, m) {
   m.impl("crf_viterbi", &crf_viterbi);
   m.impl("crf_nll", &crf_nll);
   m.impl("crf_nll_backward", &crf_nll_backward);
+  m.impl("crf_partial_nll", &crf_partial_nll);
+  m.impl("crf_partial_nll_backward", &crf_partial_nll_backward);
   m.impl("crf_nbest", &crf_nbest);
   m.impl("crf_marginals", &crf_marginals);
 }

@@ -157,31 +157,78 @@ class _DecomposeBase(nn.Module):
                                             threshold=self.args.threshold, o_idx=self.o_idx, flat_out=_flat_out)
         return flat
 
+    def _crf_only(self, what):
+        if not self.use_crf:
+            raise NotImplementedError("%s needs a CRF head (use_crf=1); %s decodes per position"
+                                      % (what, type(self).__name__))
+
+    def _decode_scores(self, input, lengths):
+        """(scores B x L x C as decode's Viterbi sees them, CE1 flag): under CE1 column C-3 clamped to the threshold."""
+        sc = self.forward_scores(input, lengths).detach().contiguous()
+        ce1 = self.args.local_loss_func == 'CE1'
+        if ce1:
+            sc = sc.clone()
+            sc[:, :, self.C - 3] = torch.minimum(sc[:, :, self.C - 3], sc.new_tensor(self.args.threshold))
+        return sc, ce1
+
+    def _report_tags(self, pred, lengths, ce1):
+        """decode's report: under CE1 tag C-3 at a valid position is o_idx."""
+        if not ce1:
+            return pred
+        valid = get_length_mask(lengths, pred.shape[1])
+        if pred.dim() == 3:
+            valid = valid[:, :, None]
+        return torch.where(valid & (pred == self.C - 3), torch.full_like(pred, self.o_idx), pred)
+
+    @staticmethod
+    def _allowed_rows(allowed, sc):
+        """A caller's mask on the scores' device and cut to their L (the CRF checks it)."""
+        if isinstance(allowed, torch.Tensor) and allowed.dim() == 3:
+            allowed = allowed.to(sc.device)[:, :sc.shape[1]]
+        return allowed
+
     def forward_nbest(self, input, lengths, nbest=1):
         """N-best CRF decoding with confidences -> (pred B x L x K int64, seq_prob B x K, marginals B x L x C).
         pred[..., 0] is what forward_local decodes (padded, in the caller's order; -1 marks a rank with no sequence,
         pads are 0), seq_prob[:, k] = P(path k | x) and marginals[b, t, c] = P(y_t = c | x), zero at pads.  Under CE1
         decode's clamp of column C-3 to the threshold applies to both, and tag C-3 is reported as o_idx in pred.
         Eager (no graph capture), no gradient."""
-        if not self.use_crf:
-            raise NotImplementedError("forward_nbest needs a CRF head (use_crf=1); %s decodes per position"
-                                      % type(self).__name__)
+        self._crf_only('forward_nbest')
         with torch.no_grad():
             dev = self._device()
             lengths = lengths.to(dev).contiguous()
-            sc = self.forward_scores(input, lengths).detach().contiguous()
-            ce1 = self.args.local_loss_func == 'CE1'
-            if ce1:
-                sc = sc.clone()
-                sc[:, :, self.C - 3] = torch.minimum(sc[:, :, self.C - 3], sc.new_tensor(self.args.threshold))
+            sc, ce1 = self._decode_scores(input, lengths)
             trans = self.crf.transitions.detach()
             pred, score = ops.crf_nbest(sc, trans, lengths, nbest)
             marg, log_z = ops.crf_marginals(sc, trans, lengths)
-            if ce1:
-                valid = get_length_mask(lengths, sc.shape[1])[:, :, None]
-                pred = torch.where(valid & (pred == self.C - 3), torch.full_like(pred, self.o_idx), pred)
+            pred = self._report_tags(pred, lengths, ce1)
             seq_prob = torch.exp(score - log_z[:, None])
         return pred, seq_prob, marg
+
+    def forward_partial(self, input, lengths, allowed):
+        """Partial-annotation CRF loss (differentiable scalar, summed over sequences like forward_local's CRF loss):
+        log Z - log Z^A per sequence, where Z^A counts only the tag sequences that keep every valid position on an
+        allowed tag.  allowed: B x L' x C bool / uint8 over the CRF's C columns (START / STOP included), L' >= the
+        longest length; crf.partial_allowed builds it from labels with an unknown marker.  With every label known it
+        is forward_local's training loss; a sequence with none known adds nothing.  Eager."""
+        self._crf_only('forward_partial')
+        dev = self._device()
+        lengths = lengths.to(dev).contiguous()
+        sc = self.forward_scores(input, lengths)
+        return self.crf.partial_neg_log_likelihood_loss(sc, None, self._allowed_rows(allowed, sc), lengths=lengths)
+
+    def forward_constrained(self, input, lengths, allowed):
+        """Constrained CRF decoding -> pred B x L int64 (padded, in the caller's order): the best tag sequence that keeps
+        every valid position on a tag allowed there (allowed as in forward_partial), e.g. tokens fixed by a person or a
+        rule.  CE1's clamp of column C-3 and its o_idx report apply as in forward_nbest, so an all-true mask gives what
+        forward_local decodes.  Eager, no gradient."""
+        self._crf_only('forward_constrained')
+        with torch.no_grad():
+            dev = self._device()
+            lengths = lengths.to(dev).contiguous()
+            sc, ce1 = self._decode_scores(input, lengths)
+            pred = self.crf.constrained_decode(sc, None, self._allowed_rows(allowed, sc), lengths=lengths)
+            return self._report_tags(pred, lengths, ce1)
 
     # ---- loss + decode tail shared by forward_local / forward (model_decompose_single.py:271-304) ---
     def _length_order(self, lengths, re_tags, L=None):

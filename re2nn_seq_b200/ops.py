@@ -296,6 +296,22 @@ def crf_nll_backward(feats, transitions, lengths, tags, part, gscale):
     return dfeats, dtrans
 
 
+def crf_partial_nll(feats, transitions, lengths, allowed, save=False):
+    """Partial-annotation CRF loss -> (loss, per_seq B = log Z - log Z^A, (free, constrained) partitions or None).
+    allowed: B x L x T bool / uint8, the tags each position may take (checked by CRF.partial_neg_log_likelihood_loss)."""
+    for t in (feats, transitions, lengths, allowed):
+        _p(t)
+    loss, per_seq, part, part_a = tops.crf_partial_nll(feats, transitions, lengths, allowed, bool(save))
+    _count(2)
+    return loss, per_seq, ((part, part_a) if save else None)
+
+
+def crf_partial_nll_backward(feats, transitions, lengths, allowed, part, part_allowed, gscale):
+    dfeats, dtrans = tops.crf_partial_nll_backward(feats, transitions, lengths, allowed, part, part_allowed, gscale)
+    _count(1)
+    return dfeats, dtrans
+
+
 def crf_nbest(feats, transitions, lengths, nbest):
     """K-best Viterbi -> (paths B x L x K int64, scores B x K): rank 0 is crf_viterbi's path; a missing rank has
     score -inf and path -1 at valid positions; pads hold 0."""

@@ -31,6 +31,39 @@ def _nl_name(name, allowed):
 class _DecomposeBase(nn.Module):
     """Shared pieces of the rank-R i-FST modules."""
 
+    def __init__(self, args, C, S, R, start_vector, final_vector, priority_mat, o_idx, fwd_params,
+                 word_embed=None, is_cuda=True):
+        """The construction sequence of every rank-R module; its order fixes the RNG draws and the parameter
+        registration order (optimizer checkpoints index parameters by position).  C x S x R are the label / state /
+        rank sizes before the CRF's two extra labels, fwd_params the subclass's init_forward_parameters arguments;
+        the token-input modules pass word_embed and so own `embedding` and `beta_vec`."""
+        super().__init__()
+        self.is_cuda = torch.cuda.is_available() if is_cuda else False
+        self.additional_states = args.additional_states
+        self.args = args
+        if word_embed is not None:
+            self.embedding = nn.Embedding.from_pretrained(torch.from_numpy(word_embed).float(),
+                                                          freeze=(not args.train_word_embed))
+        self.C, self.S, self.R = C, S, R
+        self.t = 1
+        self.use_crf = bool(args.use_crf)
+        if self.use_crf:
+            self.crf = CRF(self.C, self.is_cuda)
+            self.C += 2
+        self.priority_layer = PriorityLayer(self.C, priority_mat)
+        self.random = bool(args.random)
+        self.h0 = nn.Parameter(self.pad_additional_states(torch.from_numpy(start_vector).float()),
+                               requires_grad=bool(args.train_h0))
+        self.hT = nn.Parameter(self.pad_additional_states(torch.from_numpy(final_vector).float()),
+                               requires_grad=bool(args.train_hT))
+        self.init_forward_parameters(*fwd_params)
+        if word_embed is not None:
+            self.beta = args.beta
+            self.beta_vec = nn.Parameter(torch.tensor([self.beta] * self.R).float(), requires_grad=bool(args.train_beta))
+        self.o_idx = o_idx
+        self.not_o_idxs = [i for i in range(self.C) if i != self.o_idx]
+        self.initialize()
+
     # ---- construction helpers (model_decompose.py:191-220) ------------------------------------
     def get_random(self, sizes):
         kind = self.args.random_pad_func
@@ -71,6 +104,7 @@ class _DecomposeBase(nn.Module):
         self._cache = {}
 
     def _gate_params(self, S_full):
+        """Update (farnn >= 1) and reset (farnn == 2) gate parameters, model_decompose.py:137-171."""
         a = self.args
         if a.farnn not in (0, 1, 2):
             raise NotImplementedError()
@@ -273,7 +307,7 @@ class _DecomposeBase(nn.Module):
             offsets = offs0
         chunks = self._infer_chunks(B) if order is not None else None
         if chunks is None:
-            scores = self._scores_from(inp, lengths, (L, nmax), fuse=True)      # scores feed the decoder only
+            scores = self.forward_scores(inp, lengths, (L, nmax), fuse=True)      # scores feed the decoder only
             pred = self.decode(scores, None, None, lengths, _shape=(L, nmax), _offsets=offsets)
             return pred, true
         # Sequences are sorted longest-first, so the recurrence of a later chunk finishes earlier (its tiles stop at
@@ -291,7 +325,7 @@ class _DecomposeBase(nn.Module):
             st.wait_event(fork)
             with torch.cuda.stream(st):
                 lc = lengths[b0:b1]
-                sc = self._scores_from(inp[b0:b1], lc, (L, nmax), fuse=True)
+                sc = self.forward_scores(inp[b0:b1], lc, (L, nmax), fuse=True)
                 self.decode(sc, None, None, lc, _shape=(L, nmax), _offsets=offsets[b0:b1], _flat_out=pred)
                 done = torch.cuda.Event()
                 done.record(st)
@@ -406,6 +440,22 @@ class _DecomposeBase(nn.Module):
         return (not train) and re_tags is None and not torch.is_grad_enabled() and getattr(self, 'use_cuda_graph', True) \
             and self.args.marryup_type not in ('kd', 'pr') and not getattr(self, 'full_pad', False)
 
+    def _forward_body(self, input, label, lengths, train, re_tags, tag):
+        """forward_local / forward: a graph replay where _can_graph allows it, else the scores (longest-first when
+        _length_order sorts) and the loss + decode tail.  _device_input is the subclass's forward_scores input
+        conversion."""
+        dev = self._device()
+        lengths = lengths.to(dev).contiguous()
+        shape = self._host_shape(lengths)
+        if self._can_graph(train, re_tags):
+            return self._infer_graphed(self._device_input(input, dev), label.to(dev), lengths, shape, tag)
+        order, offsets, ls, _ = self._length_order(lengths, re_tags, shape[0])
+        if order is None:
+            all_scores = self.forward_scores(input, lengths, shape)
+            return self._finish(all_scores, label, lengths, train, re_tags, shape)
+        all_scores = self.forward_scores(input.to(dev).index_select(0, order), ls, shape)
+        return self._finish(all_scores, label, ls, train, re_tags, shape, order, offsets, lengths)
+
     def _finish(self, all_scores, label, lengths, train, re_tags, shape, order=None, offsets=None, orig=None):
         L, N = shape
         dev = all_scores.device
@@ -472,32 +522,8 @@ class FARNN_S_D_W_I_S(_DecomposeBase):
     def __init__(self, V=None, S1=None, S2=None, C_output_mat=None, wildcard_mat=None,
                  wildcard_output_vector=None, final_vector=None, start_vector=None,
                  pretrained_word_embed=None, priority_mat=None, args=None, o_idx=0, is_cuda=True):
-        super().__init__()
-        self.is_cuda = torch.cuda.is_available() if is_cuda else False
-        self.additional_states = args.additional_states
-        self.args = args
-        self.embedding = nn.Embedding.from_pretrained(torch.from_numpy(pretrained_word_embed).float(),
-                                                      freeze=(not args.train_word_embed))
-        self.C, _ = C_output_mat.shape
-        self.S, self.R = S1.shape
-        self.t = 1
-        self.use_crf = bool(args.use_crf)
-        if self.use_crf:
-            self.crf = CRF(self.C, self.is_cuda)
-            self.C += 2
-        self.priority_layer = PriorityLayer(self.C, priority_mat)
-        self.random = bool(args.random)
-        self.h0 = nn.Parameter(self.pad_additional_states(torch.from_numpy(start_vector).float()),
-                               requires_grad=bool(args.train_h0))
-        self.hT = nn.Parameter(self.pad_additional_states(torch.from_numpy(final_vector).float()),
-                               requires_grad=bool(args.train_hT))
-        self.init_forward_parameters(S1, S2, V, C_output_mat, wildcard_mat, wildcard_output_vector)
-        self.beta = args.beta
-        self.beta_vec = nn.Parameter(torch.tensor([self.beta] * self.R).float(),
-                                     requires_grad=bool(args.train_beta))
-        self.o_idx = o_idx
-        self.not_o_idxs = [i for i in range(self.C) if i != self.o_idx]
-        self.initialize()
+        super().__init__(args, C_output_mat.shape[0], *S1.shape, start_vector, final_vector, priority_mat, o_idx,
+                         (S1, S2, V, C_output_mat, wildcard_mat, wildcard_output_vector), pretrained_word_embed, is_cuda)
 
     def init_forward_parameters(self, S1, S2, V, C_o, W, W_o):
         a = self.args
@@ -533,7 +559,7 @@ class FARNN_S_D_W_I_S(_DecomposeBase):
         fuse=True (decode-only callers): rows past the length may hold anything -- the label-score operand then comes
         fused out of the recurrence (re2nn_decompose_recurrence ab_out) where the call allows it."""
         dev = self._device()
-        x = input.to(dev).contiguous()
+        x = self._device_input(input, dev)
         lengths = lengths.to(dev).contiguous()
         shape = shape or self._host_shape(lengths)
         names, tensors = self._fn_params()
@@ -544,8 +570,8 @@ class FARNN_S_D_W_I_S(_DecomposeBase):
         return autograd_fns.decompose_scores(dict(self._recurrence_consts(), fuse_scores=bool(fuse)), names, tensors, pr, x,
                                              None, lengths, shape[0], cache=self._cache)
 
-    def _scores_from(self, inp, lengths, shape, fuse=False):
-        return self.forward_scores(inp, lengths, shape, fuse=fuse)
+    def _device_input(self, input, dev):
+        return input.to(dev).contiguous()
 
     def _warm_tables(self):
         names, tensors = self._fn_params()
@@ -554,43 +580,14 @@ class FARNN_S_D_W_I_S(_DecomposeBase):
         autograd_fns._weight_prep(self._recurrence_consts(), p, self._cache)
 
     def forward_local(self, input, label, lengths, train=True, re_tags=None):
-        dev = self._device()
-        lengths = lengths.to(dev).contiguous()
-        shape = self._host_shape(lengths)
-        if self._can_graph(train, re_tags):
-            return self._infer_graphed(input.to(dev).contiguous(), label.to(dev), lengths, shape, 'tok')
-        order, offsets, ls, _ = self._length_order(lengths, re_tags, shape[0])
-        if order is None:
-            all_scores = self.forward_scores(input, lengths, shape)
-            return self._finish(all_scores, label, lengths, train, re_tags, shape)
-        all_scores = self.forward_scores(input.to(dev).index_select(0, order), ls, shape)
-        return self._finish(all_scores, label, ls, train, re_tags, shape, order, offsets, lengths)
+        return self._forward_body(input, label, lengths, train, re_tags, 'tok')
 
 
 class FARNN_S_SF(_DecomposeBase):
     def __init__(self, S1=None, S2=None, C_output_mat=None, wildcard_mat=None, wildcard_output_vector=None,
                  final_vector=None, start_vector=None, priority_mat=None, args=None, o_idx=0, is_cuda=True):
-        super().__init__()
-        self.is_cuda = torch.cuda.is_available() if is_cuda else False
-        self.additional_states = args.additional_states
-        self.args = args
-        self.C, _ = C_output_mat.shape
-        self.S, self.R = S1.shape
-        self.t = 1
-        self.use_crf = bool(args.use_crf)
-        if self.use_crf:
-            self.crf = CRF(self.C, self.is_cuda)
-            self.C += 2
-        self.priority_layer = PriorityLayer(self.C, priority_mat)
-        self.random = bool(args.random)
-        self.h0 = nn.Parameter(self.pad_additional_states(torch.from_numpy(start_vector).float()),
-                               requires_grad=bool(args.train_h0))
-        self.hT = nn.Parameter(self.pad_additional_states(torch.from_numpy(final_vector).float()),
-                               requires_grad=bool(args.train_hT))
-        self.init_forward_parameters(S1, S2, C_output_mat, wildcard_mat, wildcard_output_vector)
-        self.o_idx = o_idx
-        self.not_o_idxs = [i for i in range(self.C) if i != self.o_idx]
-        self.initialize()
+        super().__init__(args, C_output_mat.shape[0], *S1.shape, start_vector, final_vector, priority_mat, o_idx,
+                         (S1, S2, C_output_mat, wildcard_mat, wildcard_output_vector), is_cuda=is_cuda)
 
     def init_forward_parameters(self, S1, S2, C_o, W, W_o):
         a = self.args
@@ -613,7 +610,7 @@ class FARNN_S_SF(_DecomposeBase):
 
     def forward_scores(self, input, lengths, shape=None, fuse=False):
         dev = self._device()
-        v = input.to(dev).float().contiguous()
+        v = self._device_input(input, dev)
         lengths = lengths.to(dev).contiguous()
         shape = shape or self._host_shape(lengths)
         names = self._params_for_fn()
@@ -625,19 +622,9 @@ class FARNN_S_SF(_DecomposeBase):
         return autograd_fns.decompose_scores(dict(self._recurrence_consts(), fuse_scores=bool(fuse)), names, tensors, pr, None,
                                              v, lengths, shape[0], cache=self._cache)
 
-    def _scores_from(self, inp, lengths, shape, fuse=False):
-        return self.forward_scores(inp, lengths, shape, fuse=fuse)
+    def _device_input(self, input, dev):
+        return input.to(dev).float().contiguous()
 
     def forward(self, input, label, lengths, train=True, re_tags=None):
         """input: pre-computed rank factors B x L x R (model_decompose_single.py:483-580)."""
-        dev = self._device()
-        lengths = lengths.to(dev).contiguous()
-        shape = self._host_shape(lengths)
-        if self._can_graph(train, re_tags):
-            return self._infer_graphed(input.to(dev).float().contiguous(), label.to(dev), lengths, shape, 'sf')
-        order, offsets, ls, _ = self._length_order(lengths, re_tags, shape[0])
-        if order is None:
-            all_scores = self.forward_scores(input, lengths, shape)
-            return self._finish(all_scores, label, lengths, train, re_tags, shape)
-        all_scores = self.forward_scores(input.to(dev).index_select(0, order), ls, shape)
-        return self._finish(all_scores, label, ls, train, re_tags, shape, order, offsets, lengths)
+        return self._forward_body(input, label, lengths, train, re_tags, 'sf')

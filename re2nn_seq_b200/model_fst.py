@@ -29,13 +29,12 @@ import numpy as np
 import torch
 from torch import nn
 
-from . import autograd_fns, ops
+from . import ops
 from ._lib import V_TOKEN
 from .bert_embeddings import _Aggregate
-from .crf import CRF
 from .model_decompose_single import _ADD_NL, _UPDATE_NL, _DecomposeBase, _nl_name
+from .model_onehot import _OnehotBase
 from .priority import PriorityLayer
-from .utils import exclusive_offsets, flatten
 
 
 # ---- differentiable wrappers of the library primitives ----------------------------------------------------------------
@@ -129,6 +128,40 @@ def _beta_rows(hT, backward_scores, lengths):
     return full.gather(1, idx.unsqueeze(2).expand(B, L, S))
 
 
+def _apply_priority(m, scores):
+    """scores @ priority_mat + priority_bias over the last dimension (priority.py:20-30) when args.use_priority."""
+    if not m.args.use_priority:
+        return scores
+    Cn = scores.shape[-1]
+    out = matmul_nt(scores.reshape(-1, Cn), m.priority_layer.priority_mat.t().contiguous())
+    return (out + m.priority_layer.priority_bias).view(scores.shape)
+
+
+def _dense_transition(m, V_vec):
+    """Tr[b,j,s] = sum_r S1[j,r] V_vec[b,r] S2[s,r] + wildcard_mat[j,s]   (model_decompose_independent.py:172-175)"""
+    B, S = V_vec.shape[0], m._S_full
+    X = (m.S1.unsqueeze(0) * V_vec.unsqueeze(1)).reshape(B * S, m.S1.shape[1])
+    return matmul_nt(X, m.S2).view(B, S, S) + m.wildcard_mat
+
+
+def _gated_step(m, h, V_vec, h_init, inner):
+    """One step of the gated recurrence on dense transitions: hn = nl(inner(h_bar, V_vec)) between the reset gate
+    (farnn == 2: h_bar mixes h with h_init) and the update gate (farnn >= 1: hn mixes with h).  `inner` is the
+    caller's semiring product with its output mask applied."""
+    a = m.args
+    k = float(a.sigmoid_exponent)
+    h_bar = h
+    if a.farnn >= 1:
+        zt = torch.sigmoid(k * (matmul_nt(h, m.Wss1.t().contiguous()) + matmul_nt(V_vec, m.Wrs1.t().contiguous()) + m.bs1))
+    if a.farnn == 2:
+        rt = torch.sigmoid(k * (matmul_nt(h, m.Wss2.t().contiguous()) + matmul_nt(V_vec, m.Wrs2.t().contiguous()) + m.bs2))
+        h_bar = (1 - rt) * h_init + rt * h
+    hn = _apply_nl(inner(h_bar, V_vec), _nl_name(a.update_nonlinear, _UPDATE_NL))
+    if a.farnn >= 1:
+        hn = (1 - zt) * h + zt * hn
+    return hn
+
+
 class _FstRecurrence(torch.autograd.Function):
     """alpha, beta of the rank-R recurrence with no output mask, differentiable w.r.t. the (already scaled) token
     table, S1, S2, the wildcard matrix, h0 / hT and the gate parameters."""
@@ -183,8 +216,6 @@ def ifst_decompose_max_scores(m, x, dense_v, lengths, L):
     a = m.args
     S = m._S_full
     B = lengths.shape[0]
-    k = float(a.sigmoid_exponent)
-    nl = _nl_name(a.update_nonlinear, _UPDATE_NL)
     if dense_v is None:
         vt = _Aggregate.apply(m.V_embed, m.embedding.weight, m.embed_r_generalized, m.beta_vec,
                               _nl_name(a.additional_nonlinear, _ADD_NL))
@@ -203,39 +234,18 @@ def ifst_decompose_max_scores(m, x, dense_v, lengths, L):
         o = o + m.wildcard_output_vector
     h0 = m.h0.view(1, S).expand(B, S)
     hT = m.hT.view(1, S).expand(B, S)
-
-    def step(h, V_vec, h_init, is_forward):
-        h_bar = h
-        if a.farnn >= 1:
-            zt = torch.sigmoid(k * (matmul_nt(h, m.Wss1.t().contiguous()) + matmul_nt(V_vec, m.Wrs1.t().contiguous()) + m.bs1))
-        if a.farnn == 2:
-            rt = torch.sigmoid(k * (matmul_nt(h, m.Wss2.t().contiguous()) + matmul_nt(V_vec, m.Wrs2.t().contiguous()) + m.bs2))
-            h_bar = (1 - rt) * h_init + rt * h
-        if not is_forward:
-            h_bar = h_bar * o
-        X = (m.S1.unsqueeze(0) * V_vec.unsqueeze(1)).reshape(B * S, m.S1.shape[1])
-        Tr = matmul_nt(X, m.S2).view(B, S, S) + m.wildcard_mat
-        hn = vecmat(h_bar, Tr, transposed=not is_forward, maxp=True)
-        if is_forward:
-            hn = hn * o
-        hn = _apply_nl(hn, nl)
-        if a.farnn >= 1:
-            hn = (1 - zt) * h + zt * hn
-        return hn
-
+    fwd = lambda h_bar, V_vec: vecmat(h_bar, _dense_transition(m, V_vec), False, True) * o     # mask on the new state
+    bwd = lambda h_bar, V_vec: vecmat(h_bar * o, _dense_transition(m, V_vec), True, True)      # mask on the old state
     hf, hb, fw, bw = h0, hT, [], []
     for i in range(L):
-        hf = step(hf, v_at(i, False), h0, True)
+        hf = _gated_step(m, hf, v_at(i, False), h0, fwd)
         fw.append(hf)
-        hb = step(hb, v_at(i, True), hT, False)
+        hb = _gated_step(m, hb, v_at(i, True), hT, bwd)
         bw.append(hb)
     alpha = torch.stack(fw, dim=1)                                          # h0_forward_score[:, i + 1]
     beta = _beta_rows(m.hT, torch.stack(bw, dim=1), lengths)                # reversed_backward_score_x[:, i + 1]
     scores = matmul_nt((alpha * beta).reshape(B * L, S), m.C_output_mat).view(B, L, m.C)
-    if a.use_priority:
-        scores = (matmul_nt(scores.reshape(B * L, m.C), m.priority_layer.priority_mat.t().contiguous()) +
-                  m.priority_layer.priority_bias).view(B, L, m.C)
-    return scores
+    return _apply_priority(m, scores)
 
 
 def ifst_onehot_max_scores(m, x, lengths):
@@ -243,7 +253,7 @@ def ifst_onehot_max_scores(m, x, lengths):
     a = m.args
     B, L = x.shape
     S = m.S
-    nl = a.update_nonlinear if a.update_nonlinear in _UPDATE_NL else 'none'
+    nl = _nl_name(a.update_nonlinear, _UPDATE_NL)
     T = m.language_tensor + m.wildcard_mat
     o = m.output_mat.sum(0)
     if a.local_loss_func != 'CE1':
@@ -261,10 +271,7 @@ def ifst_onehot_max_scores(m, x, lengths):
     beta = _beta_rows(m.hT, torch.stack(bw, dim=1), lengths)
     Cn = m.output_mat.shape[0]
     scores = matmul_nt((alpha * beta).reshape(B * L, S), m.output_mat).view(B, L, Cn)
-    if a.use_priority:
-        scores = (matmul_nt(scores.reshape(B * L, Cn), m.priority_layer.priority_mat.t().contiguous()) +
-                  m.priority_layer.priority_bias).view(B, L, Cn)
-    return scores
+    return _apply_priority(m, scores)
 
 
 # ---- FARNN_S_D_W ------------------------------------------------------------------------------------------------------------
@@ -272,32 +279,10 @@ class FARNN_S_D_W(_DecomposeBase):
     def __init__(self, V=None, C=None, S1=None, S2=None, C_wildcard=None, S1_wildcard=None, S2_wildcard=None,
                  wildcard_wildcard=None, final_vector=None, start_vector=None, pretrained_word_embed=None,
                  priority_mat=None, args=None, o_idx=0):
-        super().__init__()
-        self.is_cuda = torch.cuda.is_available()
-        self.additional_states = args.additional_states
-        self.args = args
-        self.embedding = nn.Embedding.from_pretrained(torch.from_numpy(pretrained_word_embed).float(),
-                                                      freeze=(not args.train_word_embed))
-        self.C, self.R_W = C_wildcard.shape
-        self.S, _ = S1_wildcard.shape
-        _, self.R = C.shape
-        self.t = 1
-        self.use_crf = bool(args.use_crf)
-        if self.use_crf:
-            self.crf = CRF(self.C, self.is_cuda)
-            self.C += 2
-        self.priority_layer = PriorityLayer(self.C, priority_mat)
-        self.random = bool(args.random)
-        self.h0 = nn.Parameter(self.pad_additional_states(torch.from_numpy(start_vector).float()),
-                               requires_grad=bool(args.train_h0))
-        self.hT = nn.Parameter(self.pad_additional_states(torch.from_numpy(final_vector).float()),
-                               requires_grad=bool(args.train_hT))
-        self.init_forward_parameters(S1, S2, C, V, S1_wildcard, S2_wildcard, C_wildcard, wildcard_wildcard)
-        self.beta = args.beta
-        self.beta_vec = nn.Parameter(torch.tensor([self.beta] * self.R).float(), requires_grad=bool(args.train_beta))
-        self.o_idx = o_idx
-        self.not_o_idxs = [i for i in range(self.C) if i != self.o_idx]
-        self.initialize()
+        super().__init__(args, C_wildcard.shape[0], S1_wildcard.shape[0], C.shape[1], start_vector, final_vector,
+                         priority_mat, o_idx, (S1, S2, C, V, S1_wildcard, S2_wildcard, C_wildcard, wildcard_wildcard),
+                         pretrained_word_embed)
+        self.R_W = C_wildcard.shape[1]
 
     def init_forward_parameters(self, S1, S2, C, V, S1_w, S2_w, C_w, W):
         a = self.args
@@ -308,7 +293,7 @@ class FARNN_S_D_W(_DecomposeBase):
         self.embed_r_generalized = nn.Parameter(G, requires_grad=True)
         if a.use_crf == 1:
             C = np.concatenate((C, self.get_random((2, self.R)).numpy() * a.rand_constant), axis=0)
-            C_w = np.concatenate((C_w, self.get_random((2, self.R_W)).numpy() * a.rand_constant), axis=0)
+            C_w = np.concatenate((C_w, self.get_random((2, C_w.shape[1])).numpy() * a.rand_constant), axis=0)
         self.C_wildcard = nn.Parameter(self.pad_additional_states(torch.from_numpy(C_w).float()),
                                        requires_grad=bool(a.train_wildcard))
         self.C_embed = nn.Parameter(torch.from_numpy(C).float(), requires_grad=True)
@@ -318,35 +303,13 @@ class FARNN_S_D_W(_DecomposeBase):
                                         requires_grad=bool(a.train_wildcard))
         self.wildcard_wildcard = nn.Parameter(self.pad_additional_states(torch.from_numpy(W).float()),
                                               requires_grad=bool(a.train_wildcard_wildcard))
-        self._fst_gate_params(self.S + self.additional_states)
+        self._gate_params(self.S + self.additional_states)
         if self.random:
             for w in (self.S1, self.S2, self.C_embed, self.V_embed, self.S1_wildcard, self.S2_wildcard, self.C_wildcard,
                       self.embed_r_generalized, self.wildcard_wildcard):
                 nn.init.xavier_normal_(w)
             nn.init.normal_(self.h0)
             nn.init.normal_(self.hT)
-
-    def _fst_gate_params(self, S_full):
-        """model_decompose.py:137-171 (the farnn == 1 branch also re-initialises bs1 under xavier)."""
-        a = self.args
-        if a.farnn == 1:
-            self.Wss1 = nn.Parameter(torch.randn((S_full, S_full)).float(), requires_grad=True)
-            self.Wrs1 = nn.Parameter(torch.randn((self.R, S_full)).float(), requires_grad=True)
-            self.bs1 = nn.Parameter(torch.ones((1, S_full)).float() * a.bias_init, requires_grad=True)
-            if a.xavier:
-                nn.init.xavier_normal_(self.Wss1)
-                nn.init.xavier_normal_(self.Wrs1)
-                nn.init.xavier_normal_(self.bs1)
-        if a.farnn == 2:
-            self.Wss1 = nn.Parameter(torch.randn((S_full, S_full)).float(), requires_grad=True)
-            self.Wrs1 = nn.Parameter(torch.randn((self.R, S_full)).float(), requires_grad=True)
-            self.bs1 = nn.Parameter(torch.ones((1, S_full)).float() * a.bias_init, requires_grad=True)
-            self.Wss2 = nn.Parameter(torch.randn((S_full, S_full)).float(), requires_grad=True)
-            self.Wrs2 = nn.Parameter(torch.randn((self.R, S_full)).float(), requires_grad=True)
-            self.bs2 = nn.Parameter(torch.ones((1, S_full)).float() * a.bias_init, requires_grad=True)
-            if a.xavier:
-                for w in (self.Wss1, self.Wrs1, self.Wss2, self.Wrs2):
-                    nn.init.xavier_normal_(w)
 
     # -- shared by FARNN_S_D_W / FARNN_S_D_W_I -----------------------------------------------------------------
     def _token_table(self):
@@ -357,13 +320,6 @@ class FARNN_S_D_W(_DecomposeBase):
     def _gates(self):
         g = [getattr(self, n, None) for n in ('Wss1', 'Wrs1', 'bs1', 'Wss2', 'Wrs2', 'bs2')]
         return g
-
-    def _apply_priority(self, scores):
-        if not self.args.use_priority:
-            return scores
-        B, L, Cn = scores.shape
-        out = matmul_nt(scores.reshape(B * L, Cn), self.priority_layer.priority_mat.t().contiguous())
-        return (out + self.priority_layer.priority_bias).view(B, L, Cn)
 
     def forward_scores(self, input, lengths, shape=None):
         dev = self._device()
@@ -386,7 +342,7 @@ class FARNN_S_D_W(_DecomposeBase):
         v = vt[x[:, :L]].reshape(B * L, self.R)
         prod = torch.cat([prod[:, :self.R] * v, prod[:, self.R:]], dim=1)
         scores = matmul_nt(prod, torch.cat([self.C_embed, self.C_wildcard], dim=1)).view(B, L, self.C)
-        return self._apply_priority(scores)
+        return _apply_priority(self, scores)
 
     def forward_local(self, input, label, lengths, train=True):
         dev = self._device()
@@ -401,31 +357,10 @@ class FARNN_S_D_W_I(FARNN_S_D_W):
     def __init__(self, V=None, S1=None, S2=None, C_output=None, S1_output=None, S2_output=None, wildcard_mat=None,
                  wildcard_output=None, final_vector=None, start_vector=None, pretrained_word_embed=None, priority_mat=None,
                  args=None, o_idx=0):
-        nn.Module.__init__(self)
-        self.is_cuda = torch.cuda.is_available()
-        self.additional_states = args.additional_states
-        self.args = args
-        self.embedding = nn.Embedding.from_pretrained(torch.from_numpy(pretrained_word_embed).float(),
-                                                      freeze=(not args.train_word_embed))
-        self.C, self.R_O = C_output.shape
-        self.S, self.R = S1.shape
-        self.t = 1
-        self.use_crf = bool(args.use_crf)
-        if self.use_crf:
-            self.crf = CRF(self.C, self.is_cuda)
-            self.C += 2
-        self.priority_layer = PriorityLayer(self.C, priority_mat)
-        self.random = bool(args.random)
-        self.h0 = nn.Parameter(self.pad_additional_states(torch.from_numpy(start_vector).float()),
-                               requires_grad=bool(args.train_h0))
-        self.hT = nn.Parameter(self.pad_additional_states(torch.from_numpy(final_vector).float()),
-                               requires_grad=bool(args.train_hT))
-        self.init_forward_parameters(S1, S2, V, S1_output, S2_output, C_output, wildcard_mat, wildcard_output)
-        self.beta = args.beta
-        self.beta_vec = nn.Parameter(torch.tensor([self.beta] * self.R).float(), requires_grad=bool(args.train_beta))
-        self.o_idx = o_idx
-        self.not_o_idxs = [i for i in range(self.C) if i != self.o_idx]
-        self.initialize()
+        _DecomposeBase.__init__(self, args, C_output.shape[0], *S1.shape, start_vector, final_vector, priority_mat, o_idx,
+                                (S1, S2, V, S1_output, S2_output, C_output, wildcard_mat, wildcard_output),
+                                pretrained_word_embed)
+        self.R_O = C_output.shape[1]
 
     def init_forward_parameters(self, S1, S2, V, S1_o, S2_o, C_o, W, W_o):
         a = self.args
@@ -435,7 +370,7 @@ class FARNN_S_D_W_I(FARNN_S_D_W):
         G = torch.matmul(self.embedding.weight.data.pinverse(), self.V_embed.data)
         self.embed_r_generalized = nn.Parameter(G, requires_grad=True)
         if a.use_crf:
-            C_o = np.concatenate((C_o, self.get_random((2, self.R_O)).numpy() * a.rand_constant), axis=0)
+            C_o = np.concatenate((C_o, self.get_random((2, C_o.shape[1])).numpy() * a.rand_constant), axis=0)
         self.C_output = nn.Parameter(self.pad_additional_states(torch.from_numpy(C_o).float()),
                                      requires_grad=bool(a.train_wildcard))
         self.S1_output = nn.Parameter(self.pad_additional_states(torch.from_numpy(S1_o).float()),
@@ -446,44 +381,13 @@ class FARNN_S_D_W_I(FARNN_S_D_W):
                                          requires_grad=bool(a.train_wildcard_wildcard))
         self.wildcard_output = nn.Parameter(self.pad_additional_states(torch.from_numpy(W_o).float()),
                                             requires_grad=bool(a.train_wildcard_wildcard)) if W_o is not None else None
-        self._fst_gate_params(self.S + self.additional_states)
+        self._gate_params(self.S + self.additional_states)
         if self.random:
             for w in (self.S1, self.S2, self.V_embed, self.S1_output, self.S2_output, self.C_output,
                       self.embed_r_generalized, self.wildcard_mat):
                 nn.init.xavier_normal_(w)
             nn.init.normal_(self.h0)
             nn.init.normal_(self.hT)
-
-    def _device(self):
-        ops.require_cuda()
-        dev = self.S1.device
-        if dev.type != 'cuda':
-            raise RuntimeError("re2nn_b200: %s must live on a CUDA device (call .cuda()); there is no CPU path"
-                               % type(self).__name__)
-        return dev
-
-    def _dense_transition(self, V_vec):
-        """Tr[b,j,s] = sum_r S1[j,r] V_vec[b,r] S2[s,r] + wildcard_mat[j,s]   (model_decompose_independent.py:172-175)"""
-        B = V_vec.shape[0]
-        S = self._S_full
-        X = (self.S1.unsqueeze(0) * V_vec.unsqueeze(1)).reshape(B * S, self.R)
-        return matmul_nt(X, self.S2).view(B, S, S) + self.wildcard_mat
-
-    def _step(self, h, tok, h_init, vt, O, is_forward, maxp):
-        a = self.args
-        k = float(a.sigmoid_exponent)
-        V_vec = vt[tok]
-        h_bar = h
-        if a.farnn >= 1:
-            zt = torch.sigmoid(k * (matmul_nt(h, self.Wss1.t().contiguous()) + matmul_nt(V_vec, self.Wrs1.t().contiguous()) + self.bs1))
-        if a.farnn == 2:
-            rt = torch.sigmoid(k * (matmul_nt(h, self.Wss2.t().contiguous()) + matmul_nt(V_vec, self.Wrs2.t().contiguous()) + self.bs2))
-            h_bar = (1 - rt) * h_init + rt * h
-        Tr = self._dense_transition(V_vec) * O
-        hn = _apply_nl(vecmat(h_bar, Tr, transposed=not is_forward, maxp=maxp), _nl_name(a.update_nonlinear, _UPDATE_NL))
-        if a.farnn >= 1:
-            hn = (1 - zt) * h + zt * hn
-        return hn
 
     def forward_scores(self, input, lengths, shape=None):
         dev = self._device()
@@ -500,11 +404,13 @@ class FARNN_S_D_W_I(FARNN_S_D_W):
         xr = _reverse_tokens(x, lengths)
         h0 = self.h0.view(1, S).expand(B, S)
         hT = self.hT.view(1, S).expand(B, S)
+        fwd = lambda h_bar, V_vec: vecmat(h_bar, _dense_transition(self, V_vec) * O, False, maxp)
+        bwd = lambda h_bar, V_vec: vecmat(h_bar, _dense_transition(self, V_vec) * O, True, maxp)
         hf, hb, fw, bw = h0, hT, [], []
         for i in range(L):
-            hf = self._step(hf, x[:, i], h0, vt, O, True, maxp)
+            hf = _gated_step(self, hf, vt[x[:, i]], h0, fwd)
             fw.append(hf)
-            hb = self._step(hb, xr[:, i], hT, vt, O, False, maxp)
+            hb = _gated_step(self, hb, vt[xr[:, i]], hT, bwd)
             bw.append(hb)
         fw, bw = torch.stack(fw, dim=1), torch.stack(bw, dim=1)
         alpha = torch.cat([h0.unsqueeze(1), fw[:, :L - 1]], dim=1)          # h0_forward_score[:, i]
@@ -512,15 +418,15 @@ class FARNN_S_D_W_I(FARNN_S_D_W):
         s1s2_out = (self.S1_output.t().unsqueeze(2) * self.S2_output.t().unsqueeze(1)).reshape(self.R_O, S * S)
         scores = []
         for i in range(L):                                                  # get_final_score (:198-206)
-            bss = self._dense_transition(vt[x[:, i]])
+            bss = _dense_transition(self, vt[x[:, i]])
             M = alpha[:, i].unsqueeze(2) * beta[:, i].unsqueeze(1) * bss
             br = matmul_nt(M.reshape(B, S * S), s1s2_out)
             scores.append(matmul_nt(br, self.C_output))
-        return self._apply_priority(torch.stack(scores, dim=1))
+        return _apply_priority(self, torch.stack(scores, dim=1))
 
 
 # ---- exact (onehot) FST classes -----------------------------------------------------------------------------------------
-class FARNN_S_O(nn.Module):
+class FARNN_S_O(_OnehotBase):
     def __init__(self, language_tensor=None, wildcard_tensor=None, wildcard_wildcard_mat=None, final_vector=None,
                  start_vector=None, priority_mat=None, args=None, o_idx=0, is_cuda=False):
         super().__init__()
@@ -529,11 +435,10 @@ class FARNN_S_O(nn.Module):
         C, S, S = wildcard_tensor.shape
         self.S, self.C = S, C
         self.amp = args.rand_constant
-        noisy = lambda a: torch.from_numpy(a).float() + torch.rand_like(torch.from_numpy(a).float()) * self.amp   # utils.py:273-274
-        self.h0 = nn.Parameter(noisy(start_vector), requires_grad=False)
-        self.hT = nn.Parameter(noisy(final_vector), requires_grad=False)
-        self.language_tensor = nn.Parameter(noisy(language_tensor), requires_grad=True)                    # V x C x S x S
-        self.wildcard_tensor = nn.Parameter(noisy(wildcard_tensor), requires_grad=bool(args.train_wildcard))   # C x S x S
+        self.h0 = nn.Parameter(self._noisy(start_vector), requires_grad=False)
+        self.hT = nn.Parameter(self._noisy(final_vector), requires_grad=False)
+        self.language_tensor = nn.Parameter(self._noisy(language_tensor), requires_grad=True)                  # V x C x S x S
+        self.wildcard_tensor = nn.Parameter(self._noisy(wildcard_tensor), requires_grad=bool(args.train_wildcard))   # C x S x S
         self.wildcard_wildcard_mat = nn.Parameter(torch.from_numpy(wildcard_wildcard_mat).float(),
                                                   requires_grad=bool(args.train_wildcard_wildcard))
         self.priority_layer = PriorityLayer(self.C, priority_mat)
@@ -541,18 +446,6 @@ class FARNN_S_O(nn.Module):
         self.initialize()
         if torch.cuda.is_available():
             self.cuda()
-
-    def initialize(self):
-        a = self.args
-        self.t = 1
-        if a.local_loss_func not in ('CE', 'CE1', 'ML'):
-            raise NotImplementedError()
-
-    def _device(self):
-        ops.require_cuda()
-        if not self.language_tensor.is_cuda:
-            self.cuda()
-        return self.language_tensor.device
 
     def _recurrence(self, x, lengths, sum_tensor, mask=None):
         """h <- relu(semiring(h, sum_tensor[x_t] [* mask])) in both directions (model_onehot.py:88-103, 271-290);
@@ -577,12 +470,8 @@ class FARNN_S_O(nn.Module):
         alpha = torch.cat([self.h0.view(1, 1, S).expand(B, 1, S), fw[:, :L - 1]], dim=1)
         return alpha, _beta_rows(self.hT, bw, lengths)
 
-    def _apply_priority(self, score):
-        if not self.args.use_priority:
-            return score
-        return matmul_nt(score, self.priority_layer.priority_mat.t().contiguous()) + self.priority_layer.priority_bias
-
-    def _scores(self, x, lengths):
+    def _scores(self, x, lengths, full_pad):
+        """Every position is scored, pads included, whatever full_pad asks."""
         B, L = x.shape
         lang, wild = self.language_tensor, self.wildcard_tensor
         sum_tensor = lang.sum(1) + wild.sum(0)                                     # V x S x S   (:81-85)
@@ -594,62 +483,8 @@ class FARNN_S_O(nn.Module):
         for i in range(L):                                                         # (:119-133)
             Tr = all_tensor[x[:, i]]                                               # B x C x S x S
             sc = torch.relu(Tr * alpha[:, i].view(B, 1, self.S, 1) * beta[:, i].view(B, 1, 1, self.S)).sum(dim=(2, 3))
-            out.append(self._apply_priority(sc))
+            out.append(_apply_priority(self, sc))
         return torch.stack(out, dim=1)
-
-    def forward_score(self, input, label, lengths, train=True):
-        out_dev = input.device
-        dev = self._device()
-        return self._scores(input.to(dev).contiguous(), lengths.to(dev).contiguous()).to(out_dev)
-
-    def forward_local(self, input, label, lengths, train=True):
-        out_dev = input.device
-        dev = self._device()
-        dl = lengths.to(dev).contiguous()
-        scores = self._scores(input.to(dev).contiguous(), dl).contiguous()
-        N = int(lengths.sum())
-        label = label.to(dev)
-        flattened_true_labels = flatten(label, dl)
-        loss = None
-        if train and self.args.local_loss_func == 'ML':
-            from .kd import ml_loss
-            loss = ml_loss(scores, dl, label, self.args.margin)
-        elif train:
-            loss = autograd_fns.ce_loss(scores, dl, label.contiguous(), N)
-        with torch.no_grad():
-            ce1 = self.args.local_loss_func == 'CE1'
-            pred, _ = ops.argmax_decode(scores.detach(), dl, exclusive_offsets(dl), N, clamp_col=self.C - 1 if ce1 else -1,
-                                        threshold=self.args.threshold, o_idx=self.o_idx)
-        if loss is not None:
-            loss = loss.to(out_dev)
-        return loss, pred.to(out_dev), flattened_true_labels.to(out_dev)
-
-    def forward_RE(self, input, label, lengths, train=False):
-        out_dev = input.device
-        dev = self._device()
-        with torch.no_grad():
-            dl = lengths.to(dev).contiguous()
-            scores = self._scores(input.to(dev).contiguous(), dl).contiguous()
-            ce1 = self.args.local_loss_func == 'CE1'
-            _, pred = ops.argmax_decode(scores, dl, None, 0, clamp_col=self.C - 1 if ce1 else -1,
-                                        threshold=self.args.threshold, o_idx=self.o_idx, want_flat=False, want_padded=True)
-            if ce1:
-                scores = scores.clone()
-                scores[:, :, self.C - 1].clamp_(max=float(self.args.threshold))
-        return pred.to(out_dev), scores.to(out_dev)
-
-    def local_decode(self, all_scores=None):
-        assert torch.is_tensor(all_scores)
-        out_dev = all_scores.device
-        dev = self._device()
-        with torch.no_grad():
-            sc = all_scores.detach().to(dev).float().contiguous().unsqueeze(1)
-            N = sc.shape[0]
-            ones = torch.ones((N,), dtype=torch.int64, device=dev)
-            ce1 = self.args.local_loss_func == 'CE1'
-            pred, _ = ops.argmax_decode(sc, ones, torch.arange(N, dtype=torch.int64, device=dev), N,
-                                        clamp_col=self.C - 1 if ce1 else -1, threshold=self.args.threshold, o_idx=self.o_idx)
-        return pred.to(out_dev)
 
 
 class FARNN_S_O_I(FARNN_S_O):
@@ -661,11 +496,10 @@ class FARNN_S_O_I(FARNN_S_O):
         C, S, S = output_tensor.shape
         self.S, self.C = S, C
         self.amp = args.rand_constant
-        noisy = lambda a: torch.from_numpy(a).float() + torch.rand_like(torch.from_numpy(a).float()) * self.amp
-        self.h0 = nn.Parameter(noisy(start_vector), requires_grad=False)
-        self.hT = nn.Parameter(noisy(final_vector), requires_grad=False)
-        self.language_tensor = nn.Parameter(noisy(language_tensor), requires_grad=True)          # V x S x S
-        self.wildcard_mat = nn.Parameter(noisy(wildcard_mat), requires_grad=False)               # S x S
+        self.h0 = nn.Parameter(self._noisy(start_vector), requires_grad=False)
+        self.hT = nn.Parameter(self._noisy(final_vector), requires_grad=False)
+        self.language_tensor = nn.Parameter(self._noisy(language_tensor), requires_grad=True)    # V x S x S
+        self.wildcard_mat = nn.Parameter(self._noisy(wildcard_mat), requires_grad=False)         # S x S
         self.output_tensor = nn.Parameter(torch.from_numpy(output_tensor).float(), requires_grad=False)   # C x S x S
         self.output_wildcard_mat = nn.Parameter(torch.from_numpy(output_wildcard_mat).float(), requires_grad=False) \
             if output_wildcard_mat is not None else None
@@ -675,7 +509,7 @@ class FARNN_S_O_I(FARNN_S_O):
         if torch.cuda.is_available():
             self.cuda()
 
-    def _scores(self, x, lengths):
+    def _scores(self, x, lengths, full_pad):
         B, L = x.shape
         S = self.S
         sum_tensor = self.language_tensor + self.wildcard_mat                      # V x S x S   (:259)
@@ -688,5 +522,5 @@ class FARNN_S_O_I(FARNN_S_O):
         out = []
         for i in range(L):                                                         # get_final_score (:226-230)
             M = alpha[:, i].unsqueeze(2) * beta[:, i].unsqueeze(1) * sum_tensor[x[:, i]]
-            out.append(self._apply_priority(matmul_nt(M.reshape(B, S * S), out_flat)))
+            out.append(_apply_priority(self, matmul_nt(M.reshape(B, S * S), out_flat)))
         return torch.stack(out, dim=1)

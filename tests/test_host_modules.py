@@ -17,7 +17,8 @@ def test_state_dict_surface_and_init(name):
     m = build_module(name, z, meta, load_state=False).cpu()
     sd = m.state_dict()
     gold = {k[2:]: z[k] for k in z.files if k.startswith('p.')}
-    assert sorted(sd.keys()) == sorted(gold.keys())                  # same state_dict keys
+    assert list(sd.keys()) == list(gold)                             # same state_dict keys, in the same order
+    assert [n for n, _ in m.named_parameters()] == list(gold)        # optimizers index parameters by position
     for k, g in gold.items():
         assert tuple(sd[k].shape) == g.shape, k
         if k in _PERTURBED:
@@ -95,7 +96,8 @@ def test_fst_constructors_match_reference(name):
     m = build_fst_module(z, meta, load_state=False)
     sd = m.state_dict()
     want = {k[2:]: z[k] for k in z.files if k.startswith('p.')}
-    assert sorted(sd.keys()) == sorted(want.keys())
+    assert list(sd.keys()) == list(want)
+    assert [n for n, _ in m.named_parameters()] == list(want)
     edited = ('Wss1', 'Wrs1', 'bs1', 'Wss2', 'Wrs2', 'bs2', 'crf.transitions')
     for k, v in sd.items():
         assert tuple(v.shape) == want[k].shape, k
@@ -105,3 +107,17 @@ def test_fst_constructors_match_reference(name):
     grads = {k[2:] for k in z.files if k.startswith('g.')}
     if grads:
         assert grads <= {k for k, rg in flags.items() if rg}
+
+
+def test_fst_rank_r_rejects_unknown_farnn():
+    """FARNN_S_D_W / FARNN_S_D_W_I refuse farnn outside {0, 1, 2} at construction, as the other rank-R classes do."""
+    import json
+    import os
+    from helpers import GOLDEN
+    from test_gpu_fst import build_fst_module
+    for name in ('fst_dw_f0_tanh_crf', 'fst_dwi_f0_tanh_crf'):
+        z = np.load(os.path.join(GOLDEN, name + '.npz'), allow_pickle=False)
+        meta = json.loads(str(z['meta']))
+        meta['flags']['farnn'] = 3
+        with pytest.raises(NotImplementedError):
+            build_fst_module(z, meta, load_state=False)

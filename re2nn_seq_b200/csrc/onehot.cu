@@ -288,6 +288,8 @@ __global__ void __launch_bounds__(kOhThreads) onehot_recurrence_kernel(const re2
 // state gradient in shared memory, scatter-adds dT[x_t] += outer products and propagates g through T[x_t].
 //   fwd: pre = (h_prev . T) * o, h = phi(pre):  dacc = G*phi'(h)*o ; dT[s][j] += h_prev[s]*dacc[j] ; g_prev[s] = sum_j T[s][j]*dacc[j]
 //   bwd: pre = T . (h_prev*o),   h = phi(pre):  dacc = G*phi'(h)   ; dT[s][j] += dacc[s]*hh[j]     ; g_prev[j] = o[j]*sum_s dacc[s]*T[s][j]
+// Under full_pad the backward direction's step n-1 (token 0) produces a state that feeds the pad steps but has no output
+// row (step_pos: orow = -1); the forward keeps it in shared memory only, so this kernel recomputes it once (hb).
 __global__ void __launch_bounds__(kOhThreads) onehot_backward_kernel(const re2nn_onehot_backward_args a) {
   extern __shared__ float smem[];
   const int S = a.S;
@@ -295,6 +297,7 @@ __global__ void __launch_bounds__(kOhThreads) onehot_backward_kernel(const re2nn
   float* dacc = smem + S;     // S
   float* hprev = smem + 2 * S;  // S   operand of the step (bwd: already * o)
   float* part = smem + 3 * S;   // kOhWarps * S
+  float* hb = part + kOhWarps * S;  // S, full_pad only: bwd state after token 0
   const int b = blockIdx.x, z = blockIdx.y;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int n = (int)a.lengths[b];
@@ -302,6 +305,18 @@ __global__ void __launch_bounds__(kOhThreads) onehot_backward_kernel(const re2nn
   const float* __restrict__ o = a.o;
   const float* states = z == 0 ? a.alpha : a.beta;
   const float* dstates = z == 0 ? a.dalpha : a.dbeta;
+  if (z == 1 && a.full_pad && n >= 1) {
+    // hb = phi(T[x_0] . (prev*o)), prev = beta row 0 (the state after token 1), or hT when n == 1
+    for (int s = tid; s < S; s += kOhThreads) dacc[s] = (n >= 2 ? states[(size_t)b * a.L * S + s] : a.hT[s]) * o[s];
+    __syncthreads();
+    const float* __restrict__ T = a.language + (size_t)a.x[(size_t)b * a.Lpad] * S * S;
+    for (int s = warp; s < S; s += kOhWarps) {
+      float acc = 0.f;
+      for (int j = lane; j < S; j += 32) acc = fmaf(dacc[j], tw(T, W, (size_t)s * S + j), acc);
+      acc = warp_sum(acc);
+      if (lane == 0) hb[s] = apply_nl(acc, a.update_nonlinear);
+    }
+  }
   for (int s = tid; s < S; s += kOhThreads) g[s] = 0.f;
   __syncthreads();
   for (int k = a.L - 1; k >= 0; --k) {
@@ -316,13 +331,14 @@ __global__ void __launch_bounds__(kOhThreads) onehot_backward_kernel(const re2nn
     const int64_t tok = a.x[(size_t)b * a.Lpad + tpos];
     const float* __restrict__ T = a.language + (size_t)tok * S * S;
     float* __restrict__ dT = a.dlanguage + (size_t)tok * S * S;
+    // orow / oprev < 0 only for the state after token 0 of the bwd direction under full_pad: hb, no output gradient
     for (int s = tid; s < S; s += kOhThreads) {
-      const float h = states[((size_t)b * a.L + orow) * S + s];
-      const float G = g[s] + dstates[((size_t)b * a.L + orow) * S + s];
+      const float h = orow >= 0 ? states[((size_t)b * a.L + orow) * S + s] : hb[s];
+      const float G = orow >= 0 ? g[s] + dstates[((size_t)b * a.L + orow) * S + s] : g[s];
       float d = G * nl_grad_from_out(h, a.update_nonlinear);
       if (z == 0) d *= o[s];
       dacc[s] = d;
-      float hp = k > 0 ? states[((size_t)b * a.L + oprev) * S + s] : (z == 0 ? a.h0[s] : a.hT[s]);
+      float hp = k == 0 ? (z == 0 ? a.h0[s] : a.hT[s]) : (oprev >= 0 ? states[((size_t)b * a.L + oprev) * S + s] : hb[s]);
       hprev[s] = z == 0 ? hp : hp * o[s];
     }
     __syncthreads();
@@ -387,8 +403,9 @@ extern "C" int re2nn_onehot_backward(const re2nn_onehot_backward_args* a, void* 
   RE2NN_CHECK(a != nullptr, "onehot_backward: null args");
   RE2NN_CHECK(a->x && a->lengths && a->language && a->o && a->h0 && a->hT && a->alpha && a->beta &&
                   a->dalpha && a->dbeta && a->dlanguage, "onehot_backward: null tensor");
-  const size_t smem = (size_t)(3 + kOhWarps) * a->S * sizeof(float);
-  RE2NN_CHECK(smem <= 220 * 1024, "onehot_backward: S=%d too large", a->S);
+  // S <= 2964; under full_pad one more S-float buffer (the recomputed state after token 0): S <= 2816
+  const size_t smem = (size_t)(3 + kOhWarps + (a->full_pad ? 1 : 0)) * a->S * sizeof(float);
+  RE2NN_CHECK(smem <= 220 * 1024, "onehot_backward: S=%d too large%s", a->S, a->full_pad ? " under full_pad" : "");
   RE2NN_CUDA(cudaFuncSetAttribute(onehot_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   onehot_backward_kernel<<<dim3(a->B, 2), kOhThreads, smem, (cudaStream_t)stream>>>(*a);
   RE2NN_LAUNCH_CHECK();
